@@ -2,6 +2,7 @@
 """bench.py — BWT-forward throughput of the B200-native path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--workload c2|c3|c5|c1|c4]
+                    [--dump-outputs DIR]
 
 A "step" is one forward BWT (suffix sort + BWT emission + origin) of one synthetic block per GPU.
 Default workload = BASELINE.json configs[1]: a 256 MiB block of DNA-like 4-symbol text (C2).
@@ -21,6 +22,9 @@ batch entry) and `copy_only` (the same H2D/D2H traffic with the transform skippe
 `--impl reference` times that CPU restatement on all host cores (the reference is Rust and cannot
 be compiled in this image; see DESIGN.md), same metric/config/unit.  .dark byte identity and the C1 CLI
 round trip of the reference cannot be tested in this image (no rustc/cargo, no golden .dark file).
+
+`--dump-outputs DIR` writes what the last timed step returned to its caller (rank 0's block) as DIR/*.npy, so that
+two builds can be compared output for output on the same seeded inputs: see dump_outputs().
 """
 import argparse
 import json
@@ -231,6 +235,28 @@ def crc32_of(t):
     return "%08x" % (zlib.crc32(t.numpy().tobytes()) & 0xFFFFFFFF)
 
 
+DUMP_SAMPLE = 1 << 22   # BWT positions --dump-outputs writes: 16 MiB of float32 bytes + 32 MiB of float64 positions
+DUMP_SEED = 20261020
+
+
+def dump_outputs(out_dir, torch, d_bwt, origin):
+    """Write what one forward call returns to its caller: origin.npy (the origin, float64[1]), bwt.npy (BWT bytes as
+    float32) and bwt_index.npy (the block positions of those bytes, float64).  A block of more than DUMP_SAMPLE bytes
+    is sampled at DUMP_SAMPLE distinct positions drawn with a fixed seed, so equal arguments give equal positions;
+    the CRC-32 of the whole BWT is `config.bwt_crc32` of the JSON line."""
+    import numpy as np
+    n = d_bwt.numel()
+    if n <= DUMP_SAMPLE:
+        idx = np.arange(n, dtype=np.int64)
+    else:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_SAMPLE, replace=False))
+    vals = d_bwt[torch.from_numpy(idx).to(d_bwt.device)].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "origin.npy"), np.array([origin], dtype=np.float64))
+    np.save(os.path.join(out_dir, "bwt.npy"), vals.astype(np.float32))
+    np.save(os.path.join(out_dir, "bwt_index.npy"), idx.astype(np.float64))
+
+
 def golden_fixtures():
     try:
         with open(os.path.join(ROOT, "tests", "golden", "oracle_golden.json")) as f:
@@ -333,6 +359,8 @@ def run_native(args, rank, local_rank, world):
     ev1.record(stream)
     barrier()
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, torch, d_bwt, origin)
     ms_total = ev0.elapsed_time(ev1)
     stats = con.stats.as_dict()
     fx = gold.get("%s:%d:%d" % (kind, seed, n))
@@ -500,6 +528,7 @@ def run_native(args, rank, local_rank, world):
 
 
 def main():
+    sys.dont_write_bytecode = True   # the benchmark leaves the tree it runs from as it found it
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=10)
@@ -509,7 +538,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-side-workloads", action="store_true", help="skip the c3/c5 sub-records of the 1-GPU run")
     ap.add_argument("--c5-blocks", type=int, default=0, help="C5 blocks per rank for the `c5` sub-record (default: 4 when N > 1, none at N = 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's BWT (a seeded sample of large blocks) "
+                                                          "and origin as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes the outputs of the native path (--impl native)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -91,13 +91,18 @@ def test_null_arguments_are_rejected_before_any_device_work(lib):
 
 
 def test_no_cpu_fallback_create_fails_without_gpu(lib):
-    """On a box without a CUDA device the product path must fail loudly."""
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is present")
-    from dark_b200 import saca, DarkBwtError
-    with pytest.raises(DarkBwtError):
-        saca.Constructor(1024)
+    """Where no CUDA device is visible the product path must fail loudly.  The check runs in a fresh process that sees
+    no device, so that it also runs on a machine that has one."""
+    import subprocess
+    import sys
+    code = ("from dark_b200 import saca, DarkBwtError\n"
+            "try:\n"
+            "    saca.Constructor(1024)\n"
+            "except DarkBwtError:\n"
+            "    print('raised')\n")
+    out = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), cwd=ROOT,
+                         capture_output=True, text=True, timeout=120)
+    assert out.returncode == 0 and out.stdout.strip() == "raised", (out.stdout, out.stderr[-2000:])
 
 
 def test_product_never_touches_the_oracle():

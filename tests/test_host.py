@@ -105,3 +105,53 @@ def test_bench_reference_arm_prints_contract_line():
     line = json.loads(out.stdout.strip().splitlines()[-1])
     assert line["impl"] == "reference" and line["unit"] == "MB/s" and line["value"] > 0
     assert line["cpu_baseline"]["kind"] == "port" and line["e2e"]["h2d_bytes_per_step"] == 0
+
+
+def test_bench_rejects_bad_arguments():
+    import subprocess
+    for extra in (["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", "out"]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True, timeout=60)
+        assert out.returncode == 2 and "error" in out.stderr, (extra, out.stderr[-2000:])
+
+
+def test_bench_dump_outputs_whole_or_fixed_sample(tmp_path):
+    """bench.py --dump-outputs: a small block is written whole; a larger one at DUMP_SAMPLE distinct positions that are
+    the same on every run; float32/float64 files only, 64 MB at most."""
+    import torch
+    import bench
+    small = torch.from_numpy(np.random.default_rng(1).integers(0, 256, 1000).astype(np.uint8))
+    bench.dump_outputs(str(tmp_path / "small"), torch, small, 7)
+    assert np.load(tmp_path / "small" / "origin.npy").tolist() == [7.0]
+    assert np.array_equal(np.load(tmp_path / "small" / "bwt.npy"), small.numpy().astype(np.float32))
+    assert np.array_equal(np.load(tmp_path / "small" / "bwt_index.npy"), np.arange(1000, dtype=np.float64))
+    n = bench.DUMP_SAMPLE + 4099
+    big = torch.from_numpy(np.random.default_rng(2).integers(0, 256, n).astype(np.uint8))
+    runs = []
+    for d in ("run1", "run2"):
+        bench.dump_outputs(str(tmp_path / d), torch, big, 123456)
+        files = {f: np.load(tmp_path / d / f) for f in ("origin.npy", "bwt.npy", "bwt_index.npy")}
+        assert all(a.dtype in (np.float32, np.float64) for a in files.values())
+        assert sum(os.path.getsize(tmp_path / d / f) for f in files) <= 64 * 10**6
+        runs.append(files)
+    idx = runs[0]["bwt_index.npy"]
+    assert idx.size == bench.DUMP_SAMPLE and np.all(np.diff(idx) > 0) and idx[0] >= 0 and idx[-1] < n
+    assert np.array_equal(runs[0]["bwt.npy"], big.numpy()[idx.astype(np.int64)].astype(np.float32))
+    for f in runs[0]:
+        assert np.array_equal(runs[0][f], runs[1][f])
+
+
+@pytest.mark.gpu
+def test_bench_dumps_what_the_timed_steps_computed(oracle, tmp_path):
+    """bench.py runs exactly --steps timed steps and --dump-outputs writes the BWT and origin of the last one: on the
+    C1 block (written whole) they equal the oracle's."""
+    import json
+    import subprocess
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "c1", "--steps", "3", "--warmup", "1",
+                          "--no-cpu-baseline", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads(out.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 3 and line["gpu_launches"] == 3 * line["config"]["kernel_launches_per_step"]
+    bwt_o, origin_o = oracle.bwt_forward(oracle.gen("text", 3, 768771))
+    assert np.load(tmp_path / "origin.npy").tolist() == [origin_o]
+    assert np.array_equal(np.load(tmp_path / "bwt.npy"), bwt_o.astype(np.float32))
+    assert np.array_equal(np.load(tmp_path / "bwt_index.npy"), np.arange(bwt_o.size, dtype=np.float64))

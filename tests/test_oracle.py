@@ -12,7 +12,7 @@ import zlib
 import numpy as np
 import pytest
 
-REF_LICENSE = "/root/reference/LICENSE"
+REF_LICENSE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "mit_license.txt")
 
 
 def crc(a):
@@ -48,9 +48,9 @@ def test_block_level_string(oracle):
     assert oracle.bwt_decode(bwt, origin).tobytes() == text
 
 
-@pytest.mark.skipif(not os.path.exists(REF_LICENSE), reason="reference tree not present (GPU box)")
 def test_license_roundtrip(oracle):
-    # saca.rs:429-433 / block/dc.rs:187-192 round-trip the crate's LICENSE file (1,083 B)
+    # saca.rs:429-433 / block/dc.rs:187-192 round-trip the crate's LICENSE file (1,083 B); that file is not part of
+    # this repository, so an MIT license text of the same size stands in for it
     text = open(REF_LICENSE, "rb").read()
     assert len(text) == 1083
     sa = oracle.saca(text)
