@@ -15,7 +15,8 @@ F_DEFAULT, F_NO_ALPHABET_PACKING, F_DEVICE_ONLY = 0, 1, 2
 # every symbol include/dark_bwt.h declares (tests/test_abi.py checks the .so exports all of them)
 SYMBOLS = [
     "dark_bwt_abi_version", "dark_bwt_create", "dark_bwt_create_ex", "dark_bwt_capacity", "dark_bwt_forward",
-    "dark_bwt_forward_batch", "dark_bwt_forward_many", "dark_bwt_forward_many_device", "dark_bwt_forward_device", "dark_bwt_inverse", "dark_bwt_inverse_device", "dark_bwt_reuse", "dark_bwt_destroy", "dark_bwt_strerror", "dark_bwt_last_error",
+    "dark_bwt_forward_batch", "dark_bwt_forward_many", "dark_bwt_forward_many_device", "dark_bwt_forward_device", "dark_bwt_inverse", "dark_bwt_inverse_device",
+    "dark_bwt_inverse_batch", "dark_bwt_inverse_many", "dark_bwt_inverse_many_device", "dark_bwt_reuse", "dark_bwt_destroy", "dark_bwt_strerror", "dark_bwt_last_error",
     "dark_bwt_stream", "dark_bwt_sort_pairs_device", "dark_bwt_verify_sa_device", "dark_bwt_emit_device", "dark_bwt_lcp_profile_device",
     "dark_bwt_synth", "dark_bwt_dc_encode_device", "dark_bwt_dc_encode", "dark_bwt_forward_dc",
 ]
@@ -93,6 +94,9 @@ def lib():
     L.dark_bwt_forward_many_device.argtypes = [vp, vp, vp, u64, vp, vp, vp, ctypes.POINTER(Stats)]
     L.dark_bwt_inverse.argtypes = [vp, vp, u64, u64, vp]
     L.dark_bwt_inverse_device.argtypes = [vp, vp, u64, u64, vp, ctypes.POINTER(ctypes.c_float)]
+    L.dark_bwt_inverse_batch.argtypes = [vp, vp, vp, vp, vp, u64, vp]
+    L.dark_bwt_inverse_many.argtypes = [vp, vp, vp, vp, vp, u64, vp]
+    L.dark_bwt_inverse_many_device.argtypes = [vp, vp, vp, vp, u64, vp, vp]
     L.dark_bwt_reuse.argtypes = [vp, pp, ctypes.POINTER(u64)]
     L.dark_bwt_destroy.argtypes = [vp]
     L.dark_bwt_destroy.restype = None

@@ -59,6 +59,7 @@ struct Mailbox {  // pinned host memory the device results are copied into
     unsigned long long bad;
     u32 flag;  // pairs-mode detector: set when some group has three or more members
     u32 not_pairs;  // the same answer from the check queued behind a re-rank (read with the survivor count)
+    u32 bad_block;  // inverse_many: the lowest block whose list does not cover its rows (with `count` = how many do not)
 };
 
 struct DeviceScalars {  // mirrors Mailbox on the device
@@ -1305,6 +1306,87 @@ int inverse_device(dark_bwt_ctx* ctx, const u8* d_bwt, u64 n64, u64 origin64, u8
     return DARK_BWT_OK;
 }
 
+// Inverse BWT of B blocks in one pass (suffix_kernels.cuh, "inverse BWT of many blocks").  d_bwt holds the blocks back to
+// back (n bytes), ctx->many_starts their offsets and ctx->many_origins their origins (validated, on the device); d_text
+// receives the texts at the same offsets.  max_nb = the largest block.
+//
+// Buffers: the rows number R = n + B <= capacity (the entry points check it).  The sort moves n <= capacity pairs.  The
+// node arrays (dist and next twice, len_keep) hold `regular + B` entries, and regular = ceil(R / stride) <= (R + 1) / 2 with
+// stride >= 2 while every block has at least two rows (B <= R / 2): nodes <= R <= capacity, which the u32 arrays of the
+// arena hold.  The stash gets (8 capacity + 1024) / nodes >= 8 bytes a chunk.  So 65,536 blocks of one byte need a
+// capacity of 131,072 (rows, not bytes, are what must fit), and sum(ns) <= capacity alone would not be enough.
+int inverse_many_device(dark_bwt_ctx* ctx, const u8* d_bwt, u32 n, u32 B, u32 max_nb, u8* d_text, float* ms_out) {
+    CK(cudaSetDevice(ctx->device));
+    ctx->n_events = 0;
+    ctx->spans.clear();
+    ctx->next_counter = 0;
+    cudaEvent_t ea = ctx->events[kMaxEvents - 1], eb = ctx->events[kMaxEvents - 2];
+    CK(cudaEventRecord(ea, ctx->stream));
+    CK(cudaMemsetAsync(ctx->counters, 0, sizeof(u32) * kMaxCounters, ctx->stream));
+    CK(cudaMemsetAsync(ctx->hist, 0, sizeof(u32) * kMaxPasses * kRadix, ctx->stream));
+    // step 1: (block, last symbol) keys of the real rows, one stable sort -> psi and the first symbols
+    const int passes = 1 + (B > 1 ? (bit_length((u64)B - 1) + kRadixBits - 1) / kRadixBits : 0);
+    const u32 grid = (u32)std::min<u64>(ceil_div(n, 256), (u64)ctx->num_sms * 8);
+    k_ibwt_many_elements<256><<<grid, 256, 0, ctx->stream>>>(d_bwt, n, ctx->many_starts, B, ctx->many_origins, ctx->keys[0], ctx->ids[0],
+                                                             ctx->hist, passes);
+    LAUNCHED();
+    int cur = 0;
+    // passes whose digit is the same in every key are skipped (one-symbol blocks, a single block): the order stays the row order
+    if (int rc = run_sort(ctx, ctx->keys, ctx->ids, 0, n, 0, passes, &cur, nullptr, 0)) return rc;
+    const u32* psi = ctx->ids[cur];
+    const u64* skeys = ctx->keys[cur];
+    // step 2: sublists between splitters (buffers as in inverse_device)
+    const u32 stride = (u32)ctx->knobs.ibwt_stride;
+    const u32 regular = (u32)ceil_div((u64)n + B, stride);
+    const u32 nodes = regular + B;
+    u32* dist[2] = {ctx->ranks, ctx->sa};
+    u32* next[2] = {ctx->isa, ctx->ids[cur ^ 1]};
+    u32* len_keep = ctx->ranks_alt;
+    u32* stash = (u32*)ctx->keys[cur ^ 1];
+    const u32 cap = (u32)std::min<u64>(kIbwtStashCap, ((ctx->capacity * 8 + 1024) / nodes) & ~3ull);
+    const bool two_walks = ctx->knobs.ibwt_two_walks || cap < 8;
+    const u32 wgrid = (u32)ceil_div(nodes, 128);
+    if (two_walks)
+        k_ibwt_many_walk<0><<<wgrid, 128, 0, ctx->stream>>>(psi, skeys, ctx->many_starts, B, ctx->many_origins, stride, regular, dist[0], next[0],
+                                                            nullptr, nullptr, nullptr, nullptr, 0u, 0u);
+    else
+        k_ibwt_many_walk<2><<<wgrid, 128, 0, ctx->stream>>>(psi, skeys, ctx->many_starts, B, ctx->many_origins, stride, regular, dist[0], next[0],
+                                                            nullptr, nullptr, len_keep, stash, 0u, cap);
+    LAUNCHED();
+    // step 3: pointer jumping; a block's list holds at most ceil((max_nb + 1) / stride) + 1 splitters
+    const u64 chain = ceil_div((u64)max_nb + 1, stride) + 1;
+    int w = 0;
+    for (u64 span = 1; span < chain; span <<= 1) {
+        k_ibwt_jump<<<(u32)ceil_div(nodes, 256), 256, 0, ctx->stream>>>(dist[w], next[w], dist[w ^ 1], next[w ^ 1], nodes);
+        LAUNCHED();
+        w ^= 1;
+    }
+    k_ibwt_many_check<<<1, 1024, 0, ctx->stream>>>(dist[w], regular, ctx->many_starts, B, &ctx->mail_dev->count, &ctx->mail_dev->bad_block);
+    LAUNCHED();
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (ctx->mail->count != 0) {
+        snprintf(ctx->err, sizeof(ctx->err), "inverse BWT: block %u is not a forward transform (%u of %u blocks are not)",
+                 ctx->mail->bad_block, ctx->mail->count, B);
+        return DARK_BWT_E_INVALID_ARG;
+    }
+    // step 4: the texts
+    if (two_walks) {
+        k_ibwt_many_walk<1><<<wgrid, 128, 0, ctx->stream>>>(psi, skeys, ctx->many_starts, B, ctx->many_origins, stride, regular, nullptr, nullptr,
+                                                            dist[w], d_text, nullptr, nullptr, 0u, 0u);
+        LAUNCHED();
+    } else {
+        k_ibwt_many_unstash<<<wgrid, 128, 0, ctx->stream>>>(stash, len_keep, dist[w], ctx->many_starts, B, stride, regular, d_text, cap);
+        LAUNCHED();
+        k_ibwt_many_walk<1><<<wgrid, 128, 0, ctx->stream>>>(psi, skeys, ctx->many_starts, B, ctx->many_origins, stride, regular, nullptr, nullptr,
+                                                            dist[w], d_text, len_keep, nullptr, cap, 0u);
+        LAUNCHED();
+    }
+    CK(cudaEventRecord(eb, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (ms_out) cudaEventElapsedTime(ms_out, ea, eb);
+    return DARK_BWT_OK;
+}
+
 // Distance coding + MTF of a BWT block on device buffers (dc_kernels.cuh).  Every output pointer is nullable: the
 // context's own arena is used for what the caller does not want.  *d_dist_used / *d_pos_used etc. tell where the data is.
 struct DcBuffers {
@@ -1484,6 +1566,92 @@ int copy_out_blocking(dark_bwt_ctx* ctx, void* host, const void* dev, size_t byt
     CK(cudaMemcpyAsync(host, dev, bytes, cudaMemcpyDeviceToHost, stream));
     CK(cudaStreamSynchronize(stream));
     return 0;
+}
+
+// A second copy-out of a block that must be complete before the next block is transformed (its device buffer is single).
+struct SideCopy {
+    void* host = nullptr;
+    const void* dev = nullptr;
+    size_t bytes = 0;
+};
+
+// The pipelined loop of the batch entries: `count` host blocks ins[k] (ns[k] bytes) -> outs[k] (ns[k] bytes).  While block
+// k is transformed (transform(k, d_in[b], d_out[b], &side), synchronous on the context's stream), block k+1 is copied into
+// the other input buffer and block k-1 out of the other output buffer.  Pinned host buffers ride on the two copy
+// streams; pageable ones (>= 1 MiB) are moved by the staging lanes in a helper thread.
+template <typename Transform>
+int run_pipelined(dark_bwt_ctx* ctx, const u8* const* ins, const uint64_t* ns, u8* const* outs, uint64_t count, u8* const d_in[2],
+                  u8* const d_out[2], Transform transform) {
+    bool comp_recorded[2] = {false, false}, out_recorded[2] = {false, false};
+    std::future<int> fin[2], fout;
+    auto staged_in = [&](uint64_t k) { return ns[k] >= kStageMinBytes && is_pageable(ins[k]) && stage_prepare(ctx, ctx->stage_in) == 0; };
+    auto staged_out = [&](uint64_t k) { return ns[k] >= kStageMinBytes && is_pageable(outs[k]) && stage_prepare(ctx, ctx->stage_out) == 0; };
+    auto start_in = [&](uint64_t k, int buf) -> int {  // the transform that read d_in[buf] has returned (it is synchronous)
+        if (staged_in(k)) {
+            u8* dst = d_in[buf];
+            const u8* src = ins[k];
+            const size_t bytes = ns[k];
+            fin[buf] = std::async(std::launch::async, [ctx, dst, src, bytes] { return staged_copy(ctx, ctx->stage_in, dst, (void*)src, bytes, true); });
+            return 0;
+        }
+        if (comp_recorded[buf]) CK(cudaStreamWaitEvent(ctx->copy_in, ctx->ev_comp[buf], 0));
+        CK(cudaMemcpyAsync(d_in[buf], ins[k], ns[k], cudaMemcpyHostToDevice, ctx->copy_in));
+        CK(cudaEventRecord(ctx->ev_in[buf], ctx->copy_in));
+        return 0;
+    };
+    auto drain = [&]() {  // never leave a helper thread behind
+        int rc = 0;
+        for (int i = 0; i < 2; ++i)
+            if (fin[i].valid()) rc |= fin[i].get();
+        if (fout.valid()) rc |= fout.get();
+        return rc;
+    };
+    if (int rc = start_in(0, 0)) return rc;
+    for (uint64_t k = 0; k < count; ++k) {
+        const int b = (int)(k & 1), nb = b ^ 1;
+        if (fin[b].valid()) {
+            if (int rc = fin[b].get()) { drain(); return rc; }
+        } else {
+            CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_in[b], 0));
+        }
+        if (k + 1 < count)
+            if (int rc = start_in(k + 1, nb)) { drain(); return rc; }
+        // (a staged copy-out of block k-1 may still be reading the OTHER output buffer; this one was drained before it began)
+        if (out_recorded[b]) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_out[b], 0));  // output buffer b drained
+        SideCopy side;
+        int rc = transform(k, (const u8*)d_in[b], d_out[b], &side);
+        if (rc) { drain(); return rc; }
+        CK(cudaEventRecord(ctx->ev_comp[b], ctx->stream));
+        comp_recorded[b] = true;
+        if (fout.valid())
+            if (int rc2 = fout.get()) { drain(); return rc2; }  // one staged copy-out at a time (they share the lanes)
+        if (staged_out(k)) {
+            u8* dst = outs[k];
+            const u8* src = d_out[b];
+            const size_t bytes = ns[k];
+            fout = std::async(std::launch::async, [ctx, dst, src, bytes, side] {
+                int r = staged_copy(ctx, ctx->stage_out, (void*)src, dst, bytes, false);
+                if (r == 0 && side.host) r = staged_copy(ctx, ctx->stage_out, (void*)side.dev, side.host, side.bytes, false);
+                return r;
+            });
+            if (side.host)
+                if (int rc2 = fout.get()) { drain(); return rc2; }  // the side buffer is reused by the next block
+            out_recorded[b] = false;
+        } else {
+            CK(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_comp[b], 0));
+            CK(cudaMemcpyAsync(outs[k], d_out[b], ns[k], cudaMemcpyDeviceToHost, ctx->copy_out));
+            if (side.host) {  // the side buffer is reused by the next block: drain it before going on
+                CK(cudaMemcpyAsync(side.host, side.dev, side.bytes, cudaMemcpyDeviceToHost, ctx->copy_out));
+                CK(cudaStreamSynchronize(ctx->copy_out));
+            }
+            CK(cudaEventRecord(ctx->ev_out[b], ctx->copy_out));
+            out_recorded[b] = true;
+        }
+    }
+    if (int rc = drain()) return rc;
+    CK(cudaStreamSynchronize(ctx->copy_out));
+    CK(cudaStreamSynchronize(ctx->copy_in));
+    return DARK_BWT_OK;
 }
 
 }  // namespace
@@ -1694,83 +1862,38 @@ int dark_bwt_forward_batch(dark_bwt_ctx* ctx, const uint8_t* const* texts, const
     }
     if (count == 0) return DARK_BWT_OK;
     CK(cudaSetDevice(ctx->device));
-    u8* d_text[2] = {ctx->d_text, ctx->d_text2};
-    u8* d_bwt[2] = {ctx->d_bwt, ctx->d_bwt2};
-    bool comp_recorded[2] = {false, false}, out_recorded[2] = {false, false};
-    // Pinned host buffers ride on the two copy streams; pageable ones (>= 1 MiB) are moved by the staging lanes in a
-    // helper thread, so that either way block k+1 comes in and block k-1 goes out while block k is transformed.
-    std::future<int> fin[2], fout;
-    auto staged_in = [&](uint64_t k) { return ns[k] >= kStageMinBytes && is_pageable(texts[k]) && stage_prepare(ctx, ctx->stage_in) == 0; };
-    auto staged_out = [&](uint64_t k) { return ns[k] >= kStageMinBytes && is_pageable(bwt_outs[k]) && stage_prepare(ctx, ctx->stage_out) == 0; };
-    auto start_in = [&](uint64_t k, int buf) -> int {  // the transform that read d_text[buf] has returned (forward_device is synchronous)
-        if (staged_in(k)) {
-            u8* dst = d_text[buf];
-            const u8* src = texts[k];
-            const size_t bytes = ns[k];
-            fin[buf] = std::async(std::launch::async, [ctx, dst, src, bytes] { return staged_copy(ctx, ctx->stage_in, dst, (void*)src, bytes, true); });
-            return 0;
-        }
-        if (comp_recorded[buf]) CK(cudaStreamWaitEvent(ctx->copy_in, ctx->ev_comp[buf], 0));
-        CK(cudaMemcpyAsync(d_text[buf], texts[k], ns[k], cudaMemcpyHostToDevice, ctx->copy_in));
-        CK(cudaEventRecord(ctx->ev_in[buf], ctx->copy_in));
-        return 0;
-    };
-    auto drain = [&]() {  // never leave a helper thread behind
-        int rc = 0;
-        for (int i = 0; i < 2; ++i)
-            if (fin[i].valid()) rc |= fin[i].get();
-        if (fout.valid()) rc |= fout.get();
-        return rc;
-    };
-    if (int rc = start_in(0, 0)) return rc;
-    for (uint64_t k = 0; k < count; ++k) {
-        const int b = (int)(k & 1), nb = b ^ 1;
-        if (fin[b].valid()) {
-            if (int rc = fin[b].get()) { drain(); return rc; }
-        } else {
-            CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_in[b], 0));
-        }
-        if (k + 1 < count)
-            if (int rc = start_in(k + 1, nb)) { drain(); return rc; }
-        // (a staged copy-out of block k-1 may still be reading the OTHER BWT buffer; this one was drained before it began)
-        if (out_recorded[b]) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_out[b], 0));  // BWT buffer b drained
-        u32* sa_user = (sa_outs && sa_outs[k]) ? sa_outs[k] : nullptr;
+    u8* const d_text[2] = {ctx->d_text, ctx->d_text2};
+    u8* const d_bwt[2] = {ctx->d_bwt, ctx->d_bwt2};
+    return run_pipelined(ctx, texts, ns, bwt_outs, count, d_text, d_bwt, [&](uint64_t k, const u8* din, u8* dout, SideCopy* side) {
         dark_bwt_stats* st = stats ? stats + k : nullptr;
         if (st) st->h2d_ms = 0.f;
-        int rc = forward_device(ctx, d_text[b], ns[k], d_bwt[b], origins_out + k, nullptr, st);
-        if (rc) { drain(); return rc; }
-        CK(cudaEventRecord(ctx->ev_comp[b], ctx->stream));
-        comp_recorded[b] = true;
-        if (fout.valid())
-            if (int rc2 = fout.get()) { drain(); return rc2; }  // one staged copy-out at a time (they share the lanes)
-        if (staged_out(k)) {
-            u8* dst = bwt_outs[k];
-            const u8* src = d_bwt[b];
-            const size_t bytes = ns[k];
-            const u32* sa_src = ctx->sa;
-            fout = std::async(std::launch::async, [ctx, dst, src, bytes, sa_user, sa_src] {
-                int r = staged_copy(ctx, ctx->stage_out, (void*)src, dst, bytes, false);
-                if (r == 0 && sa_user) r = staged_copy(ctx, ctx->stage_out, (void*)sa_src, sa_user, bytes * sizeof(u32), false);
-                return r;
-            });
-            if (sa_user)
-                if (int rc2 = fout.get()) { drain(); return rc2; }  // the single SA buffer is reused by the next block
-            out_recorded[b] = false;
-        } else {
-            CK(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_comp[b], 0));
-            CK(cudaMemcpyAsync(bwt_outs[k], d_bwt[b], ns[k], cudaMemcpyDeviceToHost, ctx->copy_out));
-            if (sa_user) {  // the single SA buffer is reused by the next block: drain it before going on
-                CK(cudaMemcpyAsync(sa_user, ctx->sa, ns[k] * sizeof(u32), cudaMemcpyDeviceToHost, ctx->copy_out));
-                CK(cudaStreamSynchronize(ctx->copy_out));
-            }
-            CK(cudaEventRecord(ctx->ev_out[b], ctx->copy_out));
-            out_recorded[b] = true;
+        const int rc = forward_device(ctx, din, ns[k], dout, origins_out + k, nullptr, st);
+        if (rc == 0 && sa_outs && sa_outs[k]) {  // the SA of the block is in the context's single SA buffer
+            side->host = sa_outs[k];
+            side->dev = ctx->sa;
+            side->bytes = ns[k] * sizeof(u32);
         }
+        return rc;
+    });
+}
+
+int dark_bwt_inverse_batch(dark_bwt_ctx* ctx, const uint8_t* const* bwts, const uint64_t* ns, const uint64_t* origins,
+                           uint8_t* const* text_outs, uint64_t count, float* ms_out) {
+    if (!ctx || !bwts || !ns || !origins || !text_outs) return DARK_BWT_E_INVALID_ARG;
+    if (ctx->flags & DARK_BWT_F_DEVICE_ONLY) return DARK_BWT_E_INVALID_ARG;
+    ctx->err[0] = 0;
+    for (uint64_t k = 0; k < count; ++k) {
+        if (!bwts[k] || !text_outs[k]) return DARK_BWT_E_INVALID_ARG;
+        if (ns[k] < 1 || ns[k] > ctx->capacity || ns[k] > 0xFFFFFFFEull) return DARK_BWT_E_INVALID_N;
+        if (origins[k] >= ns[k]) return DARK_BWT_E_INVALID_ARG;
     }
-    if (int rc = drain()) return rc;
-    CK(cudaStreamSynchronize(ctx->copy_out));
-    CK(cudaStreamSynchronize(ctx->copy_in));
-    return DARK_BWT_OK;
+    if (count == 0) return DARK_BWT_OK;
+    CK(cudaSetDevice(ctx->device));
+    u8* const d_bwt[2] = {ctx->d_bwt, ctx->d_bwt2};
+    u8* const d_text[2] = {ctx->d_text, ctx->d_text2};
+    return run_pipelined(ctx, bwts, ns, text_outs, count, d_bwt, d_text, [&](uint64_t k, const u8* din, u8* dout, SideCopy*) {
+        return inverse_device(ctx, din, ns[k], origins[k], dout, ms_out ? ms_out + k : nullptr);
+    });
 }
 
 int dark_bwt_forward_many(dark_bwt_ctx* ctx, const uint8_t* const* texts, const uint64_t* ns, uint8_t* const* bwt_outs,
@@ -1852,6 +1975,66 @@ int dark_bwt_inverse(dark_bwt_ctx* ctx, const uint8_t* bwt, uint64_t n, uint64_t
     if (int rc = copy_in_blocking(ctx, ctx->d_bwt, bwt, n, ctx->stream)) return rc;
     if (int rc = inverse_device(ctx, ctx->d_bwt, n, origin, ctx->d_text, nullptr)) return rc;
     return copy_out_blocking(ctx, text_out, ctx->d_text, n, ctx->stream);
+}
+
+int dark_bwt_inverse_many(dark_bwt_ctx* ctx, const uint8_t* const* bwts, const uint64_t* ns, const uint64_t* origins,
+                          uint8_t* const* text_outs, uint64_t count, float* ms_out) {
+    if (!ctx || !bwts || !ns || !origins || !text_outs) return DARK_BWT_E_INVALID_ARG;
+    if (count > kMaxManyBlocks) return DARK_BWT_E_INVALID_ARG;
+    if (ctx->flags & DARK_BWT_F_DEVICE_ONLY) return DARK_BWT_E_INVALID_ARG;
+    ctx->err[0] = 0;
+    if (count == 0) return DARK_BWT_OK;
+    std::vector<u32> starts(count + 1);
+    u64 total = 0, max_nb = 0;
+    for (uint64_t k = 0; k < count; ++k) {
+        if (!bwts[k] || !text_outs[k]) return DARK_BWT_E_INVALID_ARG;
+        if (ns[k] < 1) return DARK_BWT_E_INVALID_N;
+        if (origins[k] >= ns[k]) return DARK_BWT_E_INVALID_ARG;
+        starts[k] = (u32)total;
+        total += ns[k];
+        max_nb = std::max<u64>(max_nb, ns[k]);
+        if (total + k + 1 > ctx->capacity) return DARK_BWT_E_INVALID_N;  // the rows (bytes + one '$' row per block) share the arena
+    }
+    starts[count] = (u32)total;
+    CK(cudaSetDevice(ctx->device));
+    static_assert(sizeof(unsigned long long) == sizeof(uint64_t), "origins are copied as they are");
+    CK(cudaMemcpyAsync(ctx->many_starts, starts.data(), sizeof(u32) * (count + 1), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->many_origins, origins, sizeof(uint64_t) * count, cudaMemcpyHostToDevice, ctx->stream));
+    for (uint64_t k = 0; k < count; ++k)
+        CK(cudaMemcpyAsync(ctx->d_bwt + starts[k], bwts[k], ns[k], cudaMemcpyHostToDevice, ctx->stream));
+    if (int rc = inverse_many_device(ctx, ctx->d_bwt, (u32)total, (u32)count, (u32)max_nb, ctx->d_text, ms_out)) return rc;
+    for (uint64_t k = 0; k < count; ++k)
+        CK(cudaMemcpyAsync(text_outs[k], ctx->d_text + starts[k], ns[k], cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return DARK_BWT_OK;
+}
+
+int dark_bwt_inverse_many_device(dark_bwt_ctx* ctx, const uint8_t* d_bwt, const uint32_t* d_starts, const uint64_t* d_origins,
+                                 uint64_t count, uint8_t* d_text_out, float* ms_out) {
+    if (!ctx || !d_bwt || !d_starts || !d_origins || !d_text_out) return DARK_BWT_E_INVALID_ARG;
+    if (count > kMaxManyBlocks) return DARK_BWT_E_INVALID_ARG;
+    ctx->err[0] = 0;
+    if (count == 0) return DARK_BWT_OK;
+    CK(cudaSetDevice(ctx->device));
+    // offsets and origins are checked on the host before any kernel reads them
+    std::vector<u32> starts(count + 1);
+    std::vector<uint64_t> origins(count);
+    CK(cudaMemcpyAsync(starts.data(), d_starts, sizeof(u32) * (count + 1), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(origins.data(), d_origins, sizeof(uint64_t) * count, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (starts[0] != 0) return DARK_BWT_E_INVALID_ARG;
+    u64 max_nb = 0;
+    for (uint64_t k = 0; k < count; ++k) {
+        if ((u64)starts[k + 1] < (u64)starts[k] + 1) return DARK_BWT_E_INVALID_N;
+        const u64 nb = (u64)starts[k + 1] - starts[k];
+        if (origins[k] >= nb) return DARK_BWT_E_INVALID_ARG;
+        max_nb = std::max(max_nb, nb);
+    }
+    const u64 total = starts[count];
+    if (total + count > ctx->capacity) return DARK_BWT_E_INVALID_N;
+    CK(cudaMemcpyAsync(ctx->many_starts, d_starts, sizeof(u32) * (count + 1), cudaMemcpyDeviceToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->many_origins, d_origins, sizeof(uint64_t) * count, cudaMemcpyDeviceToDevice, ctx->stream));
+    return inverse_many_device(ctx, d_bwt, (u32)total, (u32)count, (u32)max_nb, d_text_out, ms_out);
 }
 
 int dark_bwt_dc_encode_device(dark_bwt_ctx* ctx, const uint8_t* d_bwt, uint64_t n, uint32_t* d_dist_out, uint32_t* d_item_pos,

@@ -1646,24 +1646,13 @@ k_ibwt_walk(const u32* __restrict__ psi1 /* psi[r] for r >= 1 at psi1[r-1] */, u
     }
 }
 
-// Copy every stashed sublist (length <= kIbwtStashCap) to its place in the text: aligned 32-bit stores composed from
-// two neighbouring chunk words, single bytes only at the two ends.
-__global__ void __launch_bounds__(128)
-k_ibwt_unstash(const u32* __restrict__ stash, const u32* __restrict__ len_keep, const u32* __restrict__ dist, u32 n, u32 regular,
-               u8* __restrict__ text_out, u32 cap) {
-    const u32 s = blockIdx.x * 128 + threadIdx.x;
-    if (s > regular) return;
-    const u32 len = len_keep[s];
-    if (len == 0 || len > cap) return;  // longer sublists are written by a second walk
-    const u64 pos = (u64)(n + 1) - dist[s];
-    if (pos >= n) return;
-    const u32 L = (u32)min((u64)len, (u64)n - pos);  // the '$' row's placeholder falls off the end
-    const u32* src = stash + (size_t)s * (cap / 4);
-    u8* dst = text_out + pos;
+// Copy L bytes of a stash chunk to dst: with `words`, aligned 32-bit stores composed from two neighbouring chunk words,
+// single bytes only at the two ends.
+__device__ __forceinline__ void ibwt_copy_chunk(const u32* __restrict__ src, u8* __restrict__ dst, u32 L, bool words) {
     auto byte_at = [&](u32 i) { return (u8)(src[i >> 2] >> (8 * (i & 3))); };
     u32 i = 0;
-    if ((((uintptr_t)text_out) & 3) == 0) {
-        while (((pos + i) & 3) != 0 && i < L) {
+    if (words) {
+        while ((((uintptr_t)dst + i) & 3) != 0 && i < L) {
             dst[i] = byte_at(i);
             ++i;
         }
@@ -1674,6 +1663,20 @@ k_ibwt_unstash(const u32* __restrict__ stash, const u32* __restrict__ len_keep, 
         }
     }
     for (; i < L; ++i) dst[i] = byte_at(i);
+}
+
+// Copy every stashed sublist (length <= kIbwtStashCap) to its place in the text.
+__global__ void __launch_bounds__(128)
+k_ibwt_unstash(const u32* __restrict__ stash, const u32* __restrict__ len_keep, const u32* __restrict__ dist, u32 n, u32 regular,
+               u8* __restrict__ text_out, u32 cap) {
+    const u32 s = blockIdx.x * 128 + threadIdx.x;
+    if (s > regular) return;
+    const u32 len = len_keep[s];
+    if (len == 0 || len > cap) return;  // longer sublists are written by a second walk
+    const u64 pos = (u64)(n + 1) - dist[s];
+    if (pos >= n) return;
+    const u32 L = (u32)min((u64)len, (u64)n - pos);  // the '$' row's placeholder falls off the end
+    ibwt_copy_chunk(stash + (size_t)s * (cap / 4), text_out + pos, L, (((uintptr_t)text_out) & 3) == 0);
 }
 
 __global__ void k_ibwt_report(const u32* __restrict__ dist, u32 head_splitter, u32* __restrict__ out) { *out = dist[head_splitter]; }
@@ -2010,6 +2013,179 @@ k_many_emit(const u64* __restrict__ blk, const u32* __restrict__ ids, u32 n, con
         bwt[p] = text[id - 1];
     }
     if (sa_out != nullptr) sa_out[p] = id - first;
+}
+
+// ---- inverse BWT of many blocks in one pass (dark_bwt_inverse_many) ---------------------------------
+// The single-block method ("inverse BWT" above) over one ROW SPACE shared by B blocks.  Block b (bytes [starts[b],
+// starts[b+1]) of the concatenated BWTs, n_b of them) owns the n_b + 1 global rows [starts[b] + b, starts[b+1] + b + 1):
+// its '$' row first, then its real rows.
+//   psi    the real rows' last symbols under the key (b << 8) | symbol, sorted stably (one byte pass + 1-2 passes on
+//          the block number): the stable partition of every block at once.  Sorted slot q of block b is row q + b + 1;
+//          the row id stored there is its psi, the key's low byte its first symbol (one index for both loads, no
+//          symbol bases).  psi never leaves a block, whatever the input.
+//   walk   splitters are every stride-th global row plus each block's head row (local row origin_b + 1, splitter
+//          `regular + b`).  A walk finds its block once (binary search over the row offsets) and stops at a
+//          stride-th row or at its own block's head; reaching the head means it came through the '$' row, so that
+//          sublist ends the block's list (nil).  k_ibwt_jump then runs unchanged over the forest of lists.
+//   offset a splitter's text offset is starts[b] + n_b + 1 - dist.
+//   check  every block's list covers its n_b + 1 rows: dist[regular + b] == n_b + 1 (k_ibwt_many_check).
+__device__ __forceinline__ u32 row_block_of(const u32* __restrict__ starts, u32 B, u32 row) {  // largest b with starts[b] + b <= row
+    u32 lo = 0, hi = B - 1;
+    while (lo < hi) {
+        const u32 mid = (lo + hi + 1) >> 1;
+        if (__ldg(starts + mid) + mid <= row) lo = mid;
+        else hi = mid - 1;
+    }
+    return lo;
+}
+__device__ __forceinline__ u32 ibwt_many_block(const u32* __restrict__ starts, u32 B, u32 stride, u32 regular, u32 s) {
+    return s < regular ? row_block_of(starts, B, s * stride) : s - regular;
+}
+// (key, row) of every real row, in row order within each block (the sort is stable), and the digit histogram
+template <int THREADS>
+__global__ void __launch_bounds__(THREADS)
+k_ibwt_many_elements(const u8* __restrict__ bwt, u32 n, const u32* __restrict__ starts, u32 B,
+                     const unsigned long long* __restrict__ origins, u64* __restrict__ keys, u32* __restrict__ rows,
+                     u32* __restrict__ g_hist, int num_passes) {
+    __shared__ u32 s_hist[kMaxPasses * kRadix];
+    const int tid = threadIdx.x;
+    hist_clear(s_hist, tid, THREADS);
+    __syncthreads();
+    for (u64 e = (u64)blockIdx.x * THREADS + tid; e < n; e += (u64)gridDim.x * THREADS) {
+        const u32 b = block_of(starts, B, (u32)e);
+        const u32 first = __ldg(starts + b), origin = (u32)__ldg(origins + b);
+        const u32 le = (u32)e - first;
+        const u32 r = le == 0 ? 0u : (le <= origin ? le : le + 1u);  // local row, as in k_ibwt_elements
+        const u32 sym = le == 0 ? bwt[first + origin] : bwt[first + r - 1];
+        const u64 key = ((u64)b << 8) | sym;
+        keys[e] = key;
+        rows[e] = first + b + r;
+        hist_add_key(s_hist, key, 0, num_passes);
+    }
+    __syncthreads();
+    hist_flush(s_hist, g_hist, num_passes, tid, THREADS);
+}
+// MODE 0 / 1 / 2 as k_ibwt_walk: count / write (with only_longer_than: the sublists the stash could not hold) / count + stash.
+template <int MODE>
+__global__ void __launch_bounds__(128)
+k_ibwt_many_walk(const u32* __restrict__ psi, const u64* __restrict__ sorted_keys, const u32* __restrict__ starts, u32 B,
+                 const unsigned long long* __restrict__ origins, u32 stride, u32 regular, u32* __restrict__ len, u32* __restrict__ next,
+                 const u32* __restrict__ dist, u8* __restrict__ text_out, u32* __restrict__ len_keep, u32* __restrict__ stash,
+                 u32 only_longer_than, u32 cap) {
+    constexpr bool WRITE = MODE == 1, COUNT = MODE != 1, STASH = MODE == 2;
+    const u32 s = blockIdx.x * 128 + threadIdx.x;
+    if (s >= regular + B) return;
+    const u32 b = ibwt_many_block(starts, B, stride, regular, s);
+    const u32 first = __ldg(starts + b), nb = __ldg(starts + b + 1) - first;
+    const u32 dollar = first + b;  // the block's '$' row
+    const u32 head = dollar + (u32)__ldg(origins + b) + 1u;
+    u32 r = s < regular ? s * stride : head;
+    if (s < regular && r == head) {  // the head row is owned by its block's head splitter
+        if (COUNT) {
+            len[s] = 0;
+            next[s] = kIbwtNil;
+            if (STASH) len_keep[s] = 0;
+        }
+        return;
+    }
+    if (WRITE && only_longer_than && len_keep[s] <= only_longer_than) return;
+    u64 pos = 0;
+    if (WRITE) pos = (u64)nb + 1 - dist[s];  // block-relative text position of this splitter's row
+    u32 cnt = 0;
+    const bool word_stores = WRITE && (((uintptr_t)text_out) & 3) == 0;  // word stores as in k_ibwt_walk
+    u32 acc = 0, have = 0;
+    u64 wbase = 0;
+    u32* const chunk = STASH ? stash + (size_t)s * (cap / 4) : nullptr;
+    do {
+        u32 sym = 0, nx = head;  // the '$' row: no symbol, and its successor is the head
+        if (r != dollar) {
+            const u32 q = r - b - 1;  // sorted slot of row r
+            nx = __ldg(psi + q);
+            sym = (u32)(__ldg(sorted_keys + q) & 0xFFu);
+            DARK_ASSERT(nx >= dollar && nx <= dollar + nb && (u32)(__ldg(sorted_keys + q) >> 8) == b);
+        }
+        if (WRITE && r != dollar && pos + cnt < nb) {
+            const u64 q = (u64)first + pos + cnt;
+            DARK_ASSERT(pos <= nb);
+            if (word_stores) {
+                acc |= sym << (8 * (u32)(q & 3));
+                have |= 1u << (u32)(q & 3);
+                wbase = q & ~3ull;
+                if ((q & 3) == 3) {
+                    if (have == 0xFu) {
+                        *reinterpret_cast<u32*>(text_out + (q & ~3ull)) = acc;
+                    } else {
+                        for (u32 e = 0; e < 4; ++e)
+                            if ((have >> e) & 1u) text_out[(q & ~3ull) + e] = (u8)(acc >> (8 * e));
+                    }
+                    acc = 0;
+                    have = 0;
+                }
+            } else {
+                text_out[q] = (u8)sym;
+            }
+        }
+        if (STASH && cnt < cap) {
+            acc |= sym << (8 * (cnt & 3));
+            if ((cnt & 3) == 3) {
+                chunk[cnt >> 2] = acc;
+                acc = 0;
+            }
+        }
+        ++cnt;
+        r = nx;
+    } while (!(r % stride == 0 || r == head) && cnt <= nb);  // cnt bound: belt and braces (psi is a permutation of the block's rows)
+    if (WRITE && have) {
+        for (u32 e = 0; e < 4; ++e)
+            if ((have >> e) & 1u) text_out[wbase + e] = (u8)(acc >> (8 * e));
+    }
+    if (STASH && (cnt & 3) != 0 && cnt < cap) chunk[cnt >> 2] = acc;
+    if (COUNT) {
+        len[s] = cnt;
+        if (STASH) len_keep[s] = cnt;
+        next[s] = r == head ? kIbwtNil : r / stride;  // only the '$' row leads to the head: the list ends here
+    }
+}
+__global__ void __launch_bounds__(128)
+k_ibwt_many_unstash(const u32* __restrict__ stash, const u32* __restrict__ len_keep, const u32* __restrict__ dist,
+                    const u32* __restrict__ starts, u32 B, u32 stride, u32 regular, u8* __restrict__ text_out, u32 cap) {
+    const u32 s = blockIdx.x * 128 + threadIdx.x;
+    if (s >= regular + B) return;
+    const u32 len = len_keep[s];
+    if (len == 0 || len > cap) return;  // longer sublists are written by a second walk
+    const u32 b = ibwt_many_block(starts, B, stride, regular, s);
+    const u32 first = __ldg(starts + b), nb = __ldg(starts + b + 1) - first;
+    const u64 pos = (u64)nb + 1 - dist[s];
+    if (pos >= nb) return;
+    const u32 L = (u32)min((u64)len, (u64)nb - pos);  // the '$' row's placeholder falls off the block's end
+    ibwt_copy_chunk(stash + (size_t)s * (cap / 4), text_out + first + pos, L, (((uintptr_t)text_out) & 3) == 0);
+}
+// every block's list must cover its n_b + 1 rows: *bad_out = blocks that do not, *first_bad_out = the lowest of them
+__global__ void __launch_bounds__(1024)
+k_ibwt_many_check(const u32* __restrict__ dist, u32 regular, const u32* __restrict__ starts, u32 B, u32* __restrict__ bad_out,
+                  u32* __restrict__ first_bad_out) {
+    __shared__ u32 s_bad, s_first;
+    if (threadIdx.x == 0) {
+        s_bad = 0;
+        s_first = 0xFFFFFFFFu;
+    }
+    __syncthreads();
+    u32 bad = 0, first = 0xFFFFFFFFu;
+    for (u32 b = threadIdx.x; b < B; b += 1024) {
+        if ((u64)dist[regular + b] != (u64)__ldg(starts + b + 1) - __ldg(starts + b) + 1) {
+            ++bad;
+            first = min(first, b);
+        }
+    }
+    if (bad) {
+        atomicAdd(&s_bad, bad);
+        atomicMin(&s_first, first);
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        *bad_out = s_bad;
+        *first_bad_out = s_first;
+    }
 }
 
 // Debug statistic (DARK_BWT_GROUP_STATS=1): largest group of the active list (capped at 4096) and the

@@ -153,6 +153,57 @@ class Constructor:
                    "bwt::decode")
         return float(ms.value)
 
+    def inverse_many_into(self, bwt_ptrs, ns, origins, text_ptrs):
+        """Many small host blocks inverted in ONE device pass (dark_bwt_inverse_many): raw host addresses; returns the
+        device ms of the pass.  The blocks share the context's arena: sum(ns) + len(ns) <= capacity."""
+        cnt = len(ns)
+        assert len(bwt_ptrs) == cnt and len(origins) == cnt and len(text_ptrs) == cnt
+        B = (ctypes.c_void_p * cnt)(*bwt_ptrs)
+        T = (ctypes.c_void_p * cnt)(*text_ptrs)
+        N = (ctypes.c_uint64 * cnt)(*[int(x) for x in ns])
+        O = (ctypes.c_uint64 * cnt)(*[int(x) for x in origins])
+        ms = ctypes.c_float(0)
+        _ffi.check(self._L.dark_bwt_inverse_many(self._ctx, B, N, O, T, cnt, ctypes.byref(ms)), self._ctx, "bwt::decode (many)")
+        return float(ms.value)
+
+    def inverse_many(self, pairs):
+        """[text, ...] for a list of (bwt, origin) pairs of small blocks, inverted together in one pass over the GPU."""
+        bs = [_as_u8(b) for b, _ in pairs]
+        outs = [np.empty(b.size, dtype=np.uint8) for b in bs]
+        self.inverse_many_into([b.ctypes.data for b in bs], [b.size for b in bs], [int(o) for _, o in pairs],
+                               [o.ctypes.data for o in outs])
+        return outs
+
+    def inverse_many_device(self, d_bwt, d_starts, d_origins, count, d_text):
+        """Device-resident form, the layout bwt_many_device writes: blocks back to back in d_bwt, offsets d_starts[0..count]
+        (u32) and origins d_origins[0..count) (u64), all on the device.  Returns the device ms of the pass."""
+        ms = ctypes.c_float(0)
+        _ffi.check(self._L.dark_bwt_inverse_many_device(self._ctx, d_bwt, d_starts, d_origins, int(count), d_text, ctypes.byref(ms)),
+                   self._ctx, "bwt::decode (many)")
+        return float(ms.value)
+
+    def inverse_batch_into(self, bwt_ptrs, ns, origins, text_ptrs):
+        """Pipelined host entry over several blocks (dark_bwt_inverse_batch; raw host addresses, ideally pinned): copy-in
+        of block k+1 and copy-out of block k-1 overlap the inverse of block k.  Returns the per-block device ms."""
+        cnt = len(ns)
+        assert len(bwt_ptrs) == cnt and len(origins) == cnt and len(text_ptrs) == cnt
+        B = (ctypes.c_void_p * cnt)(*bwt_ptrs)
+        T = (ctypes.c_void_p * cnt)(*text_ptrs)
+        N = (ctypes.c_uint64 * cnt)(*[int(x) for x in ns])
+        O = (ctypes.c_uint64 * cnt)(*[int(x) for x in origins])
+        ms = (ctypes.c_float * max(cnt, 1))()
+        _ffi.check(self._L.dark_bwt_inverse_batch(self._ctx, B, N, O, T, cnt, ms), self._ctx, "bwt::decode (batch)")
+        return [float(ms[i]) for i in range(cnt)]
+
+    def inverse_blocks(self, pairs):
+        """[text, ...] for an iterable of (bwt, origin) host blocks, through the pipelined batch entry."""
+        pairs = list(pairs)
+        bs = [_as_u8(b) for b, _ in pairs]
+        outs = [np.empty(b.size, dtype=np.uint8) for b in bs]
+        self.inverse_batch_into([b.ctypes.data for b in bs], [b.size for b in bs], [int(o) for _, o in pairs],
+                                [o.ctypes.data for o in outs])
+        return outs
+
     # -- distance coding + MTF: bwt::dc::encode(&output, suf, &mut mtf) and its item stream (block/dc.rs:52, 82-85) ---------
     def _dc_result(self, info, n, dist, pos, idist, sym, rank):
         k = int(info.num_items)

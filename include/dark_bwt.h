@@ -153,6 +153,27 @@ int dark_bwt_inverse(dark_bwt_ctx *ctx, const uint8_t *bwt, uint64_t n, uint64_t
 int dark_bwt_inverse_device(dark_bwt_ctx *ctx, const uint8_t *d_bwt, uint64_t n, uint64_t origin, uint8_t *d_text_out,
                             float *ms_out /* nullable */);
 
+/* `count` independent host blocks, pipelined like dark_bwt_forward_batch: while block k is inverted, block k+1 is copied
+ * in and block k-1 copied out (double-buffered device staging, the two copy streams, pageable buffers of 1 MiB or more
+ * through the staging lanes).  Each block: 1 <= ns[k] <= capacity, origins[k] < ns[k].  ms_out (nullable) = `count`
+ * device times.  Results identical to `count` dark_bwt_inverse calls; DARK_BWT_E_INVALID_ARG with a device-only context. */
+int dark_bwt_inverse_batch(dark_bwt_ctx *ctx, const uint8_t *const *bwts, const uint64_t *ns, const uint64_t *origins,
+                           uint8_t *const *text_outs, uint64_t count, float *ms_out);
+
+/* MANY SMALL blocks inverted in ONE pass, the unpack side of dark_bwt_forward_many: `count` BWT blocks (each >= 1 byte,
+ * origins[k] < ns[k], count <= DARK_BWT_MAX_MANY_BLOCKS) give text_outs[k][0..ns[k]), what dark_bwt_inverse(bwts[k],
+ * ns[k], origins[k]) gives.  The blocks share one row space of sum(ns) + count rows (one '$' row per block), which must
+ * fit: sum(ns) + count <= capacity, else DARK_BWT_E_INVALID_N.  One H2D copy per block, one device pass, one D2H copy per
+ * block.  ms_out (nullable) = device time of the pass.  DARK_BWT_E_INVALID_ARG if some (bwt, origin) is not the forward
+ * transform of any text; dark_bwt_last_error() then names the first such block. */
+int dark_bwt_inverse_many(dark_bwt_ctx *ctx, const uint8_t *const *bwts, const uint64_t *ns, const uint64_t *origins,
+                          uint8_t *const *text_outs, uint64_t count, float *ms_out);
+/* Same on device buffers, the layout dark_bwt_forward_many_device writes: d_bwt holds the blocks back to back,
+ * d_starts[0..count] (u32) their offsets, d_origins[0..count) (u64) their origins, all on the device (offsets and origins
+ * are read back and checked before any kernel runs); d_text_out gets the texts at the same offsets. */
+int dark_bwt_inverse_many_device(dark_bwt_ctx *ctx, const uint8_t *d_bwt, const uint32_t *d_starts, const uint64_t *d_origins,
+                                 uint64_t count, uint8_t *d_text_out, float *ms_out);
+
 /* ---- distance coding + MTF (SURVEY.md 8f rank 3) ---------------------------------------------------------------
  * What `bwt::dc::encode(&output, suf, &mut self.mtf)` computes and what iterating its result yields
  * (/root/reference/src/block/dc.rs:52, 54-85).  That code is third-party (`compress::bwt::dc`, Cargo.toml:18) and absent

@@ -74,6 +74,12 @@ extern "C" {
     pub fn dark_bwt_forward_device(ctx: *mut dark_bwt_ctx, d_text: *const u8, n: u64, d_bwt_out: *mut u8,
                                    origin_out: *mut u64, d_sa_out: *mut u32, stats: *mut dark_bwt_stats) -> c_int;
     pub fn dark_bwt_inverse(ctx: *mut dark_bwt_ctx, bwt: *const u8, n: u64, origin: u64, text_out: *mut u8) -> c_int;
+    pub fn dark_bwt_inverse_batch(ctx: *mut dark_bwt_ctx, bwts: *const *const u8, ns: *const u64, origins: *const u64,
+                                  text_outs: *const *mut u8, count: u64, ms_out: *mut f32) -> c_int;
+    pub fn dark_bwt_inverse_many(ctx: *mut dark_bwt_ctx, bwts: *const *const u8, ns: *const u64, origins: *const u64,
+                                 text_outs: *const *mut u8, count: u64, ms_out: *mut f32) -> c_int;
+    pub fn dark_bwt_inverse_many_device(ctx: *mut dark_bwt_ctx, d_bwt: *const u8, d_starts: *const u32, d_origins: *const u64,
+                                        count: u64, d_text_out: *mut u8, ms_out: *mut f32) -> c_int;
     pub fn dark_bwt_reuse(ctx: *mut dark_bwt_ctx, words_out: *mut *mut u32, count_out: *mut u64) -> c_int;
     pub fn dark_bwt_destroy(ctx: *mut dark_bwt_ctx);
     pub fn dark_bwt_strerror(code: c_int) -> *const c_char;
