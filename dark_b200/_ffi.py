@@ -4,7 +4,7 @@ import os
 import subprocess
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-_LIB = os.environ.get("DARK_BWT_LIB") or os.path.join(_HERE, "lib", "libdark_bwt.so")  # DARK_BWT_LIB: tuning builds (tools/)
+_LIB = os.environ.get("DARK_BWT_LIB") or os.path.join(_HERE, "lib", "libdark_bwt.so")  # DARK_BWT_LIB: another build (e.g. `make checked`)
 _lib = None
 
 MAX_ROUNDS = 40

@@ -33,11 +33,8 @@ using namespace dark;
 
 namespace {
 
-constexpr int kSortTile = 3072;  // smallest tile of any pass variant (sizes the status buffer)
-#ifndef DARK_SCAN_THREADS
-#define DARK_SCAN_THREADS 512
-#endif
-constexpr int kScanThreads = DARK_SCAN_THREADS;  // tuning builds: -DDARK_SCAN_THREADS=256 (profiles/r1_ncu_rerank_final.md)
+constexpr int kSortTile = 3072;  // sizes the status buffer: no radix pass has a smaller tile
+constexpr int kScanThreads = 512;
 constexpr int kScanItems = 8;
 constexpr int kScanTile = kScanThreads * kScanItems;
 constexpr int kInitThreads = 256;
@@ -83,38 +80,25 @@ inline int bit_length(u64 x) {
 
 }  // namespace
 
-// Test and tuning knobs, resolved ONCE at dark_bwt_create from the environment (never on the hot path).  The test knobs
-// force code paths that the block size or content would otherwise choose; none of them changes a result, and each has
-// a parity test (tests/test_gpu_parity.py).  The tuning knobs can skip work (garbage output) or select kernels without
-// a forward-progress guarantee, so they exist only in builds with -DDARK_BWT_TUNING (tools/, never shipped).
+// Test knobs, resolved ONCE at dark_bwt_create from the environment (never on the hot path).  They force code paths
+// that the block size or content would otherwise choose; none of them changes a result, and each has a parity test
+// (tests/test_gpu_parity.py).
 struct Knobs {
     int pass_impl = 1;              // DARK_BWT_PASS_IMPL: 1 = onesweep_tma.cuh, 0 = the round-1 kernel k_onesweep_pass
     bool force_u64_status = false;  // DARK_BWT_FORCE_U64_STATUS=1
-    bool fused_init = true;         // DARK_BWT_FUSED_INIT=0 materialises the round-0 keys
-    bool gram_hist = true;          // DARK_BWT_GRAM_HIST=0 counts digits key by key
     bool check_hist = false;        // DARK_BWT_CHECK_HIST=1 counts both ways and compares
     bool inline_emit = true;        // DARK_BWT_INLINE_EMIT=0
     bool sparse_rerank = true;      // DARK_BWT_SPARSE_RERANK=0
-    int inline_gather = 0;          // DARK_BWT_INLINE_GATHER=1: unpruned blocks emit inline too, gathering T[id-1] in the re-rank
     bool fuse_round0 = true;        // DARK_BWT_FUSE_ROUND0=0: round 0 of an unpruned large block without the fused bucket sink
-    bool rerank_chainfree = false;  // DARK_BWT_RERANK_CHAINFREE=1: rounds >= 1 re-ranked by flags + scan + apply kernels (no look-back chain; measured
-                                    // equal to the single kernel on C3/C5/C4: profiles/r2_rejected.md)
     int text_div = 8;               // DARK_BWT_TEXT_BUILD=<k>: text-order key build while m > n/k (0 = never, no isa[] tag)
     bool pairs = true;              // DARK_BWT_PAIRS=0
     bool rank_search = true;        // DARK_BWT_RANK_SEARCH=0
     int bucketed = -1;              // DARK_BWT_BUCKETED=0/1 (-1: by block size)
     int host_chunk_mb = 2;          // DARK_BWT_HOST_CHUNK_MB: pinned bytes per staging lane (2 MiB chunks fill the pipeline sooner than 8: 23.1 vs 23.8 ms per C2 call)
     int host_threads = 12;          // DARK_BWT_HOST_THREADS=<t>: staging lanes per direction for pageable host buffers (0: let the driver stage)
-    int sort_variant = -1;          // DARK_BWT_SORT_VARIANT=<i>: run the round-1 kernel with tiling i
     int emit_window_mb = 64;        // DARK_BWT_EMIT_WINDOW_MB: text window of the emission
     int ibwt_stride = 48;           // DARK_BWT_IBWT_STRIDE: splitter stride of the inverse BWT
     bool ibwt_two_walks = false;    // DARK_BWT_IBWT_TWO_WALKS=1
-    // tuning builds only (-DDARK_BWT_TUNING)
-    bool tile_by_blockidx = false;  // DARK_BWT_TILE_BY_BLOCKIDX=1: tiles by blockIdx (no forward-progress guarantee)
-    unsigned knockout = 0;          // DARK_BWT_PASS_KNOCKOUT=<mask>: skip phases of k_onesweep_pass (garbage output)
-    int pass_prefetch = -1;         // DARK_BWT_PASS_PREFETCH=<tiles>
-    int rerank_prefetch = -1;       // DARK_BWT_RERANK_PREFETCH=<tiles>
-    bool group_stats = false;       // DARK_BWT_GROUP_STATS=1
 
     void read_env() {
         auto geti = [](const char* name, int dflt) {
@@ -123,14 +107,10 @@ struct Knobs {
         };
         pass_impl = geti("DARK_BWT_PASS_IMPL", pass_impl);
         force_u64_status = geti("DARK_BWT_FORCE_U64_STATUS", 0) != 0;
-        fused_init = geti("DARK_BWT_FUSED_INIT", 1) != 0;
-        gram_hist = geti("DARK_BWT_GRAM_HIST", 1) != 0;
         check_hist = geti("DARK_BWT_CHECK_HIST", 0) != 0;
         inline_emit = geti("DARK_BWT_INLINE_EMIT", 1) != 0;
         sparse_rerank = geti("DARK_BWT_SPARSE_RERANK", 1) != 0;
-        rerank_chainfree = geti("DARK_BWT_RERANK_CHAINFREE", 0) != 0;
         fuse_round0 = geti("DARK_BWT_FUSE_ROUND0", 1) != 0;
-        inline_gather = geti("DARK_BWT_INLINE_GATHER", 0);
         text_div = geti("DARK_BWT_TEXT_BUILD", text_div);
         pairs = geti("DARK_BWT_PAIRS", 1) != 0;
         rank_search = geti("DARK_BWT_RANK_SEARCH", 1) != 0;
@@ -141,17 +121,9 @@ struct Knobs {
         }
         host_threads = std::min(std::max(geti("DARK_BWT_HOST_THREADS", host_threads), 0), 16);
         host_chunk_mb = std::min(std::max(geti("DARK_BWT_HOST_CHUNK_MB", host_chunk_mb), 1), 64);
-        sort_variant = geti("DARK_BWT_SORT_VARIANT", -1);
         emit_window_mb = std::max(1, geti("DARK_BWT_EMIT_WINDOW_MB", 64));
         ibwt_stride = std::max(2, geti("DARK_BWT_IBWT_STRIDE", 48));
         ibwt_two_walks = geti("DARK_BWT_IBWT_TWO_WALKS", 0) != 0;
-#ifdef DARK_BWT_TUNING
-        tile_by_blockidx = geti("DARK_BWT_TILE_BY_BLOCKIDX", 0) != 0;
-        knockout = (unsigned)geti("DARK_BWT_PASS_KNOCKOUT", 0);
-        pass_prefetch = geti("DARK_BWT_PASS_PREFETCH", -1);
-        rerank_prefetch = geti("DARK_BWT_RERANK_PREFETCH", -1);
-        group_stats = geti("DARK_BWT_GROUP_STATS", 0) != 0;
-#endif
     }
 };
 
@@ -207,15 +179,12 @@ struct dark_bwt_ctx {
     u32 status_dirty_lo[2] = {0u, 0u}, status_dirty_hi[2] = {0u, 0u};
     u32* counters = nullptr;
     u64* scan_words = nullptr;
-    long long* pass_trace = nullptr;  // debug: per-tile phase stamps of the radix pass (dark_bwt_debug_trace)
-    long long* rerank_trace = nullptr;  // debug: per-tile phase stamps of the round-0 re-rank (dark_bwt_debug_trace_rerank)
     u32* bucket_hist = nullptr;  // 256 counters / cursors of the bucketed rank scatter
     u32* many_starts = nullptr;            // dark_bwt_forward_many: block offsets (kMaxManyBlocks + 1)
     unsigned long long* many_origins = nullptr;  // ... per-block origins
     u16* many_lut = nullptr;               // ... byte -> code 1..sigma
     DcInfoDev* dc_info = nullptr;             // dark_bwt_dc_*: device copy of the result header, followed by the run counter
-    u32* bitmap = nullptr;  // n bits: positions whose rank the next round reads; new-head flags of the chain-free re-rank
-    u32* bitmap2 = nullptr;  // old-head flags of the chain-free re-rank
+    u32* bitmap = nullptr;  // n bits: positions whose rank the next round reads; survivor flags of the sparse round-0 re-rank
     size_t scan_tiles = 0;
 
     Mailbox* mail = nullptr;      // pinned + mapped host memory: kernels write their scalar results straight into it
@@ -291,24 +260,19 @@ int next_counter(dark_bwt_ctx* ctx, u32** out) {
     return 0;
 }
 
-// Tuning variants of the radix pass (threads, items per thread, min CTAs per SM).  The default is
-// chosen from measurements (profiles/); DARK_BWT_SORT_VARIANT=<i> selects another one for sweeps.
 template <int THREADS, int ITEMS, int MINBLOCKS, int ILP, typename StatusT, bool ALIGNED, bool GEN = false>
 int launch_pass_kernel(dark_bwt_ctx* ctx, const u64* kin, const u32* vin, u64* kout, u32* vout, u32 m, int shift,
                        const u32* digit_base, u32* counter, u32 tiles, const u8* prev_text, u32 n_text, KeyGen gen = KeyGen()) {
     typedef OnesweepSmem<THREADS, ITEMS> Smem;
     auto kern = k_onesweep_pass<THREADS, ITEMS, MINBLOCKS, ILP, StatusT, ALIGNED, GEN>;
     CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)));  // per device
-    const bool by_block_index = ctx->knobs.tile_by_blockidx;
-    const u32 knock = ctx->knobs.knockout;  // tuning builds only: skip phases (1 look-back, 2 ranking, 4 stores)
     // persistent grid: as many CTAs as stay resident (SMs x MINBLOCKS), each claiming tiles until none are left
-    const u32 grid = by_block_index ? tiles : std::min<u32>(tiles, (u32)ctx->num_sms * MINBLOCKS);
+    const u32 grid = std::min<u32>(tiles, (u32)ctx->num_sms * MINBLOCKS);
     // L2 prefetch distance in tiles: two thirds of a wave of claims (the persistent grid; 148..444 measured alike, beyond
-    // one wave the gain fades) unless DARK_BWT_PASS_PREFETCH says otherwise (0 = off)
-    const u32 prefetch_ahead = by_block_index ? 0u : (ctx->knobs.pass_prefetch >= 0 ? (u32)ctx->knobs.pass_prefetch : std::max(1u, grid * 2 / 3));
-    kern<<<grid, THREADS, sizeof(Smem), ctx->stream>>>(kin, vin, kout, vout, m, shift, digit_base, (StatusT*)ctx->sort_status,
-                                                        by_block_index ? nullptr : counter, ctx->pass_trace, prev_text, n_text, knock, gen,
-                                                        prefetch_ahead);
+    // one wave the gain fades)
+    const u32 prefetch_ahead = std::max(1u, grid * 2 / 3);
+    kern<<<grid, THREADS, sizeof(Smem), ctx->stream>>>(kin, vin, kout, vout, m, shift, digit_base, (StatusT*)ctx->sort_status, counter,
+                                                        prev_text, n_text, gen, prefetch_ahead);
     LAUNCHED();
     return 0;
 }
@@ -382,7 +346,7 @@ int launch_pass_tma(dark_bwt_ctx* ctx, const u64* kin, const u32* vin, u64* kout
                        : k_onesweep_tma<THREADS, ITEMS, MINBLOCKS, ILP, ST, GEN, false>;                                     \
         CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)));                      \
         kern<<<grid, THREADS, sizeof(Smem), ctx->stream>>>(kin, vin, kout, vout, m, shift, digit_base, (ST*)st_use, (ST*)st_clean, \
-                                                           counter, g, prev_text, ctx->pass_trace);                          \
+                                                           counter, g, prev_text);                                           \
     } while (0)
     if (gen) {
         if (wide) LT(u64, true);
@@ -396,17 +360,8 @@ int launch_pass_tma(dark_bwt_ctx* ctx, const u64* kin, const u32* vin, u64* kout
     return 0;
 }
 
-#ifndef DARK_PASS_ILP
-#define DARK_PASS_ILP 2
-#endif
-#ifndef DARK_PASS_THREADS
-#define DARK_PASS_THREADS 256
-#define DARK_PASS_ITEMS 16
-#endif
-#ifndef DARK_PASS_CTAS
-#define DARK_PASS_CTAS 2
-#endif
-constexpr int kDefaultSortVariant = 1;  // 256 threads x 16 items, 3 CTAs/SM: best of the sweeps in profiles/r1_sort_variants_*.log
+// Tiling of the pipelined pass: threads, items per thread, CTAs per SM, ranking items in flight per warp
+constexpr int kPassThreads = 256, kPassItems = 16, kPassCtas = 2, kPassIlp = 2;
 
 // One onesweep pass over m pairs: buffers[cur] -> buffers[cur^1].
 int launch_pass(dark_bwt_ctx* ctx, const u64* kin, const u32* vin, u64* kout, u32* vout, u32 m, int shift,
@@ -422,27 +377,14 @@ int launch_pass(dark_bwt_ctx* ctx, const u64* kin, const u32* vin, u64* kout, u3
     // DARK_BWT_FORCE_U64_STATUS=1 exercises the wide path on small inputs (tests).
     const bool wide = !(m < (1u << 30)) || ctx->knobs.force_u64_status;
     const bool wide_tma = m > (1u << 31) || ctx->knobs.force_u64_status;  // the pipelined pass keeps 31 bits of prefix in a 4-byte word
-    const bool ev = ctx->knobs.sort_variant >= 0;
-    const int variant = ev ? ctx->knobs.sort_variant : kDefaultSortVariant;
-    {
-        // default: the TMA-staged pipelined pass; DARK_BWT_PASS_IMPL=0 keeps the round-1 kernel (k_onesweep_pass)
-        const int impl = ctx->knobs.pass_impl;
-        const bool eligible = (shift & 7) == 0 && !ev && (gen == nullptr || gen->mode == 0) &&
-                              (gen != nullptr || (prev_text == nullptr && ((uintptr_t)kin & 15) == 0 && ((uintptr_t)vin & 15) == 0));
-        if (impl != 0 && eligible) {
-            return launch_pass_tma<DARK_PASS_THREADS, DARK_PASS_ITEMS, DARK_PASS_CTAS, DARK_PASS_ILP>(ctx, kin, vin, kout, vout, m, shift, digit_base, counter, wide_tma, prev_text, gen);
-        }
-    }
-    if (gen != nullptr) return launch_pass_variant<256, 16, 3, 2>(ctx, kin, vin, kout, vout, m, shift, digit_base, counter, wide, prev_text, n_text, gen);
-#define V(T, I, B, L) return launch_pass_variant<T, I, B, L>(ctx, kin, vin, kout, vout, m, shift, digit_base, counter, wide, prev_text, n_text)
-    switch (variant) {
-        case 0: V(256, 16, 2, 2);
-        case 2: V(256, 12, 3, 2);
-        case 5: V(512, 12, 2, 2);
-        case 42: V(384, 16, 2, 2);
-        default: V(256, 16, 3, 2);  // 1
-    }
-#undef V
+    // default: the TMA-staged pipelined pass; DARK_BWT_PASS_IMPL=0 keeps the round-1 kernel (k_onesweep_pass)
+    const bool eligible = (shift & 7) == 0 && (gen == nullptr || gen->mode == 0) &&
+                          (gen != nullptr || (prev_text == nullptr && ((uintptr_t)kin & 15) == 0 && ((uintptr_t)vin & 15) == 0));
+    if (ctx->knobs.pass_impl != 0 && eligible)
+        return launch_pass_tma<kPassThreads, kPassItems, kPassCtas, kPassIlp>(ctx, kin, vin, kout, vout, m, shift, digit_base, counter, wide_tma,
+                                                                              prev_text, gen);
+    // the round-1 kernel: 256 threads x 16 items, 3 CTAs/SM, best of the tiling sweeps in profiles/r1_sort_variants_*.log
+    return launch_pass_variant<256, 16, 3, 2>(ctx, kin, vin, kout, vout, m, shift, digit_base, counter, wide, prev_text, n_text, gen);
 }
 
 // Sort passes for a histogram that is already in ctx->hist (counts).  `cur` is the index of the
@@ -533,43 +475,18 @@ int launch_rerank(dark_bwt_ctx* ctx, const u64* keys, const u32* ids, u32 m, u32
     if (tiles > ctx->scan_tiles) return ctx->fail_internal("scan tile state too small");
     ScanTileState ts{ctx->scan_words};
     constexpr size_t smem = kRerankSmem<kScanTile>;
-    if (!ROUND0 && ctx->knobs.rerank_chainfree) {
-        // rounds >= 1: flags + tile aggregates, a scan over the aggregates, apply — no chain between tiles (suffix_kernels.cuh)
-        auto kflags = k_rerank<kScanThreads, kScanItems, false, false, 1>;
-        auto kapply = k_rerank<kScanThreads, kScanItems, false, PAIRS, 2>;
-        if (smem > 48 * 1024) {
-            CK(cudaFuncSetAttribute(kflags, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            CK(cudaFuncSetAttribute(kapply, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        }
-        u8* fnew = (u8*)ctx->bitmap;
-        u8* fold = (u8*)ctx->bitmap2;
-        kflags<<<tiles, kScanThreads, 0, ctx->stream>>>(keys, ids, ctx->ranks, m, n, K, kb, ctx->isa, sa, out_ids, ctx->ranks_alt, ts, nullptr,
-                                                           &ctx->mail_dev->count, nullptr, nullptr, nullptr, 0, text, bwt_inline,
-                                                           &ctx->mail_dev->origin, 0u, ctx->tag, nullptr, fnew, fold);
-        LAUNCHED();
-        k_rerank_scan_tiles<<<1, 1024, 0, ctx->stream>>>(ctx->scan_words, tiles, &ctx->mail_dev->count);
-        LAUNCHED();
-        kapply<<<tiles, kScanThreads, smem, ctx->stream>>>(keys, ids, ctx->ranks, m, n, K, kb, ctx->isa, sa, out_ids, ctx->ranks_alt, ts, nullptr,
-                                                           &ctx->mail_dev->count, sink.ids, sink.vals, ctx->bucket_hist, sink.shift, text, bwt_inline,
-                                                           &ctx->mail_dev->origin, 0u, ctx->tag, nullptr, fnew, fold);
-        LAUNCHED();
-        std::swap(ctx->ranks, ctx->ranks_alt);
-        ctx->count_dev = nullptr;  // this form leaves the count in the mailbox only
-        return 0;
-    }
     u32 *counter = nullptr, *count_copy = nullptr;  // two consecutive words: the tile counter, then the survivor count (device copy)
     if (int rc = next_counter(ctx, &counter)) return rc;
     if (int rc = next_counter(ctx, &count_copy)) return rc;
     ctx->count_dev = count_copy;
     CK(cudaMemsetAsync(ctx->scan_words, 0, sizeof(u64) * kScanWordsPerTile * tiles, ctx->stream));
-    const u32 prefetch_ahead = ctx->knobs.rerank_prefetch >= 0 ? (u32)ctx->knobs.rerank_prefetch : 2u * (u32)ctx->num_sms;  // one wave of CTAs ahead (-2 %)
+    const u32 prefetch_ahead = 2u * (u32)ctx->num_sms;  // one wave of CTAs ahead (-2 %)
     auto kern = k_rerank<kScanThreads, kScanItems, ROUND0, PAIRS>;
     if (smem > 48 * 1024) CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kern<<<tiles, kScanThreads, smem, ctx->stream>>>(
         keys, ids, ROUND0 ? nullptr : ctx->ranks, m, n, K, kb, ctx->isa, sa, out_ids, ROUND0 ? ctx->ranks : ctx->ranks_alt, ts, counter,
         &ctx->mail_dev->count, sink.ids, sink.vals,
-        ctx->bucket_hist, sink.shift, text, bwt_inline, &ctx->mail_dev->origin, prefetch_ahead, (ROUND0 && !PAIRS) ? 0u : ctx->tag,
-        ROUND0 ? ctx->rerank_trace : nullptr, nullptr, nullptr);
+        ctx->bucket_hist, sink.shift, text, bwt_inline, &ctx->mail_dev->origin, prefetch_ahead, (ROUND0 && !PAIRS) ? 0u : ctx->tag);
     LAUNCHED();
     if (!ROUND0) std::swap(ctx->ranks, ctx->ranks_alt);
     return 0;
@@ -721,26 +638,22 @@ int forward_device(dark_bwt_ctx* ctx, const u8* d_text, u64 n64, u8* d_bwt, u64*
     }
 
     // ---- round 0: keys of K symbols, ids descending
-    // Fused initial keys (s in {1,2,4,8}): the key builder only counts digits; the first radix pass that runs
-    // rebuilds the keys from the text (radix_sort.cuh, GEN).  DARK_BWT_FUSED_INIT=0 materialises them instead.
+    // Fused initial keys (s in {1,2,4,8}): the digit histograms come from the text's q-grams (suffix_kernels.cuh) and
+    // the first radix pass that runs builds the keys from the text (radix_sort.cuh, GEN).
     const Knobs& kn = ctx->knobs;
     const bool packed_s = s_bits == 1 || s_bits == 2 || s_bits == 4 || s_bits == 8;
-    const bool fuse_init = packed_s && kn.fused_init && kn.sort_variant < 0;
-    const bool gram_hist = packed_s && kn.gram_hist;  // histograms from the text's q-grams (suffix_kernels.cuh)
     const int lg_s = s_bits == 1 ? 0 : s_bits == 2 ? 1 : s_bits == 4 ? 2 : 3;
-    auto init_keys = [&](bool write, bool hist) -> int {
+    // packed widths: the keys (write) or the digit histograms counted key by key (!write); other widths: both
+    auto init_keys = [&](bool write) -> int {
         const u32 blocks = (u32)std::min<u64>(ceil_div(n, kInitThreads * kInitItems), (u64)ctx->num_sms * 8);
 #define INIT_PACKED(S)                                                                                                              \
     do {                                                                                                                            \
-        if (write && hist)                                                                                                          \
-            k_init_keys_packed<kInitThreads, kInitItems, S, true, true><<<blocks, kInitThreads, 0, ctx->stream>>>(                  \
-                d_text, n, ctx->lut, ctx->keys[0], ctx->ids[0], ctx->hist);                                                         \
-        else if (write)                                                                                                             \
-            k_init_keys_packed<kInitThreads, kInitItems, S, true, false><<<blocks, kInitThreads, 0, ctx->stream>>>(                 \
+        if (write)                                                                                                                  \
+            k_init_keys_packed<kInitThreads, kInitItems, S, true><<<blocks, kInitThreads, 0, ctx->stream>>>(                        \
                 d_text, n, ctx->lut, ctx->keys[0], ctx->ids[0], ctx->hist);                                                         \
         else                                                                                                                        \
-            k_init_keys_packed<kInitThreads, kInitItems, S, false, true><<<blocks, kInitThreads, 0, ctx->stream>>>(d_text, n, ctx->lut, \
-                                                                                                               nullptr, nullptr, ctx->hist); \
+            k_init_keys_packed<kInitThreads, kInitItems, S, false><<<blocks, kInitThreads, 0, ctx->stream>>>(                       \
+                d_text, n, ctx->lut, nullptr, nullptr, ctx->hist);                                                                  \
     } while (0)
         switch (s_bits) {
             case 1: INIT_PACKED(1); break;
@@ -755,7 +668,7 @@ int forward_device(dark_bwt_ctx* ctx, const u8* d_text, u64 n64, u8* d_bwt, u64*
         LAUNCHED();
         return 0;
     };
-    if (gram_hist) {
+    if (packed_s) {
         u32* gram = ctx->bucket_hist;  // 256 counters, free until the first rank scatter
         CK(cudaMemsetAsync(gram, 0, sizeof(u32) * kRadix, ctx->stream));
         const u32 blocks = (u32)std::min<u64>(ceil_div(n, 256 * 16), (u64)ctx->num_sms * 8);
@@ -772,17 +685,15 @@ int forward_device(dark_bwt_ctx* ctx, const u8* d_text, u64 n64, u8* d_bwt, u64*
             std::vector<u32> a(kMaxPasses * kRadix), b(kMaxPasses * kRadix);
             CK(cudaMemcpyAsync(a.data(), ctx->hist, a.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
             CK(cudaMemsetAsync(ctx->hist, 0, sizeof(u32) * kMaxPasses * kRadix, ctx->stream));
-            if (int rc = init_keys(false, true)) return rc;
+            if (int rc = init_keys(false)) return rc;
             CK(cudaMemcpyAsync(b.data(), ctx->hist, b.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
             CK(sync_counted(ctx));
             if (a != b) return ctx->fail_internal("q-gram histogram differs from the per-key histogram");
             CK(cudaMemcpyAsync(ctx->hist, a.data(), a.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
             CK(sync_counted(ctx));
         }
-        if (!fuse_init)
-            if (int rc = init_keys(true, false)) return rc;
     } else {
-        if (int rc = init_keys(!fuse_init, true)) return rc;
+        if (int rc = init_keys(true)) return rc;
     }
     span_end(ctx, sp);
 
@@ -802,17 +713,16 @@ int forward_device(dark_bwt_ctx* ctx, const u8* d_text, u64 n64, u8* d_bwt, u64*
     gen.origin = 0;
     bool gen_used = false;
     if (int rc = run_sort(ctx, ctx->keys, ctx->ids, cur, n, 0, passes0, &cur, st, 0, /*prune=*/!no_pack, &first_pass,
-                          want_inline ? d_text : nullptr, &emit_inline, fuse_init ? &gen : nullptr, &gen_used))
+                          want_inline ? d_text : nullptr, &emit_inline, packed_s ? &gen : nullptr, &gen_used))
         return rc;
-    if (fuse_init && !gen_used) {  // every digit was trivial (one-symbol text): no pass ran, the re-rank still wants the keys
-        if (int rc = init_keys(true, false)) return rc;
+    if (packed_s && !gen_used) {  // every digit was trivial (one-symbol text): no pass ran, the re-rank still wants the keys
+        if (int rc = init_keys(true)) return rc;
         cur = 0;
     }
     span_end(ctx, sp);
-    // DARK_BWT_INLINE_GATHER=1: an unpruned block emits inline as well, the re-rank gathering T[id-1] for every suffix as it
-    // settles.  Measured equal to the final gather pass (C4: re-rank +38 ms, emission -37 ms: one random DRAM sector per
-    // suffix wherever the read is issued, profiles/r2_rejected.md), so it stays an option.
-    if (want_inline && !emit_inline && kn.inline_gather > 0) emit_inline = true;
+    // An unpruned block emits in a final gather pass.  Emitting it inline instead, the re-rank gathering T[id-1] for every
+    // suffix as it settles, measured equal (C4: re-rank +38 ms, emission -37 ms: one random DRAM sector per suffix wherever
+    // the read is issued, profiles/r2_rejected.md).
     u8* bwt_inline = emit_inline ? d_bwt : nullptr;
     // The sort covered the key bits above `drop`: K0 whole leading symbols are known equal inside a
     // tie group, Kc symbols were touched (a suffix shorter than Kc had padding compared).
@@ -991,16 +901,6 @@ int forward_device(dark_bwt_ctx* ctx, const u8* d_text, u64 n64, u8* d_bwt, u64*
             h *= 2;
             ++round;
             continue;
-        }
-        if (kn.group_stats) {  // debug: group-size statistics of the active list
-            CK(cudaMemsetAsync(ctx->bucket_hist, 0, 8, ctx->stream));
-            k_group_stats<<<(u32)ceil_div(m, 256), 256, 0, ctx->stream>>>(ctx->ranks, m, ctx->bucket_hist);
-            LAUNCHED();
-            u32 gs[2] = {0, 0};
-            CK(cudaMemcpyAsync(gs, ctx->bucket_hist, 8, cudaMemcpyDeviceToHost, ctx->stream));
-            CK(sync_counted(ctx));
-            fprintf(stderr, "[dark_bwt] round %d: h=%llu active=%u groups=%u max_group=%u%s\n", round, (unsigned long long)h, m, gs[1],
-                    gs[0], gs[0] >= 4096 ? "+" : "");
         }
         sp = span_begin(ctx, PH_KEYBUILD);
         CK(cudaMemsetAsync(ctx->hist, 0, sizeof(u32) * kMaxPasses * kRadix, ctx->stream));
@@ -1727,7 +1627,6 @@ int dark_bwt_create_ex(uint64_t max_n, int device, uint32_t flags, dark_bwt_ctx*
     const size_t o_counters = carve(sizeof(u32) * kMaxCounters);
     const size_t o_bhist = carve(sizeof(u32) * 1280);  // 256 bucket counters/cursors + 257 chunk prefixes; DC: first/last occurrences + dense alphabet
     const size_t o_bitmap = carve(sizeof(u32) * (ceil_div(N, 32) + 1) + 1024);  // + one tile of flag bytes past the end
-    const size_t o_bitmap2 = carve(sizeof(u32) * (ceil_div(N, 32) + 1) + 1024);
     const size_t o_swords = carve(sizeof(u64) * kScanWordsPerTile * ctx->scan_tiles);
     const size_t o_mstarts = carve(sizeof(u32) * (kMaxManyBlocks + 1));
     const size_t o_morigins = carve(sizeof(unsigned long long) * kMaxManyBlocks);
@@ -1766,7 +1665,6 @@ int dark_bwt_create_ex(uint64_t max_n, int device, uint32_t flags, dark_bwt_ctx*
     ctx->counters = (u32*)(base + o_counters);
     ctx->scan_words = (u64*)(base + o_swords);
     ctx->bitmap = (u32*)(base + o_bitmap);
-    ctx->bitmap2 = (u32*)(base + o_bitmap2);
     ctx->bucket_hist = (u32*)(base + o_bhist);
     ctx->many_starts = (u32*)(base + o_mstarts);
     ctx->many_origins = (unsigned long long*)(base + o_morigins);
@@ -2164,30 +2062,6 @@ int dark_bwt_verify_sa_device(dark_bwt_ctx* ctx, const uint8_t* d_text, uint64_t
     CK(cudaStreamSynchronize(ctx->stream));
     *bad_out = ctx->mail->bad;
     return DARK_BWT_OK;
-}
-
-// Debug hook (not in the public header): per-tile clock64() stamps of subsequent radix passes are
-// written to d_trace ([tiles][8] long long); nullptr switches tracing off.
-int dark_bwt_debug_trace_rerank(dark_bwt_ctx* ctx, long long* d_trace) {
-    if (!ctx) return DARK_BWT_E_INVALID_ARG;
-#if defined(DARK_BWT_TUNING) || defined(DARK_TUNE_TRACE)
-    ctx->rerank_trace = d_trace;
-    return DARK_BWT_OK;
-#else
-    (void)d_trace;
-    return DARK_BWT_E_INVALID_ARG;  // tracing exists in tuning builds only
-#endif
-}
-
-int dark_bwt_debug_trace(dark_bwt_ctx* ctx, long long* d_trace) {
-    if (!ctx) return DARK_BWT_E_INVALID_ARG;
-#if defined(DARK_BWT_TUNING) || defined(DARK_TUNE_TRACE)
-    ctx->pass_trace = d_trace;
-    return DARK_BWT_OK;
-#else
-    (void)d_trace;
-    return DARK_BWT_E_INVALID_ARG;  // tracing exists in tuning builds only
-#endif
 }
 
 int dark_bwt_lcp_profile_device(dark_bwt_ctx* ctx, const uint8_t* d_text, uint64_t n64, const uint32_t* d_sa, uint64_t* m_out,

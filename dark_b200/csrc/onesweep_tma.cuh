@@ -32,10 +32,6 @@
 
 #include "radix_sort.cuh"
 
-#ifndef DARK_SCANNERS
-#define DARK_SCANNERS 4
-#endif
-
 namespace dark {
 
 template <int THREADS, int ITEMS>
@@ -55,8 +51,8 @@ struct PipeSmem {
     u8 lut[256];
 };
 
-static_assert(DARK_SCANNERS >= 1 && 256 % DARK_SCANNERS == 0, "every digit needs a scanner: the scanner count must divide 256");
-constexpr int kScanners = DARK_SCANNERS;  // scanner CTAs per pass: each owns 256 / kScanners digits (tickets 0 .. kScanners-1)
+constexpr int kScanners = 4;  // scanner CTAs per pass: each owns 256 / kScanners digits (tickets 0 .. kScanners-1)
+static_assert(256 % kScanners == 0, "every digit needs a scanner: the scanner count must divide 256");
 constexpr int kScannerBatch = 32;      // status rows per scanner batch (three in flight: 3 * 32 zeroed rows follow the last tile)
 constexpr u32 kGenStageBytes = 4288;   // text slice of a 4,096-suffix tile: 4,096 + 64 symbols of look-ahead + alignment slack
 constexpr u32 kGenWordsOff = 8192;     // byte offset of the packed code words inside stage_keys
@@ -113,17 +109,9 @@ __global__ void __launch_bounds__(THREADS, MINBLOCKS)
 k_onesweep_tma(const u64* __restrict__ keys_in, const u32* __restrict__ vals_in, u64* __restrict__ keys_out,
                u32* __restrict__ vals_out, const u32 m, const int shift, const u32* __restrict__ digit_base,
                StatusT* __restrict__ status, StatusT* __restrict__ status_clean, u32* __restrict__ tile_counter, const KeyGen gen,
-               const u8* __restrict__ prev_text, long long* __restrict__ trace) {
+               const u8* __restrict__ prev_text) {
     // status_clean (nullable): the status buffer the NEXT pass will use.  Every worker zeroes the row of each tile it
     // processes there, so the host need not launch a memset between passes (64 MB per 2^28 pairs and a launch gap each).
-    // tuning builds only (-DDARK_TUNE_TRACE, tools/pass_trace2.py): thread 0 stamps clock64() at the phase boundaries
-#ifdef DARK_TUNE_TRACE
-#define TMA_STAMP(t, i) do { if (trace && threadIdx.x == 0) trace[(size_t)(t) * 12 + (i)] = clock64(); } while (0)
-#define TMA_GT(t, i, who) do { if (trace && threadIdx.x == (who)) { unsigned long long gt_; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt_)); trace[(size_t)(t) * 12 + (i)] = (long long)gt_; } } while (0)
-#else
-#define TMA_STAMP(t, i) do { (void)trace; } while (0)
-#define TMA_GT(t, i, who) do { } while (0)
-#endif
     static_assert(THREADS >= kRadix && THREADS % 32 == 0, "one thread per digit is assumed");
     static_assert(ITEMS % 2 == 0 && 32 * ITEMS < 65536, "ranks are packed two per register");
     typedef PipeSmem<THREADS, ITEMS> Smem;
@@ -264,13 +252,8 @@ k_onesweep_tma(const u64* __restrict__ keys_in, const u32* __restrict__ vals_in,
                 const u64 kk = s.keys[p];
                 const u32 idx = s.global_off[digit(kk)] + p;
                 DARK_ASSERT(idx < m);
-#ifdef DARK_TUNE_NO_STORES
-                if (idx == 0xFFFFFFF3u)
-#endif
-                {
-                    keys_out[idx] = kk;
-                    vals_out[idx] = s.vals[p];
-                }
+                keys_out[idx] = kk;
+                vals_out[idx] = s.vals[p];
             }
         }
     };
@@ -367,9 +350,6 @@ k_onesweep_tma(const u64* __restrict__ keys_in, const u32* __restrict__ vals_in,
                 }
             }
         }
-#ifndef DARK_TUNE_TRACE_FINE
-        TMA_STAMP(tile, 1);
-#endif
         __syncthreads();  // every thread has read the stage: it may be refilled
     };
 
@@ -431,21 +411,14 @@ k_onesweep_tma(const u64* __restrict__ keys_in, const u32* __restrict__ vals_in,
         const u32 nvalid = (u32)min((u64)TILE, (u64)m - (u64)tile * TILE);
         const bool full = nvalid == (u32)TILE;
         if (status_clean != nullptr && digit_thread) status_clean[(size_t)tile * kRadix + tid] = 0;
-        TMA_STAMP(tile, 0);
         if (full) {
             load_tile(BoolC<true>(), nvalid);
-#ifndef DARK_TUNE_TRACE_FINE
-            TMA_STAMP(tile, 2);
-#endif
             rank_tile(BoolC<true>(), nvalid);
         } else {
             load_tile(BoolC<false>(), nvalid);
-            TMA_STAMP(tile, 2);
             rank_tile(BoolC<false>(), nvalid);
         }
-        TMA_STAMP(tile, 3);
         __syncthreads();
-        TMA_STAMP(tile, 4);
 
         // ---- per digit: exclusive offsets across warps, tile total, publish the aggregate
         u32 count = 0;
@@ -461,9 +434,6 @@ k_onesweep_tma(const u64* __restrict__ keys_in, const u32* __restrict__ vals_in,
             DARK_ASSERT(tile < num_tiles && count <= nvalid);
             st_relaxed(status + (size_t)tile * kRadix + tid, ST::kPub | (StatusT)count);
         }
-#ifdef DARK_TUNE_TRACE_FINE
-        TMA_GT(tile, 1, 255);
-#endif
         u32 incl = count;
 #pragma unroll
         for (int o = 1; o < 32; o <<= 1) {
@@ -472,7 +442,6 @@ k_onesweep_tma(const u64* __restrict__ keys_in, const u32* __restrict__ vals_in,
         }
         if (digit_thread && lane == 31) s.warp_sum[warp] = incl;
         __syncthreads();
-        TMA_STAMP(tile, 5);
         u32 dstart = 0;
         if (digit_thread) {
             u32 wbase = 0;
@@ -481,21 +450,14 @@ k_onesweep_tma(const u64* __restrict__ keys_in, const u32* __restrict__ vals_in,
 #pragma unroll
             for (int w = 0; w < Smem::kWarps; ++w) s.warp_hist[w][tid] += dstart;
             if (have_prev) {
-#ifndef DARK_TUNE_NO_WAIT
                 while (!ST::resolved(my_row)) {
                     __nanosleep(32);  // the scanner is behind: do not hammer L2 with 256 polls per CTA
                     my_row = ld_relaxed(status + (size_t)prev_tile * kRadix + tid);
                 }
-#endif
                 s.global_off[tid] = digit_base[tid] + (u32)(my_row & ST::kPrefix) - prev_dstart;
-#ifdef DARK_TUNE_TRACE_FINE
-                TMA_GT(prev_tile, 2, 255);
-#endif
             }
         }
-        TMA_STAMP(tile, 6);
         __syncthreads();
-        TMA_STAMP(tile, 7);
         // The next ticket is taken only now, after the wait for the previous tile's prefix: tickets must be handed out
         // in (nearly) the order in which the tiles will publish their counts - the scanner works in tile order, so
         // every tile behind a late one waits for it - and a wait between ticket and counts would feed on itself.
@@ -519,21 +481,11 @@ k_onesweep_tma(const u64* __restrict__ keys_in, const u32* __restrict__ vals_in,
             s.next_tile = nxt;
             if (nxt < num_tiles && staged(nxt)) issue_load(nxt);
         }
-        TMA_STAMP(tile, 8);
         __syncthreads();  // the re-order buffer is free
-        TMA_STAMP(tile, 9);
         const u32 nxt_tile = s.next_tile;
 
         if (full) reorder_tile(BoolC<true>(), nvalid);
         else reorder_tile(BoolC<false>(), nvalid);
-        TMA_STAMP(tile, 10);
-#ifdef DARK_TUNE_TRACE
-        if (trace && threadIdx.x == 0) {
-            unsigned int smid;
-            asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-            trace[(size_t)tile * 12 + 11] = (long long)smid;
-        }
-#endif
         have_prev = true;
         prev_tile = tile;
         prev_nvalid = nvalid;
@@ -545,18 +497,13 @@ k_onesweep_tma(const u64* __restrict__ keys_in, const u32* __restrict__ vals_in,
     // ---- drain: the last tile of this CTA
     __syncthreads();
     if (digit_thread) {
-#ifndef DARK_TUNE_NO_WAIT
         do my_row = ld_relaxed(status + (size_t)prev_tile * kRadix + tid);
         while (!ST::resolved(my_row));
-#endif
         s.global_off[tid] = digit_base[tid] + (u32)(my_row & ST::kPrefix) - prev_dstart;
     }
     __syncthreads();
     if (prev_nvalid == (u32)TILE) scatter(BoolC<true>(), prev_nvalid);
     else scatter(BoolC<false>(), prev_nvalid);
 }
-
-#undef TMA_STAMP
-#undef TMA_GT
 
 }  // namespace dark

@@ -241,17 +241,7 @@ __device__ __forceinline__ void onesweep_tile(OnesweepSmem<THREADS, ITEMS>& s, c
                                               const u32* __restrict__ vals_in, u64* __restrict__ keys_out,
                                               u32* __restrict__ vals_out, const u32 tile, const u32 nvalid, const int shift,
                                               const u32* __restrict__ digit_base, StatusT* __restrict__ status,
-                                              long long* __restrict__ trace, const u8* __restrict__ prev_text, const u32 n_text, const u32 knock,
-                                              const KeyGen gen) {
-    // knock != 0 (tools/sort_bench.py KNOCKOUT only): phases are skipped to measure what they cost; output is garbage
-    // trace != nullptr (tools/pass_trace.py only): thread 0 stamps clock64() at the phase boundaries
-#ifdef DARK_BWT_TUNING
-#define DARK_STAMP(i) do { if (trace && threadIdx.x == 0) trace[(size_t)tile * 12 + (i)] = clock64(); } while (0)
-#define DARK_KNOCK(bit) (knock & (bit))
-#else
-#define DARK_STAMP(i) do { (void)trace; } while (0)
-#define DARK_KNOCK(bit) ((void)knock, false)
-#endif
+                                              const u8* __restrict__ prev_text, const u32 n_text, const KeyGen gen) {
     typedef OnesweepSmem<THREADS, ITEMS> Smem;
     typedef StatusTraits<StatusT> ST;
     constexpr int TILE = Smem::kTile;
@@ -364,8 +354,7 @@ __device__ __forceinline__ void onesweep_tile(OnesweepSmem<THREADS, ITEMS>& s, c
         // ILP items stay in flight per warp.
         if (k >= ILP) asm volatile("" : "+r"(d) : "r"(rank2[(k - ILP) / 2]));
         u32 peers = FULL ? 0xffffffffu : __ballot_sync(0xffffffffu, valid);
-        if (DARK_KNOCK(2u)) peers = 1u << lane;
-        else peers = match_digit_bits(peers, d);
+        peers = match_digit_bits(peers, d);
         const u32 prev = whist[d];  // every lane reads (padding lanes harmlessly), then the group's lowest lane bumps
         const u32 below = peers & lt;
         const u32 r = prev + __popc(below);
@@ -375,9 +364,7 @@ __device__ __forceinline__ void onesweep_tile(OnesweepSmem<THREADS, ITEMS>& s, c
         else rank2[k / 2] = r;
         __syncwarp();
     }
-    DARK_STAMP(2);
     __syncthreads();
-    DARK_STAMP(3);
 
     // ---- per digit: exclusive offsets across warps, tile total, publish the aggregate
     if (tid < kRadix) {
@@ -410,7 +397,6 @@ __device__ __forceinline__ void onesweep_tile(OnesweepSmem<THREADS, ITEMS>& s, c
         for (int w = 0; w < Smem::kWarps; ++w) s.warp_hist[w][tid] += dstart;
     }
     __syncthreads();
-    DARK_STAMP(4);
 
     // ---- re-order the tile by digit in shared memory (needs only tile-local offsets, so it runs
     // before the look-back and gives the predecessor tiles time to publish)
@@ -424,20 +410,18 @@ __device__ __forceinline__ void onesweep_tile(OnesweepSmem<THREADS, ITEMS>& s, c
         }
     }
 
-    DARK_STAMP(5);
     // ---- decoupled look-back over the predecessors' digit counts.  Tiles finish every ~60 cycles
     // chip-wide while a status read costs an L2 round trip (600+ cycles, more under load), so the
     // nearest inclusive prefix is 10-25 tiles back: walking them one load at a time cost 34 % of the
     // tile time (profiles/r1_pass_trace_v3.log); 8 predecessors are read per round trip.
     if (tid < kRadix) {
-        if (tile > 0 && !DARK_KNOCK(1u)) {
+        if (tile > 0) {
             lb.finish(status, tid);
             st_relaxed(status + (size_t)tile * kRadix + tid, ((StatusT)2 << ST::kShift) | (lb.excl + count));
         }
         s.global_off[tid] = digit_base[tid] + (u32)lb.excl - dstart;
     }
     __syncthreads();
-    DARK_STAMP(6);
 
     // ---- scatter: consecutive threads write consecutive addresses inside each digit run
 #pragma unroll
@@ -446,30 +430,18 @@ __device__ __forceinline__ void onesweep_tile(OnesweepSmem<THREADS, ITEMS>& s, c
         if (FULL || p < nvalid) {
             const u64 kk = s.keys[p];
             const u32 idx = s.global_off[digit(kk)] + p;
-            if (!DARK_KNOCK(4u)) {
-                keys_out[idx] = kk;
-                vals_out[idx] = s.vals[p];
-            }
+            keys_out[idx] = kk;
+            vals_out[idx] = s.vals[p];
         }
     }
-    DARK_STAMP(7);
-#ifdef DARK_BWT_TUNING
-    if (trace && threadIdx.x == 0) {
-        unsigned long long gt;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt));
-        trace[(size_t)tile * 12 + 10] = (long long)gt;
-    }
-#endif
-#undef DARK_STAMP
-#undef DARK_KNOCK
 }
 
 template <int THREADS, int ITEMS, int MINBLOCKS, int ILP, typename StatusT, bool ALIGNED, bool GEN = false>
 __global__ void __launch_bounds__(THREADS, MINBLOCKS)
 k_onesweep_pass(const u64* __restrict__ keys_in, const u32* __restrict__ vals_in, u64* __restrict__ keys_out,
                 u32* __restrict__ vals_out, u32 m, int shift, const u32* __restrict__ digit_base,
-                StatusT* __restrict__ status, u32* __restrict__ tile_counter, long long* __restrict__ trace,
-                const u8* __restrict__ prev_text, u32 n_text, u32 knock, KeyGen gen, u32 prefetch_ahead) {
+                StatusT* __restrict__ status, u32* __restrict__ tile_counter, const u8* __restrict__ prev_text, u32 n_text,
+                KeyGen gen, u32 prefetch_ahead) {
     static_assert(THREADS >= kRadix && THREADS % 32 == 0, "one thread per digit is assumed");
     typedef OnesweepSmem<THREADS, ITEMS> Smem;
     constexpr int TILE = Smem::kTile;
@@ -481,32 +453,16 @@ k_onesweep_pass(const u64* __restrict__ keys_in, const u32* __restrict__ vals_in
     // none are left.  Tiles are thereby numbered in the order they are started, so the look-back only
     // ever waits on tiles that are already running; and a CTA no longer has to drain its scattered
     // stores and be re-launched between tiles — with one tile per CTA the SMs held only 1.8 of 3
-    // resident tiles on average (tools/pass_trace.py, profiles/r1_pass_trace_v4.log).
-    // tile_counter == nullptr (test knob) falls back to one tile per CTA numbered by blockIdx.x.
+    // resident tiles on average (profiles/r1_pass_trace_v4.log).
     const u32 num_tiles = (u32)(((u64)m + TILE - 1) / TILE);
     for (;;) {
-#ifdef DARK_BWT_TUNING
-        const long long t_claim = trace ? clock64() : 0;
-#endif
-        if (tile_counter != nullptr && tid == 0) s.tile = atomicAdd(tile_counter, 1u);
+        if (tid == 0) s.tile = atomicAdd(tile_counter, 1u);
         for (int i = tid; i < Smem::kWarps * kRadix; i += THREADS) (&s.warp_hist[0][0])[i] = 0;
         __syncthreads();
-        const u32 tile = tile_counter != nullptr ? s.tile : blockIdx.x;
+        const u32 tile = s.tile;
         if (tile >= num_tiles) break;
-#ifdef DARK_BWT_TUNING
-        if (trace && tid == 0) {
-            trace[(size_t)tile * 12 + 0] = t_claim;
-            trace[(size_t)tile * 12 + 1] = clock64();
-            unsigned long long gt;
-            unsigned int smid;
-            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt));
-            asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-            trace[(size_t)tile * 12 + 8] = (long long)gt;
-            trace[(size_t)tile * 12 + 9] = (long long)smid;
-        }
-#endif
         const u32 nvalid = (u32)min((u64)TILE, (u64)m - (u64)tile * TILE);
-        if (!GEN && prefetch_ahead) {
+        if (!GEN) {
             // Pull the pairs of the tile this CTA is likely to claim next (one wave of claims ahead) into L2, a
             // 128-byte line per thread: its loads then miss only L1.  Measured: C2 sort phase 10.1 -> 9.4 ms at a
             // distance of one wave (444 tiles); no gain at two waves (profiles/r1_final.md).
@@ -518,11 +474,10 @@ k_onesweep_pass(const u64* __restrict__ keys_in, const u32* __restrict__ vals_in
         }
         if (nvalid == TILE)
             onesweep_tile<THREADS, ITEMS, ILP, StatusT, ALIGNED, true, GEN>(s, keys_in, vals_in, keys_out, vals_out, tile, nvalid,
-                                                                            shift, digit_base, status, trace, prev_text, n_text, knock, gen);
+                                                                            shift, digit_base, status, prev_text, n_text, gen);
         else
             onesweep_tile<THREADS, ITEMS, ILP, StatusT, ALIGNED, false, GEN>(s, keys_in, vals_in, keys_out, vals_out, tile, nvalid,
-                                                                             shift, digit_base, status, trace, prev_text, n_text, knock, gen);
-        if (tile_counter == nullptr) break;
+                                                                             shift, digit_base, status, prev_text, n_text, gen);
         __syncthreads();  // the scatter has read the shared tile: it may be overwritten now
     }
 }

@@ -126,9 +126,9 @@ k_init_keys(const u8* __restrict__ text, u32 n, const u8* __restrict__ lut, int 
 // packed MSB-first into 32-bit words in shared memory; a key is then a 64-bit window of that bit
 // stream (3 LDS + 2 funnel shifts instead of K byte loads — the byte loop made the first version
 // of this kernel issue-bound at K = 32, profiles/r1_ncu_c2_v1.md).
-// WRITE = false: digit histogram only (the keys are rebuilt inside the first radix pass, radix_sort.cuh GEN).
-// HIST = false: keys only (the histogram came from k_gram_hist).
-template <int THREADS, int ITEMS, int S, bool WRITE, bool HIST>
+// WRITE = true: keys only (the histograms came from k_gram_hist; the keys are needed when no radix pass builds them,
+// radix_sort.cuh GEN).  WRITE = false: the digit histograms only, counted key by key (DARK_BWT_CHECK_HIST).
+template <int THREADS, int ITEMS, int S, bool WRITE>
 __global__ void __launch_bounds__(THREADS)
 k_init_keys_packed(const u8* __restrict__ text, u32 n, const u8* __restrict__ lut, u64* __restrict__ keys_out,
                    u32* __restrict__ ids_out, u32* __restrict__ g_hist) {
@@ -175,13 +175,14 @@ k_init_keys_packed(const u8* __restrict__ text, u32 n, const u8* __restrict__ lu
                 if (WRITE) {
                     keys_out[jb + jl] = key;
                     ids_out[jb + jl] = (u32)(i_lo + x);
+                } else {
+                    hist_add_key(s_hist, key, 0, kMaxPasses);
                 }
-                if (HIST) hist_add_key(s_hist, key, 0, kMaxPasses);
             }
         }
         __syncthreads();
     }
-    if (HIST) hist_flush(s_hist, g_hist, kMaxPasses, tid, THREADS);
+    if (!WRITE) hist_flush(s_hist, g_hist, kMaxPasses, tid, THREADS);
 }
 
 // Digit histograms of the initial keys without building a key.  For s in {1,2,4,8} a radix digit is a whole
@@ -529,42 +530,23 @@ struct ScanTileState {
     u64* words;  // [tiles][4]  (gs1, hs1, cnt, pad)
 };
 constexpr int kScanWordsPerTile = 4;
-#ifndef DARK_LB_WARPS
-#define DARK_LB_WARPS 4
-#endif
-#ifndef DARK_RERANK_DEFER
-#define DARK_RERANK_DEFER 1
-#endif
-constexpr bool kRerankDeferLoads = DARK_RERANK_DEFER != 0;  // rounds >= 1: ids and old ranks are loaded after the publish
-constexpr int kLookbackWarps = DARK_LB_WARPS;  // 32 x this many predecessor tiles polled per look-back step
+constexpr int kLookbackWarps = 4;  // 32 x this many predecessor tiles polled per look-back step
 __device__ __forceinline__ u64 scan_pack(u32 flag, u32 value) { return ((u64)flag << 62) | value; }
 
 // PAIRS (large rounds >= 1): changed ranks are not scattered into isa[] here.  The tile partitions its
 // (id, new rank) updates by bucket = id >> pair_shift in shared memory and appends each bucket's run to that
 // bucket's region of pair_ids/pair_vals (region b starts at element b << pair_shift and can hold every id
 // of the bucket; pair_hist[b] is its fill cursor).  The bucketed scatter that follows reads the regions.
-#ifndef DARK_RERANK_CTAS
-#define DARK_RERANK_CTAS (1024 / THREADS)
-#endif
-// MODE 0: the single-kernel form above (decoupled look-back).
-// MODE 1 + k_rerank_scan_tiles + MODE 2 (rounds >= 1): the same result without any chain between tiles.  MODE 1 reads the
-// keys once, writes the two head-flag bitmaps (one byte per thread and bitmap) and the tile's aggregate; the scan kernel
-// turns the aggregates into exclusive prefixes; MODE 2 reads the flags, ids and old ranks and applies.  Same bytes as
-// MODE 0 plus 1/4 byte per suffix.  Measured equal to MODE 0 (C3 45.1 vs 44.6 ms, C5 33.0 vs 32.9, C4 345.5 vs 345.2:
-// what bounds the re-rank of a large round is the apply phase - shared-memory partition and scattered stores - not the
-// chain, profiles/r2_rejected.md), so MODE 0 stays the default; DARK_BWT_RERANK_CHAINFREE=1 selects this form.
-template <int THREADS, int ITEMS, bool ROUND0, bool PAIRS, int MODE = 0>
-__global__ void __launch_bounds__(THREADS, DARK_RERANK_CTAS)
+// A chain-free form of rounds >= 1 (flags and tile aggregates, a scan over the aggregates, then an apply kernel) was
+// measured equal to this one (C3 45.1 vs 44.6 ms, C5 33.0 vs 32.9, C4 345.5 vs 345.2: what bounds the re-rank of a large
+// round is the apply phase - shared-memory partition and scattered stores - not the chain, profiles/r2_rejected.md).
+template <int THREADS, int ITEMS, bool ROUND0, bool PAIRS>
+__global__ void __launch_bounds__(THREADS, 1024 / THREADS)
 k_rerank(const u64* __restrict__ keys, const u32* __restrict__ ids, const u32* __restrict__ ranks_in, u32 m, u32 n, int K, int kb,
          u32* __restrict__ isa, u32* __restrict__ sa, u32* __restrict__ out_ids, u32* __restrict__ out_ranks, ScanTileState ts,
          u32* __restrict__ tile_counter, u32* __restrict__ out_count, u32* __restrict__ pair_ids,
          u32* __restrict__ pair_vals, u32* __restrict__ pair_hist, int pair_shift, const u8* __restrict__ text,
-         u8* __restrict__ bwt_inline, u64* __restrict__ origin, u32 prefetch_ahead, u32 tag, long long* __restrict__ trace,
-         u8* __restrict__ flags_new, u8* __restrict__ flags_old) {
-    static_assert(MODE == 0 || !ROUND0, "the chain-free form serves the rounds after the initial sort");
-    // trace != nullptr (tools/rerank_trace.py only): thread 0 stamps clock64() at the phase boundaries of its tile
-#define DARK_RSTAMP(i) do { if (trace && threadIdx.x == 0) trace[(size_t)s_tile * 8 + (i)] = clock64(); } while (0)
-    const long long t_entry = trace ? clock64() : 0;
+         u8* __restrict__ bwt_inline, u64* __restrict__ origin, u32 prefetch_ahead, u32 tag) {
     constexpr int TILE = THREADS * ITEMS;
     constexpr int WARPS = THREADS / 32;
     static_assert(TILE / 8 <= THREADS, "one prefetch per thread covers the tile");
@@ -573,7 +555,7 @@ k_rerank(const u64* __restrict__ keys, const u32* __restrict__ ids, const u32* _
     __shared__ ScanTriple s_excl;
     __shared__ u32 s_tile;
     __shared__ u64 s_lb[2][kLookbackWarps][3];
-    extern __shared__ __align__(16) u32 smem_rerank[];  // kRerankSmem<TILE> bytes (dynamic: 1,024-thread tuning builds exceed 48 KB)
+    extern __shared__ __align__(16) u32 smem_rerank[];  // kRerankSmem<TILE> bytes
     u32* s_oid = smem_rerank;         // this tile's survivors, staged for coalesced stores
     u32* s_ork = smem_rerank + stage_pad32(TILE);
     __shared__ u32 s_tile_cnt;
@@ -581,15 +563,13 @@ k_rerank(const u64* __restrict__ keys, const u32* __restrict__ ids, const u32* _
     __shared__ u32 s_bwarp[8], s_btotal;
     static_assert(WARPS >= kLookbackWarps, "look-back warps");
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    if (tid == 0) s_tile = MODE == 0 ? atomicAdd(tile_counter, 1u) : blockIdx.x;  // no chain, no need for claim order
+    if (tid == 0) s_tile = atomicAdd(tile_counter, 1u);
     if (PAIRS)
         for (int i = tid; i < 256; i += THREADS) s_bhist[i] = 0;
     __syncthreads();
     const u32 tile = s_tile;
-    if (trace && tid == 0) trace[(size_t)tile * 8 + 0] = t_entry;
-    DARK_RSTAMP(1);
     const u64 p0 = (u64)tile * TILE + (u64)tid * ITEMS;  // blocked arrangement
-    if (MODE == 0 && prefetch_ahead) {
+    {
         // pull the input of the tile that will be claimed ~one wave from now into L2: a tile's lifetime is
         // load latency + look-back, and only two CTAs fit on an SM
         const u64 q0 = ((u64)tile + prefetch_ahead) * TILE;
@@ -605,10 +585,7 @@ k_rerank(const u64* __restrict__ keys, const u32* __restrict__ ids, const u32* _
     // keys[p0-1 .. p0+ITEMS], ids[p0 .. p0+ITEMS) (+ neighbours in round 0)
     u64 key[ITEMS + 2];
     u32 id[ITEMS + 2];
-    if (MODE == 2) {
-#pragma unroll
-        for (int k = 0; k < ITEMS + 2; ++k) key[k] = 0;  // the flags come from the bitmaps
-    } else if (p0 + ITEMS <= m) {
+    if (p0 + ITEMS <= m) {
         const ulonglong2* kv = reinterpret_cast<const ulonglong2*>(keys + p0);
 #pragma unroll
         for (int k = 0; k < ITEMS / 2; ++k) {
@@ -616,7 +593,7 @@ k_rerank(const u64* __restrict__ keys, const u32* __restrict__ ids, const u32* _
             key[1 + 2 * k] = q.x;
             key[2 + 2 * k] = q.y;
         }
-        if (ROUND0 || (!kRerankDeferLoads && MODE == 0)) {
+        if (ROUND0) {
             const uint4* iv = reinterpret_cast<const uint4*>(ids + p0);
 #pragma unroll
             for (int k = 0; k < ITEMS / 4; ++k) {
@@ -631,13 +608,11 @@ k_rerank(const u64* __restrict__ keys, const u32* __restrict__ ids, const u32* _
 #pragma unroll
         for (int k = 0; k < ITEMS; ++k) {
             key[1 + k] = (p0 + k < m) ? keys[p0 + k] : 0;
-            if (ROUND0 || (!kRerankDeferLoads && MODE == 0)) id[1 + k] = (p0 + k < m) ? ids[p0 + k] : 0;
+            if (ROUND0) id[1 + k] = (p0 + k < m) ? ids[p0 + k] : 0;
         }
     }
-    if (MODE != 2) {
-        key[0] = (p0 > 0 && p0 - 1 < m) ? keys[p0 - 1] : 0;
-        key[ITEMS + 1] = (p0 + ITEMS < m) ? keys[p0 + ITEMS] : 0;
-    }
+    key[0] = (p0 > 0 && p0 - 1 < m) ? keys[p0 - 1] : 0;
+    key[ITEMS + 1] = (p0 + ITEMS < m) ? keys[p0 + ITEMS] : 0;
     if (ROUND0) {
         id[0] = (p0 > 0 && p0 - 1 < m) ? ids[p0 - 1] : 0;
         id[ITEMS + 1] = (p0 + ITEMS < m) ? ids[p0 + ITEMS] : 0;
@@ -649,55 +624,6 @@ k_rerank(const u64* __restrict__ keys, const u32* __restrict__ ids, const u32* _
     // rank comes from the list itself: sorting permutes elements only inside their group, and every
     // member of a group holds the same rank, so ranks_in[p] is the rank of whatever lands at index p.
     u32 rold[ITEMS];
-    // Rounds >= 1: the head flags need the keys only.  The ids and the old ranks are fetched AFTER the tile's
-    // aggregate is on its way (below), so that fewer bytes stand between a tile's start and its publish — every later
-    // tile's look-back waits for the slowest recent tile to publish (profiles/r1_ncu_rerank_final.md) — and their
-    // latency hides behind the look-back.
-    auto load_ids_and_ranks = [&]() {
-        if (p0 + ITEMS <= m) {
-            const uint4* iv = reinterpret_cast<const uint4*>(ids + p0);
-#pragma unroll
-            for (int k = 0; k < ITEMS / 4; ++k) {
-                const uint4 q = iv[k];
-                id[1 + 4 * k] = q.x;
-                id[2 + 4 * k] = q.y;
-                id[3 + 4 * k] = q.z;
-                id[4 + 4 * k] = q.w;
-            }
-            const uint4* rv = reinterpret_cast<const uint4*>(ranks_in + p0);
-#pragma unroll
-            for (int k = 0; k < ITEMS / 4; ++k) {
-                const uint4 q = rv[k];
-                rold[4 * k] = q.x;
-                rold[4 * k + 1] = q.y;
-                rold[4 * k + 2] = q.z;
-                rold[4 * k + 3] = q.w;
-            }
-        } else {
-#pragma unroll
-            for (int k = 0; k < ITEMS; ++k) {
-                id[1 + k] = (p0 + k < m) ? ids[p0 + k] : 0u;
-                rold[k] = (p0 + k < m) ? ranks_in[p0 + k] : 0u;
-            }
-        }
-    };
-    if (!ROUND0 && !kRerankDeferLoads && MODE == 0) {
-        if (p0 + ITEMS <= m) {
-            const uint4* rv = reinterpret_cast<const uint4*>(ranks_in + p0);
-#pragma unroll
-            for (int k = 0; k < ITEMS / 4; ++k) {
-                const uint4 q = rv[k];
-                rold[4 * k] = q.x;
-                rold[4 * k + 1] = q.y;
-                rold[4 * k + 2] = q.z;
-                rold[4 * k + 3] = q.w;
-            }
-        } else {
-#pragma unroll
-            for (int k = 0; k < ITEMS; ++k) rold[k] = (p0 + k < m) ? ranks_in[p0 + k] : 0u;
-        }
-    }
-
     // head flags for p0 .. p0+ITEMS (the last one is the look-ahead of item ITEMS-1)
     const u32 short_from = n >= (u32)K ? n - (u32)K + 1u : 0u;  // suffix i is "short" (key padded) iff i >= short_from
     const u32 navail = p0 >= m ? 0u : (u32)min((u64)ITEMS + 1, (u64)m - p0);  // of p0 .. p0+ITEMS, how many are inside the list
@@ -731,18 +657,6 @@ k_rerank(const u64* __restrict__ keys, const u32* __restrict__ ids, const u32* _
         oldh |= tail;
     }
 
-    if (MODE == 2) {  // flags of p0 .. p0+ITEMS-1 from this thread's byte, the look-ahead flag from the next byte
-        static_assert(MODE != 2 || ITEMS == 8, "one flag byte per thread");
-        const u64 b = p0 >> 3;
-        const bool ahead_in_list = p0 + ITEMS < m;
-        newh = (u32)flags_new[b] | ((ahead_in_list ? ((u32)flags_new[b + 1] & 1u) : 1u) << ITEMS);
-        oldh = (u32)flags_old[b] | ((ahead_in_list ? ((u32)flags_old[b + 1] & 1u) : 1u) << ITEMS);
-    }
-    if (MODE == 1) {
-        flags_new[p0 >> 3] = (u8)(newh & 0xFFu);
-        flags_old[p0 >> 3] = (u8)(oldh & 0xFFu);
-    }
-    DARK_RSTAMP(2);
     // thread aggregate, from the flag words: latest old/new head among the valid elements, survivors
     ScanTriple agg = {0u, 0u, 0u};
     {
@@ -762,18 +676,38 @@ k_rerank(const u64* __restrict__ keys, const u32* __restrict__ ids, const u32* _
     }
     if (lane == 31) s_warp[warp] = incl;
     __syncthreads();
-    if (MODE == 1) {  // the tile's aggregate, and done
-        if (tid == 0) {
-            ScanTriple tile_agg = {0u, 0u, 0u};
-            for (int w = 0; w < WARPS; ++w) tile_agg = scan_combine(tile_agg, s_warp[w]);
-            u64* mine = ts.words + (size_t)tile * kScanWordsPerTile;
-            mine[0] = tile_agg.gs1;
-            mine[1] = tile_agg.hs1;
-            mine[2] = tile_agg.cnt;
+    if (!ROUND0) {
+        // Rounds >= 1: the head flags need the keys only.  The ids and the old ranks are fetched AFTER the tile's
+        // aggregate is on its way (below), so that fewer bytes stand between a tile's start and its publish — every later
+        // tile's look-back waits for the slowest recent tile to publish (profiles/r1_ncu_rerank_final.md) — and their
+        // latency hides behind the look-back.
+        if (p0 + ITEMS <= m) {
+            const uint4* iv = reinterpret_cast<const uint4*>(ids + p0);
+#pragma unroll
+            for (int k = 0; k < ITEMS / 4; ++k) {
+                const uint4 q = iv[k];
+                id[1 + 4 * k] = q.x;
+                id[2 + 4 * k] = q.y;
+                id[3 + 4 * k] = q.z;
+                id[4 + 4 * k] = q.w;
+            }
+            const uint4* rv = reinterpret_cast<const uint4*>(ranks_in + p0);
+#pragma unroll
+            for (int k = 0; k < ITEMS / 4; ++k) {
+                const uint4 q = rv[k];
+                rold[4 * k] = q.x;
+                rold[4 * k + 1] = q.y;
+                rold[4 * k + 2] = q.z;
+                rold[4 * k + 3] = q.w;
+            }
+        } else {
+#pragma unroll
+            for (int k = 0; k < ITEMS; ++k) {
+                id[1 + k] = (p0 + k < m) ? ids[p0 + k] : 0u;
+                rold[k] = (p0 + k < m) ? ranks_in[p0 + k] : 0u;
+            }
         }
-        return;
     }
-    if (!ROUND0 && (kRerankDeferLoads || MODE == 2)) load_ids_and_ranks();
     ScanTriple wprefix = {0u, 0u, 0u};
     for (int w = 0; w < warp; ++w) wprefix = scan_combine(wprefix, s_warp[w]);
     ScanTriple texcl = shfl_up_triple(incl, 1);
@@ -785,14 +719,7 @@ k_rerank(const u64* __restrict__ keys, const u32* __restrict__ ids, const u32* _
     // L2 round trip: the "inclusive prefix known" frontier advances one window per polling step.  A
     // 32-tile window of 2,048-element tiles ran at 1.5-1.9 TB/s (profiles/r1_ncu_c5_c3_v2.md), hence
     // kLookbackWarps warps poll kLookbackWarps*32 predecessors per step and the tiles are 4,096 wide.
-    DARK_RSTAMP(3);
-    if (MODE == 2) {
-        if (tid == 0) {  // exclusive prefix and survivor count of this tile, from k_rerank_scan_tiles
-            const u64* mine = ts.words + (size_t)tile * kScanWordsPerTile;
-            s_excl = ScanTriple{(u32)mine[0], (u32)mine[1], (u32)mine[2]};
-            s_tile_cnt = (u32)mine[3];
-        }
-    } else if (warp < kLookbackWarps) {
+    if (warp < kLookbackWarps) {
         ScanTriple tile_agg = {0u, 0u, 0u};
         for (int w = 0; w < WARPS; ++w) tile_agg = scan_combine(tile_agg, s_warp[w]);
         ScanTriple excl = {0u, 0u, 0u};
@@ -871,10 +798,8 @@ k_rerank(const u64* __restrict__ keys, const u32* __restrict__ ids, const u32* _
                 tile_counter[1] = excl.cnt + tile_agg.cnt;
             }
         }
-        DARK_RSTAMP(4);
     }
     __syncthreads();
-    DARK_RSTAMP(5);
     ScanTriple run = scan_combine(s_excl, texcl);
 
     // apply.  Stores are shaped for L2: a thread's 8 consecutive words leave as two 128-bit stores,
@@ -882,8 +807,8 @@ k_rerank(const u64* __restrict__ keys, const u32* __restrict__ ids, const u32* _
     // (per-lane 4-byte stores at a 32 B stride cost one L2 sector operation each; the first version
     // spent its time there: 3 sector writes per element, profiles/r1_ncu_c5_c3_v2.md).
     const u32 tile_cnt0 = s_excl.cnt;  // survivors before this tile
-    // bwt_inline != nullptr: BWT bytes are emitted as suffixes settle.  In round 0 the byte T[id-1] sits
-    // in the low key byte (pruned initial sort, see the radix pass); later rounds gather it.
+    // bwt_inline != nullptr: BWT bytes are emitted as suffixes settle.  Round 0 emits only after a pruned initial sort
+    // (kb >= 8), where the byte T[id-1] sits in the low key byte (see the radix pass); later rounds gather it.
     u32 v_sa[ITEMS], v_pid[ITEMS], v_pval[ITEMS];
     u32 v_b0 = 0, v_b1 = 0;  // round 0: the 8 BWT bytes of this thread's slots
 #pragma unroll
@@ -920,8 +845,7 @@ k_rerank(const u64* __restrict__ keys, const u32* __restrict__ ids, const u32* _
             if (ROUND0 && single) v_sa[k] = sid;
             if (bwt_inline != nullptr && single) {
                 if (ROUND0) {
-                    // pruned initial sort (kb >= 8): the byte rides in the low key byte; otherwise it is gathered here
-                    const u32 byte = kb >= 8 ? ((u32)key[k + 1] & 0xFFu) : (u32)__ldg(text + (sid == 0 ? n - 1 : sid - 1));
+                    const u32 byte = (u32)key[k + 1] & 0xFFu;
                     if (k < 4) v_b0 |= byte << (8 * k);
                     else v_b1 |= byte << (8 * (k - 4));
                     if (sid == 0) *origin = p;
@@ -962,7 +886,6 @@ k_rerank(const u64* __restrict__ keys, const u32* __restrict__ ids, const u32* _
                 if (p0 + k < m) bwt_inline[p0 + k] = (u8)((k < 4 ? v_b0 >> (8 * k) : v_b1 >> (8 * (k - 4))) & 0xFFu);
         }
     }
-    DARK_RSTAMP(6);
     __syncthreads();
     {
         const u32 tile_cnt = s_tile_cnt;
@@ -971,8 +894,6 @@ k_rerank(const u64* __restrict__ keys, const u32* __restrict__ ids, const u32* _
             out_ranks[tile_cnt0 + i] = s_ork[stage_pad32(i)];
         }
     }
-    DARK_RSTAMP(7);
-#undef DARK_RSTAMP
     if (PAIRS) {
         static_assert(!PAIRS || THREADS >= 256, "one thread per bucket");
         // bucket starts inside the tile; one global atomicAdd per (tile, bucket) reserves the run
@@ -1011,48 +932,6 @@ k_rerank(const u64* __restrict__ keys, const u32* __restrict__ ids, const u32* _
             pair_vals[o] = s_ork[i];
         }
     }
-}
-
-// Exclusive scan of the tile aggregates of k_rerank<MODE 1>: words[t] = (latest old head + 1, latest new head + 1,
-// survivors) of tile t  ->  the same over tiles 0 .. t-1, and word 3 = the tile's own survivor count.  One CTA.
-__global__ void __launch_bounds__(1024) k_rerank_scan_tiles(u64* __restrict__ words, u32 tiles, u32* __restrict__ out_count) {
-    __shared__ ScanTriple s_warp[32];
-    __shared__ ScanTriple s_carry;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    if (tid == 0) s_carry = ScanTriple{0u, 0u, 0u};
-    __syncthreads();
-    for (u32 t0 = 0; t0 < tiles; t0 += 1024) {
-        const u32 t = t0 + tid;
-        ScanTriple v = {0u, 0u, 0u};
-        if (t < tiles) {
-            const u64* w = words + (size_t)t * kScanWordsPerTile;
-            v = ScanTriple{(u32)w[0], (u32)w[1], (u32)w[2]};
-        }
-        ScanTriple incl = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const ScanTriple u = shfl_up_triple(incl, o);
-            if (lane >= o) incl = scan_combine(u, incl);
-        }
-        if (lane == 31) s_warp[warp] = incl;
-        __syncthreads();
-        ScanTriple base = s_carry;
-        for (int w = 0; w < warp; ++w) base = scan_combine(base, s_warp[w]);
-        ScanTriple excl = shfl_up_triple(incl, 1);
-        if (lane == 0) excl = ScanTriple{0u, 0u, 0u};
-        excl = scan_combine(base, excl);
-        if (t < tiles) {
-            u64* w = words + (size_t)t * kScanWordsPerTile;
-            w[0] = excl.gs1;
-            w[1] = excl.hs1;
-            w[2] = excl.cnt;
-            w[3] = v.cnt;
-        }
-        __syncthreads();
-        if (tid == 1023) s_carry = scan_combine(base, incl);
-        __syncthreads();
-    }
-    if (tid == 0) *out_count = s_carry.cnt;
 }
 
 // ---- sparse round-0 re-rank (pruned initial sort: almost every suffix settles) -------------------------------
@@ -2186,19 +2065,6 @@ k_ibwt_many_check(const u32* __restrict__ dist, u32 regular, const u32* __restri
         *bad_out = s_bad;
         *first_bad_out = s_first;
     }
-}
-
-// Debug statistic (DARK_BWT_GROUP_STATS=1): largest group of the active list (capped at 4096) and the
-// number of groups, from the rank list (equal rank = same group, groups are contiguous).
-__global__ void __launch_bounds__(256) k_group_stats(const u32* __restrict__ ranks, u32 m, u32* __restrict__ out /* [0]=max size, [1]=groups */) {
-    const u64 p = (u64)blockIdx.x * 256 + threadIdx.x;
-    if (p >= m) return;
-    const u32 r = ranks[p];
-    if (p > 0 && ranks[p - 1] == r) return;  // not a head
-    u32 len = 1;
-    while (p + len < m && len < 4096 && ranks[p + len] == r) ++len;
-    atomicMax(out, len);
-    atomicAdd(out + 1, 1u);
 }
 
 // ---- verification (independent of the construction kernels) ------------------------------------

@@ -163,13 +163,6 @@ FORCED_PATHS = [
     ({"DARK_BWT_BUCKETED": "1"}, "dna", 5, 2000003),
     ({"DARK_BWT_EMIT_WINDOW_MB": "1"}, "mixed", 7, 5000011),         # windowed BWT emission (text larger than L2)
     ({"DARK_BWT_EMIT_WINDOW_MB": "1", "DARK_BWT_BUCKETED": "1"}, "text", 3, 2500000),
-    ({"DARK_BWT_SORT_VARIANT": "0"}, "mixed", 4, 700001),            # the other radix-pass tilings
-    ({"DARK_BWT_SORT_VARIANT": "2"}, "mixed", 4, 700001),
-    ({"DARK_BWT_SORT_VARIANT": "5"}, "dna", 1, 700001),
-    ({"DARK_BWT_RERANK_CHAINFREE": "1"}, "mixed", 4, 1300001),        # rounds >= 1 re-ranked by flags + scan + apply (no look-back chain)
-    ({"DARK_BWT_RERANK_CHAINFREE": "1"}, "rep17", 2, 800001),
-    ({"DARK_BWT_RERANK_CHAINFREE": "1", "DARK_BWT_BUCKETED": "1"}, "mixed", 6, 2100001),
-    ({"DARK_BWT_RERANK_CHAINFREE": "1", "DARK_BWT_TEXT_BUILD": "1000000"}, "text", 6, 800001),
     ({"DARK_BWT_FUSE_ROUND0": "0", "DARK_BWT_BUCKETED": "1"}, "mixed", 4, 3300001),   # round 0 followed by separate partition passes
     ({"DARK_BWT_FUSE_ROUND0": "0", "DARK_BWT_BUCKETED": "1"}, "text", 3, 2500000),
     ({"DARK_BWT_PASS_IMPL": "0"}, "mixed", 9, 900001),               # the round-1 pass kernel (fallback of unaligned inputs / digits)
@@ -186,15 +179,11 @@ FORCED_PATHS = [
     ({"DARK_BWT_TEXT_BUILD": "1000000", "DARK_BWT_BUCKETED": "1"}, "mixed", 6, 2100001),
     ({"DARK_BWT_TEXT_BUILD": "1000000", "DARK_BWT_BUCKETED": "1"}, "rep17", 4, 1000001),
     ({"DARK_BWT_TEXT_BUILD": "1000000", "DARK_BWT_RANK_SEARCH": "0"}, "dna", 6, 1500003),
-    ({"DARK_BWT_FUSED_INIT": "0"}, "mixed", 4, 900001),              # initial keys materialised instead of built inside pass 1
-    ({"DARK_BWT_FUSED_INIT": "0"}, "dna", 2, 1100003),
-    ({"DARK_BWT_FORCE_U64_STATUS": "1"}, "dna", 8, 600011),          # key-generating pass with 64-bit tile status                  # late rounds WITHOUT the pairs kernel
+    ({"DARK_BWT_CHECK_HIST": "1"}, "mixed", 4, 900001),              # q-gram histogram compared with the per-key count
+    ({"DARK_BWT_CHECK_HIST": "1"}, "dna", 2, 1100003),
+    ({"DARK_BWT_FORCE_U64_STATUS": "1"}, "dna", 8, 600011),          # key-generating pass with 64-bit tile status
     ({"DARK_BWT_INLINE_EMIT": "0"}, "dna", 3, 1200007),              # pruned initial sort WITHOUT inline emission
-    ({"DARK_BWT_INLINE_GATHER": "1"}, "mixed", 7, 1300003),           # unpruned block emitting inline: T[id-1] gathered as suffixes settle
-    ({"DARK_BWT_INLINE_GATHER": "1"}, "rep17", 8, 700001),
-    ({"DARK_BWT_INLINE_GATHER": "1", "DARK_BWT_TEXT_BUILD": "1000000", "DARK_BWT_BUCKETED": "1"}, "text", 9, 2200003),  # ... with the fused round-0 bucket sink
-    ({"DARK_BWT_INLINE_GATHER": "1", "DARK_BWT_PAIRS": "0"}, "text", 10, 500009),
-    ({"DARK_BWT_INLINE_EMIT": "0", "DARK_BWT_EMIT_WINDOW_MB": "1"}, "dna", 4, 3000001),        # tiles ordered by blockIdx instead of the claim counter
+    ({"DARK_BWT_INLINE_EMIT": "0", "DARK_BWT_EMIT_WINDOW_MB": "1"}, "dna", 4, 3000001),        # ... emitted by the windowed gather
 ]
 
 

@@ -1,5 +1,5 @@
 #!/usr/bin/env python3
-"""One device-resident forward BWT of a named workload (for ncu / quick timing).
+"""One device-resident forward BWT of a named workload (quick timing).
     python tools/profile_step.py <c1|c2|c3|c4|c5> [reps] [n_override]"""
 import json
 import os
@@ -30,7 +30,7 @@ for _ in range(reps):
 # the timing is only worth reading if the bytes are right: CRC-32 of the BWT against the committed oracle fixture
 gold = json.load(open(os.path.join(ROOT, "tests", "golden", "oracle_golden.json")))
 key = "%s:%d:%d" % (kind, seed, n)
-if key in gold and not os.environ.get("DARK_BWT_PASS_KNOCKOUT"):
+if key in gold:
     crc = "%08x" % (zlib.crc32(db.cpu().numpy().tobytes()) & 0xFFFFFFFF)
     ok = crc == gold[key]["bwt_crc32"] and origin == gold[key]["origin"]
     print(json.dumps({"workload": name, "parity": "ok" if ok else "MISMATCH", "bwt_crc32": crc}))
