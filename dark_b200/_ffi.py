@@ -18,7 +18,8 @@ SYMBOLS = [
     "dark_bwt_forward_batch", "dark_bwt_forward_many", "dark_bwt_forward_many_device", "dark_bwt_forward_device", "dark_bwt_inverse", "dark_bwt_inverse_device",
     "dark_bwt_inverse_batch", "dark_bwt_inverse_many", "dark_bwt_inverse_many_device", "dark_bwt_reuse", "dark_bwt_destroy", "dark_bwt_strerror", "dark_bwt_last_error",
     "dark_bwt_stream", "dark_bwt_sort_pairs_device", "dark_bwt_verify_sa_device", "dark_bwt_emit_device", "dark_bwt_lcp_profile_device",
-    "dark_bwt_synth", "dark_bwt_dc_encode_device", "dark_bwt_dc_encode", "dark_bwt_forward_dc",
+    "dark_bwt_synth", "dark_bwt_dc_encode_device", "dark_bwt_dc_encode", "dark_bwt_forward_dc", "dark_bwt_dc_encode_many",
+    "dark_bwt_dc_encode_many_device", "dark_bwt_forward_dc_many",
 ]
 
 
@@ -115,6 +116,9 @@ def lib():
     L.dark_bwt_dc_encode_device.argtypes = [vp, vp, u64, vp, vp, vp, vp, vp, ctypes.POINTER(DcInfo)]
     L.dark_bwt_dc_encode.argtypes = [vp, vp, u64, vp, vp, vp, vp, vp, ctypes.POINTER(DcInfo)]
     L.dark_bwt_forward_dc.argtypes = [vp, vp, u64, vp, ctypes.POINTER(u64), vp, vp, vp, vp, vp, ctypes.POINTER(DcInfo), ctypes.POINTER(Stats)]
+    L.dark_bwt_dc_encode_many.argtypes = [vp, vp, vp, u64, vp, vp, vp, vp, vp, vp, vp, ctypes.POINTER(ctypes.c_float)]
+    L.dark_bwt_dc_encode_many_device.argtypes = [vp, vp, vp, u64, vp, vp, vp, vp, vp, vp, vp, ctypes.POINTER(ctypes.c_float)]
+    L.dark_bwt_forward_dc_many.argtypes = [vp, vp, vp, u64, vp, vp, vp, vp, vp, vp, vp, vp, vp, ctypes.POINTER(Stats)]
     _lib = L
     return L
 

@@ -1322,7 +1322,8 @@ int dc_device(dark_bwt_ctx* ctx, const u8* d_bwt, u64 n64, DcBuffers* io, dark_b
     CK(cudaEventRecord(ea, ctx->stream));
     CK(cudaMemsetAsync(first, 0xFF, sizeof(u32) * 256, ctx->stream));
     CK(cudaMemsetAsync(total_runs, 0, sizeof(unsigned long long), ctx->stream));
-    k_dc_tables<<<nblocks, 256, 0, ctx->stream>>>(d_bwt, n, tab, first, run_counts, io->dist, total_runs);
+    const DcMany none{};
+    k_dc_tables<false><<<nblocks, 256, 0, ctx->stream>>>(d_bwt, n, tab, first, run_counts, io->dist, total_runs, none);
     LAUNCHED();
     const u32 ngroups = (u32)ceil_div(nblocks, kDcGroup);
     u32* group_last = tab + (size_t)nblocks * 256;  // ngroups x 256 words behind the table (n/4 + n/1024 bytes of the 4n)
@@ -1335,17 +1336,104 @@ int dc_device(dark_bwt_ctx* ctx, const u8* d_bwt, u64 n64, DcBuffers* io, dark_b
     u32* alpha = ctx->bucket_hist + 512;  // 513 words: dense codes of the symbols that occur
     k_dc_alphabet<<<1, 256, 0, ctx->stream>>>(first, alpha);
     LAUNCHED();
-    k_dc_ranks<<<(u32)ceil_div(nblocks, 8), 256, 0, ctx->stream>>>(d_bwt, n, tab, group_last, run_counts, nblocks, alpha, io->dist, run_start, io->item_sym, io->item_rank);
+    k_dc_ranks<false><<<(u32)ceil_div(nblocks, 8), 256, 0, ctx->stream>>>(d_bwt, n, tab, group_last, run_counts, nblocks, alpha, io->dist, run_start,
+                                                                         io->item_sym, io->item_rank, none);
     LAUNCHED();
     k_dc_final<<<1, 256, 0, ctx->stream>>>(n, final_last, first, io->dist, total_runs, ctx->dc_info);
     LAUNCHED();
-    k_dc_stream<<<(u32)std::min<u64>(ceil_div(n, 256), (u64)ctx->num_sms * 16), 256, 0, ctx->stream>>>(run_start, total_runs, n, io->dist, io->item_pos, io->item_dist);
+    k_dc_stream<false><<<(u32)std::min<u64>(ceil_div(n, 256), (u64)ctx->num_sms * 16), 256, 0, ctx->stream>>>(run_start, total_runs, n, io->dist,
+                                                                                                              io->item_pos, io->item_dist, none);
     LAUNCHED();
     CK(cudaEventRecord(eb, ctx->stream));
     static_assert(offsetof(dark_bwt_dc_info, num_items) == offsetof(DcInfoDev, num_items), "DcInfoDev mirrors the head of dark_bwt_dc_info");
     CK(cudaMemcpyAsync(info, ctx->dc_info, sizeof(DcInfoDev), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     cudaEventElapsedTime(&info->device_ms, ea, eb);
+    return DARK_BWT_OK;
+}
+
+// The per-block records of dc_many_device are staged in the sort's second key buffer (8 N + 1 KiB bytes), which distance
+// coding leaves free: count * sizeof(DcRecDev) <= 8 * capacity + 1024.
+bool dc_many_records_fit(const dark_bwt_ctx* ctx, u64 count) {
+    return count * sizeof(DcRecDev) <= ctx->capacity * 8 + 1024;
+}
+
+// Distance coding of `count` BWT blocks back to back in d_bwt (n bytes in all), in one pass.  ctx->many_starts holds the
+// offsets [0..count] and the caller has checked them (each block >= 1 byte, n <= capacity, the records fit).  Outputs in
+// `io` are nullable like dc_device's; item_starts (count + 1 words) likewise.  infos[0..count) and *item_starts_host
+// (count + 1 words) are filled on the host.
+struct DcManyBuffers {
+    DcBuffers dc;
+    u32* item_starts = nullptr;
+};
+int dc_many_device(dark_bwt_ctx* ctx, const u8* d_bwt, u32 n, u32 count, DcManyBuffers* io, dark_bwt_dc_info* infos,
+                   std::vector<u32>* item_starts_host) {
+    const u32 nblocks = (u32)ceil_div(n, kDcBlock);
+    u32* tab = ctx->ranks;
+    if (n <= 65536u) {  // as in dc_device: tiny totals borrow the status buffer
+        tab = (u32*)ctx->sort_status;
+        for (int h = 0; h < 2; ++h) ctx->status_dirty_lo[h] = 0u, ctx->status_dirty_hi[h] = (u32)(ctx->sort_status_bytes / 2 / (kRadix * sizeof(u32)));
+    }
+    u32* run_counts = ctx->ranks_alt;
+    u32* first = ctx->bucket_hist;
+    u32* final_last = ctx->bucket_hist + 256;
+    DcBuffers& b = io->dc;
+    if (!b.dist) b.dist = (u32*)ctx->keys[0];
+    if (!b.item_pos) b.item_pos = ctx->isa;
+    if (!b.item_dist) b.item_dist = ctx->sa;
+    u32* run_start = ctx->ids[0];
+    if (!b.item_sym) b.item_sym = (u8*)ctx->ids[1];
+    if (!b.item_rank) b.item_rank = (u8*)ctx->ids[1] + (size_t)n;
+    // behind the run counts (4 N + 16 bytes): align4(nblocks) + count + 1 words fit, as the records bound count to capacity / 160
+    if (!io->item_starts) io->item_starts = ctx->ranks_alt + align_up(nblocks, 4);
+    DcRecDev* recs = (DcRecDev*)ctx->keys[1];
+    unsigned long long* total_runs = (unsigned long long*)((char*)ctx->dc_info + align_up(sizeof(DcInfoDev), 8));
+    DcMany many{ctx->many_starts, count, ctx->bitmap, recs, io->item_starts};
+    cudaEvent_t ea = ctx->events[kMaxEvents - 1], eb = ctx->events[kMaxEvents - 2];
+    CK(cudaEventRecord(ea, ctx->stream));
+    CK(cudaMemsetAsync(first, 0xFF, sizeof(u32) * 256, ctx->stream));
+    CK(cudaMemsetAsync(total_runs, 0, sizeof(unsigned long long), ctx->stream));
+    CK(cudaMemsetAsync(ctx->bitmap, 0, sizeof(u32) * ceil_div(n, 32), ctx->stream));
+    k_dc_mark_starts<<<(u32)ceil_div(count, 256), 256, 0, ctx->stream>>>(ctx->many_starts, count, ctx->bitmap, io->item_starts);
+    LAUNCHED();
+    k_dc_tables<true><<<nblocks, 256, 0, ctx->stream>>>(d_bwt, n, tab, first, run_counts, b.dist, total_runs, many);
+    LAUNCHED();
+    const u32 ngroups = (u32)ceil_div(nblocks, kDcGroup);
+    u32* group_last = tab + (size_t)nblocks * 256;
+    k_dc_scan_groups<<<ngroups, 256, 0, ctx->stream>>>(tab, nblocks, group_last);
+    LAUNCHED();
+    k_dc_scan_carry<<<1, 256, 0, ctx->stream>>>(group_last, ngroups, final_last);
+    LAUNCHED();
+    k_sparse_scan<<<1, 1024, 0, ctx->stream>>>(run_counts, nblocks);
+    LAUNCHED();
+    u32* alpha = ctx->bucket_hist + 512;  // dense codes over the union of the blocks' alphabets
+    k_dc_alphabet<<<1, 256, 0, ctx->stream>>>(first, alpha);
+    LAUNCHED();
+    k_dc_ranks<true><<<(u32)ceil_div(nblocks, 8), 256, 0, ctx->stream>>>(d_bwt, n, tab, group_last, run_counts, nblocks, alpha, b.dist, run_start,
+                                                                        b.item_sym, b.item_rank, many);
+    LAUNCHED();
+    k_dc_stream<true><<<(u32)std::min<u64>(ceil_div(n, 256), (u64)ctx->num_sms * 16), 256, 0, ctx->stream>>>(run_start, total_runs, n, b.dist,
+                                                                                                             b.item_pos, b.item_dist, many);
+    LAUNCHED();
+    CK(cudaEventRecord(eb, ctx->stream));
+    std::vector<DcRecDev> recs_host(count);
+    item_starts_host->resize((size_t)count + 1);
+    CK(cudaMemcpyAsync(recs_host.data(), recs, sizeof(DcRecDev) * count, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(item_starts_host->data(), io->item_starts, sizeof(u32) * ((size_t)count + 1), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    float ms = 0.f;
+    cudaEventElapsedTime(&ms, ea, eb);
+    const std::vector<u32>& hs = *item_starts_host;
+    for (u32 k = 0; k < count; ++k) {
+        dark_bwt_dc_info& info = infos[k];
+        for (int c = 0; c < 256; ++c) info.init[c] = recs_host[k].init[c];
+        memcpy(info.mtf_symbols, recs_host[k].mtf_symbols, 256);
+        info.num_unique = recs_host[k].num_unique;
+        info.reserved_ = 0;
+        info.num_items = hs[k + 1] - hs[k];
+        info.device_ms = ms;
+        info.reserved2_ = 0;
+    }
     return DARK_BWT_OK;
 }
 
@@ -1794,23 +1882,27 @@ int dark_bwt_inverse_batch(dark_bwt_ctx* ctx, const uint8_t* const* bwts, const 
     });
 }
 
-int dark_bwt_forward_many(dark_bwt_ctx* ctx, const uint8_t* const* texts, const uint64_t* ns, uint8_t* const* bwt_outs,
-                          uint64_t* origins_out, uint64_t count, dark_bwt_stats* stats) {
-    if (!ctx || !texts || !ns || !bwt_outs || !origins_out) return DARK_BWT_E_INVALID_ARG;
-    if (ctx->flags & DARK_BWT_F_DEVICE_ONLY) return DARK_BWT_E_INVALID_ARG;
-    ctx->err[0] = 0;
-    if (count == 0) return DARK_BWT_OK;
-    if (count > kMaxManyBlocks) return DARK_BWT_E_INVALID_ARG;
-    std::vector<u32> starts(count + 1);
+// Offsets of `count` host blocks of at least min_n bytes each that share the arena (sum <= capacity, <= 2^32-2).  `outs`,
+// if given, must have an entry for every block.
+static int many_starts_of(const dark_bwt_ctx* ctx, const uint8_t* const* blocks, uint8_t* const* outs, const uint64_t* ns, uint64_t count,
+                          uint64_t min_n, std::vector<u32>* starts) {
+    starts->resize(count + 1);
     u64 total = 0;
     for (uint64_t k = 0; k < count; ++k) {
-        if (!texts[k] || !bwt_outs[k]) return DARK_BWT_E_INVALID_ARG;
-        if (ns[k] < 2) return DARK_BWT_E_INVALID_N;
-        starts[k] = (u32)total;
+        if (!blocks[k] || (outs && !outs[k])) return DARK_BWT_E_INVALID_ARG;
+        if (ns[k] < min_n) return DARK_BWT_E_INVALID_N;
+        (*starts)[k] = (u32)total;
         total += ns[k];
         if (total > ctx->capacity || total > 0xFFFFFFFEull) return DARK_BWT_E_INVALID_N;  // the blocks share one arena
     }
-    starts[count] = (u32)total;
+    (*starts)[count] = (u32)total;
+    return DARK_BWT_OK;
+}
+
+// dark_bwt_forward_many after its argument checks; bwt_outs (and its entries) may be null: the BWTs stay in ctx->d_bwt.
+static int forward_many_host(dark_bwt_ctx* ctx, const uint8_t* const* texts, const uint64_t* ns, uint8_t* const* bwt_outs,
+                             uint64_t* origins_out, uint64_t count, const std::vector<u32>& starts, dark_bwt_stats* stats) {
+    const u64 total = starts[count];
     CK(cudaSetDevice(ctx->device));
     cudaEvent_t a = ctx->events[kMaxEvents - 1], b = ctx->events[kMaxEvents - 2];
     CK(cudaEventRecord(a, ctx->stream));
@@ -1825,13 +1917,25 @@ int dark_bwt_forward_many(dark_bwt_ctx* ctx, const uint8_t* const* texts, const 
     if (int rc = forward_many_device(ctx, ctx->d_text, (u32)total, (u32)count, ctx->d_bwt, nullptr, stats)) return rc;
     CK(cudaEventRecord(a, ctx->stream));
     for (uint64_t k = 0; k < count; ++k)
-        CK(cudaMemcpyAsync(bwt_outs[k], ctx->d_bwt + starts[k], ns[k], cudaMemcpyDeviceToHost, ctx->stream));
+        if (bwt_outs && bwt_outs[k]) CK(cudaMemcpyAsync(bwt_outs[k], ctx->d_bwt + starts[k], ns[k], cudaMemcpyDeviceToHost, ctx->stream));
     static_assert(sizeof(unsigned long long) == sizeof(uint64_t), "origins are copied as they are");
     CK(cudaMemcpyAsync(origins_out, ctx->many_origins, sizeof(uint64_t) * count, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaEventRecord(b, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     if (stats) cudaEventElapsedTime(&stats->d2h_ms, a, b);
     return DARK_BWT_OK;
+}
+
+int dark_bwt_forward_many(dark_bwt_ctx* ctx, const uint8_t* const* texts, const uint64_t* ns, uint8_t* const* bwt_outs,
+                          uint64_t* origins_out, uint64_t count, dark_bwt_stats* stats) {
+    if (!ctx || !texts || !ns || !bwt_outs || !origins_out) return DARK_BWT_E_INVALID_ARG;
+    if (ctx->flags & DARK_BWT_F_DEVICE_ONLY) return DARK_BWT_E_INVALID_ARG;
+    ctx->err[0] = 0;
+    if (count == 0) return DARK_BWT_OK;
+    if (count > kMaxManyBlocks) return DARK_BWT_E_INVALID_ARG;
+    std::vector<u32> starts;
+    if (int rc = many_starts_of(ctx, texts, bwt_outs, ns, count, 2, &starts)) return rc;
+    return forward_many_host(ctx, texts, ns, bwt_outs, origins_out, count, starts, stats);
 }
 
 int dark_bwt_forward_many_device(dark_bwt_ctx* ctx, const uint8_t* d_text, const uint32_t* d_starts, uint64_t count,
@@ -1994,6 +2098,103 @@ int dark_bwt_forward_dc(dark_bwt_ctx* ctx, const uint8_t* text, uint64_t n, uint
         if (int rc = copy_out_blocking(ctx, bwt_out, ctx->d_bwt, n, ctx->stream)) return rc;
     // the BWT is still in HBM: distance coding reads it there
     return dc_host(ctx, nullptr, n, dist_out, item_pos, item_dist, item_sym, item_rank, info);
+}
+
+// Host copies of what dc_many_device left in `io` (one copy per array); null host pointers are skipped.
+static int dc_many_copy_out(dark_bwt_ctx* ctx, u64 n, const DcManyBuffers& io, const std::vector<u32>& hs, uint32_t* dist_out,
+                            uint32_t* item_starts, uint32_t* item_pos, uint32_t* item_dist, uint8_t* item_sym, uint8_t* item_rank) {
+    const size_t items = hs.back();
+    if (dist_out)
+        if (int rc = copy_out_blocking(ctx, dist_out, io.dc.dist, n * sizeof(u32), ctx->stream)) return rc;
+    if (item_starts) memcpy(item_starts, hs.data(), hs.size() * sizeof(u32));
+    if (item_pos && items)
+        if (int rc = copy_out_blocking(ctx, item_pos, io.dc.item_pos, items * sizeof(u32), ctx->stream)) return rc;
+    if (item_dist && items)
+        if (int rc = copy_out_blocking(ctx, item_dist, io.dc.item_dist, items * sizeof(u32), ctx->stream)) return rc;
+    if (item_sym && items)
+        if (int rc = copy_out_blocking(ctx, item_sym, io.dc.item_sym, items, ctx->stream)) return rc;
+    if (item_rank && items)
+        if (int rc = copy_out_blocking(ctx, item_rank, io.dc.item_rank, items, ctx->stream)) return rc;
+    return DARK_BWT_OK;
+}
+
+int dark_bwt_dc_encode_many_device(dark_bwt_ctx* ctx, const uint8_t* d_bwt, const uint32_t* d_starts, uint64_t count, uint32_t* d_dist_out,
+                                   uint32_t* d_item_starts, uint32_t* d_item_pos, uint32_t* d_item_dist, uint8_t* d_item_sym,
+                                   uint8_t* d_item_rank, dark_bwt_dc_info* infos, float* ms_out) {
+    if (!ctx || !d_bwt || !d_starts || !infos) return DARK_BWT_E_INVALID_ARG;
+    if (count > kMaxManyBlocks) return DARK_BWT_E_INVALID_ARG;
+    ctx->err[0] = 0;
+    if (count == 0) return DARK_BWT_OK;
+    if (!dc_many_records_fit(ctx, count)) return DARK_BWT_E_INVALID_N;
+    CK(cudaSetDevice(ctx->device));
+    // the offsets are checked on the host before any kernel reads them
+    std::vector<u32> starts(count + 1);
+    CK(cudaMemcpyAsync(starts.data(), d_starts, sizeof(u32) * (count + 1), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (starts[0] != 0) return DARK_BWT_E_INVALID_ARG;
+    for (uint64_t k = 0; k < count; ++k)
+        if ((u64)starts[k + 1] < (u64)starts[k] + 1) return DARK_BWT_E_INVALID_N;
+    const u64 total = starts[count];
+    if (total > ctx->capacity || total > 0xFFFFFFFEull) return DARK_BWT_E_INVALID_N;
+    CK(cudaMemcpyAsync(ctx->many_starts, d_starts, sizeof(u32) * (count + 1), cudaMemcpyDeviceToDevice, ctx->stream));
+    DcManyBuffers io;
+    io.dc.dist = d_dist_out;
+    io.item_starts = d_item_starts;
+    io.dc.item_pos = d_item_pos;
+    io.dc.item_dist = d_item_dist;
+    io.dc.item_sym = d_item_sym;
+    io.dc.item_rank = d_item_rank;
+    std::vector<u32> hs;
+    if (int rc = dc_many_device(ctx, d_bwt, (u32)total, (u32)count, &io, infos, &hs)) return rc;
+    if (ms_out) *ms_out = infos[0].device_ms;
+    return DARK_BWT_OK;
+}
+
+int dark_bwt_dc_encode_many(dark_bwt_ctx* ctx, const uint8_t* const* bwts, const uint64_t* ns, uint64_t count, uint32_t* dist_out,
+                            uint32_t* item_starts, uint32_t* item_pos, uint32_t* item_dist, uint8_t* item_sym, uint8_t* item_rank,
+                            dark_bwt_dc_info* infos, float* ms_out) {
+    if (!ctx || !bwts || !ns || !infos) return DARK_BWT_E_INVALID_ARG;
+    if (count > kMaxManyBlocks) return DARK_BWT_E_INVALID_ARG;
+    if (ctx->flags & DARK_BWT_F_DEVICE_ONLY) return DARK_BWT_E_INVALID_ARG;
+    ctx->err[0] = 0;
+    if (count == 0) {
+        if (item_starts) item_starts[0] = 0;
+        return DARK_BWT_OK;
+    }
+    std::vector<u32> starts;
+    if (int rc = many_starts_of(ctx, bwts, nullptr, ns, count, 1, &starts)) return rc;
+    if (!dc_many_records_fit(ctx, count)) return DARK_BWT_E_INVALID_N;
+    CK(cudaSetDevice(ctx->device));
+    CK(cudaMemcpyAsync(ctx->many_starts, starts.data(), sizeof(u32) * (count + 1), cudaMemcpyHostToDevice, ctx->stream));
+    for (uint64_t k = 0; k < count; ++k)
+        CK(cudaMemcpyAsync(ctx->d_bwt + starts[k], bwts[k], ns[k], cudaMemcpyHostToDevice, ctx->stream));
+    DcManyBuffers io;
+    std::vector<u32> hs;
+    if (int rc = dc_many_device(ctx, ctx->d_bwt, starts[count], (u32)count, &io, infos, &hs)) return rc;  // synchronises: `starts` may go
+    if (ms_out) *ms_out = infos[0].device_ms;
+    return dc_many_copy_out(ctx, starts[count], io, hs, dist_out, item_starts, item_pos, item_dist, item_sym, item_rank);
+}
+
+int dark_bwt_forward_dc_many(dark_bwt_ctx* ctx, const uint8_t* const* texts, const uint64_t* ns, uint64_t count, uint8_t* const* bwt_outs,
+                             uint64_t* origins_out, uint32_t* dist_out, uint32_t* item_starts, uint32_t* item_pos, uint32_t* item_dist,
+                             uint8_t* item_sym, uint8_t* item_rank, dark_bwt_dc_info* infos, dark_bwt_stats* stats) {
+    if (!ctx || !texts || !ns || !origins_out || !infos) return DARK_BWT_E_INVALID_ARG;
+    if (count > kMaxManyBlocks) return DARK_BWT_E_INVALID_ARG;
+    if (ctx->flags & DARK_BWT_F_DEVICE_ONLY) return DARK_BWT_E_INVALID_ARG;
+    ctx->err[0] = 0;
+    if (count == 0) {
+        if (item_starts) item_starts[0] = 0;
+        return DARK_BWT_OK;
+    }
+    std::vector<u32> starts;
+    if (int rc = many_starts_of(ctx, texts, nullptr, ns, count, 2, &starts)) return rc;
+    if (!dc_many_records_fit(ctx, count)) return DARK_BWT_E_INVALID_N;
+    if (int rc = forward_many_host(ctx, texts, ns, bwt_outs, origins_out, count, starts, stats)) return rc;
+    // the BWTs are still in HBM at the same offsets, and ctx->many_starts still holds them
+    DcManyBuffers io;
+    std::vector<u32> hs;
+    if (int rc = dc_many_device(ctx, ctx->d_bwt, starts[count], (u32)count, &io, infos, &hs)) return rc;
+    return dc_many_copy_out(ctx, starts[count], io, hs, dist_out, item_starts, item_pos, item_dist, item_sym, item_rank);
 }
 
 int dark_bwt_reuse(dark_bwt_ctx* ctx, uint32_t** words_out, uint64_t* count_out) {

@@ -22,6 +22,12 @@
 //                 32 symbols: one shuffle, one compare, one ballot per run) or in shared memory (8 entries per lane, one
 //                 compare each, one warp reduction): rank, distance of the previous run of s, run record
 //   k_dc_final    last runs and the final MTF order;   k_dc_stream   run ends + their distances, compacted
+//
+// MANY = true: many BWT blocks back to back (DESIGN.md §3.5).  The 4,096-byte chunks stay chunks of the concatenation and
+// the scans run unchanged over global positions; a reader clamps a last occurrence against the start s_b of its own
+// block (a value v <= s_b reads as "none": the symbol has not occurred in the block yet).  Every block start is a run
+// start, so runs never cross a boundary.  k_dc_ranks finalises each block at its end (what k_dc_final does for one
+// block) into a DcRecDev record; k_dc_final is not used.
 #pragma once
 
 #include "common.cuh"
@@ -38,10 +44,49 @@ struct DcInfoDev {  // mirrors the head of dark_bwt_dc_info
     unsigned long long num_items;
 };
 
-// first[256] must be preset to 0xFFFFFFFF, *total_runs to 0.
+// Per-block result of the many-block pass, expanded into dark_bwt_dc_info on the host (num_items from the item starts).
+struct DcRecDev {
+    u32 init[256];
+    u8 mtf_symbols[256];
+    u32 num_unique;
+    u32 reserved_;
+};
+static_assert(sizeof(DcRecDev) == 1288, "include/dark_bwt.h states the record size");
+
+// What the many-block instantiations read besides the single-block arguments (zero in the single-block ones).
+struct DcMany {
+    const u32* starts;      // block offsets [0..count], starts[count] = n
+    u32 count;
+    const u32* start_bits;  // bit p set: a block starts at position p
+    DcRecDev* recs;         // [count]
+    u32* item_starts;       // [0..count]: index of each block's first run; [count] = total runs
+};
+
+// the block holding position pos: the largest b < count with starts[b] <= pos
+__device__ __forceinline__ u32 dc_block_of(const u32* __restrict__ starts, u32 count, u32 pos) {
+    u32 lo = 0, hi = count - 1;
+    while (lo < hi) {
+        const u32 mid = (lo + hi + 1) >> 1;
+        if (starts[mid] <= pos) lo = mid;
+        else hi = mid - 1;
+    }
+    return lo;
+}
+
+// Block-start bitmap of the many-block pass (bits zeroed before), and item_starts[0] = 0.
+__global__ void __launch_bounds__(256) k_dc_mark_starts(const u32* __restrict__ starts, u32 count, u32* __restrict__ bits,
+                                                        u32* __restrict__ item_starts) {
+    const u32 b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b < count) atomicOr(&bits[starts[b] >> 5], 1u << (starts[b] & 31));
+    if (b == 0) item_starts[0] = 0u;
+}
+
+// first[256] must be preset to 0xFFFFFFFF, *total_runs to 0.  MANY: the filler is the length of the position's block,
+// and a block start is a run start even where its byte equals the previous block's last byte.
+template <bool MANY>
 __global__ void __launch_bounds__(256)
 k_dc_tables(const u8* __restrict__ bwt, u32 n, u32* __restrict__ tab, u32* __restrict__ first, u32* __restrict__ run_counts,
-            u32* __restrict__ dist, unsigned long long* __restrict__ total_runs) {
+            u32* __restrict__ dist, unsigned long long* __restrict__ total_runs, DcMany many) {
     __shared__ u32 s_last[256], s_first[256];
     __shared__ u32 s_runs;
     const int tid = threadIdx.x;
@@ -54,19 +99,34 @@ k_dc_tables(const u8* __restrict__ bwt, u32 n, u32* __restrict__ tab, u32* __res
     if (base < n) {
         u32 prev = base > 0 ? (u32)bwt[base - 1] : 0x100u;
         u32 last_pos = 0;
+        u32 b = 0, bs = 0, be = n;  // MANY: the block [bs, be) holding pos
+        if constexpr (MANY) {
+            b = dc_block_of(many.starts, many.count, (u32)base);
+            bs = many.starts[b];
+            be = many.starts[b + 1];
+        }
 #pragma unroll 4
         for (int k = 0; k < 16; ++k) {
             const u64 pos = base + k;
             if (pos < n) {
                 const u32 s = bwt[pos];
-                if (s != prev) {
+                bool run_start = s != prev;
+                if constexpr (MANY) {
+                    if ((u32)pos == be) {  // blocks hold >= 1 byte: one step at most
+                        bs = be;
+                        be = many.starts[++b + 1];
+                    }
+                    run_start |= (u32)pos == bs;
+                }
+                if (run_start) {
                     ++runs;
                     atomicMin(&s_first[s], (u32)pos);
                     if (k > 0) atomicMax(&s_last[prev], (u32)pos);  // the run of prev ended at pos-1 (stored +1)
                 }
                 prev = s;
                 last_pos = (u32)pos;
-                dist[pos] = n;
+                if constexpr (MANY) dist[pos] = be - bs;
+                else dist[pos] = n;
             }
         }
         atomicMax(&s_last[prev], last_pos + 1u);  // this thread's last byte (its run may go on in the next thread's bytes)
@@ -144,10 +204,14 @@ __global__ void __launch_bounds__(256) k_dc_alphabet(const u32* __restrict__ fir
 // One warp per block.  run_offsets = exclusive scan of the blocks' run counts.
 // Alphabets of up to 32 symbols (DNA, most text) keep the table in registers, one symbol per lane: the rank of a run start
 // is one shuffle, one compare and one ballot.  Larger alphabets keep 256 entries in shared memory, 8 per lane.
-__global__ void __launch_bounds__(256)
+// MANY: the warp tracks the text block [bs, be) of its position, found once by binary search.  At the run start i == be
+// (or at the chunk's end when be is there) the table holds the block's final runs, and the warp finalises the block:
+// last-run distances, MTF list, init of absent symbols, item_starts[b + 1].  A first run in the block records init.
+template <bool MANY>
+__global__ void __launch_bounds__(256, MANY ? 6 : 1)
 k_dc_ranks(const u8* __restrict__ bwt, u32 n, const u32* __restrict__ tab, const u32* __restrict__ group_carry,
            const u32* __restrict__ run_offsets, u32 nblocks, const u32* __restrict__ alpha, u32* __restrict__ dist, u32* __restrict__ run_start, u8* __restrict__ run_sym,
-           u8* __restrict__ run_rank) {
+           u8* __restrict__ run_rank, DcMany many) {
     __shared__ u32 s_tab[8][256];
     __shared__ u8 s_dense[256];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -176,6 +240,71 @@ k_dc_ranks(const u8* __restrict__ bwt, u32 n, const u32* __restrict__ tab, const
     __syncwarp();
     u32 run_idx = run_offsets[block];
     const u64 block_base = (u64)block * kDcBlock;
+    u32 tb = 0, bs = 0, be = n;  // MANY: the text block [bs, be) of the current position
+    if constexpr (MANY) {
+        tb = dc_block_of(many.starts, many.count, (u32)block_base);
+        bs = many.starts[tb];
+        be = many.starts[tb + 1];
+    }
+    // MANY: finalise text block tb (the table holds its final runs; next_run = index of the run after its last), step to
+    // the next.  Symbols with v > bs occur in the block; a later v is in the block too, so their ranks need no clamping.
+    auto finish = [&](u32 next_run) {
+        DcRecDev* rec = many.recs + tb;
+        const u32 nb = be - bs;
+        u32 nu = 0, below;
+        if (small) {
+            const bool present = lastreg > bs;  // lanes >= sigma hold 0
+            u32 rank = 0;
+            for (int t = 0; t < 32; ++t) rank += __shfl_sync(0xffffffffu, lastreg, t) > lastreg ? 1u : 0u;
+            nu = __popc(__ballot_sync(0xffffffffu, present));
+            if (present) {
+                dist[lastreg - 1] = be - lastreg - rank;
+                rec->mtf_symbols[rank] = (u8)alpha[256 + lane];
+            }
+        } else {
+#pragma unroll 1
+            for (int k = 0; k < 8; ++k) {
+                const u32 v = last[lane + 32 * k];
+                if (v > bs) {
+                    u32 rank = 0;
+                    for (int c = 0; c < 256; ++c) rank += last[c] > v ? 1u : 0u;
+                    dist[v - 1] = be - v - rank;
+                    rec->mtf_symbols[rank] = (u8)(lane + 32 * k);
+                    ++nu;
+                }
+            }
+            nu = __reduce_add_sync(0xffffffffu, nu);
+        }
+        below = nu;  // absent symbols: the tail of the list in ascending order, init = block length
+#pragma unroll 1
+        for (int k = 0; k < 8; ++k) {
+            const u32 c = (u32)lane + 32u * k;
+            bool absent;
+            if (small) {
+                const u32 d = s_dense[c];
+                const u32 v = __shfl_sync(0xffffffffu, lastreg, (int)(d & 31u));
+                absent = d == 0xFFu || v <= bs;
+            } else {
+                absent = last[c] <= bs;
+            }
+            const u32 ab = __ballot_sync(0xffffffffu, absent);
+            if (absent) {
+                rec->mtf_symbols[below + __popc(ab & ((1u << lane) - 1u))] = (u8)c;
+                rec->init[c] = nb;
+            }
+            below += __popc(ab);
+        }
+        if (lane == 0) {
+            rec->num_unique = nu;
+            rec->reserved_ = 0u;
+            many.item_starts[tb + 1] = next_run;
+        }
+        __syncwarp();
+        ++tb;
+        bs = be;
+        if (tb < many.count) be = many.starts[tb + 1];
+    };
+    (void)finish;
     u32 carry = block_base > 0 ? (u32)bwt[block_base - 1] : 0x100u;
     for (int chunk = 0; chunk < kDcBlock / 32; ++chunk) {
         const u64 pos0 = block_base + (u64)chunk * 32;
@@ -186,6 +315,7 @@ k_dc_ranks(const u8* __restrict__ bwt, u32 n, const u32* __restrict__ tab, const
         u32 prevb = __shfl_up_sync(0xffffffffu, byte, 1);
         if (lane == 0) prevb = carry;
         u32 mask = __ballot_sync(0xffffffffu, valid && byte != prevb);
+        if constexpr (MANY) mask |= many.start_bits[pos0 >> 5];  // pos0 is a multiple of 32; no block starts at or past n
         // run records of this chunk are written together: lane q keeps the q-th run start of the chunk
         const u32 nruns = __popc(mask);
         u32 rec_start = 0, rec_sym = 0, rec_rank = 0;
@@ -198,12 +328,20 @@ k_dc_ranks(const u8* __restrict__ bwt, u32 n, const u32* __restrict__ tab, const
             u32 old, rank;
             if (small) {
                 if (ps < 0x100u && (u32)lane == (u32)s_dense[ps]) lastreg = i;  // the run before this one ended at i-1 (stored +1)
+                if constexpr (MANY)
+                    if (i == be) finish(run_idx + q);
                 old = __shfl_sync(0xffffffffu, lastreg, (int)s_dense[s]);
+                if constexpr (MANY)
+                    if (old <= bs) old = 0u;  // last seen in an earlier block: the first run of s in this one
                 rank = __popc(__ballot_sync(0xffffffffu, lastreg > old));
             } else {
                 if (lane == 0 && ps < 0x100u) last[ps] = i;
                 __syncwarp();
+                if constexpr (MANY)
+                    if (i == be) finish(run_idx + q);
                 old = last[s];  // end + 1 of the previous run of s (0: this is its first)
+                if constexpr (MANY)
+                    if (old <= bs) old = 0u;
                 u32 cnt = 0;
 #pragma unroll
                 for (int k = 0; k < 8; ++k) cnt += last[lane + 32 * k] > old ? 1u : 0u;
@@ -211,6 +349,8 @@ k_dc_ranks(const u8* __restrict__ bwt, u32 n, const u32* __restrict__ tab, const
                 __syncwarp();
             }
             DARK_ASSERT(old <= i && (old == 0 || i >= old + rank));
+            if constexpr (MANY)
+                if (lane == 0 && !old) many.recs[tb].init[s] = i - bs;
             if (lane == 0 && old) dist[old - 1] = i - (old - 1u) - rank - 1u;
             if ((u32)lane == q) {
                 rec_start = i;
@@ -227,6 +367,19 @@ k_dc_ranks(const u8* __restrict__ bwt, u32 n, const u32* __restrict__ tab, const
         }
         run_idx += nruns;
         carry = __shfl_sync(0xffffffffu, byte, 31);
+    }
+    if constexpr (MANY) {
+        const u32 chunk_end = block_base + kDcBlock < (u64)n ? (u32)(block_base + kDcBlock) : n;
+        if (be == chunk_end) {  // the text block ends with this chunk: its final run goes into the table first
+            const u32 ps = bwt[chunk_end - 1];
+            if (small) {
+                if ((u32)lane == (u32)s_dense[ps]) lastreg = chunk_end;
+            } else {
+                if (lane == 0) last[ps] = chunk_end;
+                __syncwarp();
+            }
+            finish(run_idx);
+        }
     }
 }
 
@@ -262,15 +415,18 @@ k_dc_final(u32 n, const u32* __restrict__ final_last, const u32* __restrict__ fi
     }
 }
 
-// The item stream: run r ends just before run r+1 starts.
+// The item stream: run r ends just before run r+1 starts (MANY: runs never cross a block; positions are block-relative).
+template <bool MANY>
 __global__ void __launch_bounds__(256)
 k_dc_stream(const u32* __restrict__ run_start, const unsigned long long* __restrict__ total_runs, u32 n, const u32* __restrict__ dist,
-            u32* __restrict__ out_pos, u32* __restrict__ out_dist) {
+            u32* __restrict__ out_pos, u32* __restrict__ out_dist, DcMany many) {
     const u64 R = *total_runs;
     const u64 stride = (u64)gridDim.x * blockDim.x;
     for (u64 r = (u64)blockIdx.x * blockDim.x + threadIdx.x; r < R; r += stride) {
         const u32 end = (r + 1 < R ? run_start[r + 1] : n) - 1u;
-        out_pos[r] = end;
+        u32 pos = end;
+        if constexpr (MANY) pos -= many.starts[dc_block_of(many.starts, many.count, end)];
+        out_pos[r] = pos;
         out_dist[r] = dist[end];
     }
 }

@@ -245,6 +245,67 @@ class Constructor:
                                                      ctypes.byref(info)), self._ctx, "dc::encode")
         return info
 
+    # -- distance coding of many small blocks in one device pass -----------------------------------------------------
+    def _dc_many_results(self, infos, ns, dist, item_starts, pos, idist, sym, rank):
+        """Per-block dicts shaped like _dc_result, cut out of the concatenated outputs."""
+        out, off = [], 0
+        for k, n in enumerate(ns):
+            a, e = int(item_starts[k]), int(item_starts[k + 1])
+            d = dist[off:off + n] if dist is not None else None
+            res = self._dc_result(infos[k], n, d, pos[a:e], idist[a:e], sym[a:e], rank[a:e])
+            assert res["num_items"] == e - a
+            out.append(res)
+            off += n
+        return out
+
+    def _dc_many_outputs(self, total, count, want_dist):
+        dist = np.empty(total, dtype=np.uint32) if want_dist else None
+        starts = np.empty(count + 1, dtype=np.uint32)
+        pos, idist = np.empty(total, dtype=np.uint32), np.empty(total, dtype=np.uint32)
+        sym, rank = np.empty(total, dtype=np.uint8), np.empty(total, dtype=np.uint8)
+        ptrs = [dist.ctypes.data if want_dist else None] + [a.ctypes.data for a in (starts, pos, idist, sym, rank)]
+        return (dist, starts, pos, idist, sym, rank), ptrs
+
+    def dc_encode_many(self, bwts, want_dist=True):
+        """Distance coding of many small BWT blocks (host buffers) in ONE device pass (dark_bwt_dc_encode_many): a list of
+        dicts shaped like dc_encode's, one per block, each what dc_encode gives on that block alone."""
+        bs = [_as_u8(b) for b in bwts]
+        cnt, ns = len(bs), [b.size for b in bs]
+        arrays, ptrs = self._dc_many_outputs(sum(ns), cnt, want_dist)
+        infos = (_ffi.DcInfo * max(cnt, 1))()
+        ms = ctypes.c_float(0)
+        _ffi.check(self._L.dark_bwt_dc_encode_many(self._ctx, (ctypes.c_void_p * max(cnt, 1))(*[b.ctypes.data for b in bs]),
+                                                   (ctypes.c_uint64 * max(cnt, 1))(*ns), cnt, *ptrs, infos, ctypes.byref(ms)),
+                   self._ctx, "dc::encode (many)")
+        return self._dc_many_results(infos, ns, *arrays)
+
+    def bwt_dc_many(self, texts, want_dist=True, want_bwt=True):
+        """block/dc.rs:45-52 for many small blocks (dark_bwt_forward_dc_many): one sort of all blocks, then one DC pass over
+        the BWTs while they are still in HBM.  [(bwt or None, origin, dc dict), ...]."""
+        ts = [_as_u8(t) for t in texts]
+        cnt, ns = len(ts), [t.size for t in ts]
+        outs = [np.empty(n, dtype=np.uint8) for n in ns] if want_bwt else None
+        arrays, ptrs = self._dc_many_outputs(sum(ns), cnt, want_dist)
+        infos = (_ffi.DcInfo * max(cnt, 1))()
+        origins = (ctypes.c_uint64 * max(cnt, 1))()
+        bwt_ptrs = (ctypes.c_void_p * max(cnt, 1))(*[o.ctypes.data for o in outs]) if want_bwt else None
+        _ffi.check(self._L.dark_bwt_forward_dc_many(self._ctx, (ctypes.c_void_p * max(cnt, 1))(*[t.ctypes.data for t in ts]),
+                                                    (ctypes.c_uint64 * max(cnt, 1))(*ns), cnt, bwt_ptrs, origins, *ptrs, infos,
+                                                    ctypes.byref(self.stats)), self._ctx, "bwt + dc::encode (many)")
+        res = self._dc_many_results(infos, ns, *arrays)
+        return [(outs[k] if want_bwt else None, int(origins[k]), res[k]) for k in range(cnt)]
+
+    def dc_encode_many_device(self, d_bwt, d_starts, count, d_dist=None, d_item_starts=None, d_item_pos=None, d_item_dist=None,
+                              d_item_sym=None, d_item_rank=None):
+        """Device-resident form, the layout bwt_many_device writes: blocks back to back in d_bwt at the offsets d_starts[0..count]
+        (u32, on the device); outputs are device pointers (all optional).  Returns (list of DcInfo headers, device ms)."""
+        infos = (_ffi.DcInfo * max(int(count), 1))()
+        ms = ctypes.c_float(0)
+        _ffi.check(self._L.dark_bwt_dc_encode_many_device(self._ctx, d_bwt, d_starts, int(count), d_dist, d_item_starts, d_item_pos,
+                                                          d_item_dist, d_item_sym, d_item_rank, infos, ctypes.byref(ms)),
+                   self._ctx, "dc::encode (many)")
+        return [infos[k] for k in range(int(count))], float(ms.value)
+
     # -- device-resident form (benches, pipelines that keep the block in HBM) ------------------
     def bwt_device(self, d_text, n, d_bwt, d_sa=None):
         """Raw device pointers (ints).  Returns origin; self.stats holds the device timings."""

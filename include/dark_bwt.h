@@ -208,6 +208,34 @@ int dark_bwt_forward_dc(dark_bwt_ctx *ctx, const uint8_t *text, uint64_t n, uint
                         uint32_t *dist_out, uint32_t *item_pos, uint32_t *item_dist, uint8_t *item_sym, uint8_t *item_rank,
                         dark_bwt_dc_info *info, dark_bwt_stats *stats);
 
+/* MANY SMALL blocks distance-coded in ONE pass.  Block k gives exactly what dark_bwt_dc_encode gives on that block alone:
+ * every value is block-relative (filler and last-run distances use n_k, init[c] is the first occurrence inside the block
+ * or n_k, item_pos is the run end inside the block, runs never merge across a boundary).  Outputs:
+ *   infos[0..count)          host array, one record per block; device_ms is the time of the one pass (also *ms_out);
+ *   dist                     the blocks' distances at their byte offsets (room for sum(ns) words);
+ *   item_starts[0..count]    u32 offsets of each block's items, item_starts[count] = total runs;
+ *   item_pos/dist/sym/rank   the items of all blocks in block order (room for sum(ns) entries each).
+ * Every output but `infos` is nullable.  Limits: count <= DARK_BWT_MAX_MANY_BLOCKS (else DARK_BWT_E_INVALID_ARG), each
+ * block >= 1 byte, sum(ns) <= capacity and <= 2^32-2, and the per-block records (1,288 bytes each) are staged in an
+ * 8 * capacity + 1 KiB buffer: count * 1288 <= 8 * capacity + 1024 (blocks of about 161 bytes or more on average at full
+ * capacity), else DARK_BWT_E_INVALID_N.  One H2D copy per block, one device pass, one D2H copy per output array.
+ * DARK_BWT_E_INVALID_ARG with a device-only context. */
+int dark_bwt_dc_encode_many(dark_bwt_ctx *ctx, const uint8_t *const *bwts, const uint64_t *ns, uint64_t count, uint32_t *dist_out,
+                            uint32_t *item_starts, uint32_t *item_pos, uint32_t *item_dist, uint8_t *item_sym, uint8_t *item_rank,
+                            dark_bwt_dc_info *infos, float *ms_out);
+/* Same on device buffers, the layout dark_bwt_forward_many_device writes: d_bwt holds the blocks back to back at the u32
+ * offsets d_starts[0..count] (on the device; read back and checked before any kernel runs: d_starts[0] = 0, offsets
+ * increasing).  The outputs are device buffers with the layout above; `infos` and `ms_out` are host pointers. */
+int dark_bwt_dc_encode_many_device(dark_bwt_ctx *ctx, const uint8_t *d_bwt, const uint32_t *d_starts, uint64_t count,
+                                   uint32_t *d_dist_out, uint32_t *d_item_starts, uint32_t *d_item_pos, uint32_t *d_item_dist,
+                                   uint8_t *d_item_sym, uint8_t *d_item_rank, dark_bwt_dc_info *infos, float *ms_out);
+/* block/dc.rs:45-52 for many small blocks: dark_bwt_forward_many, then the pass above over the BWTs while they are still in
+ * HBM.  Each block >= 2 bytes; bwt_outs (and its entries) nullable; stats reports the sort as dark_bwt_forward_many does. */
+int dark_bwt_forward_dc_many(dark_bwt_ctx *ctx, const uint8_t *const *texts, const uint64_t *ns, uint64_t count,
+                             uint8_t *const *bwt_outs, uint64_t *origins_out, uint32_t *dist_out, uint32_t *item_starts,
+                             uint32_t *item_pos, uint32_t *item_dist, uint8_t *item_sym, uint8_t *item_rank,
+                             dark_bwt_dc_info *infos, dark_bwt_stats *stats);
+
 /* Constructor::reuse — lends >= capacity host u32 words of scratch (DC distances in
  * block/dc.rs:51).  Allocated on first use; owned by the context. */
 int dark_bwt_reuse(dark_bwt_ctx *ctx, uint32_t **words_out, uint64_t *count_out);

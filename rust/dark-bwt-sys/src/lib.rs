@@ -59,6 +59,17 @@ extern "C" {
     pub fn dark_bwt_forward_dc(ctx: *mut dark_bwt_ctx, text: *const u8, n: u64, bwt_out: *mut u8, origin_out: *mut u64,
                                dist_out: *mut u32, item_pos: *mut u32, item_dist: *mut u32, item_sym: *mut u8, item_rank: *mut u8,
                                info: *mut dark_bwt_dc_info, stats: *mut dark_bwt_stats) -> c_int;
+    pub fn dark_bwt_dc_encode_many(ctx: *mut dark_bwt_ctx, bwts: *const *const u8, ns: *const u64, count: u64, dist_out: *mut u32,
+                                   item_starts: *mut u32, item_pos: *mut u32, item_dist: *mut u32, item_sym: *mut u8,
+                                   item_rank: *mut u8, infos: *mut dark_bwt_dc_info, ms_out: *mut f32) -> c_int;
+    pub fn dark_bwt_dc_encode_many_device(ctx: *mut dark_bwt_ctx, d_bwt: *const u8, d_starts: *const u32, count: u64,
+                                          d_dist_out: *mut u32, d_item_starts: *mut u32, d_item_pos: *mut u32, d_item_dist: *mut u32,
+                                          d_item_sym: *mut u8, d_item_rank: *mut u8, infos: *mut dark_bwt_dc_info,
+                                          ms_out: *mut f32) -> c_int;
+    pub fn dark_bwt_forward_dc_many(ctx: *mut dark_bwt_ctx, texts: *const *const u8, ns: *const u64, count: u64,
+                                    bwt_outs: *const *mut u8, origins_out: *mut u64, dist_out: *mut u32, item_starts: *mut u32,
+                                    item_pos: *mut u32, item_dist: *mut u32, item_sym: *mut u8, item_rank: *mut u8,
+                                    infos: *mut dark_bwt_dc_info, stats: *mut dark_bwt_stats) -> c_int;
     pub fn dark_bwt_create(max_n: u64, device: c_int, out: *mut *mut dark_bwt_ctx) -> c_int;
     pub fn dark_bwt_create_ex(max_n: u64, device: c_int, flags: u32, out: *mut *mut dark_bwt_ctx) -> c_int;
     pub fn dark_bwt_capacity(ctx: *const dark_bwt_ctx) -> u64;
