@@ -59,15 +59,6 @@ struct Mailbox {  // pinned host memory the device results are copied into
     u32 bad_block;  // inverse_many: the lowest block whose list does not cover its rows (with `count` = how many do not)
 };
 
-struct DeviceScalars {  // mirrors Mailbox on the device
-    u32 sigma;
-    u32 count;
-    u32 trivial[kMaxPasses];
-    float collide[kMaxPasses];
-    u64 origin;
-    unsigned long long bad;
-};
-
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 inline int bit_length(u64 x) {
     int b = 0;
@@ -169,7 +160,7 @@ struct dark_bwt_ctx {
     u32* hist = nullptr;
     u32* present = nullptr;
     u8* lut = nullptr;
-    DeviceScalars* scalars = nullptr;
+    unsigned long long* bad = nullptr;  // dark_bwt_verify_sa_device: violation counter (device atomics)
     void* sort_status = nullptr;
     size_t sort_status_bytes = 0;
     // Sorts of at most 2^31 pairs use 32-bit status words and the buffer as two halves in turn: the workers of a pass zero
@@ -193,6 +184,7 @@ struct dark_bwt_ctx {
     u64 reuse_count = 0;
 
     cudaEvent_t events[kMaxEvents];
+    cudaEvent_t call_start = nullptr, call_stop = nullptr;  // the last two events: time a whole call (span_begin leaves them free)
     int n_events = 0;
     struct Span {
         int phase, e0, e1;
@@ -234,8 +226,40 @@ inline cudaError_t sync_counted(dark_bwt_ctx* ctx) {
     return cudaStreamSynchronize(ctx->stream);
 }
 
+// The start of a call that sorts or inverts: the context's device, fresh per-call bookkeeping (events and spans, tile
+// counters, launch and sync counts, the isa[] tag), the call's clock (call_start) and zeroed tile counters.
+int begin_call(dark_bwt_ctx* ctx) {
+    CK(cudaSetDevice(ctx->device));
+    ctx->n_events = 0;
+    ctx->spans.clear();
+    ctx->next_counter = 0;
+    ctx->launches = 0;
+    ctx->syncs = 0;
+    ctx->tag = 0;
+    CK(cudaEventRecord(ctx->call_start, ctx->stream));
+    CK(cudaMemsetAsync(ctx->counters, 0, sizeof(u32) * kMaxCounters, ctx->stream));
+    return 0;
+}
+
+// Device time from call_start to call_stop; both have completed.
+float call_ms(const dark_bwt_ctx* ctx) {
+    float ms = 0.f;
+    cudaEventElapsedTime(&ms, ctx->call_start, ctx->call_stop);
+    return ms;
+}
+
+// The stats of a forward call start from zero, but for the host entry's h2d_ms, measured before the transform.
+void reset_stats(dark_bwt_stats* st, u32 n) {
+    if (!st) return;
+    const float h2d = st->h2d_ms;
+    memset(st, 0, sizeof(*st));
+    st->h2d_ms = h2d;
+    st->n = n;
+    st->active[0] = n;
+}
+
 int span_begin(dark_bwt_ctx* ctx, int phase) {
-    if (ctx->n_events + 2 > kMaxEvents - 4) return -1;  // the last events are reserved for the entry points
+    if (ctx->n_events + 2 > kMaxEvents - 4) return -1;  // the last events are reserved (call_start, call_stop)
     int e0 = ctx->n_events++;
     cudaEventRecord(ctx->events[e0], ctx->stream);
     ctx->spans.push_back({phase, e0, -1});
@@ -566,11 +590,9 @@ int emit(dark_bwt_ctx* ctx, const u8* d_text, u32 n, const u32* d_sa, u8* d_bwt)
     return 0;
 }
 
-void finish_stats(dark_bwt_ctx* ctx, dark_bwt_stats* st, int e_first, int e_last) {
+void finish_stats(dark_bwt_ctx* ctx, dark_bwt_stats* st) {
     if (!st) return;
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, ctx->events[e_first], ctx->events[e_last]);
-    st->device_ms = ms;
+    st->device_ms = call_ms(ctx);
     for (const auto& s : ctx->spans) {
         if (s.e1 < 0) continue;
         float t = 0.f;
@@ -589,32 +611,14 @@ void finish_stats(dark_bwt_ctx* ctx, dark_bwt_stats* st, int e_first, int e_last
     st->host_syncs = ctx->syncs;
 }
 
-// The whole forward transform on device buffers.  d_sa_user nullable.
-int forward_device(dark_bwt_ctx* ctx, const u8* d_text, u64 n64, u8* d_bwt, u64* origin_out, u32* d_sa_user,
-                   dark_bwt_stats* st) {
-    if (n64 < 2 || n64 > ctx->capacity || n64 > 0xFFFFFFFEull) return DARK_BWT_E_INVALID_N;
-    const u32 n = (u32)n64;
-    CK(cudaSetDevice(ctx->device));
-    ctx->n_events = 0;
-    ctx->spans.clear();
-    ctx->next_counter = 0;
-    ctx->launches = 0;
-    ctx->syncs = 0;
-    if (st) {
-        const float h2d = st->h2d_ms;
-        memset(st, 0, sizeof(*st));
-        st->h2d_ms = h2d;
-        st->n = n;
-        st->active[0] = n;
-    }
+// The whole forward transform on device buffers (2 <= n <= capacity).  d_sa_user nullable.
+int forward_device(dark_bwt_ctx* ctx, const u8* d_text, u32 n, u8* d_bwt, u64* origin_out, u32* d_sa_user, dark_bwt_stats* st) {
+    if (int rc = begin_call(ctx)) return rc;
+    reset_stats(st, n);
     u32* sa = d_sa_user ? d_sa_user : ctx->sa;
-
-    const int e_first = ctx->n_events++;
-    CK(cudaEventRecord(ctx->events[e_first], ctx->stream));
 
     // ---- alphabet: sigma, dense codes, symbols per key
     int sp = span_begin(ctx, PH_INIT);
-    CK(cudaMemsetAsync(ctx->counters, 0, sizeof(u32) * kMaxCounters, ctx->stream));
     CK(cudaMemsetAsync(ctx->present, 0, sizeof(u32) * 256, ctx->stream));
     CK(cudaMemsetAsync(ctx->hist, 0, sizeof(u32) * kMaxPasses * kRadix, ctx->stream));
     const int no_pack = (ctx->flags & DARK_BWT_F_NO_ALPHABET_PACKING) ? 1 : 0;
@@ -992,11 +996,10 @@ int forward_device(dark_bwt_ctx* ctx, const u8* d_text, u64 n64, u8* d_bwt, u64*
     if (!emit_inline)
         if (int rc = emit(ctx, d_text, n, sa, d_bwt)) return rc;
     span_end(ctx, sp);
-    const int e_last = ctx->n_events++;
-    CK(cudaEventRecord(ctx->events[e_last], ctx->stream));
+    CK(cudaEventRecord(ctx->call_stop, ctx->stream));
     CK(sync_counted(ctx));
     *origin_out = ctx->mail->origin;
-    finish_stats(ctx, st, e_first, e_last);
+    finish_stats(ctx, st);
     return DARK_BWT_OK;
 }
 
@@ -1004,23 +1007,9 @@ int forward_device(dark_bwt_ctx* ctx, const u8* d_text, u64 n64, u8* d_bwt, u64*
 // to back, ctx->many_starts their offsets (B + 1 values, already on the device); d_bwt receives the per-block BWTs
 // at the same offsets, ctx->many_origins the origins.
 int forward_many_device(dark_bwt_ctx* ctx, const u8* d_text, u32 n, u32 B, u8* d_bwt, u32* d_sa_out, dark_bwt_stats* st) {
-    CK(cudaSetDevice(ctx->device));
-    ctx->n_events = 0;
-    ctx->spans.clear();
-    ctx->next_counter = 0;
-    ctx->launches = 0;
-    ctx->tag = 0;
-    if (st) {
-        const float h2d = st->h2d_ms;
-        memset(st, 0, sizeof(*st));
-        st->h2d_ms = h2d;
-        st->n = n;
-        st->active[0] = n;
-    }
-    const int e_first = ctx->n_events++;
-    CK(cudaEventRecord(ctx->events[e_first], ctx->stream));
+    if (int rc = begin_call(ctx)) return rc;
+    reset_stats(st, n);
     int sp = span_begin(ctx, PH_INIT);
-    CK(cudaMemsetAsync(ctx->counters, 0, sizeof(u32) * kMaxCounters, ctx->stream));
     CK(cudaMemsetAsync(ctx->present, 0, sizeof(u32) * 256, ctx->stream));
     CK(cudaMemsetAsync(ctx->hist, 0, sizeof(u32) * kMaxPasses * kRadix, ctx->stream));
     {
@@ -1030,7 +1019,7 @@ int forward_many_device(dark_bwt_ctx* ctx, const u8* d_text, u32 n, u32 B, u8* d
         k_many_lut<<<1, 256, 0, ctx->stream>>>(ctx->present, ctx->many_lut, &ctx->mail_dev->sigma);
         LAUNCHED();
     }
-    CK(cudaStreamSynchronize(ctx->stream));
+    CK(sync_counted(ctx));
     const u32 sigma = ctx->mail->sigma;
     if (sigma < 1 || sigma > 256) return ctx->fail_internal("alphabet scan returned an impossible sigma");
     const int s_bits = bit_length(sigma);  // codes 1..sigma, 0 = past the end of the block
@@ -1105,25 +1094,15 @@ int forward_many_device(dark_bwt_ctx* ctx, const u8* d_text, u32 n, u32 B, u8* d
                                                                ctx->many_origins, d_sa_out);
     LAUNCHED();
     span_end(ctx, sp);
-    const int e_last = ctx->n_events++;
-    CK(cudaEventRecord(ctx->events[e_last], ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    finish_stats(ctx, st, e_first, e_last);
+    CK(cudaEventRecord(ctx->call_stop, ctx->stream));
+    CK(sync_counted(ctx));
+    finish_stats(ctx, st);
     return DARK_BWT_OK;
 }
 
-// Inverse BWT on device buffers (kernels and method: suffix_kernels.cuh, "inverse BWT").
-int inverse_device(dark_bwt_ctx* ctx, const u8* d_bwt, u64 n64, u64 origin64, u8* d_text, float* ms_out) {
-    if (n64 < 1 || n64 > ctx->capacity || n64 > 0xFFFFFFFEull) return DARK_BWT_E_INVALID_N;
-    if (origin64 >= n64) return DARK_BWT_E_INVALID_ARG;
-    const u32 n = (u32)n64, origin = (u32)origin64;
-    CK(cudaSetDevice(ctx->device));
-    ctx->n_events = 0;
-    ctx->spans.clear();
-    ctx->next_counter = 0;
-    cudaEvent_t ea = ctx->events[kMaxEvents - 1], eb = ctx->events[kMaxEvents - 2];
-    CK(cudaEventRecord(ea, ctx->stream));
-    CK(cudaMemsetAsync(ctx->counters, 0, sizeof(u32) * kMaxCounters, ctx->stream));
+// Inverse BWT on device buffers (kernels and method: suffix_kernels.cuh, "inverse BWT"); 1 <= n <= capacity, origin < n.
+int inverse_device(dark_bwt_ctx* ctx, const u8* d_bwt, u32 n, u32 origin, u8* d_text, float* ms_out) {
+    if (int rc = begin_call(ctx)) return rc;
     CK(cudaMemsetAsync(ctx->hist, 0, sizeof(u32) * kMaxPasses * kRadix, ctx->stream));
     // step 1: (last-column symbol, row) pairs; stable partition by symbol -> psi.  The pairs are built inside the
     // radix pass (GEN mode 1) and their digit histogram is the byte histogram of the BWT.
@@ -1200,9 +1179,9 @@ int inverse_device(dark_bwt_ctx* ctx, const u8* d_bwt, u64 n64, u64 origin64, u8
                                                                          d_text, len_keep, nullptr, cap, 0u);
         LAUNCHED();
     }
-    CK(cudaEventRecord(eb, ctx->stream));
+    CK(cudaEventRecord(ctx->call_stop, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    if (ms_out) cudaEventElapsedTime(ms_out, ea, eb);
+    if (ms_out) *ms_out = call_ms(ctx);
     return DARK_BWT_OK;
 }
 
@@ -1216,13 +1195,7 @@ int inverse_device(dark_bwt_ctx* ctx, const u8* d_bwt, u64 n64, u64 origin64, u8
 // arena hold.  The stash gets (8 capacity + 1024) / nodes >= 8 bytes a chunk.  So 65,536 blocks of one byte need a
 // capacity of 131,072 (rows, not bytes, are what must fit), and sum(ns) <= capacity alone would not be enough.
 int inverse_many_device(dark_bwt_ctx* ctx, const u8* d_bwt, u32 n, u32 B, u32 max_nb, u8* d_text, float* ms_out) {
-    CK(cudaSetDevice(ctx->device));
-    ctx->n_events = 0;
-    ctx->spans.clear();
-    ctx->next_counter = 0;
-    cudaEvent_t ea = ctx->events[kMaxEvents - 1], eb = ctx->events[kMaxEvents - 2];
-    CK(cudaEventRecord(ea, ctx->stream));
-    CK(cudaMemsetAsync(ctx->counters, 0, sizeof(u32) * kMaxCounters, ctx->stream));
+    if (int rc = begin_call(ctx)) return rc;
     CK(cudaMemsetAsync(ctx->hist, 0, sizeof(u32) * kMaxPasses * kRadix, ctx->stream));
     // step 1: (block, last symbol) keys of the real rows, one stable sort -> psi and the first symbols
     const int passes = 1 + (B > 1 ? (bit_length((u64)B - 1) + kRadixBits - 1) / kRadixBits : 0);
@@ -1281,24 +1254,113 @@ int inverse_many_device(dark_bwt_ctx* ctx, const u8* d_bwt, u32 n, u32 B, u32 ma
                                                             dist[w], d_text, len_keep, nullptr, cap, 0u);
         LAUNCHED();
     }
-    CK(cudaEventRecord(eb, ctx->stream));
+    CK(cudaEventRecord(ctx->call_stop, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    if (ms_out) cudaEventElapsedTime(ms_out, ea, eb);
+    if (ms_out) *ms_out = call_ms(ctx);
     return DARK_BWT_OK;
 }
 
-// Distance coding + MTF of a BWT block on device buffers (dc_kernels.cuh).  Every output pointer is nullable: the
-// context's own arena is used for what the caller does not want.  *d_dist_used / *d_pos_used etc. tell where the data is.
+// ---- argument checks of the entry points --------------------------------------------------------
+// The length of a single block: min_n (1 or 2) <= n <= capacity, and n <= 2^32-2 (suffixes and rows are u32).
+int check_n(const dark_bwt_ctx* ctx, u64 n, u64 min_n) {
+    return (n < min_n || n > ctx->capacity || n > 0xFFFFFFFEull) ? DARK_BWT_E_INVALID_N : DARK_BWT_OK;
+}
+
+// The host-buffer entries stage through device buffers that a DARK_BWT_F_DEVICE_ONLY context does not have.
+int check_staging(const dark_bwt_ctx* ctx) { return (ctx->flags & DARK_BWT_F_DEVICE_ONLY) ? DARK_BWT_E_INVALID_ARG : DARK_BWT_OK; }
+
+// The blocks of a many-block entry, back to back: block k is [starts[k], starts[k+1]).
+struct BlockList {
+    std::vector<u32> starts;              // count + 1 offsets
+    std::vector<uint64_t> origins;        // the inverse's, one per block
+    const u32* d_starts = nullptr;        // device entries: the caller's offsets and origins, which load_blocks copies
+    const uint64_t* d_origins = nullptr;
+    u64 max_nb = 0;                       // the largest block
+    u32 count() const { return (u32)starts.size() - 1; }
+    u32 total() const { return starts.back(); }
+};
+
+// The one check of a many-block list, before any kernel reads it.  The offsets come from the host lengths `ns`, or from
+// `d_starts` on the device, read back here; `origins` (the inverse's, else null) lives where the offsets do.  `ins` and
+// `outs` (nullable) are host blocks and outputs, one per block.  Every block has at least min_n bytes and adds `extra_rows`
+// rows beyond them (the inverse's '$' row); the rows must fit the arena and u32 offsets.  u64 arithmetic throughout, so
+// no offset, length or sum wraps.  In the order checked: count > DARK_BWT_MAX_MANY_BLOCKS, starts[0] != 0, a null block or
+// output pointer or an origin outside its block is DARK_BWT_E_INVALID_ARG; a shorter block (decreasing offsets included)
+// or too many rows is DARK_BWT_E_INVALID_N.
+int check_blocks(dark_bwt_ctx* ctx, u64 count, const uint64_t* ns, const u32* d_starts, const uint64_t* origins, u64 min_n,
+                 u64 extra_rows, const uint8_t* const* ins, uint8_t* const* outs, BlockList* bl) {
+    if (count > kMaxManyBlocks) return DARK_BWT_E_INVALID_ARG;
+    std::vector<u64> s(count + 1, 0);
+    bl->starts.resize(count + 1);
+    bl->origins.resize(origins ? count : 0);
+    if (d_starts) {
+        CK(cudaSetDevice(ctx->device));
+        CK(cudaMemcpyAsync(bl->starts.data(), d_starts, sizeof(u32) * (count + 1), cudaMemcpyDeviceToHost, ctx->stream));
+        if (origins) CK(cudaMemcpyAsync(bl->origins.data(), origins, sizeof(uint64_t) * count, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        std::copy(bl->starts.begin(), bl->starts.end(), s.begin());
+        bl->d_starts = d_starts;
+        bl->d_origins = origins;
+    } else {
+        // a block of 2^32 bytes or more fails below whatever its length: clamped there, the lengths add up without wrapping
+        for (u64 k = 0; k < count; ++k) s[k + 1] = s[k] + std::min<u64>(ns[k], 1ull << 32);
+        if (origins) std::copy(origins, origins + count, bl->origins.begin());
+    }
+    if (s[0] != 0) return DARK_BWT_E_INVALID_ARG;
+    const u64 max_rows = std::min<u64>(ctx->capacity, 0xFFFFFFFEull);
+    bl->max_nb = 0;
+    for (u64 k = 0; k < count; ++k) {
+        if ((ins && !ins[k]) || (outs && !outs[k])) return DARK_BWT_E_INVALID_ARG;
+        if (s[k + 1] < s[k] + min_n) return DARK_BWT_E_INVALID_N;
+        const u64 nb = s[k + 1] - s[k];
+        if (origins && bl->origins[k] >= nb) return DARK_BWT_E_INVALID_ARG;
+        bl->max_nb = std::max(bl->max_nb, nb);
+        if (s[k + 1] + extra_rows * (k + 1) > max_rows) return DARK_BWT_E_INVALID_N;  // the blocks share one arena
+    }
+    for (u64 k = 0; k <= count; ++k) bl->starts[k] = (u32)s[k];
+    return DARK_BWT_OK;
+}
+
+// Puts a checked list where the kernels read it: the offsets into ctx->many_starts, the inverse's origins into ctx->many_origins,
+// and the host blocks `ins` (if given) into `dst` at their offsets.
+int load_blocks(dark_bwt_ctx* ctx, const BlockList& bl, const uint8_t* const* ins = nullptr, u8* dst = nullptr) {
+    const size_t count = bl.count();
+    if (bl.d_starts) CK(cudaMemcpyAsync(ctx->many_starts, bl.d_starts, sizeof(u32) * (count + 1), cudaMemcpyDeviceToDevice, ctx->stream));
+    else CK(cudaMemcpyAsync(ctx->many_starts, bl.starts.data(), sizeof(u32) * (count + 1), cudaMemcpyHostToDevice, ctx->stream));
+    static_assert(sizeof(unsigned long long) == sizeof(uint64_t), "origins are copied as they are");
+    if (bl.d_origins) CK(cudaMemcpyAsync(ctx->many_origins, bl.d_origins, sizeof(uint64_t) * count, cudaMemcpyDeviceToDevice, ctx->stream));
+    else if (!bl.origins.empty())
+        CK(cudaMemcpyAsync(ctx->many_origins, bl.origins.data(), sizeof(uint64_t) * count, cudaMemcpyHostToDevice, ctx->stream));
+    if (ins)
+        for (size_t k = 0; k < count; ++k)
+            CK(cudaMemcpyAsync(dst + bl.starts[k], ins[k], bl.starts[k + 1] - bl.starts[k], cudaMemcpyHostToDevice, ctx->stream));
+    return 0;
+}
+
+// ---- distance coding ----------------------------------------------------------------------------
+// Where distance coding writes.  Every device pointer is nullable: the context's own arena is used for what the caller does
+// not want, and dc_device sets the pointer to where the data is.
 struct DcBuffers {
-    u32* dist = nullptr;     // n
-    u32* item_pos = nullptr; // num_items
+    u32* dist = nullptr;         // n
+    u32* item_pos = nullptr;     // num_items
     u32* item_dist = nullptr;
     u8* item_sym = nullptr;
     u8* item_rank = nullptr;
+    u32* item_starts = nullptr;  // many blocks: count + 1
+    std::vector<u32> item_starts_host;  // many blocks: item_starts, read back
 };
-int dc_device(dark_bwt_ctx* ctx, const u8* d_bwt, u64 n64, DcBuffers* io, dark_bwt_dc_info* info) {
-    if (n64 < 1 || n64 > ctx->capacity || n64 > 0xFFFFFFFEull) return DARK_BWT_E_INVALID_N;
-    const u32 n = (u32)n64;
+
+// The per-block records of the many-block pass are staged in the sort's second key buffer (8 N + 1 KiB bytes), which distance
+// coding leaves free: count * sizeof(DcRecDev) <= 8 * capacity + 1024.
+bool dc_many_records_fit(const dark_bwt_ctx* ctx, u64 count) {
+    return count * sizeof(DcRecDev) <= ctx->capacity * 8 + 1024;
+}
+
+// Distance coding + MTF on device buffers (dc_kernels.cuh) of one BWT block d_bwt[0..n) (`blocks` null; 1 <= n <= capacity),
+// or in one pass of the checked list `blocks`, back to back in d_bwt and loaded into ctx->many_starts (the records fit).
+// One block: infos[0] gets the result header.  Many: infos[0..count) get the per-block records, io->item_starts_host the
+// item offsets.
+int dc_device(dark_bwt_ctx* ctx, const u8* d_bwt, u32 n, const BlockList* blocks, DcBuffers* io, dark_bwt_dc_info* infos) {
     CK(cudaSetDevice(ctx->device));
     const u32 nblocks = (u32)ceil_div(n, kDcBlock);
     // last-occurrence tables: (nblocks + ngroups) x 256 words = n/4 + n/1024 bytes (+ 2 KB): inside the 4n-byte rank buffer for
@@ -1318,13 +1380,27 @@ int dc_device(dark_bwt_ctx* ctx, const u8* d_bwt, u64 n64, DcBuffers* io, dark_b
     if (!io->item_sym) io->item_sym = (u8*)ctx->ids[1];
     if (!io->item_rank) io->item_rank = (u8*)ctx->ids[1] + (size_t)n;
     unsigned long long* total_runs = (unsigned long long*)((char*)ctx->dc_info + align_up(sizeof(DcInfoDev), 8));
-    cudaEvent_t ea = ctx->events[kMaxEvents - 1], eb = ctx->events[kMaxEvents - 2];
-    CK(cudaEventRecord(ea, ctx->stream));
+    DcMany many{};  // zero in the single-block instantiations
+    if (blocks) {
+        // behind the run counts (4 N + 16 bytes): align4(nblocks) + count + 1 words fit, as the records bound count to capacity / 160
+        if (!io->item_starts) io->item_starts = ctx->ranks_alt + align_up(nblocks, 4);
+        many = DcMany{ctx->many_starts, blocks->count(), ctx->bitmap, (DcRecDev*)ctx->keys[1], io->item_starts};
+    }
+    CK(cudaEventRecord(ctx->call_start, ctx->stream));
     CK(cudaMemsetAsync(first, 0xFF, sizeof(u32) * 256, ctx->stream));
     CK(cudaMemsetAsync(total_runs, 0, sizeof(unsigned long long), ctx->stream));
-    const DcMany none{};
-    k_dc_tables<false><<<nblocks, 256, 0, ctx->stream>>>(d_bwt, n, tab, first, run_counts, io->dist, total_runs, none);
-    LAUNCHED();
+    if (blocks) {
+        CK(cudaMemsetAsync(ctx->bitmap, 0, sizeof(u32) * ceil_div(n, 32), ctx->stream));
+        k_dc_mark_starts<<<(u32)ceil_div(many.count, 256), 256, 0, ctx->stream>>>(ctx->many_starts, many.count, ctx->bitmap, io->item_starts);
+        LAUNCHED();
+    }
+#define DC_LAUNCH(KERNEL, GRID, ...)                                                          \
+    do {                                                                                      \
+        if (blocks) KERNEL<true><<<GRID, 256, 0, ctx->stream>>>(__VA_ARGS__, many);           \
+        else KERNEL<false><<<GRID, 256, 0, ctx->stream>>>(__VA_ARGS__, many);                 \
+        LAUNCHED();                                                                           \
+    } while (0)
+    DC_LAUNCH(k_dc_tables, nblocks, d_bwt, n, tab, first, run_counts, io->dist, total_runs);
     const u32 ngroups = (u32)ceil_div(nblocks, kDcGroup);
     u32* group_last = tab + (size_t)nblocks * 256;  // ngroups x 256 words behind the table (n/4 + n/1024 bytes of the 4n)
     k_dc_scan_groups<<<ngroups, 256, 0, ctx->stream>>>(tab, nblocks, group_last);
@@ -1333,102 +1409,39 @@ int dc_device(dark_bwt_ctx* ctx, const u8* d_bwt, u64 n64, DcBuffers* io, dark_b
     LAUNCHED();
     k_sparse_scan<<<1, 1024, 0, ctx->stream>>>(run_counts, nblocks);  // in place: exclusive run offsets
     LAUNCHED();
-    u32* alpha = ctx->bucket_hist + 512;  // 513 words: dense codes of the symbols that occur
+    u32* alpha = ctx->bucket_hist + 512;  // 513 words: dense codes of the symbols that occur (in any block)
     k_dc_alphabet<<<1, 256, 0, ctx->stream>>>(first, alpha);
     LAUNCHED();
-    k_dc_ranks<false><<<(u32)ceil_div(nblocks, 8), 256, 0, ctx->stream>>>(d_bwt, n, tab, group_last, run_counts, nblocks, alpha, io->dist, run_start,
-                                                                         io->item_sym, io->item_rank, none);
-    LAUNCHED();
-    k_dc_final<<<1, 256, 0, ctx->stream>>>(n, final_last, first, io->dist, total_runs, ctx->dc_info);
-    LAUNCHED();
-    k_dc_stream<false><<<(u32)std::min<u64>(ceil_div(n, 256), (u64)ctx->num_sms * 16), 256, 0, ctx->stream>>>(run_start, total_runs, n, io->dist,
-                                                                                                              io->item_pos, io->item_dist, none);
-    LAUNCHED();
-    CK(cudaEventRecord(eb, ctx->stream));
-    static_assert(offsetof(dark_bwt_dc_info, num_items) == offsetof(DcInfoDev, num_items), "DcInfoDev mirrors the head of dark_bwt_dc_info");
-    CK(cudaMemcpyAsync(info, ctx->dc_info, sizeof(DcInfoDev), cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    cudaEventElapsedTime(&info->device_ms, ea, eb);
-    return DARK_BWT_OK;
-}
-
-// The per-block records of dc_many_device are staged in the sort's second key buffer (8 N + 1 KiB bytes), which distance
-// coding leaves free: count * sizeof(DcRecDev) <= 8 * capacity + 1024.
-bool dc_many_records_fit(const dark_bwt_ctx* ctx, u64 count) {
-    return count * sizeof(DcRecDev) <= ctx->capacity * 8 + 1024;
-}
-
-// Distance coding of `count` BWT blocks back to back in d_bwt (n bytes in all), in one pass.  ctx->many_starts holds the
-// offsets [0..count] and the caller has checked them (each block >= 1 byte, n <= capacity, the records fit).  Outputs in
-// `io` are nullable like dc_device's; item_starts (count + 1 words) likewise.  infos[0..count) and *item_starts_host
-// (count + 1 words) are filled on the host.
-struct DcManyBuffers {
-    DcBuffers dc;
-    u32* item_starts = nullptr;
-};
-int dc_many_device(dark_bwt_ctx* ctx, const u8* d_bwt, u32 n, u32 count, DcManyBuffers* io, dark_bwt_dc_info* infos,
-                   std::vector<u32>* item_starts_host) {
-    const u32 nblocks = (u32)ceil_div(n, kDcBlock);
-    u32* tab = ctx->ranks;
-    if (n <= 65536u) {  // as in dc_device: tiny totals borrow the status buffer
-        tab = (u32*)ctx->sort_status;
-        for (int h = 0; h < 2; ++h) ctx->status_dirty_lo[h] = 0u, ctx->status_dirty_hi[h] = (u32)(ctx->sort_status_bytes / 2 / (kRadix * sizeof(u32)));
+    const u32 rgrid = (u32)ceil_div(nblocks, 8);
+    DC_LAUNCH(k_dc_ranks, rgrid, d_bwt, n, tab, group_last, run_counts, nblocks, alpha, io->dist, run_start, io->item_sym, io->item_rank);
+    if (!blocks) {  // many blocks: k_dc_ranks finalises each block at its end
+        k_dc_final<<<1, 256, 0, ctx->stream>>>(n, final_last, first, io->dist, total_runs, ctx->dc_info);
+        LAUNCHED();
     }
-    u32* run_counts = ctx->ranks_alt;
-    u32* first = ctx->bucket_hist;
-    u32* final_last = ctx->bucket_hist + 256;
-    DcBuffers& b = io->dc;
-    if (!b.dist) b.dist = (u32*)ctx->keys[0];
-    if (!b.item_pos) b.item_pos = ctx->isa;
-    if (!b.item_dist) b.item_dist = ctx->sa;
-    u32* run_start = ctx->ids[0];
-    if (!b.item_sym) b.item_sym = (u8*)ctx->ids[1];
-    if (!b.item_rank) b.item_rank = (u8*)ctx->ids[1] + (size_t)n;
-    // behind the run counts (4 N + 16 bytes): align4(nblocks) + count + 1 words fit, as the records bound count to capacity / 160
-    if (!io->item_starts) io->item_starts = ctx->ranks_alt + align_up(nblocks, 4);
-    DcRecDev* recs = (DcRecDev*)ctx->keys[1];
-    unsigned long long* total_runs = (unsigned long long*)((char*)ctx->dc_info + align_up(sizeof(DcInfoDev), 8));
-    DcMany many{ctx->many_starts, count, ctx->bitmap, recs, io->item_starts};
-    cudaEvent_t ea = ctx->events[kMaxEvents - 1], eb = ctx->events[kMaxEvents - 2];
-    CK(cudaEventRecord(ea, ctx->stream));
-    CK(cudaMemsetAsync(first, 0xFF, sizeof(u32) * 256, ctx->stream));
-    CK(cudaMemsetAsync(total_runs, 0, sizeof(unsigned long long), ctx->stream));
-    CK(cudaMemsetAsync(ctx->bitmap, 0, sizeof(u32) * ceil_div(n, 32), ctx->stream));
-    k_dc_mark_starts<<<(u32)ceil_div(count, 256), 256, 0, ctx->stream>>>(ctx->many_starts, count, ctx->bitmap, io->item_starts);
-    LAUNCHED();
-    k_dc_tables<true><<<nblocks, 256, 0, ctx->stream>>>(d_bwt, n, tab, first, run_counts, b.dist, total_runs, many);
-    LAUNCHED();
-    const u32 ngroups = (u32)ceil_div(nblocks, kDcGroup);
-    u32* group_last = tab + (size_t)nblocks * 256;
-    k_dc_scan_groups<<<ngroups, 256, 0, ctx->stream>>>(tab, nblocks, group_last);
-    LAUNCHED();
-    k_dc_scan_carry<<<1, 256, 0, ctx->stream>>>(group_last, ngroups, final_last);
-    LAUNCHED();
-    k_sparse_scan<<<1, 1024, 0, ctx->stream>>>(run_counts, nblocks);
-    LAUNCHED();
-    u32* alpha = ctx->bucket_hist + 512;  // dense codes over the union of the blocks' alphabets
-    k_dc_alphabet<<<1, 256, 0, ctx->stream>>>(first, alpha);
-    LAUNCHED();
-    k_dc_ranks<true><<<(u32)ceil_div(nblocks, 8), 256, 0, ctx->stream>>>(d_bwt, n, tab, group_last, run_counts, nblocks, alpha, b.dist, run_start,
-                                                                        b.item_sym, b.item_rank, many);
-    LAUNCHED();
-    k_dc_stream<true><<<(u32)std::min<u64>(ceil_div(n, 256), (u64)ctx->num_sms * 16), 256, 0, ctx->stream>>>(run_start, total_runs, n, b.dist,
-                                                                                                             b.item_pos, b.item_dist, many);
-    LAUNCHED();
-    CK(cudaEventRecord(eb, ctx->stream));
-    std::vector<DcRecDev> recs_host(count);
-    item_starts_host->resize((size_t)count + 1);
-    CK(cudaMemcpyAsync(recs_host.data(), recs, sizeof(DcRecDev) * count, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(item_starts_host->data(), io->item_starts, sizeof(u32) * ((size_t)count + 1), cudaMemcpyDeviceToHost, ctx->stream));
+    const u32 sgrid = (u32)std::min<u64>(ceil_div(n, 256), (u64)ctx->num_sms * 16);
+    DC_LAUNCH(k_dc_stream, sgrid, run_start, total_runs, n, io->dist, io->item_pos, io->item_dist);
+#undef DC_LAUNCH
+    CK(cudaEventRecord(ctx->call_stop, ctx->stream));
+    if (!blocks) {
+        static_assert(offsetof(dark_bwt_dc_info, num_items) == offsetof(DcInfoDev, num_items), "DcInfoDev mirrors the head of dark_bwt_dc_info");
+        CK(cudaMemcpyAsync(infos, ctx->dc_info, sizeof(DcInfoDev), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        infos->device_ms = call_ms(ctx);
+        return DARK_BWT_OK;
+    }
+    const u32 count = many.count;
+    std::vector<DcRecDev> recs(count);
+    std::vector<u32>& hs = io->item_starts_host;
+    hs.resize((size_t)count + 1);
+    CK(cudaMemcpyAsync(recs.data(), many.recs, sizeof(DcRecDev) * count, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(hs.data(), io->item_starts, sizeof(u32) * ((size_t)count + 1), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, ea, eb);
-    const std::vector<u32>& hs = *item_starts_host;
+    const float ms = call_ms(ctx);
     for (u32 k = 0; k < count; ++k) {
         dark_bwt_dc_info& info = infos[k];
-        for (int c = 0; c < 256; ++c) info.init[c] = recs_host[k].init[c];
-        memcpy(info.mtf_symbols, recs_host[k].mtf_symbols, 256);
-        info.num_unique = recs_host[k].num_unique;
+        for (int c = 0; c < 256; ++c) info.init[c] = recs[k].init[c];
+        memcpy(info.mtf_symbols, recs[k].mtf_symbols, 256);
+        info.num_unique = recs[k].num_unique;
         info.reserved_ = 0;
         info.num_items = hs[k + 1] - hs[k];
         info.device_ms = ms;
@@ -1710,7 +1723,7 @@ int dark_bwt_create_ex(uint64_t max_n, int device, uint32_t flags, dark_bwt_ctx*
     const size_t o_hist = carve(sizeof(u32) * kMaxPasses * kRadix);
     const size_t o_present = carve(sizeof(u32) * 256);
     const size_t o_lut = carve(256);
-    const size_t o_scalars = carve(sizeof(DeviceScalars));
+    const size_t o_bad = carve(sizeof(unsigned long long));
     const size_t o_status = carve(ctx->sort_status_bytes);
     const size_t o_counters = carve(sizeof(u32) * kMaxCounters);
     const size_t o_bhist = carve(sizeof(u32) * 1280);  // 256 bucket counters/cursors + 257 chunk prefixes; DC: first/last occurrences + dense alphabet
@@ -1747,7 +1760,7 @@ int dark_bwt_create_ex(uint64_t max_n, int device, uint32_t flags, dark_bwt_ctx*
     ctx->hist = (u32*)(base + o_hist);
     ctx->present = (u32*)(base + o_present);
     ctx->lut = (u8*)(base + o_lut);
-    ctx->scalars = (DeviceScalars*)(base + o_scalars);
+    ctx->bad = (unsigned long long*)(base + o_bad);
     ctx->sort_status = base + o_status;
     for (int h = 0; h < 2; ++h) ctx->status_dirty_lo[h] = 0u, ctx->status_dirty_hi[h] = (u32)(ctx->sort_status_bytes / 2 / (kRadix * sizeof(u32)));
     ctx->counters = (u32*)(base + o_counters);
@@ -1777,8 +1790,8 @@ int dark_bwt_create_ex(uint64_t max_n, int device, uint32_t flags, dark_bwt_ctx*
         ctx->events[i] = nullptr;
         if (cudaEventCreate(&ctx->events[i]) != cudaSuccess) return bail(DARK_BWT_E_CUDA);
     }
-    if (cudaMemsetAsync(ctx->scalars, 0, sizeof(DeviceScalars), ctx->stream) != cudaSuccess) return bail(DARK_BWT_E_CUDA);
-    if (cudaStreamSynchronize(ctx->stream) != cudaSuccess) return bail(DARK_BWT_E_CUDA);
+    ctx->call_start = ctx->events[kMaxEvents - 1];
+    ctx->call_stop = ctx->events[kMaxEvents - 2];
     *out = ctx;
     return DARK_BWT_OK;
 }
@@ -1808,43 +1821,50 @@ void dark_bwt_destroy(dark_bwt_ctx* ctx) {
 int dark_bwt_forward_device(dark_bwt_ctx* ctx, const uint8_t* d_text, uint64_t n, uint8_t* d_bwt_out, uint64_t* origin_out,
                             uint32_t* d_sa_out, dark_bwt_stats* stats) {
     if (!ctx || !d_text || !d_bwt_out || !origin_out) return DARK_BWT_E_INVALID_ARG;
+    if (int rc = check_n(ctx, n, 2)) return rc;
     ctx->err[0] = 0;
     if (stats) stats->h2d_ms = 0.f;
-    return forward_device(ctx, d_text, n, d_bwt_out, origin_out, d_sa_out, stats);
+    return forward_device(ctx, d_text, (u32)n, d_bwt_out, origin_out, d_sa_out, stats);
 }
 
-int dark_bwt_forward(dark_bwt_ctx* ctx, const uint8_t* text, uint64_t n, uint8_t* bwt_out, uint64_t* origin_out,
-                     uint32_t* sa_out, dark_bwt_stats* stats) {
-    if (!ctx || !text || !bwt_out || !origin_out) return DARK_BWT_E_INVALID_ARG;
-    ctx->err[0] = 0;
-    if (ctx->flags & DARK_BWT_F_DEVICE_ONLY) return DARK_BWT_E_INVALID_ARG;
-    if (n < 2 || n > ctx->capacity || n > 0xFFFFFFFEull) return DARK_BWT_E_INVALID_N;
+// dark_bwt_forward and dark_bwt_forward_dc after their argument checks: the host text in, the transform, the BWT (bwt_out
+// nullable) and the SA (sa_out nullable) out, h2d_ms and d2h_ms on the host clock.  The BWT stays in ctx->d_bwt.
+static int forward_host(dark_bwt_ctx* ctx, const uint8_t* text, uint64_t n, uint8_t* bwt_out, uint64_t* origin_out, uint32_t* sa_out,
+                        dark_bwt_stats* stats) {
     CK(cudaSetDevice(ctx->device));
     // pinned (or registered) buffers are copied directly, pageable ones through the context's pinned staging lanes
     typedef std::chrono::steady_clock Clock;
     auto ms_since = [](Clock::time_point t0) { return std::chrono::duration<float, std::milli>(Clock::now() - t0).count(); };
     Clock::time_point t0 = Clock::now();
     if (int rc = copy_in_blocking(ctx, ctx->d_text, text, n, ctx->stream)) return rc;
-    const float h2d = ms_since(t0);
-    if (stats) stats->h2d_ms = h2d;
-    int rc = forward_device(ctx, ctx->d_text, n, ctx->d_bwt, origin_out, nullptr, stats);
-    if (rc) return rc;
+    if (stats) stats->h2d_ms = ms_since(t0);
+    if (int rc = forward_device(ctx, ctx->d_text, (u32)n, ctx->d_bwt, origin_out, nullptr, stats)) return rc;
     t0 = Clock::now();
-    if (int rc2 = copy_out_blocking(ctx, bwt_out, ctx->d_bwt, n, ctx->stream)) return rc2;
+    if (bwt_out)
+        if (int rc = copy_out_blocking(ctx, bwt_out, ctx->d_bwt, n, ctx->stream)) return rc;
     if (sa_out)
-        if (int rc2 = copy_out_blocking(ctx, sa_out, ctx->sa, n * sizeof(u32), ctx->stream)) return rc2;
+        if (int rc = copy_out_blocking(ctx, sa_out, ctx->sa, n * sizeof(u32), ctx->stream)) return rc;
     if (stats) stats->d2h_ms = ms_since(t0);
     return DARK_BWT_OK;
+}
+
+int dark_bwt_forward(dark_bwt_ctx* ctx, const uint8_t* text, uint64_t n, uint8_t* bwt_out, uint64_t* origin_out,
+                     uint32_t* sa_out, dark_bwt_stats* stats) {
+    if (!ctx || !text || !bwt_out || !origin_out) return DARK_BWT_E_INVALID_ARG;
+    if (int rc = check_staging(ctx)) return rc;
+    if (int rc = check_n(ctx, n, 2)) return rc;
+    ctx->err[0] = 0;
+    return forward_host(ctx, text, n, bwt_out, origin_out, sa_out, stats);
 }
 
 int dark_bwt_forward_batch(dark_bwt_ctx* ctx, const uint8_t* const* texts, const uint64_t* ns, uint8_t* const* bwt_outs,
                            uint64_t* origins_out, uint32_t* const* sa_outs, uint64_t count, dark_bwt_stats* stats) {
     if (!ctx || !texts || !ns || !bwt_outs || !origins_out) return DARK_BWT_E_INVALID_ARG;
-    if (ctx->flags & DARK_BWT_F_DEVICE_ONLY) return DARK_BWT_E_INVALID_ARG;
+    if (int rc = check_staging(ctx)) return rc;
     ctx->err[0] = 0;
     for (uint64_t k = 0; k < count; ++k) {
         if (!texts[k] || !bwt_outs[k]) return DARK_BWT_E_INVALID_ARG;
-        if (ns[k] < 2 || ns[k] > ctx->capacity || ns[k] > 0xFFFFFFFEull) return DARK_BWT_E_INVALID_N;
+        if (int rc = check_n(ctx, ns[k], 2)) return rc;
     }
     if (count == 0) return DARK_BWT_OK;
     CK(cudaSetDevice(ctx->device));
@@ -1853,7 +1873,7 @@ int dark_bwt_forward_batch(dark_bwt_ctx* ctx, const uint8_t* const* texts, const
     return run_pipelined(ctx, texts, ns, bwt_outs, count, d_text, d_bwt, [&](uint64_t k, const u8* din, u8* dout, SideCopy* side) {
         dark_bwt_stats* st = stats ? stats + k : nullptr;
         if (st) st->h2d_ms = 0.f;
-        const int rc = forward_device(ctx, din, ns[k], dout, origins_out + k, nullptr, st);
+        const int rc = forward_device(ctx, din, (u32)ns[k], dout, origins_out + k, nullptr, st);
         if (rc == 0 && sa_outs && sa_outs[k]) {  // the SA of the block is in the context's single SA buffer
             side->host = sa_outs[k];
             side->dev = ctx->sa;
@@ -1866,11 +1886,11 @@ int dark_bwt_forward_batch(dark_bwt_ctx* ctx, const uint8_t* const* texts, const
 int dark_bwt_inverse_batch(dark_bwt_ctx* ctx, const uint8_t* const* bwts, const uint64_t* ns, const uint64_t* origins,
                            uint8_t* const* text_outs, uint64_t count, float* ms_out) {
     if (!ctx || !bwts || !ns || !origins || !text_outs) return DARK_BWT_E_INVALID_ARG;
-    if (ctx->flags & DARK_BWT_F_DEVICE_ONLY) return DARK_BWT_E_INVALID_ARG;
+    if (int rc = check_staging(ctx)) return rc;
     ctx->err[0] = 0;
     for (uint64_t k = 0; k < count; ++k) {
         if (!bwts[k] || !text_outs[k]) return DARK_BWT_E_INVALID_ARG;
-        if (ns[k] < 1 || ns[k] > ctx->capacity || ns[k] > 0xFFFFFFFEull) return DARK_BWT_E_INVALID_N;
+        if (int rc = check_n(ctx, ns[k], 1)) return rc;
         if (origins[k] >= ns[k]) return DARK_BWT_E_INVALID_ARG;
     }
     if (count == 0) return DARK_BWT_OK;
@@ -1878,64 +1898,42 @@ int dark_bwt_inverse_batch(dark_bwt_ctx* ctx, const uint8_t* const* bwts, const 
     u8* const d_bwt[2] = {ctx->d_bwt, ctx->d_bwt2};
     u8* const d_text[2] = {ctx->d_text, ctx->d_text2};
     return run_pipelined(ctx, bwts, ns, text_outs, count, d_bwt, d_text, [&](uint64_t k, const u8* din, u8* dout, SideCopy*) {
-        return inverse_device(ctx, din, ns[k], origins[k], dout, ms_out ? ms_out + k : nullptr);
+        return inverse_device(ctx, din, (u32)ns[k], (u32)origins[k], dout, ms_out ? ms_out + k : nullptr);
     });
 }
 
-// Offsets of `count` host blocks of at least min_n bytes each that share the arena (sum <= capacity, <= 2^32-2).  `outs`,
-// if given, must have an entry for every block.
-static int many_starts_of(const dark_bwt_ctx* ctx, const uint8_t* const* blocks, uint8_t* const* outs, const uint64_t* ns, uint64_t count,
-                          uint64_t min_n, std::vector<u32>* starts) {
-    starts->resize(count + 1);
-    u64 total = 0;
-    for (uint64_t k = 0; k < count; ++k) {
-        if (!blocks[k] || (outs && !outs[k])) return DARK_BWT_E_INVALID_ARG;
-        if (ns[k] < min_n) return DARK_BWT_E_INVALID_N;
-        (*starts)[k] = (u32)total;
-        total += ns[k];
-        if (total > ctx->capacity || total > 0xFFFFFFFEull) return DARK_BWT_E_INVALID_N;  // the blocks share one arena
-    }
-    (*starts)[count] = (u32)total;
-    return DARK_BWT_OK;
-}
-
-// dark_bwt_forward_many after its argument checks; bwt_outs (and its entries) may be null: the BWTs stay in ctx->d_bwt.
-static int forward_many_host(dark_bwt_ctx* ctx, const uint8_t* const* texts, const uint64_t* ns, uint8_t* const* bwt_outs,
-                             uint64_t* origins_out, uint64_t count, const std::vector<u32>& starts, dark_bwt_stats* stats) {
-    const u64 total = starts[count];
+// dark_bwt_forward_many and dark_bwt_forward_dc_many after their argument checks; bwt_outs (and its entries) may be null: the
+// BWTs stay in ctx->d_bwt, and ctx->many_starts keeps their offsets.
+static int forward_many_host(dark_bwt_ctx* ctx, const uint8_t* const* texts, uint8_t* const* bwt_outs, uint64_t* origins_out,
+                             const BlockList& bl, dark_bwt_stats* stats) {
+    const u32 count = bl.count();
     CK(cudaSetDevice(ctx->device));
-    cudaEvent_t a = ctx->events[kMaxEvents - 1], b = ctx->events[kMaxEvents - 2];
-    CK(cudaEventRecord(a, ctx->stream));
-    CK(cudaMemcpyAsync(ctx->many_starts, starts.data(), sizeof(u32) * (count + 1), cudaMemcpyHostToDevice, ctx->stream));
-    for (uint64_t k = 0; k < count; ++k)
-        CK(cudaMemcpyAsync(ctx->d_text + starts[k], texts[k], ns[k], cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaEventRecord(b, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));  // `starts` may go out of scope only after the copy
-    float h2d = 0.f;
-    cudaEventElapsedTime(&h2d, a, b);
-    if (stats) stats->h2d_ms = h2d;
-    if (int rc = forward_many_device(ctx, ctx->d_text, (u32)total, (u32)count, ctx->d_bwt, nullptr, stats)) return rc;
-    CK(cudaEventRecord(a, ctx->stream));
-    for (uint64_t k = 0; k < count; ++k)
-        if (bwt_outs && bwt_outs[k]) CK(cudaMemcpyAsync(bwt_outs[k], ctx->d_bwt + starts[k], ns[k], cudaMemcpyDeviceToHost, ctx->stream));
-    static_assert(sizeof(unsigned long long) == sizeof(uint64_t), "origins are copied as they are");
-    CK(cudaMemcpyAsync(origins_out, ctx->many_origins, sizeof(uint64_t) * count, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaEventRecord(b, ctx->stream));
+    CK(cudaEventRecord(ctx->call_start, ctx->stream));
+    if (int rc = load_blocks(ctx, bl, texts, ctx->d_text)) return rc;
+    CK(cudaEventRecord(ctx->call_stop, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    if (stats) cudaEventElapsedTime(&stats->d2h_ms, a, b);
+    if (stats) stats->h2d_ms = call_ms(ctx);
+    if (int rc = forward_many_device(ctx, ctx->d_text, bl.total(), count, ctx->d_bwt, nullptr, stats)) return rc;
+    CK(cudaEventRecord(ctx->call_start, ctx->stream));
+    for (u32 k = 0; k < count; ++k)
+        if (bwt_outs && bwt_outs[k])
+            CK(cudaMemcpyAsync(bwt_outs[k], ctx->d_bwt + bl.starts[k], bl.starts[k + 1] - bl.starts[k], cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(origins_out, ctx->many_origins, sizeof(uint64_t) * count, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaEventRecord(ctx->call_stop, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (stats) stats->d2h_ms = call_ms(ctx);
     return DARK_BWT_OK;
 }
 
 int dark_bwt_forward_many(dark_bwt_ctx* ctx, const uint8_t* const* texts, const uint64_t* ns, uint8_t* const* bwt_outs,
                           uint64_t* origins_out, uint64_t count, dark_bwt_stats* stats) {
     if (!ctx || !texts || !ns || !bwt_outs || !origins_out) return DARK_BWT_E_INVALID_ARG;
-    if (ctx->flags & DARK_BWT_F_DEVICE_ONLY) return DARK_BWT_E_INVALID_ARG;
+    if (int rc = check_staging(ctx)) return rc;
     ctx->err[0] = 0;
     if (count == 0) return DARK_BWT_OK;
-    if (count > kMaxManyBlocks) return DARK_BWT_E_INVALID_ARG;
-    std::vector<u32> starts;
-    if (int rc = many_starts_of(ctx, texts, bwt_outs, ns, count, 2, &starts)) return rc;
-    return forward_many_host(ctx, texts, ns, bwt_outs, origins_out, count, starts, stats);
+    BlockList bl;
+    if (int rc = check_blocks(ctx, count, ns, nullptr, nullptr, 2, 0, texts, bwt_outs, &bl)) return rc;
+    return forward_many_host(ctx, texts, bwt_outs, origins_out, bl, stats);
 }
 
 int dark_bwt_forward_many_device(dark_bwt_ctx* ctx, const uint8_t* d_text, const uint32_t* d_starts, uint64_t count,
@@ -1943,19 +1941,11 @@ int dark_bwt_forward_many_device(dark_bwt_ctx* ctx, const uint8_t* d_text, const
     if (!ctx || !d_text || !d_starts || !d_bwt_out || !d_origins_out) return DARK_BWT_E_INVALID_ARG;
     ctx->err[0] = 0;
     if (count == 0) return DARK_BWT_OK;
-    if (count > kMaxManyBlocks) return DARK_BWT_E_INVALID_ARG;
-    CK(cudaSetDevice(ctx->device));
-    std::vector<u32> starts(count + 1);
-    CK(cudaMemcpyAsync(starts.data(), d_starts, sizeof(u32) * (count + 1), cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    if (starts[0] != 0) return DARK_BWT_E_INVALID_ARG;
-    for (uint64_t k = 0; k < count; ++k)
-        if (starts[k + 1] < starts[k] + 2) return DARK_BWT_E_INVALID_N;
-    const u64 total = starts[count];
-    if (total > ctx->capacity || total > 0xFFFFFFFEull) return DARK_BWT_E_INVALID_N;
-    CK(cudaMemcpyAsync(ctx->many_starts, d_starts, sizeof(u32) * (count + 1), cudaMemcpyDeviceToDevice, ctx->stream));
+    BlockList bl;
+    if (int rc = check_blocks(ctx, count, nullptr, d_starts, nullptr, 2, 0, nullptr, nullptr, &bl)) return rc;
+    if (int rc = load_blocks(ctx, bl)) return rc;
     if (stats) stats->h2d_ms = 0.f;
-    if (int rc = forward_many_device(ctx, d_text, (u32)total, (u32)count, d_bwt_out, d_sa_out, stats)) return rc;
+    if (int rc = forward_many_device(ctx, d_text, bl.total(), bl.count(), d_bwt_out, d_sa_out, stats)) return rc;
     CK(cudaMemcpyAsync(d_origins_out, ctx->many_origins, sizeof(uint64_t) * count, cudaMemcpyDeviceToDevice, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     return DARK_BWT_OK;
@@ -1964,49 +1954,37 @@ int dark_bwt_forward_many_device(dark_bwt_ctx* ctx, const uint8_t* d_text, const
 int dark_bwt_inverse_device(dark_bwt_ctx* ctx, const uint8_t* d_bwt, uint64_t n, uint64_t origin, uint8_t* d_text_out,
                             float* ms_out) {
     if (!ctx || !d_bwt || !d_text_out) return DARK_BWT_E_INVALID_ARG;
+    if (int rc = check_n(ctx, n, 1)) return rc;
+    if (origin >= n) return DARK_BWT_E_INVALID_ARG;
     ctx->err[0] = 0;
-    return inverse_device(ctx, d_bwt, n, origin, d_text_out, ms_out);
+    return inverse_device(ctx, d_bwt, (u32)n, (u32)origin, d_text_out, ms_out);
 }
 
 int dark_bwt_inverse(dark_bwt_ctx* ctx, const uint8_t* bwt, uint64_t n, uint64_t origin, uint8_t* text_out) {
     if (!ctx || !bwt || !text_out) return DARK_BWT_E_INVALID_ARG;
-    if (ctx->flags & DARK_BWT_F_DEVICE_ONLY) return DARK_BWT_E_INVALID_ARG;
-    if (n < 1 || n > ctx->capacity || n > 0xFFFFFFFEull) return DARK_BWT_E_INVALID_N;
+    if (int rc = check_staging(ctx)) return rc;
+    if (int rc = check_n(ctx, n, 1)) return rc;
+    if (origin >= n) return DARK_BWT_E_INVALID_ARG;
     ctx->err[0] = 0;
     CK(cudaSetDevice(ctx->device));
     if (int rc = copy_in_blocking(ctx, ctx->d_bwt, bwt, n, ctx->stream)) return rc;
-    if (int rc = inverse_device(ctx, ctx->d_bwt, n, origin, ctx->d_text, nullptr)) return rc;
+    if (int rc = inverse_device(ctx, ctx->d_bwt, (u32)n, (u32)origin, ctx->d_text, nullptr)) return rc;
     return copy_out_blocking(ctx, text_out, ctx->d_text, n, ctx->stream);
 }
 
 int dark_bwt_inverse_many(dark_bwt_ctx* ctx, const uint8_t* const* bwts, const uint64_t* ns, const uint64_t* origins,
                           uint8_t* const* text_outs, uint64_t count, float* ms_out) {
     if (!ctx || !bwts || !ns || !origins || !text_outs) return DARK_BWT_E_INVALID_ARG;
-    if (count > kMaxManyBlocks) return DARK_BWT_E_INVALID_ARG;
-    if (ctx->flags & DARK_BWT_F_DEVICE_ONLY) return DARK_BWT_E_INVALID_ARG;
+    if (int rc = check_staging(ctx)) return rc;
     ctx->err[0] = 0;
     if (count == 0) return DARK_BWT_OK;
-    std::vector<u32> starts(count + 1);
-    u64 total = 0, max_nb = 0;
-    for (uint64_t k = 0; k < count; ++k) {
-        if (!bwts[k] || !text_outs[k]) return DARK_BWT_E_INVALID_ARG;
-        if (ns[k] < 1) return DARK_BWT_E_INVALID_N;
-        if (origins[k] >= ns[k]) return DARK_BWT_E_INVALID_ARG;
-        starts[k] = (u32)total;
-        total += ns[k];
-        max_nb = std::max<u64>(max_nb, ns[k]);
-        if (total + k + 1 > ctx->capacity) return DARK_BWT_E_INVALID_N;  // the rows (bytes + one '$' row per block) share the arena
-    }
-    starts[count] = (u32)total;
+    BlockList bl;
+    if (int rc = check_blocks(ctx, count, ns, nullptr, origins, 1, 1, bwts, text_outs, &bl)) return rc;
     CK(cudaSetDevice(ctx->device));
-    static_assert(sizeof(unsigned long long) == sizeof(uint64_t), "origins are copied as they are");
-    CK(cudaMemcpyAsync(ctx->many_starts, starts.data(), sizeof(u32) * (count + 1), cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(ctx->many_origins, origins, sizeof(uint64_t) * count, cudaMemcpyHostToDevice, ctx->stream));
+    if (int rc = load_blocks(ctx, bl, bwts, ctx->d_bwt)) return rc;
+    if (int rc = inverse_many_device(ctx, ctx->d_bwt, bl.total(), bl.count(), (u32)bl.max_nb, ctx->d_text, ms_out)) return rc;
     for (uint64_t k = 0; k < count; ++k)
-        CK(cudaMemcpyAsync(ctx->d_bwt + starts[k], bwts[k], ns[k], cudaMemcpyHostToDevice, ctx->stream));
-    if (int rc = inverse_many_device(ctx, ctx->d_bwt, (u32)total, (u32)count, (u32)max_nb, ctx->d_text, ms_out)) return rc;
-    for (uint64_t k = 0; k < count; ++k)
-        CK(cudaMemcpyAsync(text_outs[k], ctx->d_text + starts[k], ns[k], cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaMemcpyAsync(text_outs[k], ctx->d_text + bl.starts[k], ns[k], cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     return DARK_BWT_OK;
 }
@@ -2014,54 +1992,20 @@ int dark_bwt_inverse_many(dark_bwt_ctx* ctx, const uint8_t* const* bwts, const u
 int dark_bwt_inverse_many_device(dark_bwt_ctx* ctx, const uint8_t* d_bwt, const uint32_t* d_starts, const uint64_t* d_origins,
                                  uint64_t count, uint8_t* d_text_out, float* ms_out) {
     if (!ctx || !d_bwt || !d_starts || !d_origins || !d_text_out) return DARK_BWT_E_INVALID_ARG;
-    if (count > kMaxManyBlocks) return DARK_BWT_E_INVALID_ARG;
     ctx->err[0] = 0;
     if (count == 0) return DARK_BWT_OK;
-    CK(cudaSetDevice(ctx->device));
-    // offsets and origins are checked on the host before any kernel reads them
-    std::vector<u32> starts(count + 1);
-    std::vector<uint64_t> origins(count);
-    CK(cudaMemcpyAsync(starts.data(), d_starts, sizeof(u32) * (count + 1), cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(origins.data(), d_origins, sizeof(uint64_t) * count, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    if (starts[0] != 0) return DARK_BWT_E_INVALID_ARG;
-    u64 max_nb = 0;
-    for (uint64_t k = 0; k < count; ++k) {
-        if ((u64)starts[k + 1] < (u64)starts[k] + 1) return DARK_BWT_E_INVALID_N;
-        const u64 nb = (u64)starts[k + 1] - starts[k];
-        if (origins[k] >= nb) return DARK_BWT_E_INVALID_ARG;
-        max_nb = std::max(max_nb, nb);
-    }
-    const u64 total = starts[count];
-    if (total + count > ctx->capacity) return DARK_BWT_E_INVALID_N;
-    CK(cudaMemcpyAsync(ctx->many_starts, d_starts, sizeof(u32) * (count + 1), cudaMemcpyDeviceToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(ctx->many_origins, d_origins, sizeof(uint64_t) * count, cudaMemcpyDeviceToDevice, ctx->stream));
-    return inverse_many_device(ctx, d_bwt, (u32)total, (u32)count, (u32)max_nb, d_text_out, ms_out);
+    BlockList bl;
+    if (int rc = check_blocks(ctx, count, nullptr, d_starts, d_origins, 1, 1, nullptr, nullptr, &bl)) return rc;
+    if (int rc = load_blocks(ctx, bl)) return rc;
+    return inverse_many_device(ctx, d_bwt, bl.total(), bl.count(), (u32)bl.max_nb, d_text_out, ms_out);
 }
 
-int dark_bwt_dc_encode_device(dark_bwt_ctx* ctx, const uint8_t* d_bwt, uint64_t n, uint32_t* d_dist_out, uint32_t* d_item_pos,
-                              uint32_t* d_item_dist, uint8_t* d_item_sym, uint8_t* d_item_rank, dark_bwt_dc_info* info) {
-    if (!ctx || !d_bwt || !info) return DARK_BWT_E_INVALID_ARG;
-    ctx->err[0] = 0;
-    DcBuffers io;
-    io.dist = d_dist_out;
-    io.item_pos = d_item_pos;
-    io.item_dist = d_item_dist;
-    io.item_sym = d_item_sym;
-    io.item_rank = d_item_rank;
-    return dc_device(ctx, d_bwt, n, &io, info);
-}
-
-// host buffers; ctx->d_bwt already holds the block when `bwt` is null (dark_bwt_forward_dc)
-static int dc_host(dark_bwt_ctx* ctx, const uint8_t* bwt, uint64_t n, uint32_t* dist_out, uint32_t* item_pos, uint32_t* item_dist,
-                   uint8_t* item_sym, uint8_t* item_rank, dark_bwt_dc_info* info) {
-    if (bwt)
-        if (int rc = copy_in_blocking(ctx, ctx->d_bwt, bwt, n, ctx->stream)) return rc;
-    DcBuffers io;
-    if (int rc = dc_device(ctx, ctx->d_bwt, n, &io, info)) return rc;
-    const size_t items = (size_t)info->num_items;
+// Host copies of what dc_device left in `io`, one copy per array (`items` runs in all); null host pointers are skipped.
+static int dc_copy_out(dark_bwt_ctx* ctx, u64 n, u64 items, const DcBuffers& io, uint32_t* dist_out, uint32_t* item_starts,
+                       uint32_t* item_pos, uint32_t* item_dist, uint8_t* item_sym, uint8_t* item_rank) {
     if (dist_out)
         if (int rc = copy_out_blocking(ctx, dist_out, io.dist, n * sizeof(u32), ctx->stream)) return rc;
+    if (item_starts) memcpy(item_starts, io.item_starts_host.data(), io.item_starts_host.size() * sizeof(u32));
     if (item_pos && items)
         if (int rc = copy_out_blocking(ctx, item_pos, io.item_pos, items * sizeof(u32), ctx->stream)) return rc;
     if (item_dist && items)
@@ -2073,79 +2017,65 @@ static int dc_host(dark_bwt_ctx* ctx, const uint8_t* bwt, uint64_t n, uint32_t* 
     return DARK_BWT_OK;
 }
 
+int dark_bwt_dc_encode_device(dark_bwt_ctx* ctx, const uint8_t* d_bwt, uint64_t n, uint32_t* d_dist_out, uint32_t* d_item_pos,
+                              uint32_t* d_item_dist, uint8_t* d_item_sym, uint8_t* d_item_rank, dark_bwt_dc_info* info) {
+    if (!ctx || !d_bwt || !info) return DARK_BWT_E_INVALID_ARG;
+    if (int rc = check_n(ctx, n, 1)) return rc;
+    ctx->err[0] = 0;
+    DcBuffers io;
+    io.dist = d_dist_out;
+    io.item_pos = d_item_pos;
+    io.item_dist = d_item_dist;
+    io.item_sym = d_item_sym;
+    io.item_rank = d_item_rank;
+    return dc_device(ctx, d_bwt, (u32)n, nullptr, &io, info);
+}
+
 int dark_bwt_dc_encode(dark_bwt_ctx* ctx, const uint8_t* bwt, uint64_t n, uint32_t* dist_out, uint32_t* item_pos, uint32_t* item_dist,
                        uint8_t* item_sym, uint8_t* item_rank, dark_bwt_dc_info* info) {
     if (!ctx || !bwt || !info) return DARK_BWT_E_INVALID_ARG;
-    if (ctx->flags & DARK_BWT_F_DEVICE_ONLY) return DARK_BWT_E_INVALID_ARG;
-    if (n < 1 || n > ctx->capacity || n > 0xFFFFFFFEull) return DARK_BWT_E_INVALID_N;
+    if (int rc = check_staging(ctx)) return rc;
+    if (int rc = check_n(ctx, n, 1)) return rc;
     ctx->err[0] = 0;
     CK(cudaSetDevice(ctx->device));
-    return dc_host(ctx, bwt, n, dist_out, item_pos, item_dist, item_sym, item_rank, info);
+    if (int rc = copy_in_blocking(ctx, ctx->d_bwt, bwt, n, ctx->stream)) return rc;
+    DcBuffers io;
+    if (int rc = dc_device(ctx, ctx->d_bwt, (u32)n, nullptr, &io, info)) return rc;
+    return dc_copy_out(ctx, n, info->num_items, io, dist_out, nullptr, item_pos, item_dist, item_sym, item_rank);
 }
 
 int dark_bwt_forward_dc(dark_bwt_ctx* ctx, const uint8_t* text, uint64_t n, uint8_t* bwt_out, uint64_t* origin_out, uint32_t* dist_out,
                         uint32_t* item_pos, uint32_t* item_dist, uint8_t* item_sym, uint8_t* item_rank, dark_bwt_dc_info* info,
                         dark_bwt_stats* stats) {
     if (!ctx || !text || !origin_out || !info) return DARK_BWT_E_INVALID_ARG;
-    if (ctx->flags & DARK_BWT_F_DEVICE_ONLY) return DARK_BWT_E_INVALID_ARG;
-    if (n < 2 || n > ctx->capacity || n > 0xFFFFFFFEull) return DARK_BWT_E_INVALID_N;
+    if (int rc = check_staging(ctx)) return rc;
+    if (int rc = check_n(ctx, n, 2)) return rc;
     ctx->err[0] = 0;
-    CK(cudaSetDevice(ctx->device));
-    if (int rc = copy_in_blocking(ctx, ctx->d_text, text, n, ctx->stream)) return rc;
-    if (stats) stats->h2d_ms = 0.f;
-    if (int rc = forward_device(ctx, ctx->d_text, n, ctx->d_bwt, origin_out, nullptr, stats)) return rc;
-    if (bwt_out)
-        if (int rc = copy_out_blocking(ctx, bwt_out, ctx->d_bwt, n, ctx->stream)) return rc;
+    if (int rc = forward_host(ctx, text, n, bwt_out, origin_out, nullptr, stats)) return rc;
     // the BWT is still in HBM: distance coding reads it there
-    return dc_host(ctx, nullptr, n, dist_out, item_pos, item_dist, item_sym, item_rank, info);
-}
-
-// Host copies of what dc_many_device left in `io` (one copy per array); null host pointers are skipped.
-static int dc_many_copy_out(dark_bwt_ctx* ctx, u64 n, const DcManyBuffers& io, const std::vector<u32>& hs, uint32_t* dist_out,
-                            uint32_t* item_starts, uint32_t* item_pos, uint32_t* item_dist, uint8_t* item_sym, uint8_t* item_rank) {
-    const size_t items = hs.back();
-    if (dist_out)
-        if (int rc = copy_out_blocking(ctx, dist_out, io.dc.dist, n * sizeof(u32), ctx->stream)) return rc;
-    if (item_starts) memcpy(item_starts, hs.data(), hs.size() * sizeof(u32));
-    if (item_pos && items)
-        if (int rc = copy_out_blocking(ctx, item_pos, io.dc.item_pos, items * sizeof(u32), ctx->stream)) return rc;
-    if (item_dist && items)
-        if (int rc = copy_out_blocking(ctx, item_dist, io.dc.item_dist, items * sizeof(u32), ctx->stream)) return rc;
-    if (item_sym && items)
-        if (int rc = copy_out_blocking(ctx, item_sym, io.dc.item_sym, items, ctx->stream)) return rc;
-    if (item_rank && items)
-        if (int rc = copy_out_blocking(ctx, item_rank, io.dc.item_rank, items, ctx->stream)) return rc;
-    return DARK_BWT_OK;
+    DcBuffers io;
+    if (int rc = dc_device(ctx, ctx->d_bwt, (u32)n, nullptr, &io, info)) return rc;
+    return dc_copy_out(ctx, n, info->num_items, io, dist_out, nullptr, item_pos, item_dist, item_sym, item_rank);
 }
 
 int dark_bwt_dc_encode_many_device(dark_bwt_ctx* ctx, const uint8_t* d_bwt, const uint32_t* d_starts, uint64_t count, uint32_t* d_dist_out,
                                    uint32_t* d_item_starts, uint32_t* d_item_pos, uint32_t* d_item_dist, uint8_t* d_item_sym,
                                    uint8_t* d_item_rank, dark_bwt_dc_info* infos, float* ms_out) {
     if (!ctx || !d_bwt || !d_starts || !infos) return DARK_BWT_E_INVALID_ARG;
-    if (count > kMaxManyBlocks) return DARK_BWT_E_INVALID_ARG;
     ctx->err[0] = 0;
     if (count == 0) return DARK_BWT_OK;
+    BlockList bl;
+    if (int rc = check_blocks(ctx, count, nullptr, d_starts, nullptr, 1, 0, nullptr, nullptr, &bl)) return rc;
     if (!dc_many_records_fit(ctx, count)) return DARK_BWT_E_INVALID_N;
-    CK(cudaSetDevice(ctx->device));
-    // the offsets are checked on the host before any kernel reads them
-    std::vector<u32> starts(count + 1);
-    CK(cudaMemcpyAsync(starts.data(), d_starts, sizeof(u32) * (count + 1), cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    if (starts[0] != 0) return DARK_BWT_E_INVALID_ARG;
-    for (uint64_t k = 0; k < count; ++k)
-        if ((u64)starts[k + 1] < (u64)starts[k] + 1) return DARK_BWT_E_INVALID_N;
-    const u64 total = starts[count];
-    if (total > ctx->capacity || total > 0xFFFFFFFEull) return DARK_BWT_E_INVALID_N;
-    CK(cudaMemcpyAsync(ctx->many_starts, d_starts, sizeof(u32) * (count + 1), cudaMemcpyDeviceToDevice, ctx->stream));
-    DcManyBuffers io;
-    io.dc.dist = d_dist_out;
+    if (int rc = load_blocks(ctx, bl)) return rc;
+    DcBuffers io;
+    io.dist = d_dist_out;
     io.item_starts = d_item_starts;
-    io.dc.item_pos = d_item_pos;
-    io.dc.item_dist = d_item_dist;
-    io.dc.item_sym = d_item_sym;
-    io.dc.item_rank = d_item_rank;
-    std::vector<u32> hs;
-    if (int rc = dc_many_device(ctx, d_bwt, (u32)total, (u32)count, &io, infos, &hs)) return rc;
+    io.item_pos = d_item_pos;
+    io.item_dist = d_item_dist;
+    io.item_sym = d_item_sym;
+    io.item_rank = d_item_rank;
+    if (int rc = dc_device(ctx, d_bwt, bl.total(), &bl, &io, infos)) return rc;
     if (ms_out) *ms_out = infos[0].device_ms;
     return DARK_BWT_OK;
 }
@@ -2154,47 +2084,41 @@ int dark_bwt_dc_encode_many(dark_bwt_ctx* ctx, const uint8_t* const* bwts, const
                             uint32_t* item_starts, uint32_t* item_pos, uint32_t* item_dist, uint8_t* item_sym, uint8_t* item_rank,
                             dark_bwt_dc_info* infos, float* ms_out) {
     if (!ctx || !bwts || !ns || !infos) return DARK_BWT_E_INVALID_ARG;
-    if (count > kMaxManyBlocks) return DARK_BWT_E_INVALID_ARG;
-    if (ctx->flags & DARK_BWT_F_DEVICE_ONLY) return DARK_BWT_E_INVALID_ARG;
+    if (int rc = check_staging(ctx)) return rc;
     ctx->err[0] = 0;
     if (count == 0) {
         if (item_starts) item_starts[0] = 0;
         return DARK_BWT_OK;
     }
-    std::vector<u32> starts;
-    if (int rc = many_starts_of(ctx, bwts, nullptr, ns, count, 1, &starts)) return rc;
+    BlockList bl;
+    if (int rc = check_blocks(ctx, count, ns, nullptr, nullptr, 1, 0, bwts, nullptr, &bl)) return rc;
     if (!dc_many_records_fit(ctx, count)) return DARK_BWT_E_INVALID_N;
     CK(cudaSetDevice(ctx->device));
-    CK(cudaMemcpyAsync(ctx->many_starts, starts.data(), sizeof(u32) * (count + 1), cudaMemcpyHostToDevice, ctx->stream));
-    for (uint64_t k = 0; k < count; ++k)
-        CK(cudaMemcpyAsync(ctx->d_bwt + starts[k], bwts[k], ns[k], cudaMemcpyHostToDevice, ctx->stream));
-    DcManyBuffers io;
-    std::vector<u32> hs;
-    if (int rc = dc_many_device(ctx, ctx->d_bwt, starts[count], (u32)count, &io, infos, &hs)) return rc;  // synchronises: `starts` may go
+    if (int rc = load_blocks(ctx, bl, bwts, ctx->d_bwt)) return rc;
+    DcBuffers io;
+    if (int rc = dc_device(ctx, ctx->d_bwt, bl.total(), &bl, &io, infos)) return rc;
     if (ms_out) *ms_out = infos[0].device_ms;
-    return dc_many_copy_out(ctx, starts[count], io, hs, dist_out, item_starts, item_pos, item_dist, item_sym, item_rank);
+    return dc_copy_out(ctx, bl.total(), io.item_starts_host.back(), io, dist_out, item_starts, item_pos, item_dist, item_sym, item_rank);
 }
 
 int dark_bwt_forward_dc_many(dark_bwt_ctx* ctx, const uint8_t* const* texts, const uint64_t* ns, uint64_t count, uint8_t* const* bwt_outs,
                              uint64_t* origins_out, uint32_t* dist_out, uint32_t* item_starts, uint32_t* item_pos, uint32_t* item_dist,
                              uint8_t* item_sym, uint8_t* item_rank, dark_bwt_dc_info* infos, dark_bwt_stats* stats) {
     if (!ctx || !texts || !ns || !origins_out || !infos) return DARK_BWT_E_INVALID_ARG;
-    if (count > kMaxManyBlocks) return DARK_BWT_E_INVALID_ARG;
-    if (ctx->flags & DARK_BWT_F_DEVICE_ONLY) return DARK_BWT_E_INVALID_ARG;
+    if (int rc = check_staging(ctx)) return rc;
     ctx->err[0] = 0;
     if (count == 0) {
         if (item_starts) item_starts[0] = 0;
         return DARK_BWT_OK;
     }
-    std::vector<u32> starts;
-    if (int rc = many_starts_of(ctx, texts, nullptr, ns, count, 2, &starts)) return rc;
+    BlockList bl;
+    if (int rc = check_blocks(ctx, count, ns, nullptr, nullptr, 2, 0, texts, nullptr, &bl)) return rc;
     if (!dc_many_records_fit(ctx, count)) return DARK_BWT_E_INVALID_N;
-    if (int rc = forward_many_host(ctx, texts, ns, bwt_outs, origins_out, count, starts, stats)) return rc;
+    if (int rc = forward_many_host(ctx, texts, bwt_outs, origins_out, bl, stats)) return rc;
     // the BWTs are still in HBM at the same offsets, and ctx->many_starts still holds them
-    DcManyBuffers io;
-    std::vector<u32> hs;
-    if (int rc = dc_many_device(ctx, ctx->d_bwt, starts[count], (u32)count, &io, infos, &hs)) return rc;
-    return dc_many_copy_out(ctx, starts[count], io, hs, dist_out, item_starts, item_pos, item_dist, item_sym, item_rank);
+    DcBuffers io;
+    if (int rc = dc_device(ctx, ctx->d_bwt, bl.total(), &bl, &io, infos)) return rc;
+    return dc_copy_out(ctx, bl.total(), io.item_starts_host.back(), io, dist_out, item_starts, item_pos, item_dist, item_sym, item_rank);
 }
 
 int dark_bwt_reuse(dark_bwt_ctx* ctx, uint32_t** words_out, uint64_t* count_out) {
@@ -2217,18 +2141,12 @@ int dark_bwt_sort_pairs_device(dark_bwt_ctx* ctx, uint64_t* d_keys, uint32_t* d_
                                float* ms_out) {
     if (!ctx || !d_keys || !d_vals || !d_keys_alt || !d_vals_alt || !in_alt_out) return DARK_BWT_E_INVALID_ARG;
     if (begin_bit < 0 || end_bit > 64 || begin_bit >= end_bit) return DARK_BWT_E_INVALID_ARG;
-    if (count == 0 || count > ctx->capacity) return DARK_BWT_E_INVALID_N;
+    if (int rc = check_n(ctx, count, 1)) return rc;
     ctx->err[0] = 0;
-    CK(cudaSetDevice(ctx->device));
     const u32 m = (u32)count;
     const int num_passes = (end_bit - begin_bit + kRadixBits - 1) / kRadixBits;
-    ctx->next_counter = 0;
-    ctx->n_events = 0;
-    ctx->spans.clear();
-    CK(cudaMemsetAsync(ctx->counters, 0, sizeof(u32) * kMaxCounters, ctx->stream));
+    if (int rc = begin_call(ctx)) return rc;
     CK(cudaMemsetAsync(ctx->hist, 0, sizeof(u32) * kMaxPasses * kRadix, ctx->stream));
-    cudaEvent_t a = ctx->events[kMaxEvents - 1], b = ctx->events[kMaxEvents - 2];
-    CK(cudaEventRecord(a, ctx->stream));
     const u32 blocks = (u32)std::min<u64>(ceil_div(m, 256 * 8), 148 * 8);
     k_digit_hist<256><<<blocks, 256, 0, ctx->stream>>>(d_keys, m, begin_bit, num_passes, ctx->hist);
     LAUNCHED();
@@ -2238,9 +2156,9 @@ int dark_bwt_sort_pairs_device(dark_bwt_ctx* ctx, uint64_t* d_keys, uint32_t* d_
     // note: a partial top digit needs no masking as long as the bits above end_bit are equal in
     // all keys or meant to take part; callers pass end_bit = 64 or keys with zero upper bits.
     if (int rc = run_sort(ctx, keys, vals, 0, m, begin_bit, num_passes, &cur, nullptr, 0)) return rc;
-    CK(cudaEventRecord(b, ctx->stream));
+    CK(cudaEventRecord(ctx->call_stop, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    if (ms_out) cudaEventElapsedTime(ms_out, a, b);
+    if (ms_out) *ms_out = call_ms(ctx);
     *in_alt_out = cur;
     return DARK_BWT_OK;
 }
@@ -2248,18 +2166,18 @@ int dark_bwt_sort_pairs_device(dark_bwt_ctx* ctx, uint64_t* d_keys, uint32_t* d_
 int dark_bwt_verify_sa_device(dark_bwt_ctx* ctx, const uint8_t* d_text, uint64_t n64, const uint32_t* d_sa,
                               uint64_t* bad_out) {
     if (!ctx || !d_text || !d_sa || !bad_out) return DARK_BWT_E_INVALID_ARG;
-    if (n64 < 1 || n64 > ctx->capacity) return DARK_BWT_E_INVALID_N;
+    if (int rc = check_n(ctx, n64, 1)) return rc;
     ctx->err[0] = 0;
     CK(cudaSetDevice(ctx->device));
     const u32 n = (u32)n64;
-    CK(cudaMemsetAsync(&ctx->scalars->bad, 0, sizeof(unsigned long long), ctx->stream));
+    CK(cudaMemsetAsync(ctx->bad, 0, sizeof(unsigned long long), ctx->stream));
     CK(cudaMemsetAsync(ctx->isa, 0xFF, sizeof(u32) * (size_t)n, ctx->stream));
     const u32 blocks = (u32)ceil_div(n, 256);
-    k_verify_scatter<256><<<blocks, 256, 0, ctx->stream>>>(d_sa, n, ctx->isa, &ctx->scalars->bad);
+    k_verify_scatter<256><<<blocks, 256, 0, ctx->stream>>>(d_sa, n, ctx->isa, ctx->bad);
     LAUNCHED();
-    k_verify_order<256><<<blocks, 256, 0, ctx->stream>>>(d_text, d_sa, n, ctx->isa, &ctx->scalars->bad);
+    k_verify_order<256><<<blocks, 256, 0, ctx->stream>>>(d_text, d_sa, n, ctx->isa, ctx->bad);
     LAUNCHED();
-    CK(cudaMemcpyAsync(&ctx->mail->bad, &ctx->scalars->bad, sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&ctx->mail->bad, ctx->bad, sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     *bad_out = ctx->mail->bad;
     return DARK_BWT_OK;
@@ -2268,7 +2186,7 @@ int dark_bwt_verify_sa_device(dark_bwt_ctx* ctx, const uint8_t* d_text, uint64_t
 int dark_bwt_lcp_profile_device(dark_bwt_ctx* ctx, const uint8_t* d_text, uint64_t n64, const uint32_t* d_sa, uint64_t* m_out,
                                 uint32_t* rounds_out, uint64_t* max_lcp_out) {
     if (!ctx || !d_text || !d_sa || !m_out || !rounds_out || !max_lcp_out) return DARK_BWT_E_INVALID_ARG;
-    if (n64 < 2 || n64 > ctx->capacity) return DARK_BWT_E_INVALID_N;
+    if (int rc = check_n(ctx, n64, 2)) return rc;
     if (((uintptr_t)d_text) & 7) return DARK_BWT_E_INVALID_ARG;  // 64-bit text loads
     ctx->err[0] = 0;
     CK(cudaSetDevice(ctx->device));
@@ -2300,7 +2218,7 @@ int dark_bwt_lcp_profile_device(dark_bwt_ctx* ctx, const uint8_t* d_text, uint64
 int dark_bwt_emit_device(dark_bwt_ctx* ctx, const uint8_t* d_text, uint64_t n, const uint32_t* d_sa, uint8_t* d_bwt_out,
                          uint64_t* origin_out) {
     if (!ctx || !d_text || !d_sa || !d_bwt_out || !origin_out) return DARK_BWT_E_INVALID_ARG;
-    if (n < 1 || n > ctx->capacity || n > 0xFFFFFFFEull) return DARK_BWT_E_INVALID_N;
+    if (int rc = check_n(ctx, n, 1)) return rc;
     ctx->err[0] = 0;
     CK(cudaSetDevice(ctx->device));
     if (int rc = emit(ctx, d_text, (u32)n, d_sa, d_bwt_out)) return rc;
