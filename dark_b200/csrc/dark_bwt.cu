@@ -56,7 +56,8 @@ struct Mailbox {  // pinned host memory the device results are copied into
     unsigned long long bad;
     u32 flag;  // pairs-mode detector: set when some group has three or more members
     u32 not_pairs;  // the same answer from the check queued behind a re-rank (read with the survivor count)
-    u32 bad_block;  // inverse_many: the lowest block whose list does not cover its rows (with `count` = how many do not)
+    u32 bad_block;  // inverse: the lowest block whose list does not cover its rows (with `count` = how many do not)
+    u32 bad_dist;   // inverse: the rows that block's list covers
 };
 
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
@@ -1100,166 +1101,6 @@ int forward_many_device(dark_bwt_ctx* ctx, const u8* d_text, u32 n, u32 B, u8* d
     return DARK_BWT_OK;
 }
 
-// Inverse BWT on device buffers (kernels and method: suffix_kernels.cuh, "inverse BWT"); 1 <= n <= capacity, origin < n.
-int inverse_device(dark_bwt_ctx* ctx, const u8* d_bwt, u32 n, u32 origin, u8* d_text, float* ms_out) {
-    if (int rc = begin_call(ctx)) return rc;
-    CK(cudaMemsetAsync(ctx->hist, 0, sizeof(u32) * kMaxPasses * kRadix, ctx->stream));
-    // step 1: (last-column symbol, row) pairs; stable partition by symbol -> psi.  The pairs are built inside the
-    // radix pass (GEN mode 1) and their digit histogram is the byte histogram of the BWT.
-    int cur = 0;
-    {
-        k_build_lut<<<1, 256, 0, ctx->stream>>>(ctx->present, ctx->lut, &ctx->mail_dev->sigma, 1);  // identity codes
-        LAUNCHED();
-        u32* gram = ctx->bucket_hist;
-        CK(cudaMemsetAsync(gram, 0, sizeof(u32) * kRadix, ctx->stream));
-        const u32 blocks = (u32)std::min<u64>(ceil_div(n, 256 * 16), (u64)ctx->num_sms * 8);
-        k_gram_hist<256, 8><<<std::max(blocks, 1u), 256, 0, ctx->stream>>>(d_bwt, n, ctx->lut, gram);
-        LAUNCHED();
-        CK(cudaMemcpyAsync(ctx->hist, gram, sizeof(u32) * kRadix, cudaMemcpyDeviceToDevice, ctx->stream));
-        KeyGen gen;
-        gen.text = d_bwt;
-        gen.lut = ctx->lut;
-        gen.n = n;
-        gen.lg_s = 3;
-        gen.mode = 1;
-        gen.origin = origin;
-        bool gen_used = false;
-        if (int rc = run_sort(ctx, ctx->keys, ctx->ids, 0, n, 0, 1, &cur, nullptr, 0, false, nullptr, nullptr, nullptr, &gen, &gen_used)) return rc;
-        if (!gen_used) {  // one-symbol BWT: the pass is the identity and did not run; psi is the row list itself
-            k_ibwt_elements<<<(u32)ceil_div(n, 256), 256, 0, ctx->stream>>>(d_bwt, n, origin, ctx->keys[0], ctx->ids[0]);
-            LAUNCHED();
-            cur = 0;
-        }
-    }
-    const u32* psi1 = ctx->ids[cur];
-    // step 2: sublists between splitters
-    const u32 stride = (u32)ctx->knobs.ibwt_stride;  // rows between splitters; swept 24..128 with the single walk: 48 (profiles/r1_final.md)
-    const u32 head = origin + 1;
-    const u32 regular = (u32)ceil_div((u64)n + 1, stride);
-    const u32 nodes = regular + 1;
-    u32* dist[2] = {ctx->ranks, ctx->sa};
-    u32* next[2] = {ctx->isa, ctx->ids[cur ^ 1]};
-    // one walk: count the sublists and stash their symbols (DARK_BWT_IBWT_TWO_WALKS=1: count, then a second walk writes)
-    u32* len_keep = ctx->ranks_alt;
-    u32* stash = (u32*)ctx->keys[cur ^ 1];  // the sort's other key buffer (8 n + 1024 bytes) is free: nodes * 384 <= 6 n + 768
-    const u32 cap = (u32)std::min<u64>(kIbwtStashCap, (((u64)n * 8 + 1024) / nodes) & ~3ull);  // smaller strides: smaller chunks
-    const bool two_walks = ctx->knobs.ibwt_two_walks || cap < 8;
-    // k_ibwt_walk needs the symbol bases (exclusive digit counts of pass 0, left in ctx->hist by run_sort)
-    if (two_walks)
-        k_ibwt_walk<0><<<(u32)ceil_div(nodes, 128), 128, 0, ctx->stream>>>(psi1, n, head, stride, regular, dist[0], next[0], nullptr, nullptr,
-                                                                         nullptr, nullptr, nullptr, 0u, 0u);
-    else
-        k_ibwt_walk<2><<<(u32)ceil_div(nodes, 128), 128, 0, ctx->stream>>>(psi1, n, head, stride, regular, dist[0], next[0], nullptr, ctx->hist,
-                                                                         nullptr, len_keep, stash, 0u, cap);
-    LAUNCHED();
-    // step 3: suffix sums of the sublist lengths along the splitter list (pointer jumping)
-    int w = 0;
-    for (u32 span = 1; span < nodes; span <<= 1) {
-        k_ibwt_jump<<<(u32)ceil_div(nodes, 256), 256, 0, ctx->stream>>>(dist[w], next[w], dist[w ^ 1], next[w ^ 1], nodes);
-        LAUNCHED();
-        w ^= 1;
-    }
-    k_ibwt_report<<<1, 1, 0, ctx->stream>>>(dist[w], regular, &ctx->mail_dev->count);
-    LAUNCHED();
-    CK(cudaStreamSynchronize(ctx->stream));
-    if ((u64)ctx->mail->count != (u64)n + 1) {
-        snprintf(ctx->err, sizeof(ctx->err), "inverse BWT: (bwt, origin) is not a forward transform (list covers %u of %llu rows)",
-                 ctx->mail->count, (unsigned long long)n + 1);
-        return DARK_BWT_E_INVALID_ARG;
-    }
-    // step 4: the text.  Stashed sublists are copied to their offsets; the few longer ones are walked again.
-    if (two_walks) {
-        k_ibwt_walk<1><<<(u32)ceil_div(nodes, 128), 128, 0, ctx->stream>>>(psi1, n, head, stride, regular, nullptr, nullptr, dist[w], ctx->hist,
-                                                                         d_text, nullptr, nullptr, 0u, 0u);
-        LAUNCHED();
-    } else {
-        k_ibwt_unstash<<<(u32)ceil_div(nodes, 128), 128, 0, ctx->stream>>>(stash, len_keep, dist[w], n, regular, d_text, cap);
-        LAUNCHED();
-        k_ibwt_walk<1><<<(u32)ceil_div(nodes, 128), 128, 0, ctx->stream>>>(psi1, n, head, stride, regular, nullptr, nullptr, dist[w], ctx->hist,
-                                                                         d_text, len_keep, nullptr, cap, 0u);
-        LAUNCHED();
-    }
-    CK(cudaEventRecord(ctx->call_stop, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    if (ms_out) *ms_out = call_ms(ctx);
-    return DARK_BWT_OK;
-}
-
-// Inverse BWT of B blocks in one pass (suffix_kernels.cuh, "inverse BWT of many blocks").  d_bwt holds the blocks back to
-// back (n bytes), ctx->many_starts their offsets and ctx->many_origins their origins (validated, on the device); d_text
-// receives the texts at the same offsets.  max_nb = the largest block.
-//
-// Buffers: the rows number R = n + B <= capacity (the entry points check it).  The sort moves n <= capacity pairs.  The
-// node arrays (dist and next twice, len_keep) hold `regular + B` entries, and regular = ceil(R / stride) <= (R + 1) / 2 with
-// stride >= 2 while every block has at least two rows (B <= R / 2): nodes <= R <= capacity, which the u32 arrays of the
-// arena hold.  The stash gets (8 capacity + 1024) / nodes >= 8 bytes a chunk.  So 65,536 blocks of one byte need a
-// capacity of 131,072 (rows, not bytes, are what must fit), and sum(ns) <= capacity alone would not be enough.
-int inverse_many_device(dark_bwt_ctx* ctx, const u8* d_bwt, u32 n, u32 B, u32 max_nb, u8* d_text, float* ms_out) {
-    if (int rc = begin_call(ctx)) return rc;
-    CK(cudaMemsetAsync(ctx->hist, 0, sizeof(u32) * kMaxPasses * kRadix, ctx->stream));
-    // step 1: (block, last symbol) keys of the real rows, one stable sort -> psi and the first symbols
-    const int passes = 1 + (B > 1 ? (bit_length((u64)B - 1) + kRadixBits - 1) / kRadixBits : 0);
-    const u32 grid = (u32)std::min<u64>(ceil_div(n, 256), (u64)ctx->num_sms * 8);
-    k_ibwt_many_elements<256><<<grid, 256, 0, ctx->stream>>>(d_bwt, n, ctx->many_starts, B, ctx->many_origins, ctx->keys[0], ctx->ids[0],
-                                                             ctx->hist, passes);
-    LAUNCHED();
-    int cur = 0;
-    // passes whose digit is the same in every key are skipped (one-symbol blocks, a single block): the order stays the row order
-    if (int rc = run_sort(ctx, ctx->keys, ctx->ids, 0, n, 0, passes, &cur, nullptr, 0)) return rc;
-    const u32* psi = ctx->ids[cur];
-    const u64* skeys = ctx->keys[cur];
-    // step 2: sublists between splitters (buffers as in inverse_device)
-    const u32 stride = (u32)ctx->knobs.ibwt_stride;
-    const u32 regular = (u32)ceil_div((u64)n + B, stride);
-    const u32 nodes = regular + B;
-    u32* dist[2] = {ctx->ranks, ctx->sa};
-    u32* next[2] = {ctx->isa, ctx->ids[cur ^ 1]};
-    u32* len_keep = ctx->ranks_alt;
-    u32* stash = (u32*)ctx->keys[cur ^ 1];
-    const u32 cap = (u32)std::min<u64>(kIbwtStashCap, ((ctx->capacity * 8 + 1024) / nodes) & ~3ull);
-    const bool two_walks = ctx->knobs.ibwt_two_walks || cap < 8;
-    const u32 wgrid = (u32)ceil_div(nodes, 128);
-    if (two_walks)
-        k_ibwt_many_walk<0><<<wgrid, 128, 0, ctx->stream>>>(psi, skeys, ctx->many_starts, B, ctx->many_origins, stride, regular, dist[0], next[0],
-                                                            nullptr, nullptr, nullptr, nullptr, 0u, 0u);
-    else
-        k_ibwt_many_walk<2><<<wgrid, 128, 0, ctx->stream>>>(psi, skeys, ctx->many_starts, B, ctx->many_origins, stride, regular, dist[0], next[0],
-                                                            nullptr, nullptr, len_keep, stash, 0u, cap);
-    LAUNCHED();
-    // step 3: pointer jumping; a block's list holds at most ceil((max_nb + 1) / stride) + 1 splitters
-    const u64 chain = ceil_div((u64)max_nb + 1, stride) + 1;
-    int w = 0;
-    for (u64 span = 1; span < chain; span <<= 1) {
-        k_ibwt_jump<<<(u32)ceil_div(nodes, 256), 256, 0, ctx->stream>>>(dist[w], next[w], dist[w ^ 1], next[w ^ 1], nodes);
-        LAUNCHED();
-        w ^= 1;
-    }
-    k_ibwt_many_check<<<1, 1024, 0, ctx->stream>>>(dist[w], regular, ctx->many_starts, B, &ctx->mail_dev->count, &ctx->mail_dev->bad_block);
-    LAUNCHED();
-    CK(cudaStreamSynchronize(ctx->stream));
-    if (ctx->mail->count != 0) {
-        snprintf(ctx->err, sizeof(ctx->err), "inverse BWT: block %u is not a forward transform (%u of %u blocks are not)",
-                 ctx->mail->bad_block, ctx->mail->count, B);
-        return DARK_BWT_E_INVALID_ARG;
-    }
-    // step 4: the texts
-    if (two_walks) {
-        k_ibwt_many_walk<1><<<wgrid, 128, 0, ctx->stream>>>(psi, skeys, ctx->many_starts, B, ctx->many_origins, stride, regular, nullptr, nullptr,
-                                                            dist[w], d_text, nullptr, nullptr, 0u, 0u);
-        LAUNCHED();
-    } else {
-        k_ibwt_many_unstash<<<wgrid, 128, 0, ctx->stream>>>(stash, len_keep, dist[w], ctx->many_starts, B, stride, regular, d_text, cap);
-        LAUNCHED();
-        k_ibwt_many_walk<1><<<wgrid, 128, 0, ctx->stream>>>(psi, skeys, ctx->many_starts, B, ctx->many_origins, stride, regular, nullptr, nullptr,
-                                                            dist[w], d_text, len_keep, nullptr, cap, 0u);
-        LAUNCHED();
-    }
-    CK(cudaEventRecord(ctx->call_stop, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    if (ms_out) *ms_out = call_ms(ctx);
-    return DARK_BWT_OK;
-}
-
 // ---- argument checks of the entry points --------------------------------------------------------
 // The length of a single block: min_n (1 or 2) <= n <= capacity, and n <= 2^32-2 (suffixes and rows are u32).
 int check_n(const dark_bwt_ctx* ctx, u64 n, u64 min_n) {
@@ -1335,6 +1176,124 @@ int load_blocks(dark_bwt_ctx* ctx, const BlockList& bl, const uint8_t* const* in
         for (size_t k = 0; k < count; ++k)
             CK(cudaMemcpyAsync(dst + bl.starts[k], ins[k], bl.starts[k + 1] - bl.starts[k], cudaMemcpyHostToDevice, ctx->stream));
     return 0;
+}
+
+// ---- inverse BWT --------------------------------------------------------------------------------
+// Inverse BWT on device buffers (kernels and method: suffix_kernels.cuh, "inverse BWT") of one block d_bwt[0..n) with origin
+// `origin` (`blocks` null; 1 <= n <= capacity, origin < n), or in one pass of the checked list `blocks`, back to back in d_bwt
+// (n bytes) and loaded into ctx->many_starts and ctx->many_origins ("inverse BWT of many blocks"; `origin` unused).  d_text
+// receives the texts at the same offsets.
+//
+// Buffers: the rows number R = n + B <= capacity (the entry points check it).  The sort moves n <= capacity pairs.  The
+// node arrays (dist and next twice, len_keep) hold `regular + B` entries, and regular = ceil(R / stride) <= (R + 1) / 2 with
+// stride >= 2 while every block has at least two rows (B <= R / 2; one block: regular + 1 <= R): nodes <= R <= capacity,
+// which the u32 arrays of the arena hold.  The stash gets (8 capacity + 1024) / nodes >= 8 bytes a chunk.  So 65,536 blocks
+// of one byte need a capacity of 131,072 (rows, not bytes, are what must fit), and sum(ns) <= capacity alone would not be
+// enough.
+int inverse_device(dark_bwt_ctx* ctx, const u8* d_bwt, u32 n, u32 origin, const BlockList* blocks, u8* d_text, float* ms_out) {
+    if (int rc = begin_call(ctx)) return rc;
+    CK(cudaMemsetAsync(ctx->hist, 0, sizeof(u32) * kMaxPasses * kRadix, ctx->stream));
+    const u32 B = blocks ? blocks->count() : 1u;
+    int cur = 0;
+    IbwtMany many{};  // zero in the single-block instantiations
+    if (!blocks) {
+        // step 1: (last-column symbol, row) pairs; stable partition by symbol -> psi.  The pairs are built inside the
+        // radix pass (GEN mode 1) and their digit histogram is the byte histogram of the BWT.
+        k_build_lut<<<1, 256, 0, ctx->stream>>>(ctx->present, ctx->lut, &ctx->mail_dev->sigma, 1);  // identity codes
+        LAUNCHED();
+        u32* gram = ctx->bucket_hist;
+        CK(cudaMemsetAsync(gram, 0, sizeof(u32) * kRadix, ctx->stream));
+        const u32 grid = (u32)std::min<u64>(ceil_div(n, 256 * 16), (u64)ctx->num_sms * 8);
+        k_gram_hist<256, 8><<<std::max(grid, 1u), 256, 0, ctx->stream>>>(d_bwt, n, ctx->lut, gram);
+        LAUNCHED();
+        CK(cudaMemcpyAsync(ctx->hist, gram, sizeof(u32) * kRadix, cudaMemcpyDeviceToDevice, ctx->stream));
+        KeyGen gen;
+        gen.text = d_bwt;
+        gen.lut = ctx->lut;
+        gen.n = n;
+        gen.lg_s = 3;
+        gen.mode = 1;
+        gen.origin = origin;
+        bool gen_used = false;
+        if (int rc = run_sort(ctx, ctx->keys, ctx->ids, 0, n, 0, 1, &cur, nullptr, 0, false, nullptr, nullptr, nullptr, &gen, &gen_used)) return rc;
+        if (!gen_used) {  // one-symbol BWT: the pass is the identity and did not run; psi is the row list itself
+            k_ibwt_elements<<<(u32)ceil_div(n, 256), 256, 0, ctx->stream>>>(d_bwt, n, origin, ctx->keys[0], ctx->ids[0]);
+            LAUNCHED();
+            cur = 0;
+        }
+        // k_ibwt_walk finds first symbols in the symbol bases (exclusive digit counts of pass 0, left in ctx->hist by run_sort)
+    } else {
+        // step 1: (block, last symbol) keys of the real rows, one stable sort -> psi and the first symbols
+        const int passes = 1 + (B > 1 ? (bit_length((u64)B - 1) + kRadixBits - 1) / kRadixBits : 0);
+        const u32 grid = (u32)std::min<u64>(ceil_div(n, 256), (u64)ctx->num_sms * 8);
+        k_ibwt_many_elements<256><<<grid, 256, 0, ctx->stream>>>(d_bwt, n, ctx->many_starts, B, ctx->many_origins, ctx->keys[0],
+                                                                 ctx->ids[0], ctx->hist, passes);
+        LAUNCHED();
+        // passes whose digit is the same in every key are skipped (one-symbol blocks, a single block): the order stays the row order
+        if (int rc = run_sort(ctx, ctx->keys, ctx->ids, 0, n, 0, passes, &cur, nullptr, 0)) return rc;
+        many = IbwtMany{ctx->many_starts, ctx->many_origins, B, ctx->keys[cur]};
+    }
+    const u32* psi = ctx->ids[cur];
+// Launches a kernel template on MANY: with MANY = true for a block list, false for one block.
+#define IBWT_LAUNCH(...)                                \
+    do {                                                \
+        if (blocks) { constexpr bool MANY = true; __VA_ARGS__; }   \
+        else { constexpr bool MANY = false; __VA_ARGS__; }         \
+        LAUNCHED();                                     \
+    } while (0)
+    // step 2: sublists between splitters
+    const u32 stride = (u32)ctx->knobs.ibwt_stride;  // rows between splitters; swept 24..128 with the single walk: 48 (profiles/r1_final.md)
+    const u32 regular = (u32)ceil_div((u64)n + B, stride);
+    const u32 nodes = regular + B;
+    const u32 grid = (u32)ceil_div(nodes, 128);
+    u32* dist[2] = {ctx->ranks, ctx->sa};
+    u32* next[2] = {ctx->isa, ctx->ids[cur ^ 1]};
+    // one walk: count the sublists and stash their symbols (DARK_BWT_IBWT_TWO_WALKS=1: count, then a second walk writes)
+    u32* len_keep = ctx->ranks_alt;
+    u32* stash = (u32*)ctx->keys[cur ^ 1];  // the sort's other key buffer (8 capacity + 1024 bytes) is free
+    const u32 cap = (u32)std::min<u64>(kIbwtStashCap, ((ctx->capacity * 8 + 1024) / nodes) & ~3ull);  // smaller strides: smaller chunks
+    const bool two_walks = ctx->knobs.ibwt_two_walks || cap < 8;
+    if (two_walks)
+        IBWT_LAUNCH(k_ibwt_walk<0, MANY><<<grid, 128, 0, ctx->stream>>>(psi, n, origin, stride, regular, dist[0], next[0], nullptr, nullptr,
+                                                                       nullptr, nullptr, nullptr, 0u, 0u, many));
+    else
+        IBWT_LAUNCH(k_ibwt_walk<2, MANY><<<grid, 128, 0, ctx->stream>>>(psi, n, origin, stride, regular, dist[0], next[0], nullptr, ctx->hist,
+                                                                       nullptr, len_keep, stash, 0u, cap, many));
+    // step 3: suffix sums of the sublist lengths along the splitter lists (pointer jumping); a list holds at most
+    // ceil((max n_b + 1) / stride) + 1 splitters (one block: all of them)
+    const u64 chain = ceil_div((u64)(blocks ? blocks->max_nb : n) + 1, stride) + 1;
+    int w = 0;
+    for (u64 span = 1; span < chain; span <<= 1) {
+        k_ibwt_jump<<<(u32)ceil_div(nodes, 256), 256, 0, ctx->stream>>>(dist[w], next[w], dist[w ^ 1], next[w ^ 1], nodes);
+        LAUNCHED();
+        w ^= 1;
+    }
+    IBWT_LAUNCH(k_ibwt_check<MANY><<<1, 1024, 0, ctx->stream>>>(dist[w], n, regular, &ctx->mail_dev->count, &ctx->mail_dev->bad_block,
+                                                                &ctx->mail_dev->bad_dist, many));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (ctx->mail->count != 0) {
+        if (blocks)
+            snprintf(ctx->err, sizeof(ctx->err), "inverse BWT: block %u is not a forward transform (%u of %u blocks are not)",
+                     ctx->mail->bad_block, ctx->mail->count, B);
+        else
+            snprintf(ctx->err, sizeof(ctx->err), "inverse BWT: (bwt, origin) is not a forward transform (list covers %u of %llu rows)",
+                     ctx->mail->bad_dist, (unsigned long long)n + 1);
+        return DARK_BWT_E_INVALID_ARG;
+    }
+    // step 4: the text.  Stashed sublists are copied to their offsets; the few longer ones are walked again.
+    if (two_walks) {
+        IBWT_LAUNCH(k_ibwt_walk<1, MANY><<<grid, 128, 0, ctx->stream>>>(psi, n, origin, stride, regular, nullptr, nullptr, dist[w], ctx->hist,
+                                                                       d_text, nullptr, nullptr, 0u, 0u, many));
+    } else {
+        IBWT_LAUNCH(k_ibwt_unstash<MANY><<<grid, 128, 0, ctx->stream>>>(stash, len_keep, dist[w], n, stride, regular, d_text, cap, many));
+        IBWT_LAUNCH(k_ibwt_walk<1, MANY><<<grid, 128, 0, ctx->stream>>>(psi, n, origin, stride, regular, nullptr, nullptr, dist[w], ctx->hist,
+                                                                       d_text, len_keep, nullptr, cap, 0u, many));
+    }
+#undef IBWT_LAUNCH
+    CK(cudaEventRecord(ctx->call_stop, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (ms_out) *ms_out = call_ms(ctx);
+    return DARK_BWT_OK;
 }
 
 // ---- distance coding ----------------------------------------------------------------------------
@@ -1898,7 +1857,7 @@ int dark_bwt_inverse_batch(dark_bwt_ctx* ctx, const uint8_t* const* bwts, const 
     u8* const d_bwt[2] = {ctx->d_bwt, ctx->d_bwt2};
     u8* const d_text[2] = {ctx->d_text, ctx->d_text2};
     return run_pipelined(ctx, bwts, ns, text_outs, count, d_bwt, d_text, [&](uint64_t k, const u8* din, u8* dout, SideCopy*) {
-        return inverse_device(ctx, din, (u32)ns[k], (u32)origins[k], dout, ms_out ? ms_out + k : nullptr);
+        return inverse_device(ctx, din, (u32)ns[k], (u32)origins[k], nullptr, dout, ms_out ? ms_out + k : nullptr);
     });
 }
 
@@ -1957,7 +1916,7 @@ int dark_bwt_inverse_device(dark_bwt_ctx* ctx, const uint8_t* d_bwt, uint64_t n,
     if (int rc = check_n(ctx, n, 1)) return rc;
     if (origin >= n) return DARK_BWT_E_INVALID_ARG;
     ctx->err[0] = 0;
-    return inverse_device(ctx, d_bwt, (u32)n, (u32)origin, d_text_out, ms_out);
+    return inverse_device(ctx, d_bwt, (u32)n, (u32)origin, nullptr, d_text_out, ms_out);
 }
 
 int dark_bwt_inverse(dark_bwt_ctx* ctx, const uint8_t* bwt, uint64_t n, uint64_t origin, uint8_t* text_out) {
@@ -1968,7 +1927,7 @@ int dark_bwt_inverse(dark_bwt_ctx* ctx, const uint8_t* bwt, uint64_t n, uint64_t
     ctx->err[0] = 0;
     CK(cudaSetDevice(ctx->device));
     if (int rc = copy_in_blocking(ctx, ctx->d_bwt, bwt, n, ctx->stream)) return rc;
-    if (int rc = inverse_device(ctx, ctx->d_bwt, (u32)n, (u32)origin, ctx->d_text, nullptr)) return rc;
+    if (int rc = inverse_device(ctx, ctx->d_bwt, (u32)n, (u32)origin, nullptr, ctx->d_text, nullptr)) return rc;
     return copy_out_blocking(ctx, text_out, ctx->d_text, n, ctx->stream);
 }
 
@@ -1982,7 +1941,7 @@ int dark_bwt_inverse_many(dark_bwt_ctx* ctx, const uint8_t* const* bwts, const u
     if (int rc = check_blocks(ctx, count, ns, nullptr, origins, 1, 1, bwts, text_outs, &bl)) return rc;
     CK(cudaSetDevice(ctx->device));
     if (int rc = load_blocks(ctx, bl, bwts, ctx->d_bwt)) return rc;
-    if (int rc = inverse_many_device(ctx, ctx->d_bwt, bl.total(), bl.count(), (u32)bl.max_nb, ctx->d_text, ms_out)) return rc;
+    if (int rc = inverse_device(ctx, ctx->d_bwt, bl.total(), 0, &bl, ctx->d_text, ms_out)) return rc;
     for (uint64_t k = 0; k < count; ++k)
         CK(cudaMemcpyAsync(text_outs[k], ctx->d_text + bl.starts[k], ns[k], cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
@@ -1997,7 +1956,7 @@ int dark_bwt_inverse_many_device(dark_bwt_ctx* ctx, const uint8_t* d_bwt, const 
     BlockList bl;
     if (int rc = check_blocks(ctx, count, nullptr, d_starts, d_origins, 1, 1, nullptr, nullptr, &bl)) return rc;
     if (int rc = load_blocks(ctx, bl)) return rc;
-    return inverse_many_device(ctx, d_bwt, bl.total(), bl.count(), (u32)bl.max_nb, d_text_out, ms_out);
+    return inverse_device(ctx, d_bwt, bl.total(), 0, &bl, d_text_out, ms_out);
 }
 
 // Host copies of what dc_device left in `io`, one copy per array (`items` runs in all); null host pointers are skipped.

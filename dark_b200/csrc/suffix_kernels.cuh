@@ -1413,10 +1413,12 @@ k_emit_bwt_window(const u8* __restrict__ text, u32 n, const u32* __restrict__ sa
 // gives psi: sorted slot q (= row q+1) <- the row whose last symbol it is.  Following psi from row
 // origin+1 spells T forwards: T[i] = first symbol of the i-th row visited.
 //   step 1  k_ibwt_elements: (symbol, row) pairs in row order            -> one radix pass -> psi
-//   step 2  k_ibwt_walk<false>: every STRIDE-th row (and the head) is a splitter; one thread walks from each
+//   step 2  k_ibwt_walk<2>: every STRIDE-th row (and the head) is a splitter; one thread walks from each
 //           splitter to the next: sublist length + successor splitter      (dependent random reads)
 //   step 3  k_ibwt_jump: pointer jumping over the splitter list only        (n/STRIDE nodes)
-//   step 4  k_ibwt_walk<true>: walk again, now writing T at the known offset
+//   check   k_ibwt_check: the list from the head covers all n + 1 rows
+//   step 4  k_ibwt_unstash, k_ibwt_walk<1>: the text at the known offsets
+// The walk, unstash and check kernels serve the many-block form too (MANY = true, "inverse BWT of many blocks" below).
 __global__ void __launch_bounds__(256)
 k_ibwt_elements(const u8* __restrict__ bwt, u32 n, u32 origin, u64* __restrict__ keys, u32* __restrict__ rows) {
     const u64 e = (u64)blockIdx.x * 256 + threadIdx.x;
@@ -1440,28 +1442,74 @@ __device__ __forceinline__ u32 ibwt_first_symbol(const u32* s_base, u32 r) {
     return lo;
 }
 
+// What only the many-block form reads (zero in the single-block instantiations; "inverse BWT of many blocks" below): block b
+// is bytes [starts[b], starts[b+1]) of the BWTs with origin origins[b], and sorted slot q holds the key (b << 8) | symbol.
+struct IbwtMany {
+    const u32* starts;  // count + 1
+    const unsigned long long* origins;
+    u32 count;
+    const u64* sorted_keys;
+};
+
+__device__ __forceinline__ u32 row_block_of(const u32* __restrict__ starts, u32 B, u32 row) {  // largest b with starts[b] + b <= row
+    u32 lo = 0, hi = B - 1;
+    while (lo < hi) {
+        const u32 mid = (lo + hi + 1) >> 1;
+        if (__ldg(starts + mid) + mid <= row) lo = mid;
+        else hi = mid - 1;
+    }
+    return lo;
+}
+__device__ __forceinline__ u32 ibwt_many_block(const u32* __restrict__ starts, u32 B, u32 stride, u32 regular, u32 s) {
+    return s < regular ? row_block_of(starts, B, s * stride) : s - regular;
+}
+
 // MODE 0: count only (sublist length + successor splitter).
 // MODE 1: write the text at the known offset (second walk; with `only_longer_than` > 0 just the sublists longer than that).
 // MODE 2: count AND stash the symbols of the sublist in the splitter's private chunk of `stash` (kIbwtStashCap bytes):
 //         the text offset is not known yet, k_ibwt_unstash copies the chunk once it is.  One walk instead of two —
 //         a walk is n dependent random reads of psi and runs at the memory system's transaction rate (~55 G/s).
+// Splitter s < regular starts at row s * stride, splitter regular + b at the head row of block b.  A block b owns the rows from
+// its '$' row starts[b] + b on, and psi of its row r is at psi[r - b - 1], its sorted slot.  One block (MANY = false) is block
+// 0 of n bytes with origin `origin`: '$' row 0, head row origin + 1, and the first symbol of a row is found in the symbol
+// bases `base` (no second load per step).  Many blocks read it from the sorted key; `n` and `origin` are then unused.
 constexpr u32 kIbwtStashCap = 384;  // bytes per chunk at the default stride: sublists are ~geometric with mean `stride` (48 by default),
                                     // 0.03 % are longer and are walked again (the driver passes min(this, what the buffer allows))
-template <int MODE>
+template <int MODE, bool MANY>
 __global__ void __launch_bounds__(128)
-k_ibwt_walk(const u32* __restrict__ psi1 /* psi[r] for r >= 1 at psi1[r-1] */, u32 n, u32 head, u32 stride, u32 regular,
-            u32* __restrict__ len, u32* __restrict__ next, const u32* __restrict__ dist, const u32* __restrict__ base,
-            u8* __restrict__ text_out, u32* __restrict__ len_keep, u32* __restrict__ stash, u32 only_longer_than, u32 cap) {
+k_ibwt_walk(const u32* __restrict__ psi, u32 n, u32 origin, u32 stride, u32 regular, u32* __restrict__ len, u32* __restrict__ next,
+            const u32* __restrict__ dist, const u32* __restrict__ base, u8* __restrict__ text_out, u32* __restrict__ len_keep,
+            u32* __restrict__ stash, u32 only_longer_than, u32 cap, IbwtMany many) {
     constexpr bool WRITE = MODE == 1, COUNT = MODE != 1, STASH = MODE == 2;
     __shared__ u32 s_base[256];
-    if (!COUNT || STASH) {
-        for (int i = threadIdx.x; i < 256; i += 128) s_base[i] = base[i];
-        __syncthreads();
+    if constexpr (!MANY) {
+        if (!COUNT || STASH) {
+            for (int i = threadIdx.x; i < 256; i += 128) s_base[i] = base[i];
+            __syncthreads();
+        }
     }
     const u32 s = blockIdx.x * 128 + threadIdx.x;
-    if (s > regular) return;  // splitters 0..regular-1 are rows s*stride; splitter `regular` is the head row
+    if (s > regular + (MANY ? many.count - 1 : 0u)) return;
+    u32 b = 0, first = 0, nb = n, head = origin + 1;  // the block of splitter s: bytes [first, first + nb)
+    if constexpr (MANY) {
+        b = ibwt_many_block(many.starts, many.count, stride, regular, s);
+        first = __ldg(many.starts + b);
+        nb = __ldg(many.starts + b + 1) - first;
+        head = first + b + (u32)__ldg(many.origins + b) + 1u;
+    }
+    const u32 dollar = first + b;  // the block's '$' row
+    // the first symbol of row r (not the '$' row)
+    auto first_symbol = [&](u32 r) -> u32 {
+        if constexpr (MANY) {
+            const u64 key = __ldg(many.sorted_keys + (r - b - 1));
+            DARK_ASSERT((u32)(key >> 8) == b);
+            return (u32)(key & 0xFFu);
+        } else {
+            return ibwt_first_symbol(s_base, r);
+        }
+    };
     u32 r = s < regular ? s * stride : head;
-    if (s < regular && r == head) {  // the head row is owned by its own splitter
+    if (s < regular && r == head) {  // the head row is owned by its block's head splitter
         if (COUNT) {
             len[s] = 0;
             next[s] = kIbwtNil;
@@ -1471,7 +1519,7 @@ k_ibwt_walk(const u32* __restrict__ psi1 /* psi[r] for r >= 1 at psi1[r-1] */, u
     }
     if (WRITE && only_longer_than && len_keep[s] <= only_longer_than) return;
     u64 pos = 0;
-    if (WRITE) pos = (u64)(n + 1) - dist[s];  // text position of this splitter's row
+    if (WRITE) pos = (u64)(nb + 1) - dist[s];  // block-relative text position of this splitter's row
     u32 cnt = 0;
     // WRITE: a sublist spells consecutive text positions; the bytes are gathered into aligned 32-bit words and
     // stored once per word (a byte store per step made the writing walk 9.3 ms against 5.2 ms for the counting one)
@@ -1480,9 +1528,12 @@ k_ibwt_walk(const u32* __restrict__ psi1 /* psi[r] for r >= 1 at psi1[r-1] */, u
     u64 wbase = 0;  // text offset of the word being gathered
     u32* const chunk = STASH ? stash + (size_t)s * (cap / 4) : nullptr;  // cap: chunk bytes, a multiple of 4
     do {
-        if (WRITE && r != 0 && pos + cnt < n) {
-            const u64 q = pos + cnt;
-            const u32 sym = ibwt_first_symbol(s_base, r);
+        const u32 nx = r == dollar ? head : __ldg(psi + (r - b - 1));  // issued before the symbol is found, so the two overlap
+        DARK_ASSERT(nx >= dollar && nx <= dollar + nb);
+        if (WRITE && r != dollar && pos + cnt < nb) {
+            const u64 q = (u64)first + pos + cnt;
+            DARK_ASSERT(pos <= nb);
+            const u32 sym = first_symbol(r);
             if (word_stores) {
                 acc |= sym << (8 * (u32)(q & 3));
                 have |= 1u << (u32)(q & 3);
@@ -1501,8 +1552,8 @@ k_ibwt_walk(const u32* __restrict__ psi1 /* psi[r] for r >= 1 at psi1[r-1] */, u
                 text_out[q] = (u8)sym;
             }
         }
-        if (STASH && cnt < cap) {  // byte cnt of the chunk (row 0, the '$' row, leaves a placeholder)
-            const u32 sym = r != 0 ? ibwt_first_symbol(s_base, r) : 0u;
+        if (STASH && cnt < cap) {  // byte cnt of the chunk (the '$' row leaves a placeholder)
+            const u32 sym = r != dollar ? first_symbol(r) : 0u;
             acc |= sym << (8 * (cnt & 3));
             if ((cnt & 3) == 3) {
                 chunk[cnt >> 2] = acc;
@@ -1510,8 +1561,8 @@ k_ibwt_walk(const u32* __restrict__ psi1 /* psi[r] for r >= 1 at psi1[r-1] */, u
             }
         }
         ++cnt;
-        r = r == 0 ? head : __ldg(psi1 + (r - 1));
-    } while (!(r % stride == 0 || r == head) && cnt <= n);  // cnt bound: corrupt input must not hang
+        r = nx;
+    } while (!(r % stride == 0 || r == head) && cnt <= nb);  // cnt bound: corrupt input must not hang
     if (WRITE && have) {  // the last, partial word of the sublist
         for (u32 e = 0; e < 4; ++e)
             if ((have >> e) & 1u) text_out[wbase + e] = (u8)(acc >> (8 * e));
@@ -1520,8 +1571,10 @@ k_ibwt_walk(const u32* __restrict__ psi1 /* psi[r] for r >= 1 at psi1[r-1] */, u
     if (COUNT) {
         len[s] = cnt;
         if (STASH) len_keep[s] = cnt;
-        // the sublist of row 0 ('$', the last node) ends the list: psi[0] wraps to the head
-        next[s] = (s == 0) ? kIbwtNil : (r == head ? regular : r / stride);
+        // Only the '$' row leads to the head, so the walk that reaches it ends its block's list.  This holds for any input:
+        // the rows psi lists are fixed by the origins, and the head row is not among them.  With one block that walk is
+        // the one from splitter 0, the '$' row.
+        next[s] = r == head ? kIbwtNil : r / stride;
     }
 }
 
@@ -1544,21 +1597,26 @@ __device__ __forceinline__ void ibwt_copy_chunk(const u32* __restrict__ src, u8*
     for (; i < L; ++i) dst[i] = byte_at(i);
 }
 
-// Copy every stashed sublist (length <= kIbwtStashCap) to its place in the text.
+// Copy every stashed sublist (length <= cap) to its place in the text.
+template <bool MANY>
 __global__ void __launch_bounds__(128)
-k_ibwt_unstash(const u32* __restrict__ stash, const u32* __restrict__ len_keep, const u32* __restrict__ dist, u32 n, u32 regular,
-               u8* __restrict__ text_out, u32 cap) {
+k_ibwt_unstash(const u32* __restrict__ stash, const u32* __restrict__ len_keep, const u32* __restrict__ dist, u32 n, u32 stride,
+               u32 regular, u8* __restrict__ text_out, u32 cap, IbwtMany many) {
     const u32 s = blockIdx.x * 128 + threadIdx.x;
-    if (s > regular) return;
+    if (s > regular + (MANY ? many.count - 1 : 0u)) return;
     const u32 len = len_keep[s];
     if (len == 0 || len > cap) return;  // longer sublists are written by a second walk
-    const u64 pos = (u64)(n + 1) - dist[s];
-    if (pos >= n) return;
-    const u32 L = (u32)min((u64)len, (u64)n - pos);  // the '$' row's placeholder falls off the end
-    ibwt_copy_chunk(stash + (size_t)s * (cap / 4), text_out + pos, L, (((uintptr_t)text_out) & 3) == 0);
+    u32 first = 0, nb = n;
+    if constexpr (MANY) {
+        const u32 b = ibwt_many_block(many.starts, many.count, stride, regular, s);
+        first = __ldg(many.starts + b);
+        nb = __ldg(many.starts + b + 1) - first;
+    }
+    const u64 pos = (u64)(nb + 1) - dist[s];
+    if (pos >= nb) return;
+    const u32 L = (u32)min((u64)len, (u64)nb - pos);  // the '$' row's placeholder falls off the block's end
+    ibwt_copy_chunk(stash + (size_t)s * (cap / 4), text_out + first + pos, L, (((uintptr_t)text_out) & 3) == 0);
 }
-
-__global__ void k_ibwt_report(const u32* __restrict__ dist, u32 head_splitter, u32* __restrict__ out) { *out = dist[head_splitter]; }
 
 // one pointer-jumping round over the splitter list: suffix sums of the sublist lengths
 __global__ void __launch_bounds__(256)
@@ -1575,6 +1633,38 @@ k_ibwt_jump(const u32* __restrict__ dist_in, const u32* __restrict__ next_in, u3
     }
     dist_out[s] = d;
     next_out[s] = nn;
+}
+
+// Every block's list must cover its n_b + 1 rows: dist[regular + b] == n_b + 1.  *bad_out = the blocks whose list does not,
+// *first_bad_out = the lowest of them and *first_dist_out = the rows its list covers.
+template <bool MANY>
+__global__ void __launch_bounds__(1024)
+k_ibwt_check(const u32* __restrict__ dist, u32 n, u32 regular, u32* __restrict__ bad_out, u32* __restrict__ first_bad_out,
+             u32* __restrict__ first_dist_out, IbwtMany many) {
+    __shared__ u32 s_bad, s_first;
+    if (threadIdx.x == 0) {
+        s_bad = 0;
+        s_first = 0xFFFFFFFFu;
+    }
+    __syncthreads();
+    u32 bad = 0, first = 0xFFFFFFFFu;
+    for (u32 b = threadIdx.x; b < (MANY ? many.count : 1u); b += 1024) {
+        const u64 nb = MANY ? (u64)__ldg(many.starts + b + 1) - __ldg(many.starts + b) : (u64)n;
+        if ((u64)dist[regular + b] != nb + 1) {
+            ++bad;
+            first = min(first, b);
+        }
+    }
+    if (bad) {
+        atomicAdd(&s_bad, bad);
+        atomicMin(&s_first, first);
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        *bad_out = s_bad;
+        *first_bad_out = s_first;
+        *first_dist_out = s_bad ? dist[regular + s_first] : 0u;
+    }
 }
 
 // ---- LCP profile (SURVEY.md 8d / 8f rank 4): the data-defined round structure m_r ------------------------
@@ -1902,24 +1992,12 @@ k_many_emit(const u64* __restrict__ blk, const u32* __restrict__ ids, u32 n, con
 //          the block number): the stable partition of every block at once.  Sorted slot q of block b is row q + b + 1;
 //          the row id stored there is its psi, the key's low byte its first symbol (one index for both loads, no
 //          symbol bases).  psi never leaves a block, whatever the input.
-//   walk   splitters are every stride-th global row plus each block's head row (local row origin_b + 1, splitter
-//          `regular + b`).  A walk finds its block once (binary search over the row offsets) and stops at a
-//          stride-th row or at its own block's head; reaching the head means it came through the '$' row, so that
-//          sublist ends the block's list (nil).  k_ibwt_jump then runs unchanged over the forest of lists.
-//   offset a splitter's text offset is starts[b] + n_b + 1 - dist.
-//   check  every block's list covers its n_b + 1 rows: dist[regular + b] == n_b + 1 (k_ibwt_many_check).
-__device__ __forceinline__ u32 row_block_of(const u32* __restrict__ starts, u32 B, u32 row) {  // largest b with starts[b] + b <= row
-    u32 lo = 0, hi = B - 1;
-    while (lo < hi) {
-        const u32 mid = (lo + hi + 1) >> 1;
-        if (__ldg(starts + mid) + mid <= row) lo = mid;
-        else hi = mid - 1;
-    }
-    return lo;
-}
-__device__ __forceinline__ u32 ibwt_many_block(const u32* __restrict__ starts, u32 B, u32 stride, u32 regular, u32 s) {
-    return s < regular ? row_block_of(starts, B, s * stride) : s - regular;
-}
+//   walk   k_ibwt_walk<MODE, true>: splitters are every stride-th global row plus each block's head row (local row
+//          origin_b + 1, splitter `regular + b`).  A walk finds its block once (binary search over the row offsets) and
+//          stops at a stride-th row or at its own block's head; reaching the head means it came through the '$' row, so
+//          that sublist ends the block's list (nil).  k_ibwt_jump then runs unchanged over the forest of lists.
+//   offset a splitter's text offset is starts[b] + n_b + 1 - dist (k_ibwt_unstash<true>, k_ibwt_walk<1, true>).
+//   check  every block's list covers its n_b + 1 rows: dist[regular + b] == n_b + 1 (k_ibwt_check<true>).
 // (key, row) of every real row, in row order within each block (the sort is stable), and the digit histogram
 template <int THREADS>
 __global__ void __launch_bounds__(THREADS)
@@ -1943,128 +2021,6 @@ k_ibwt_many_elements(const u8* __restrict__ bwt, u32 n, const u32* __restrict__ 
     }
     __syncthreads();
     hist_flush(s_hist, g_hist, num_passes, tid, THREADS);
-}
-// MODE 0 / 1 / 2 as k_ibwt_walk: count / write (with only_longer_than: the sublists the stash could not hold) / count + stash.
-template <int MODE>
-__global__ void __launch_bounds__(128)
-k_ibwt_many_walk(const u32* __restrict__ psi, const u64* __restrict__ sorted_keys, const u32* __restrict__ starts, u32 B,
-                 const unsigned long long* __restrict__ origins, u32 stride, u32 regular, u32* __restrict__ len, u32* __restrict__ next,
-                 const u32* __restrict__ dist, u8* __restrict__ text_out, u32* __restrict__ len_keep, u32* __restrict__ stash,
-                 u32 only_longer_than, u32 cap) {
-    constexpr bool WRITE = MODE == 1, COUNT = MODE != 1, STASH = MODE == 2;
-    const u32 s = blockIdx.x * 128 + threadIdx.x;
-    if (s >= regular + B) return;
-    const u32 b = ibwt_many_block(starts, B, stride, regular, s);
-    const u32 first = __ldg(starts + b), nb = __ldg(starts + b + 1) - first;
-    const u32 dollar = first + b;  // the block's '$' row
-    const u32 head = dollar + (u32)__ldg(origins + b) + 1u;
-    u32 r = s < regular ? s * stride : head;
-    if (s < regular && r == head) {  // the head row is owned by its block's head splitter
-        if (COUNT) {
-            len[s] = 0;
-            next[s] = kIbwtNil;
-            if (STASH) len_keep[s] = 0;
-        }
-        return;
-    }
-    if (WRITE && only_longer_than && len_keep[s] <= only_longer_than) return;
-    u64 pos = 0;
-    if (WRITE) pos = (u64)nb + 1 - dist[s];  // block-relative text position of this splitter's row
-    u32 cnt = 0;
-    const bool word_stores = WRITE && (((uintptr_t)text_out) & 3) == 0;  // word stores as in k_ibwt_walk
-    u32 acc = 0, have = 0;
-    u64 wbase = 0;
-    u32* const chunk = STASH ? stash + (size_t)s * (cap / 4) : nullptr;
-    do {
-        u32 sym = 0, nx = head;  // the '$' row: no symbol, and its successor is the head
-        if (r != dollar) {
-            const u32 q = r - b - 1;  // sorted slot of row r
-            nx = __ldg(psi + q);
-            sym = (u32)(__ldg(sorted_keys + q) & 0xFFu);
-            DARK_ASSERT(nx >= dollar && nx <= dollar + nb && (u32)(__ldg(sorted_keys + q) >> 8) == b);
-        }
-        if (WRITE && r != dollar && pos + cnt < nb) {
-            const u64 q = (u64)first + pos + cnt;
-            DARK_ASSERT(pos <= nb);
-            if (word_stores) {
-                acc |= sym << (8 * (u32)(q & 3));
-                have |= 1u << (u32)(q & 3);
-                wbase = q & ~3ull;
-                if ((q & 3) == 3) {
-                    if (have == 0xFu) {
-                        *reinterpret_cast<u32*>(text_out + (q & ~3ull)) = acc;
-                    } else {
-                        for (u32 e = 0; e < 4; ++e)
-                            if ((have >> e) & 1u) text_out[(q & ~3ull) + e] = (u8)(acc >> (8 * e));
-                    }
-                    acc = 0;
-                    have = 0;
-                }
-            } else {
-                text_out[q] = (u8)sym;
-            }
-        }
-        if (STASH && cnt < cap) {
-            acc |= sym << (8 * (cnt & 3));
-            if ((cnt & 3) == 3) {
-                chunk[cnt >> 2] = acc;
-                acc = 0;
-            }
-        }
-        ++cnt;
-        r = nx;
-    } while (!(r % stride == 0 || r == head) && cnt <= nb);  // cnt bound: belt and braces (psi is a permutation of the block's rows)
-    if (WRITE && have) {
-        for (u32 e = 0; e < 4; ++e)
-            if ((have >> e) & 1u) text_out[wbase + e] = (u8)(acc >> (8 * e));
-    }
-    if (STASH && (cnt & 3) != 0 && cnt < cap) chunk[cnt >> 2] = acc;
-    if (COUNT) {
-        len[s] = cnt;
-        if (STASH) len_keep[s] = cnt;
-        next[s] = r == head ? kIbwtNil : r / stride;  // only the '$' row leads to the head: the list ends here
-    }
-}
-__global__ void __launch_bounds__(128)
-k_ibwt_many_unstash(const u32* __restrict__ stash, const u32* __restrict__ len_keep, const u32* __restrict__ dist,
-                    const u32* __restrict__ starts, u32 B, u32 stride, u32 regular, u8* __restrict__ text_out, u32 cap) {
-    const u32 s = blockIdx.x * 128 + threadIdx.x;
-    if (s >= regular + B) return;
-    const u32 len = len_keep[s];
-    if (len == 0 || len > cap) return;  // longer sublists are written by a second walk
-    const u32 b = ibwt_many_block(starts, B, stride, regular, s);
-    const u32 first = __ldg(starts + b), nb = __ldg(starts + b + 1) - first;
-    const u64 pos = (u64)nb + 1 - dist[s];
-    if (pos >= nb) return;
-    const u32 L = (u32)min((u64)len, (u64)nb - pos);  // the '$' row's placeholder falls off the block's end
-    ibwt_copy_chunk(stash + (size_t)s * (cap / 4), text_out + first + pos, L, (((uintptr_t)text_out) & 3) == 0);
-}
-// every block's list must cover its n_b + 1 rows: *bad_out = blocks that do not, *first_bad_out = the lowest of them
-__global__ void __launch_bounds__(1024)
-k_ibwt_many_check(const u32* __restrict__ dist, u32 regular, const u32* __restrict__ starts, u32 B, u32* __restrict__ bad_out,
-                  u32* __restrict__ first_bad_out) {
-    __shared__ u32 s_bad, s_first;
-    if (threadIdx.x == 0) {
-        s_bad = 0;
-        s_first = 0xFFFFFFFFu;
-    }
-    __syncthreads();
-    u32 bad = 0, first = 0xFFFFFFFFu;
-    for (u32 b = threadIdx.x; b < B; b += 1024) {
-        if ((u64)dist[regular + b] != (u64)__ldg(starts + b + 1) - __ldg(starts + b) + 1) {
-            ++bad;
-            first = min(first, b);
-        }
-    }
-    if (bad) {
-        atomicAdd(&s_bad, bad);
-        atomicMin(&s_first, first);
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        *bad_out = s_bad;
-        *first_bad_out = s_first;
-    }
 }
 
 // ---- verification (independent of the construction kernels) ------------------------------------
