@@ -10,7 +10,7 @@ _lib = None
 MAX_ROUNDS = 40
 
 OK, E_INVALID_N, E_INVALID_ARG, E_CUDA, E_NOMEM, E_INTERNAL = range(6)
-F_DEFAULT, F_NO_ALPHABET_PACKING, F_DEVICE_ONLY = 0, 1, 2
+F_DEFAULT, F_NO_ALPHABET_PACKING, F_DEVICE_ONLY, F_DC_BATCH = 0, 1, 2, 4
 
 # every symbol include/dark_bwt.h declares (tests/test_abi.py checks the .so exports all of them)
 SYMBOLS = [
@@ -19,7 +19,7 @@ SYMBOLS = [
     "dark_bwt_inverse_batch", "dark_bwt_inverse_many", "dark_bwt_inverse_many_device", "dark_bwt_reuse", "dark_bwt_destroy", "dark_bwt_strerror", "dark_bwt_last_error",
     "dark_bwt_stream", "dark_bwt_sort_pairs_device", "dark_bwt_verify_sa_device", "dark_bwt_emit_device", "dark_bwt_lcp_profile_device",
     "dark_bwt_synth", "dark_bwt_dc_encode_device", "dark_bwt_dc_encode", "dark_bwt_forward_dc", "dark_bwt_dc_encode_many",
-    "dark_bwt_dc_encode_many_device", "dark_bwt_forward_dc_many",
+    "dark_bwt_dc_encode_many_device", "dark_bwt_forward_dc_many", "dark_bwt_forward_dc_batch",
 ]
 
 
@@ -119,6 +119,7 @@ def lib():
     L.dark_bwt_dc_encode_many.argtypes = [vp, vp, vp, u64, vp, vp, vp, vp, vp, vp, vp, ctypes.POINTER(ctypes.c_float)]
     L.dark_bwt_dc_encode_many_device.argtypes = [vp, vp, vp, u64, vp, vp, vp, vp, vp, vp, vp, ctypes.POINTER(ctypes.c_float)]
     L.dark_bwt_forward_dc_many.argtypes = [vp, vp, vp, u64, vp, vp, vp, vp, vp, vp, vp, vp, vp, ctypes.POINTER(Stats)]
+    L.dark_bwt_forward_dc_batch.argtypes = [vp, vp, vp, u64, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     _lib = L
     return L
 

@@ -135,6 +135,15 @@ struct HostStage {
     cudaEvent_t slot_done[kMaxLanes][2] = {{nullptr}};  // the DMA out of / into a lane's slot has completed
 };
 
+// One distance-coding output slot of dark_bwt_forward_dc_batch (DARK_BWT_F_DC_BATCH): room for N entries in each array.
+struct DcSlot {
+    u32* dist = nullptr;
+    u32* item_pos = nullptr;
+    u32* item_dist = nullptr;
+    u8* item_sym = nullptr;
+    u8* item_rank = nullptr;
+};
+
 struct dark_bwt_ctx {
     int device = 0;
     Knobs knobs;
@@ -156,6 +165,7 @@ struct dark_bwt_ctx {
     u8* d_bwt = nullptr;
     u8* d_text2 = nullptr;  // second pair for the pipelined batch entry
     u8* d_bwt2 = nullptr;
+    DcSlot dc_slot[2];  // DARK_BWT_F_DC_BATCH: block k of a pipelined DC batch is coded into slot k & 1
     cudaStream_t copy_in = nullptr, copy_out = nullptr;
     cudaEvent_t ev_in[2] = {nullptr, nullptr}, ev_comp[2] = {nullptr, nullptr}, ev_out[2] = {nullptr, nullptr};
     u32* hist = nullptr;
@@ -1528,24 +1538,38 @@ int copy_out_blocking(dark_bwt_ctx* ctx, void* host, const void* dev, size_t byt
     return 0;
 }
 
-// A second copy-out of a block that must be complete before the next block is transformed (its device buffer is single).
-struct SideCopy {
-    void* host = nullptr;
-    const void* dev = nullptr;
-    size_t bytes = 0;
+// The device -> host copies of one block's results, issued in order.  Absent outputs (null host pointers) and empty copies
+// are left out.  `serial`: a source is single-buffered (the next block overwrites it), so the copies must be complete
+// before the next block is transformed.
+struct OutCopies {
+    struct Copy {
+        void* host;
+        const void* dev;
+        size_t bytes;
+    };
+    Copy list[6];  // the most any entry copies: BWT, distances and the four item arrays
+    int count = 0;
+    bool serial = false;
+    void add(void* host, const void* dev, size_t bytes) {
+        if (host && bytes) list[count++] = Copy{host, dev, bytes};
+    }
 };
 
-// The pipelined loop of the batch entries: `count` host blocks ins[k] (ns[k] bytes) -> outs[k] (ns[k] bytes).  While block
-// k is transformed (transform(k, d_in[b], d_out[b], &side), synchronous on the context's stream), block k+1 is copied into
-// the other input buffer and block k-1 out of the other output buffer.  Pinned host buffers ride on the two copy
-// streams; pageable ones (>= 1 MiB) are moved by the staging lanes in a helper thread.
+// The pipelined loop of the batch entries: `count` host blocks ins[k] (ns[k] bytes).  While block k is transformed
+// (transform(k, b, d_in[b], &copies), synchronous on the context's stream; b = k & 1 selects the block's device buffers),
+// block k+1 is copied into the other input buffer and the copies of block k-1 run out of the other buffers.  Pinned host
+// buffers ride on the two copy streams; a list with a pageable buffer of 1 MiB or more is sent one copy after another by a
+// helper thread, the pageable copies through the staging lanes.
 template <typename Transform>
-int run_pipelined(dark_bwt_ctx* ctx, const u8* const* ins, const uint64_t* ns, u8* const* outs, uint64_t count, u8* const d_in[2],
-                  u8* const d_out[2], Transform transform) {
+int run_pipelined(dark_bwt_ctx* ctx, const u8* const* ins, const uint64_t* ns, uint64_t count, u8* const d_in[2], Transform transform) {
     bool comp_recorded[2] = {false, false}, out_recorded[2] = {false, false};
     std::future<int> fin[2], fout;
     auto staged_in = [&](uint64_t k) { return ns[k] >= kStageMinBytes && is_pageable(ins[k]) && stage_prepare(ctx, ctx->stage_in) == 0; };
-    auto staged_out = [&](uint64_t k) { return ns[k] >= kStageMinBytes && is_pageable(outs[k]) && stage_prepare(ctx, ctx->stage_out) == 0; };
+    auto staged_out = [&](const OutCopies& oc) {
+        for (int i = 0; i < oc.count; ++i)
+            if (oc.list[i].bytes >= kStageMinBytes && is_pageable(oc.list[i].host) && stage_prepare(ctx, ctx->stage_out) == 0) return true;
+        return false;
+    };
     auto start_in = [&](uint64_t k, int buf) -> int {  // the transform that read d_in[buf] has returned (it is synchronous)
         if (staged_in(k)) {
             u8* dst = d_in[buf];
@@ -1576,34 +1600,30 @@ int run_pipelined(dark_bwt_ctx* ctx, const u8* const* ins, const uint64_t* ns, u
         }
         if (k + 1 < count)
             if (int rc = start_in(k + 1, nb)) { drain(); return rc; }
-        // (a staged copy-out of block k-1 may still be reading the OTHER output buffer; this one was drained before it began)
-        if (out_recorded[b]) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_out[b], 0));  // output buffer b drained
-        SideCopy side;
-        int rc = transform(k, (const u8*)d_in[b], d_out[b], &side);
+        // (a staged copy-out of block k-1 may still be reading the OTHER buffers; these were drained before it began)
+        if (out_recorded[b]) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_out[b], 0));  // output buffers b drained
+        OutCopies oc;
+        int rc = transform(k, b, (const u8*)d_in[b], &oc);
         if (rc) { drain(); return rc; }
         CK(cudaEventRecord(ctx->ev_comp[b], ctx->stream));
         comp_recorded[b] = true;
         if (fout.valid())
             if (int rc2 = fout.get()) { drain(); return rc2; }  // one staged copy-out at a time (they share the lanes)
-        if (staged_out(k)) {
-            u8* dst = outs[k];
-            const u8* src = d_out[b];
-            const size_t bytes = ns[k];
-            fout = std::async(std::launch::async, [ctx, dst, src, bytes, side] {
-                int r = staged_copy(ctx, ctx->stage_out, (void*)src, dst, bytes, false);
-                if (r == 0 && side.host) r = staged_copy(ctx, ctx->stage_out, (void*)side.dev, side.host, side.bytes, false);
-                return r;
+        if (staged_out(oc)) {
+            fout = std::async(std::launch::async, [ctx, oc] {
+                if (cudaSetDevice(ctx->device) != cudaSuccess) return ctx->fail_cuda(cudaGetLastError(), "helper thread device", __LINE__);
+                for (int i = 0; i < oc.count; ++i)
+                    if (int r = copy_out_blocking(ctx, oc.list[i].host, oc.list[i].dev, oc.list[i].bytes, ctx->copy_out)) return r;
+                return 0;
             });
-            if (side.host)
-                if (int rc2 = fout.get()) { drain(); return rc2; }  // the side buffer is reused by the next block
+            if (oc.serial)
+                if (int rc2 = fout.get()) { drain(); return rc2; }
             out_recorded[b] = false;
         } else {
             CK(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_comp[b], 0));
-            CK(cudaMemcpyAsync(outs[k], d_out[b], ns[k], cudaMemcpyDeviceToHost, ctx->copy_out));
-            if (side.host) {  // the side buffer is reused by the next block: drain it before going on
-                CK(cudaMemcpyAsync(side.host, side.dev, side.bytes, cudaMemcpyDeviceToHost, ctx->copy_out));
-                CK(cudaStreamSynchronize(ctx->copy_out));
-            }
+            for (int i = 0; i < oc.count; ++i)
+                CK(cudaMemcpyAsync(oc.list[i].host, oc.list[i].dev, oc.list[i].bytes, cudaMemcpyDeviceToHost, ctx->copy_out));
+            if (oc.serial) CK(cudaStreamSynchronize(ctx->copy_out));
             CK(cudaEventRecord(ctx->ev_out[b], ctx->copy_out));
             out_recorded[b] = true;
         }
@@ -1644,7 +1664,9 @@ int dark_bwt_create(uint64_t max_n, int device, dark_bwt_ctx** out) {
 int dark_bwt_create_ex(uint64_t max_n, int device, uint32_t flags, dark_bwt_ctx** out) {
     if (!out) return DARK_BWT_E_INVALID_ARG;
     *out = nullptr;
-    if (flags & ~(DARK_BWT_F_NO_ALPHABET_PACKING | DARK_BWT_F_DEVICE_ONLY)) return DARK_BWT_E_INVALID_ARG;
+    if (flags & ~(DARK_BWT_F_NO_ALPHABET_PACKING | DARK_BWT_F_DEVICE_ONLY | DARK_BWT_F_DC_BATCH)) return DARK_BWT_E_INVALID_ARG;
+    // the DC batch is a host-buffer entry: it needs the staging a device-only context does not have
+    if ((flags & DARK_BWT_F_DC_BATCH) && (flags & DARK_BWT_F_DEVICE_ONLY)) return DARK_BWT_E_INVALID_ARG;
     if (max_n < 2 || max_n > 0xFFFFFFFEull) return DARK_BWT_E_INVALID_N;
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return DARK_BWT_E_CUDA;  // no CPU fallback
@@ -1692,6 +1714,13 @@ int dark_bwt_create_ex(uint64_t max_n, int device, uint32_t flags, dark_bwt_ctx*
     const size_t o_morigins = carve(sizeof(unsigned long long) * kMaxManyBlocks);
     const size_t o_mlut = carve(sizeof(u16) * 256);
     const size_t o_dcinfo = carve(sizeof(DcInfoDev) + 16);
+    const bool dc_batch = flags & DARK_BWT_F_DC_BATCH;
+    size_t o_slot[2][5] = {};  // dist, item_pos, item_dist, item_sym, item_rank
+    if (dc_batch)
+        for (auto& s : o_slot) {
+            for (int a = 0; a < 3; ++a) s[a] = carve(N * 4 + 16);
+            for (int a = 3; a < 5; ++a) s[a] = carve(N + 16);
+        }
     ctx->arena_bytes = off;
 
     auto bail = [&](int code) {
@@ -1730,6 +1759,10 @@ int dark_bwt_create_ex(uint64_t max_n, int device, uint32_t flags, dark_bwt_ctx*
     ctx->many_origins = (unsigned long long*)(base + o_morigins);
     ctx->many_lut = (u16*)(base + o_mlut);
     ctx->dc_info = (DcInfoDev*)(base + o_dcinfo);
+    if (dc_batch)
+        for (int b = 0; b < 2; ++b)
+            ctx->dc_slot[b] = DcSlot{(u32*)(base + o_slot[b][0]), (u32*)(base + o_slot[b][1]), (u32*)(base + o_slot[b][2]),
+                                     (u8*)(base + o_slot[b][3]), (u8*)(base + o_slot[b][4])};
 
     if (cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking) != cudaSuccess) return bail(DARK_BWT_E_CUDA);
     if (staging) {
@@ -1829,16 +1862,16 @@ int dark_bwt_forward_batch(dark_bwt_ctx* ctx, const uint8_t* const* texts, const
     CK(cudaSetDevice(ctx->device));
     u8* const d_text[2] = {ctx->d_text, ctx->d_text2};
     u8* const d_bwt[2] = {ctx->d_bwt, ctx->d_bwt2};
-    return run_pipelined(ctx, texts, ns, bwt_outs, count, d_text, d_bwt, [&](uint64_t k, const u8* din, u8* dout, SideCopy* side) {
+    return run_pipelined(ctx, texts, ns, count, d_text, [&](uint64_t k, int b, const u8* din, OutCopies* out) {
         dark_bwt_stats* st = stats ? stats + k : nullptr;
         if (st) st->h2d_ms = 0.f;
-        const int rc = forward_device(ctx, din, (u32)ns[k], dout, origins_out + k, nullptr, st);
-        if (rc == 0 && sa_outs && sa_outs[k]) {  // the SA of the block is in the context's single SA buffer
-            side->host = sa_outs[k];
-            side->dev = ctx->sa;
-            side->bytes = ns[k] * sizeof(u32);
+        if (int rc = forward_device(ctx, din, (u32)ns[k], d_bwt[b], origins_out + k, nullptr, st)) return rc;
+        out->add(bwt_outs[k], d_bwt[b], ns[k]);
+        if (sa_outs && sa_outs[k]) {  // the SA of the block is in the context's single SA buffer
+            out->add(sa_outs[k], ctx->sa, ns[k] * sizeof(u32));
+            out->serial = true;
         }
-        return rc;
+        return 0;
     });
 }
 
@@ -1856,8 +1889,10 @@ int dark_bwt_inverse_batch(dark_bwt_ctx* ctx, const uint8_t* const* bwts, const 
     CK(cudaSetDevice(ctx->device));
     u8* const d_bwt[2] = {ctx->d_bwt, ctx->d_bwt2};
     u8* const d_text[2] = {ctx->d_text, ctx->d_text2};
-    return run_pipelined(ctx, bwts, ns, text_outs, count, d_bwt, d_text, [&](uint64_t k, const u8* din, u8* dout, SideCopy*) {
-        return inverse_device(ctx, din, (u32)ns[k], (u32)origins[k], nullptr, dout, ms_out ? ms_out + k : nullptr);
+    return run_pipelined(ctx, bwts, ns, count, d_bwt, [&](uint64_t k, int b, const u8* din, OutCopies* out) {
+        if (int rc = inverse_device(ctx, din, (u32)ns[k], (u32)origins[k], nullptr, d_text[b], ms_out ? ms_out + k : nullptr)) return rc;
+        out->add(text_outs[k], d_text[b], ns[k]);
+        return 0;
     });
 }
 
@@ -2015,6 +2050,48 @@ int dark_bwt_forward_dc(dark_bwt_ctx* ctx, const uint8_t* text, uint64_t n, uint
     DcBuffers io;
     if (int rc = dc_device(ctx, ctx->d_bwt, (u32)n, nullptr, &io, info)) return rc;
     return dc_copy_out(ctx, n, info->num_items, io, dist_out, nullptr, item_pos, item_dist, item_sym, item_rank);
+}
+
+int dark_bwt_forward_dc_batch(dark_bwt_ctx* ctx, const uint8_t* const* texts, const uint64_t* ns, uint64_t count, uint8_t* const* bwt_outs,
+                              uint64_t* origins_out, uint32_t* const* dist_outs, uint32_t* const* item_pos, uint32_t* const* item_dist,
+                              uint8_t* const* item_sym, uint8_t* const* item_rank, dark_bwt_dc_info* infos, dark_bwt_stats* stats) {
+    if (!ctx || !texts || !ns || !origins_out || !infos) return DARK_BWT_E_INVALID_ARG;
+    if (int rc = check_staging(ctx)) return rc;
+    if (!(ctx->flags & DARK_BWT_F_DC_BATCH)) return DARK_BWT_E_INVALID_ARG;  // no DC output slots
+    ctx->err[0] = 0;
+    for (uint64_t k = 0; k < count; ++k) {
+        if (!texts[k]) return DARK_BWT_E_INVALID_ARG;
+        if (int rc = check_n(ctx, ns[k], 2)) return rc;
+    }
+    if (count == 0) return DARK_BWT_OK;
+    CK(cudaSetDevice(ctx->device));
+    u8* const d_text[2] = {ctx->d_text, ctx->d_text2};
+    u8* const d_bwt[2] = {ctx->d_bwt, ctx->d_bwt2};
+    // Block k: the forward into d_bwt[b], then distance coding of it into slot b (b = k & 1).  Its scratch (run starts,
+    // tables, run counts, the status buffer a small block borrows) is consumed before block k+1's forward starts on the
+    // same stream; what the copies read stays untouched until the wait on ev_out[b] before block k+2.
+    return run_pipelined(ctx, texts, ns, count, d_text, [&](uint64_t k, int b, const u8* din, OutCopies* out) {
+        const u64 n = ns[k];
+        dark_bwt_stats* st = stats ? stats + k : nullptr;
+        if (st) st->h2d_ms = 0.f;
+        if (int rc = forward_device(ctx, din, (u32)n, d_bwt[b], origins_out + k, nullptr, st)) return rc;
+        const DcSlot& slot = ctx->dc_slot[b];
+        DcBuffers io;
+        io.dist = slot.dist;
+        io.item_pos = slot.item_pos;
+        io.item_dist = slot.item_dist;
+        io.item_sym = slot.item_sym;
+        io.item_rank = slot.item_rank;
+        if (int rc = dc_device(ctx, d_bwt[b], (u32)n, nullptr, &io, infos + k)) return rc;
+        const u64 items = infos[k].num_items;
+        out->add(bwt_outs ? bwt_outs[k] : nullptr, d_bwt[b], n);
+        out->add(dist_outs ? dist_outs[k] : nullptr, slot.dist, n * sizeof(u32));
+        out->add(item_pos ? item_pos[k] : nullptr, slot.item_pos, items * sizeof(u32));
+        out->add(item_dist ? item_dist[k] : nullptr, slot.item_dist, items * sizeof(u32));
+        out->add(item_sym ? item_sym[k] : nullptr, slot.item_sym, items);
+        out->add(item_rank ? item_rank[k] : nullptr, slot.item_rank, items);
+        return 0;
+    });
 }
 
 int dark_bwt_dc_encode_many_device(dark_bwt_ctx* ctx, const uint8_t* d_bwt, const uint32_t* d_starts, uint64_t count, uint32_t* d_dist_out,

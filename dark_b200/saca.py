@@ -238,6 +238,44 @@ class Constructor:
                                                rank.ctypes.data, ctypes.byref(info), ctypes.byref(self.stats)), self._ctx, "bwt + dc::encode")
         return out, int(origin.value), self._dc_result(info, n, dist, pos, idist, sym, rank)
 
+    def bwt_dc_batch_into(self, text_ptrs, ns, bwt_ptrs=None, dist_ptrs=None, pos_ptrs=None, idist_ptrs=None, sym_ptrs=None,
+                          rank_ptrs=None, want_stats=False):
+        """Pipelined block/dc.rs:45-52 over several blocks (dark_bwt_forward_dc_batch; raw host addresses, ideally pinned; needs
+        a Constructor made with flags including _ffi.F_DC_BATCH): copy-in of block k+1 and copy-out of block k-1 overlap the
+        forward + DC of block k.  Each output list is optional, and so is each entry (None).  The item arrays need room for n
+        entries.  Returns (origins, DcInfo records) and the per-block stats if asked."""
+        cnt = len(ns)
+        assert len(text_ptrs) == cnt
+
+        def arr(ptrs):
+            if ptrs is None:
+                return None
+            assert len(ptrs) == cnt
+            return (ctypes.c_void_p * max(cnt, 1))(*ptrs)
+        O = (ctypes.c_uint64 * max(cnt, 1))()
+        infos = (_ffi.DcInfo * max(cnt, 1))()
+        S = (_ffi.Stats * max(cnt, 1))() if want_stats else None
+        _ffi.check(self._L.dark_bwt_forward_dc_batch(self._ctx, arr(text_ptrs), (ctypes.c_uint64 * max(cnt, 1))(*[int(x) for x in ns]), cnt,
+                                                     arr(bwt_ptrs), O, arr(dist_ptrs), arr(pos_ptrs), arr(idist_ptrs), arr(sym_ptrs),
+                                                     arr(rank_ptrs), infos, S), self._ctx, "bwt + dc::encode (batch)")
+        res = ([int(O[i]) for i in range(cnt)], [infos[i] for i in range(cnt)])
+        return res + ([S[i].as_dict() for i in range(cnt)],) if want_stats else res
+
+    def bwt_dc_blocks(self, texts, want_dist=True, want_bwt=True):
+        """block/dc.rs:45-52 for a run of host blocks through the pipelined batch entry: [(bwt or None, origin, dc dict), ...],
+        each what bwt_dc gives on that block alone."""
+        ts = [_as_u8(t) for t in texts]
+        ns = [t.size for t in ts]
+        bwts = [np.empty(n, dtype=np.uint8) for n in ns] if want_bwt else None
+        dists = [np.empty(n, dtype=np.uint32) for n in ns] if want_dist else None
+        pos, idist = [np.empty(n, dtype=np.uint32) for n in ns], [np.empty(n, dtype=np.uint32) for n in ns]
+        sym, rank = [np.empty(n, dtype=np.uint8) for n in ns], [np.empty(n, dtype=np.uint8) for n in ns]
+        ptrs = lambda arrays: [a.ctypes.data for a in arrays] if arrays is not None else None  # noqa: E731
+        origins, infos = self.bwt_dc_batch_into(ptrs(ts), ns, ptrs(bwts), ptrs(dists), ptrs(pos), ptrs(idist), ptrs(sym), ptrs(rank))
+        return [(bwts[k] if want_bwt else None, origins[k],
+                 self._dc_result(infos[k], ns[k], dists[k] if want_dist else None, pos[k], idist[k], sym[k], rank[k]))
+                for k in range(len(ts))]
+
     def dc_encode_device(self, d_bwt, n, d_dist=None, d_item_pos=None, d_item_dist=None, d_item_sym=None, d_item_rank=None):
         """Device pointers in, device pointers out (all outputs optional); returns the DcInfo header."""
         info = _ffi.DcInfo()

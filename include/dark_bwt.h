@@ -60,6 +60,10 @@ extern "C" {
 /* Do not allocate the host-entry staging (device text/BWT/SA-out buffers, pinned memory):
  * for callers that only use dark_bwt_forward_device. */
 #define DARK_BWT_F_DEVICE_ONLY 2u
+/* Reserve two distance-coding output slots (dist 4N + item_pos 4N + item_dist 4N + item_sym N + item_rank N, twice:
+ * 28 N bytes more, 73 N in all; 18.3 GiB for a 256 MiB block, 146 GiB for 2 GiB) for dark_bwt_forward_dc_batch.
+ * Not combinable with DARK_BWT_F_DEVICE_ONLY. */
+#define DARK_BWT_F_DC_BATCH 4u
 
 #define DARK_BWT_MAX_ROUNDS 40
 
@@ -98,8 +102,8 @@ typedef struct dark_bwt_stats {
 } dark_bwt_stats;
 
 /* Constructor::new — allocates every device buffer for blocks of up to max_n bytes on
- * CUDA device `device`: one arena of 45 * max_n bytes of HBM (41 * max_n with DARK_BWT_F_DEVICE_ONLY; 11.2 GiB for a
- * 256 MiB block, 89.8 GiB for 2 GiB).  No device memory is allocated later; the pinned staging lanes for pageable host
+ * CUDA device `device`: one arena of 45 * max_n bytes of HBM (41 * max_n with DARK_BWT_F_DEVICE_ONLY, 73 * max_n with
+ * DARK_BWT_F_DC_BATCH; 11.2 GiB for a 256 MiB block, 89.8 GiB for 2 GiB).  No device memory is allocated later; the pinned staging lanes for pageable host
  * buffers (12 lanes x 2 slots x 2 MiB per direction) and the `reuse` scratch are allocated by the first call that needs them. */
 int dark_bwt_create(uint64_t max_n, int device, dark_bwt_ctx **out);
 int dark_bwt_create_ex(uint64_t max_n, int device, uint32_t flags, dark_bwt_ctx **out);
@@ -207,6 +211,21 @@ int dark_bwt_dc_encode(dark_bwt_ctx *ctx, const uint8_t *bwt, uint64_t n, uint32
 int dark_bwt_forward_dc(dark_bwt_ctx *ctx, const uint8_t *text, uint64_t n, uint8_t *bwt_out, uint64_t *origin_out,
                         uint32_t *dist_out, uint32_t *item_pos, uint32_t *item_dist, uint8_t *item_sym, uint8_t *item_rank,
                         dark_bwt_dc_info *info, dark_bwt_stats *stats);
+/* `count` independent host blocks through dark_bwt_forward_dc, pipelined like dark_bwt_forward_batch: while block k is
+ * transformed and distance-coded, block k+1 is copied in and the outputs of block k-1 are copied out (two device BWT
+ * buffers and the two DC output slots of a context created with DARK_BWT_F_DC_BATCH).  This is how the reference's
+ * per-block loop (src/main.rs:87-113 -> block/dc.rs:45-85) feeds a run of large blocks.  Block k gets exactly what
+ * dark_bwt_forward_dc(texts[k], ...) gives: bwt_outs[k][0..ns[k]), origins_out[k], dist_outs[k][0..ns[k]), the
+ * infos[k].num_items items, and infos[k] (device_ms = that block's DC time).  Required: texts (and every entry), ns,
+ * origins_out, infos (`count` records).  Nullable: every output array and every entry of one (a caller that codes the
+ * item stream passes neither BWT nor distances: then only the items cross PCIe), and stats (`count` records).  Pinned
+ * host buffers overlap fully; pageable ones of 1 MiB or more go through the staging lanes.  DARK_BWT_E_INVALID_ARG,
+ * before any device work, for a context without DARK_BWT_F_DC_BATCH or a null required pointer; DARK_BWT_E_INVALID_N
+ * for any ns[k] outside [2, capacity].  count == 0 is DARK_BWT_OK. */
+int dark_bwt_forward_dc_batch(dark_bwt_ctx *ctx, const uint8_t *const *texts, const uint64_t *ns, uint64_t count,
+                              uint8_t *const *bwt_outs, uint64_t *origins_out, uint32_t *const *dist_outs,
+                              uint32_t *const *item_pos, uint32_t *const *item_dist, uint8_t *const *item_sym,
+                              uint8_t *const *item_rank, dark_bwt_dc_info *infos, dark_bwt_stats *stats);
 
 /* MANY SMALL blocks distance-coded in ONE pass.  Block k gives exactly what dark_bwt_dc_encode gives on that block alone:
  * every value is block-relative (filler and last-run distances use n_k, init[c] is the first occurrence inside the block

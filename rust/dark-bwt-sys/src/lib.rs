@@ -5,6 +5,8 @@ use libc::{c_char, c_int, c_void};
 
 pub const DARK_BWT_OK: c_int = 0;
 pub const DARK_BWT_MAX_ROUNDS: usize = 40;
+/// dark_bwt_create_ex flag: the two DC output slots dark_bwt_forward_dc_batch needs (73 N bytes of HBM in all).
+pub const DARK_BWT_F_DC_BATCH: u32 = 4;
 
 #[repr(C)]
 pub struct dark_bwt_ctx { _private: [u8; 0] }
@@ -70,6 +72,10 @@ extern "C" {
                                     bwt_outs: *const *mut u8, origins_out: *mut u64, dist_out: *mut u32, item_starts: *mut u32,
                                     item_pos: *mut u32, item_dist: *mut u32, item_sym: *mut u8, item_rank: *mut u8,
                                     infos: *mut dark_bwt_dc_info, stats: *mut dark_bwt_stats) -> c_int;
+    pub fn dark_bwt_forward_dc_batch(ctx: *mut dark_bwt_ctx, texts: *const *const u8, ns: *const u64, count: u64,
+                                     bwt_outs: *const *mut u8, origins_out: *mut u64, dist_outs: *const *mut u32,
+                                     item_pos: *const *mut u32, item_dist: *const *mut u32, item_sym: *const *mut u8,
+                                     item_rank: *const *mut u8, infos: *mut dark_bwt_dc_info, stats: *mut dark_bwt_stats) -> c_int;
     pub fn dark_bwt_create(max_n: u64, device: c_int, out: *mut *mut dark_bwt_ctx) -> c_int;
     pub fn dark_bwt_create_ex(max_n: u64, device: c_int, flags: u32, out: *mut *mut dark_bwt_ctx) -> c_int;
     pub fn dark_bwt_capacity(ctx: *const dark_bwt_ctx) -> u64;
