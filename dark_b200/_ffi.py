@@ -14,7 +14,7 @@ F_DEFAULT, F_NO_ALPHABET_PACKING, F_DEVICE_ONLY, F_DC_BATCH = 0, 1, 2, 4
 
 # every symbol include/dark_bwt.h declares (tests/test_abi.py checks the .so exports all of them)
 SYMBOLS = [
-    "dark_bwt_abi_version", "dark_bwt_create", "dark_bwt_create_ex", "dark_bwt_capacity", "dark_bwt_forward",
+    "dark_bwt_abi_version", "dark_bwt_create", "dark_bwt_create_ex", "dark_bwt_arena_bytes", "dark_bwt_capacity", "dark_bwt_forward",
     "dark_bwt_forward_batch", "dark_bwt_forward_many", "dark_bwt_forward_many_device", "dark_bwt_forward_device", "dark_bwt_inverse", "dark_bwt_inverse_device",
     "dark_bwt_inverse_batch", "dark_bwt_inverse_many", "dark_bwt_inverse_many_device", "dark_bwt_reuse", "dark_bwt_destroy", "dark_bwt_strerror", "dark_bwt_last_error",
     "dark_bwt_stream", "dark_bwt_sort_pairs_device", "dark_bwt_verify_sa_device", "dark_bwt_emit_device", "dark_bwt_lcp_profile_device",
@@ -86,6 +86,8 @@ def lib():
     L.dark_bwt_abi_version.restype = i32
     L.dark_bwt_create.argtypes = [u64, i32, pp]
     L.dark_bwt_create_ex.argtypes = [u64, i32, u32, pp]
+    L.dark_bwt_arena_bytes.argtypes = [u64, u32]
+    L.dark_bwt_arena_bytes.restype = u64
     L.dark_bwt_capacity.argtypes = [vp]
     L.dark_bwt_capacity.restype = u64
     L.dark_bwt_forward.argtypes = [vp, vp, u64, vp, ctypes.POINTER(u64), vp, ctypes.POINTER(Stats)]

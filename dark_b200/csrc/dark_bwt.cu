@@ -163,8 +163,9 @@ struct dark_bwt_ctx {
     u32* sa = nullptr;
     u8* d_text = nullptr;  // host-entry staging
     u8* d_bwt = nullptr;
-    u8* d_text2 = nullptr;  // second pair for the pipelined batch entry
+    u8* d_text2 = nullptr;  // second pair for the pipelined batch entries (== d_text, d_bwt on a one-pair context)
     u8* d_bwt2 = nullptr;
+    int pipeline_depth = 0;  // staging pairs: 2, or 1 above 2^31 (the batch entries then run their blocks serially)
     DcSlot dc_slot[2];  // DARK_BWT_F_DC_BATCH: block k of a pipelined DC batch is coded into slot k & 1
     cudaStream_t copy_in = nullptr, copy_out = nullptr;
     cudaEvent_t ev_in[2] = {nullptr, nullptr}, ev_comp[2] = {nullptr, nullptr}, ev_out[2] = {nullptr, nullptr};
@@ -1559,7 +1560,8 @@ struct OutCopies {
 // (transform(k, b, d_in[b], &copies), synchronous on the context's stream; b = k & 1 selects the block's device buffers),
 // block k+1 is copied into the other input buffer and the copies of block k-1 run out of the other buffers.  Pinned host
 // buffers ride on the two copy streams; a list with a pageable buffer of 1 MiB or more is sent one copy after another by a
-// helper thread, the pageable copies through the staging lanes.
+// helper thread, the pageable copies through the staging lanes.  A context with one staging pair (pipeline_depth 1: above
+// 2^31) has only b = 0: the copy-in of block k+1 starts once transform k has returned and the copies of block k have drained.
 template <typename Transform>
 int run_pipelined(dark_bwt_ctx* ctx, const u8* const* ins, const uint64_t* ns, uint64_t count, u8* const d_in[2], Transform transform) {
     bool comp_recorded[2] = {false, false}, out_recorded[2] = {false, false};
@@ -1590,21 +1592,23 @@ int run_pipelined(dark_bwt_ctx* ctx, const u8* const* ins, const uint64_t* ns, u
         if (fout.valid()) rc |= fout.get();
         return rc;
     };
+    const uint64_t depth = (uint64_t)ctx->pipeline_depth;
     if (int rc = start_in(0, 0)) return rc;
     for (uint64_t k = 0; k < count; ++k) {
-        const int b = (int)(k & 1), nb = b ^ 1;
+        const int b = (int)(k % depth), nb = (int)((k + 1) % depth);
         if (fin[b].valid()) {
             if (int rc = fin[b].get()) { drain(); return rc; }
         } else {
             CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_in[b], 0));
         }
-        if (k + 1 < count)
+        if (depth == 2 && k + 1 < count)
             if (int rc = start_in(k + 1, nb)) { drain(); return rc; }
         // (a staged copy-out of block k-1 may still be reading the OTHER buffers; these were drained before it began)
         if (out_recorded[b]) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_out[b], 0));  // output buffers b drained
         OutCopies oc;
         int rc = transform(k, b, (const u8*)d_in[b], &oc);
         if (rc) { drain(); return rc; }
+        if (depth == 1) oc.serial = true;
         CK(cudaEventRecord(ctx->ev_comp[b], ctx->stream));
         comp_recorded[b] = true;
         if (fout.valid())
@@ -1627,11 +1631,73 @@ int run_pipelined(dark_bwt_ctx* ctx, const u8* const* ins, const uint64_t* ns, u
             CK(cudaEventRecord(ctx->ev_out[b], ctx->copy_out));
             out_recorded[b] = true;
         }
+        if (depth == 1 && k + 1 < count)
+            if (int rc2 = start_in(k + 1, nb)) { drain(); return rc2; }
     }
     if (int rc = drain()) return rc;
     CK(cudaStreamSynchronize(ctx->copy_out));
     CK(cudaStreamSynchronize(ctx->copy_in));
     return DARK_BWT_OK;
+}
+
+// Where dark_bwt_create_ex carves each buffer of the arena: byte offsets, and `bytes` in all.  Pure host arithmetic, shared
+// with dark_bwt_arena_bytes.  Returns false for a capacity or flags create rejects.
+struct ArenaLayout {
+    size_t keys[2], ids[2], ranks, ranks2, isa, sa;
+    size_t text, bwt, text2, bwt2;  // host-entry staging pairs (none with DARK_BWT_F_DEVICE_ONLY); text2 == text with one pair
+    size_t hist, present, lut, bad, status, counters, bhist, bitmap, swords, mstarts, morigins, mlut, dcinfo;
+    size_t slot[2][5];  // DARK_BWT_F_DC_BATCH: dist, item_pos, item_dist, item_sym, item_rank
+    size_t sort_status_bytes, scan_tiles, bytes;
+    int staging_pairs;
+};
+
+bool arena_layout(uint64_t max_n, uint32_t flags, ArenaLayout* L) {
+    *L = ArenaLayout{};
+    if (flags & ~(DARK_BWT_F_NO_ALPHABET_PACKING | DARK_BWT_F_DEVICE_ONLY | DARK_BWT_F_DC_BATCH)) return false;
+    // the DC batch is a host-buffer entry: it needs the staging a device-only context does not have
+    if ((flags & DARK_BWT_F_DC_BATCH) && (flags & DARK_BWT_F_DEVICE_ONLY)) return false;
+    if (max_n < 2 || max_n > 0xFFFFFFFEull) return false;
+    const size_t N = (size_t)max_n;
+    const size_t sort_tiles = ceil_div(N, kSortTile);
+    L->sort_status_bytes = (sort_tiles + 128) * kRadix * sizeof(u64);  // + rows the scanner CTA reads ahead
+    L->scan_tiles = ceil_div(N, std::min(kScanTile, 4096));  // the pairs kernel and the text-order builder scan 4,096-suffix tiles
+    const bool staging = !(flags & DARK_BWT_F_DEVICE_ONLY);
+    const bool dc_batch = flags & DARK_BWT_F_DC_BATCH;
+    // Above 2^31 the second pair (2 N bytes) is what keeps a context of 2^32 - 2 inside a B200: the batch entries then run
+    // their blocks one after another through one pair.  The DC batch keeps two pairs: its output slots pair with them.
+    L->staging_pairs = !staging ? 0 : (max_n > (1ull << 31) && !dc_batch) ? 1 : 2;
+
+    size_t off = 0;
+    auto carve = [&](size_t bytes) {
+        size_t o = off;
+        off = align_up(off + bytes, 256);
+        return o;
+    };
+    L->keys[0] = carve(N * 8 + 1024), L->keys[1] = carve(N * 8 + 1024);  // slack: pair lists are split at a 64-aligned offset
+    L->ids[0] = carve(N * 4 + 16), L->ids[1] = carve(N * 4 + 16);
+    L->ranks = carve(N * 4 + 16), L->ranks2 = carve(N * 4 + 16), L->isa = carve(N * 4 + 16), L->sa = carve(N * 4 + 16);
+    L->text = staging ? carve(N + 16) : 0, L->bwt = staging ? carve(N + 16) : 0;
+    L->text2 = L->staging_pairs == 2 ? carve(N + 16) : L->text, L->bwt2 = L->staging_pairs == 2 ? carve(N + 16) : L->bwt;
+    L->hist = carve(sizeof(u32) * kMaxPasses * kRadix);
+    L->present = carve(sizeof(u32) * 256);
+    L->lut = carve(256);
+    L->bad = carve(sizeof(unsigned long long));
+    L->status = carve(L->sort_status_bytes);
+    L->counters = carve(sizeof(u32) * kMaxCounters);
+    L->bhist = carve(sizeof(u32) * 1280);  // 256 bucket counters/cursors + 257 chunk prefixes; DC: first/last occurrences + dense alphabet
+    L->bitmap = carve(sizeof(u32) * (ceil_div(N, 32) + 1) + 1024);  // + one tile of flag bytes past the end
+    L->swords = carve(sizeof(u64) * kScanWordsPerTile * L->scan_tiles);
+    L->mstarts = carve(sizeof(u32) * (kMaxManyBlocks + 1));
+    L->morigins = carve(sizeof(unsigned long long) * kMaxManyBlocks);
+    L->mlut = carve(sizeof(u16) * 256);
+    L->dcinfo = carve(sizeof(DcInfoDev) + 16);
+    if (dc_batch)
+        for (auto& s : L->slot) {
+            for (int a = 0; a < 3; ++a) s[a] = carve(N * 4 + 16);
+            for (int a = 3; a < 5; ++a) s[a] = carve(N + 16);
+        }
+    L->bytes = off;
+    return true;
 }
 
 }  // namespace
@@ -1657,6 +1723,11 @@ const char* dark_bwt_last_error(const dark_bwt_ctx* ctx) { return ctx ? ctx->err
 uint64_t dark_bwt_capacity(const dark_bwt_ctx* ctx) { return ctx ? ctx->capacity : 0; }
 void* dark_bwt_stream(const dark_bwt_ctx* ctx) { return ctx ? (void*)ctx->stream : nullptr; }
 
+uint64_t dark_bwt_arena_bytes(uint64_t max_n, uint32_t flags) {
+    ArenaLayout L;
+    return arena_layout(max_n, flags, &L) ? (uint64_t)L.bytes : 0;
+}
+
 int dark_bwt_create(uint64_t max_n, int device, dark_bwt_ctx** out) {
     return dark_bwt_create_ex(max_n, device, DARK_BWT_F_DEFAULT, out);
 }
@@ -1665,7 +1736,6 @@ int dark_bwt_create_ex(uint64_t max_n, int device, uint32_t flags, dark_bwt_ctx*
     if (!out) return DARK_BWT_E_INVALID_ARG;
     *out = nullptr;
     if (flags & ~(DARK_BWT_F_NO_ALPHABET_PACKING | DARK_BWT_F_DEVICE_ONLY | DARK_BWT_F_DC_BATCH)) return DARK_BWT_E_INVALID_ARG;
-    // the DC batch is a host-buffer entry: it needs the staging a device-only context does not have
     if ((flags & DARK_BWT_F_DC_BATCH) && (flags & DARK_BWT_F_DEVICE_ONLY)) return DARK_BWT_E_INVALID_ARG;
     if (max_n < 2 || max_n > 0xFFFFFFFEull) return DARK_BWT_E_INVALID_N;
     int ndev = 0;
@@ -1684,44 +1754,13 @@ int dark_bwt_create_ex(uint64_t max_n, int device, uint32_t flags, dark_bwt_ctx*
     ctx->flags = flags;
     ctx->knobs.read_env();
 
-    const size_t N = (size_t)max_n;
-    const size_t sort_tiles = ceil_div(N, kSortTile);
-    ctx->sort_status_bytes = (sort_tiles + 128) * kRadix * sizeof(u64);  // + rows the scanner CTA reads ahead
-    ctx->scan_tiles = ceil_div(N, std::min(kScanTile, 4096));  // the pairs kernel and the text-order builder scan 4,096-suffix tiles
+    ArenaLayout L;
+    arena_layout(max_n, flags, &L);
+    ctx->sort_status_bytes = L.sort_status_bytes;
+    ctx->scan_tiles = L.scan_tiles;
     const bool staging = !(flags & DARK_BWT_F_DEVICE_ONLY);
-
-    size_t off = 0;
-    auto carve = [&](size_t bytes) {
-        size_t o = off;
-        off = align_up(off + bytes, 256);
-        return o;
-    };
-    const size_t o_keys0 = carve(N * 8 + 1024), o_keys1 = carve(N * 8 + 1024);  // slack: pair lists are split at a 64-aligned offset
-    const size_t o_ids0 = carve(N * 4 + 16), o_ids1 = carve(N * 4 + 16);
-    const size_t o_ranks = carve(N * 4 + 16), o_ranks2 = carve(N * 4 + 16), o_isa = carve(N * 4 + 16), o_sa = carve(N * 4 + 16);
-    const size_t o_text = staging ? carve(N + 16) : 0, o_bwt = staging ? carve(N + 16) : 0;
-    const size_t o_text2 = staging ? carve(N + 16) : 0, o_bwt2 = staging ? carve(N + 16) : 0;
-    const size_t o_hist = carve(sizeof(u32) * kMaxPasses * kRadix);
-    const size_t o_present = carve(sizeof(u32) * 256);
-    const size_t o_lut = carve(256);
-    const size_t o_bad = carve(sizeof(unsigned long long));
-    const size_t o_status = carve(ctx->sort_status_bytes);
-    const size_t o_counters = carve(sizeof(u32) * kMaxCounters);
-    const size_t o_bhist = carve(sizeof(u32) * 1280);  // 256 bucket counters/cursors + 257 chunk prefixes; DC: first/last occurrences + dense alphabet
-    const size_t o_bitmap = carve(sizeof(u32) * (ceil_div(N, 32) + 1) + 1024);  // + one tile of flag bytes past the end
-    const size_t o_swords = carve(sizeof(u64) * kScanWordsPerTile * ctx->scan_tiles);
-    const size_t o_mstarts = carve(sizeof(u32) * (kMaxManyBlocks + 1));
-    const size_t o_morigins = carve(sizeof(unsigned long long) * kMaxManyBlocks);
-    const size_t o_mlut = carve(sizeof(u16) * 256);
-    const size_t o_dcinfo = carve(sizeof(DcInfoDev) + 16);
     const bool dc_batch = flags & DARK_BWT_F_DC_BATCH;
-    size_t o_slot[2][5] = {};  // dist, item_pos, item_dist, item_sym, item_rank
-    if (dc_batch)
-        for (auto& s : o_slot) {
-            for (int a = 0; a < 3; ++a) s[a] = carve(N * 4 + 16);
-            for (int a = 3; a < 5; ++a) s[a] = carve(N + 16);
-        }
-    ctx->arena_bytes = off;
+    ctx->arena_bytes = L.bytes;
 
     auto bail = [&](int code) {
         dark_bwt_destroy(ctx);
@@ -1733,36 +1772,37 @@ int dark_bwt_create_ex(uint64_t max_n, int device, uint32_t flags, dark_bwt_ctx*
         return bail(DARK_BWT_E_NOMEM);
     }
     char* base = (char*)ctx->arena;
-    ctx->keys[0] = (u64*)(base + o_keys0);
-    ctx->keys[1] = (u64*)(base + o_keys1);
-    ctx->ids[0] = (u32*)(base + o_ids0);
-    ctx->ids[1] = (u32*)(base + o_ids1);
-    ctx->ranks = (u32*)(base + o_ranks);
-    ctx->ranks_alt = (u32*)(base + o_ranks2);
-    ctx->isa = (u32*)(base + o_isa);
-    ctx->sa = (u32*)(base + o_sa);
-    ctx->d_text = staging ? (u8*)(base + o_text) : nullptr;
-    ctx->d_bwt = staging ? (u8*)(base + o_bwt) : nullptr;
-    ctx->d_text2 = staging ? (u8*)(base + o_text2) : nullptr;
-    ctx->d_bwt2 = staging ? (u8*)(base + o_bwt2) : nullptr;
-    ctx->hist = (u32*)(base + o_hist);
-    ctx->present = (u32*)(base + o_present);
-    ctx->lut = (u8*)(base + o_lut);
-    ctx->bad = (unsigned long long*)(base + o_bad);
-    ctx->sort_status = base + o_status;
+    ctx->keys[0] = (u64*)(base + L.keys[0]);
+    ctx->keys[1] = (u64*)(base + L.keys[1]);
+    ctx->ids[0] = (u32*)(base + L.ids[0]);
+    ctx->ids[1] = (u32*)(base + L.ids[1]);
+    ctx->ranks = (u32*)(base + L.ranks);
+    ctx->ranks_alt = (u32*)(base + L.ranks2);
+    ctx->isa = (u32*)(base + L.isa);
+    ctx->sa = (u32*)(base + L.sa);
+    ctx->d_text = staging ? (u8*)(base + L.text) : nullptr;
+    ctx->d_bwt = staging ? (u8*)(base + L.bwt) : nullptr;
+    ctx->d_text2 = staging ? (u8*)(base + L.text2) : nullptr;  // one pair: the same buffers as d_text and d_bwt
+    ctx->d_bwt2 = staging ? (u8*)(base + L.bwt2) : nullptr;
+    ctx->pipeline_depth = L.staging_pairs;
+    ctx->hist = (u32*)(base + L.hist);
+    ctx->present = (u32*)(base + L.present);
+    ctx->lut = (u8*)(base + L.lut);
+    ctx->bad = (unsigned long long*)(base + L.bad);
+    ctx->sort_status = base + L.status;
     for (int h = 0; h < 2; ++h) ctx->status_dirty_lo[h] = 0u, ctx->status_dirty_hi[h] = (u32)(ctx->sort_status_bytes / 2 / (kRadix * sizeof(u32)));
-    ctx->counters = (u32*)(base + o_counters);
-    ctx->scan_words = (u64*)(base + o_swords);
-    ctx->bitmap = (u32*)(base + o_bitmap);
-    ctx->bucket_hist = (u32*)(base + o_bhist);
-    ctx->many_starts = (u32*)(base + o_mstarts);
-    ctx->many_origins = (unsigned long long*)(base + o_morigins);
-    ctx->many_lut = (u16*)(base + o_mlut);
-    ctx->dc_info = (DcInfoDev*)(base + o_dcinfo);
+    ctx->counters = (u32*)(base + L.counters);
+    ctx->scan_words = (u64*)(base + L.swords);
+    ctx->bitmap = (u32*)(base + L.bitmap);
+    ctx->bucket_hist = (u32*)(base + L.bhist);
+    ctx->many_starts = (u32*)(base + L.mstarts);
+    ctx->many_origins = (unsigned long long*)(base + L.morigins);
+    ctx->many_lut = (u16*)(base + L.mlut);
+    ctx->dc_info = (DcInfoDev*)(base + L.dcinfo);
     if (dc_batch)
         for (int b = 0; b < 2; ++b)
-            ctx->dc_slot[b] = DcSlot{(u32*)(base + o_slot[b][0]), (u32*)(base + o_slot[b][1]), (u32*)(base + o_slot[b][2]),
-                                     (u8*)(base + o_slot[b][3]), (u8*)(base + o_slot[b][4])};
+            ctx->dc_slot[b] = DcSlot{(u32*)(base + L.slot[b][0]), (u32*)(base + L.slot[b][1]), (u32*)(base + L.slot[b][2]),
+                                     (u8*)(base + L.slot[b][3]), (u8*)(base + L.slot[b][4])};
 
     if (cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking) != cudaSuccess) return bail(DARK_BWT_E_CUDA);
     if (staging) {

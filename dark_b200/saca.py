@@ -406,6 +406,12 @@ class Constructor:
         self.close()
 
 
+def arena_bytes(max_n, flags=_ffi.F_DEFAULT):
+    """Device bytes a Constructor(max_n, flags=flags) allocates, or 0 for a max_n or flags it rejects.  Touches no device:
+    a caller can check that a block fits a card before creating the context."""
+    return int(_ffi.lib().dark_bwt_arena_bytes(int(max_n), int(flags)))
+
+
 def decode(bwt, origin, device=0):
     """`compress::bwt::decode(&input, origin, &mut suffixes)` collected: the original bytes."""
     b = _as_u8(bwt)

@@ -102,11 +102,19 @@ typedef struct dark_bwt_stats {
 } dark_bwt_stats;
 
 /* Constructor::new — allocates every device buffer for blocks of up to max_n bytes on
- * CUDA device `device`: one arena of 45 * max_n bytes of HBM (41 * max_n with DARK_BWT_F_DEVICE_ONLY, 73 * max_n with
- * DARK_BWT_F_DC_BATCH; 11.2 GiB for a 256 MiB block, 89.8 GiB for 2 GiB).  No device memory is allocated later; the pinned staging lanes for pageable host
- * buffers (12 lanes x 2 slots x 2 MiB per direction) and the `reuse` scratch are allocated by the first call that needs them. */
+ * CUDA device `device`: one arena of dark_bwt_arena_bytes(max_n, flags) bytes of HBM, about 44.8 * max_n (40.8 * max_n with
+ * DARK_BWT_F_DEVICE_ONLY, 72.8 * max_n with DARK_BWT_F_DC_BATCH; 12.0 GB for a 256 MiB block, 96.2 GB for 2^31).  Above
+ * 2^31 bytes, without DARK_BWT_F_DEVICE_ONLY or DARK_BWT_F_DC_BATCH, the context keeps one host-entry staging pair instead
+ * of two (about 42.8 * max_n: 183.8 GB for 2^32-2, which a 180 GB B200 holds); the batch entries then run their blocks one
+ * after another.  DARK_BWT_F_DC_BATCH tops out near 2.4 GiB on a B200.  No device memory is allocated later; the pinned
+ * staging lanes for pageable host buffers (12 lanes x 2 slots x 2 MiB per direction) and the `reuse` scratch are allocated
+ * by the first call that needs them. */
 int dark_bwt_create(uint64_t max_n, int device, dark_bwt_ctx **out);
 int dark_bwt_create_ex(uint64_t max_n, int device, uint32_t flags, dark_bwt_ctx **out);
+
+/* The exact bytes dark_bwt_create_ex(max_n, ., flags, .) allocates in its arena, or 0 for a max_n or flags it rejects.
+ * Host arithmetic only: touches no device.  Lets a caller learn before create whether a block fits a card. */
+uint64_t dark_bwt_arena_bytes(uint64_t max_n, uint32_t flags);
 
 /* Constructor::capacity */
 uint64_t dark_bwt_capacity(const dark_bwt_ctx *ctx);
@@ -123,7 +131,8 @@ int dark_bwt_forward(dark_bwt_ctx *ctx, const uint8_t *text, uint64_t n, uint8_t
  * k+1 is copied in and block k-1 is copied out (two copy streams beside the compute stream, double-
  * buffered device staging).  This is how a corpus of blocks is fed — the reference encodes one block
  * per Encoder (src/main.rs:95-113) and blocks share nothing.  Pinned host buffers overlap fully;
- * pageable ones still work.  sa_outs and stats are nullable (entries of sa_outs too); stats, if
+ * pageable ones still work.  A context above 2^31 has one staging pair (dark_bwt_create) and does not overlap
+ * blocks: each is copied in, transformed and copied out before the next is copied in.  sa_outs and stats are nullable (entries of sa_outs too); stats, if
  * given, is an array of `count` records.  Results are identical to `count` dark_bwt_forward calls. */
 int dark_bwt_forward_batch(dark_bwt_ctx *ctx, const uint8_t *const *texts, const uint64_t *ns, uint8_t *const *bwt_outs,
                            uint64_t *origins_out, uint32_t *const *sa_outs, uint64_t count, dark_bwt_stats *stats);
@@ -159,7 +168,8 @@ int dark_bwt_inverse_device(dark_bwt_ctx *ctx, const uint8_t *d_bwt, uint64_t n,
 
 /* `count` independent host blocks, pipelined like dark_bwt_forward_batch: while block k is inverted, block k+1 is copied
  * in and block k-1 copied out (double-buffered device staging, the two copy streams, pageable buffers of 1 MiB or more
- * through the staging lanes).  Each block: 1 <= ns[k] <= capacity, origins[k] < ns[k].  ms_out (nullable) = `count`
+ * through the staging lanes; no overlap on a context above 2^31, as in dark_bwt_forward_batch).  Each block:
+ * 1 <= ns[k] <= capacity, origins[k] < ns[k].  ms_out (nullable) = `count`
  * device times.  Results identical to `count` dark_bwt_inverse calls; DARK_BWT_E_INVALID_ARG with a device-only context. */
 int dark_bwt_inverse_batch(dark_bwt_ctx *ctx, const uint8_t *const *bwts, const uint64_t *ns, const uint64_t *origins,
                            uint8_t *const *text_outs, uint64_t count, float *ms_out);

@@ -78,6 +78,7 @@ extern "C" {
                                      item_rank: *const *mut u8, infos: *mut dark_bwt_dc_info, stats: *mut dark_bwt_stats) -> c_int;
     pub fn dark_bwt_create(max_n: u64, device: c_int, out: *mut *mut dark_bwt_ctx) -> c_int;
     pub fn dark_bwt_create_ex(max_n: u64, device: c_int, flags: u32, out: *mut *mut dark_bwt_ctx) -> c_int;
+    pub fn dark_bwt_arena_bytes(max_n: u64, flags: u32) -> u64;
     pub fn dark_bwt_capacity(ctx: *const dark_bwt_ctx) -> u64;
     pub fn dark_bwt_forward(ctx: *mut dark_bwt_ctx, text: *const u8, n: u64, bwt_out: *mut u8,
                             origin_out: *mut u64, sa_out: *mut u32, stats: *mut dark_bwt_stats) -> c_int;

@@ -52,6 +52,12 @@ impl Constructor {
         Constructor { ctx: ctx, n: max_n, sa: Vec::new(), out: Vec::new(), origin: 0 }
     }
 
+    /// Device bytes `Constructor::new(max_n)` allocates (0 if max_n is out of range): whether a block fits a card can be
+    /// checked before creating a context.  Touches no device.
+    pub fn arena_bytes(max_n: usize) -> u64 {
+        unsafe { sys::dark_bwt_arena_bytes(max_n as u64, 0) }
+    }
+
     /// Return maximum block size
     pub fn capacity(&self) -> usize {
         unsafe { sys::dark_bwt_capacity(self.ctx) as usize }
