@@ -3,9 +3,15 @@
 // Host-side control flow of one block (replaces saca::Constructor::compute + TransformIterator,
 // /root/reference/src/saca.rs:368-378 and src/block/dc.rs:45-50):
 //
-//   alphabet scan -> initial keys (K symbols per 64-bit key) -> radix sort -> re-rank/compact
-//   while (unsettled suffixes remain):  keys (rank[i], rank[i+h]) -> radix sort -> re-rank/compact;  h *= 2
-//   BWT gather + origin
+//   scan_alphabet                   sigma, dense codes, K symbols per 64-bit key
+//   round0_keys, round0_sort        initial keys / digit histograms -> radix sort (top digits only if high-entropy)
+//   round0_rerank                   re-rank/compact (sparse or scan kernel)
+//   while (unsettled suffixes remain):
+//     doubling_round                keys (rank[i], rank[i+h]) -> radix sort -> re-rank/compact, or pairs_round;  h *= 2
+//   emit                            BWT gather + origin (unless the re-ranks emitted the bytes inline)
+//
+// forward_device drives these phases.  What crosses them lives in one Fwd record; RankFill owns which ranks isa[]
+// holds, PairsMode owns pairs mode.
 //
 // All device memory is carved from one arena allocated at create (Constructor::new allocates its
 // arena up front too, saca.rs:351-360); the forward calls allocate nothing.
@@ -203,8 +209,6 @@ struct dark_bwt_ctx {
     };
     std::vector<Span> spans;
     int next_counter = 0;
-    u32* count_dev = nullptr;  // device copy of the survivor count of the last re-rank launched (nullptr: none)
-    u32 tag = 0;  // bit carried by isa[] entries of active suffixes during forward_device (0: not used)
     u32 launches = 0;
     u32 syncs = 0;
     char err[320] = {0};
@@ -239,7 +243,7 @@ inline cudaError_t sync_counted(dark_bwt_ctx* ctx) {
 }
 
 // The start of a call that sorts or inverts: the context's device, fresh per-call bookkeeping (events and spans, tile
-// counters, launch and sync counts, the isa[] tag), the call's clock (call_start) and zeroed tile counters.
+// counters, launch and sync counts), the call's clock (call_start) and zeroed tile counters.
 int begin_call(dark_bwt_ctx* ctx) {
     CK(cudaSetDevice(ctx->device));
     ctx->n_events = 0;
@@ -247,7 +251,6 @@ int begin_call(dark_bwt_ctx* ctx) {
     ctx->next_counter = 0;
     ctx->launches = 0;
     ctx->syncs = 0;
-    ctx->tag = 0;
     CK(cudaEventRecord(ctx->call_start, ctx->stream));
     CK(cudaMemsetAsync(ctx->counters, 0, sizeof(u32) * kMaxCounters, ctx->stream));
     return 0;
@@ -423,57 +426,31 @@ int launch_pass(dark_bwt_ctx* ctx, const u64* kin, const u32* vin, u64* kout, u3
     return launch_pass_variant<256, 16, 3, 2>(ctx, kin, vin, kout, vout, m, shift, digit_base, counter, wide, prev_text, n_text, gen);
 }
 
-// Sort passes for a histogram that is already in ctx->hist (counts).  `cur` is the index of the
-// (keys, ids) pair holding the input; returns the index holding the output through *cur_out.
-//
-// Pass pruning (round 0 only, `prune`): an LSD sort of the top t digits alone orders the keys by
-// their leading 8t bits; whatever stays tied is finished by the doubling rounds.  With S_p the
-// probability that two keys share digit p (from the histogram), about m * prod(S_p) of the keys
-// keep a partner after the top t digits, IF the digits are independent.  That holds for
-// high-entropy blocks (packed DNA, random bytes) and fails badly for text, where a shallower
-// initial sort also slows every later round (h starts smaller).  So the low digits are dropped
-// only when every digit is close to uniform (S_p <= 1.5/256) and the estimate leaves < 1/64 of the
-// block tied; measured: C2 8 -> 5 passes + one 65,792-element round; C1/C5 unchanged.
-// *first_pass_out = index of the lowest digit that was sorted.
-int run_sort(dark_bwt_ctx* ctx, u64* const keys[2], u32* const vals[2], int cur, u32 m, int begin_bit, int num_passes,
-             int* cur_out, dark_bwt_stats* st, int round, bool prune = false, int* first_pass_out = nullptr,
-             const u8* patch_text = nullptr, bool* patched_out = nullptr, const KeyGen* gen = nullptr, bool* gen_used_out = nullptr,
-             bool all_passes = false) {
+// The digit statistics of the histograms in ctx->hist: mail->trivial[p] (every key has the same digit p) and
+// mail->collide[p] (the probability that two keys share it).  `wait`: the host reads them (one round trip).
+int scan_digits(dark_bwt_ctx* ctx, u32 m, int num_passes, bool wait) {
     // Scalar results (flags, counts, origin) are written by the kernels directly into mapped pinned host
     // memory and read after a stream sync.  A cudaMemcpy D2H would queue on the copy engine behind the
     // 256 MB block transfers of the pipelined batch entry (measured: +5 ms per block).
     k_scan_hist<<<num_passes, kRadix, 0, ctx->stream>>>(ctx->hist, m, ctx->mail_dev->trivial, ctx->mail_dev->collide);
     LAUNCHED();
-    // all_passes (a round that still holds more than n/8 suffixes): their ranks span at least m slots, so at most the
-    // top digit could be constant; every pass runs and the host does not wait for the flags (one round trip less per round)
-    if (!all_passes) CK(sync_counted(ctx));
-    int first = 0;
-    if (prune) {
-        for (int p = 0; p < num_passes; ++p)
-            if (ctx->mail->collide[p] > 1.5f / 256.0f) prune = false;  // not a high-entropy block
-    }
-    if (prune) {
-        double tied = (double)m;  // m * P(two keys agree on the top t digits) ~ fraction of keys left with a partner
-        int t = 0;
-        for (int p = num_passes - 1; p >= 0; --p) {
-            tied *= (double)ctx->mail->collide[p];
-            ++t;
-            if (tied * 64.0 <= 1.0) break;
-        }
-        first = num_passes - t;
-        if (first < 0) first = 0;
-    }
-    if (first_pass_out) *first_pass_out = first;
-    // pruned by at least one digit: the first pass that runs also drops the BWT byte into the low key byte
-    const u8* patch = (first >= 1) ? patch_text : nullptr;
+    if (wait) CK(sync_counted(ctx));
+    return 0;
+}
+
+// Radix passes first..num_passes-1 over the (keys, vals) pair *cur, for digits scanned by scan_digits; *cur follows the
+// data.  A trivial digit's pass is the identity and is skipped, unless `all_passes` (the flags were not waited for).
+// The first pass that runs builds its input from `gen` (if given) and drops the BWT byte from `patch_text` (if given)
+// into the low key byte.
+int sort_passes(dark_bwt_ctx* ctx, u64* const keys[2], u32* const vals[2], int* cur, u32 m, int begin_bit, int first, int num_passes,
+                dark_bwt_stats* st, int round, bool all_passes, const u8* patch_text, const KeyGen* gen) {
     int sp = span_begin(ctx, gen ? PH_GENPASS : PH_PASS);
     for (int p = first; p < num_passes; ++p) {
         if (!all_passes && ctx->mail->trivial[p]) continue;  // every key has the same digit: the pass is the identity
-        if (int rc = launch_pass(ctx, keys[cur], vals[cur], keys[cur ^ 1], vals[cur ^ 1], m, begin_bit + p * kRadixBits,
-                                 ctx->hist + p * kRadix, patch, m, gen))
+        if (int rc = launch_pass(ctx, keys[*cur], vals[*cur], keys[*cur ^ 1], vals[*cur ^ 1], m, begin_bit + p * kRadixBits,
+                                 ctx->hist + p * kRadix, patch_text, m, gen))
             return rc;
         if (gen) {  // only the first pass that runs builds its input; the later ones read what it wrote
-            if (gen_used_out) *gen_used_out = true;
             gen = nullptr;
             if (st) {
                 st->gen_passes += 1;
@@ -482,11 +459,8 @@ int run_sort(dark_bwt_ctx* ctx, u64* const keys[2], u32* const vals[2], int cur,
             span_end(ctx, sp);  // the key-generating launch is timed on its own (13 B per suffix, not 24)
             sp = span_begin(ctx, PH_PASS);
         }
-        if (patch) {
-            if (patched_out) *patched_out = true;
-            patch = nullptr;
-        }
-        cur ^= 1;
+        patch_text = nullptr;
+        *cur ^= 1;
         if (st) {
             st->sort_passes += 1;
             st->sorted_elements += m;
@@ -494,8 +468,18 @@ int run_sort(dark_bwt_ctx* ctx, u64* const keys[2], u32* const vals[2], int cur,
         }
     }
     span_end(ctx, sp);
-    *cur_out = cur;
     return 0;
+}
+
+// Sort passes for a histogram that is already in ctx->hist (counts).  `cur` is the index of the
+// (keys, ids) pair holding the input; returns the index holding the output through *cur_out.
+// all_passes (a round that still holds more than n/8 suffixes): their ranks span at least m slots, so at most the top digit
+// could be constant; every pass runs and the host does not wait for the flags (one round trip less per round).
+int run_sort(dark_bwt_ctx* ctx, u64* const keys[2], u32* const vals[2], int cur, u32 m, int begin_bit, int num_passes,
+             int* cur_out, dark_bwt_stats* st, int round, const KeyGen* gen = nullptr, bool all_passes = false) {
+    if (int rc = scan_digits(ctx, m, num_passes, !all_passes)) return rc;
+    *cur_out = cur;
+    return sort_passes(ctx, keys, vals, cur_out, m, begin_bit, 0, num_passes, st, round, all_passes, nullptr, gen);
 }
 
 struct PairSink {  // where a PAIRS re-rank puts its (id, rank) updates
@@ -504,9 +488,11 @@ struct PairSink {  // where a PAIRS re-rank puts its (id, rank) updates
     int shift = 0;
 };
 
+// `tag`: the bit isa[] entries of active suffixes carry (0: none).  *count_dev (if asked): the device copy of the
+// survivor count, beside the tile counter.
 template <bool ROUND0, bool PAIRS>
 int launch_rerank(dark_bwt_ctx* ctx, const u64* keys, const u32* ids, u32 m, u32 n, int K, int kb, u32* sa, u32* out_ids,
-                  const u8* text, u8* bwt_inline, PairSink sink = PairSink()) {
+                  const u8* text, u8* bwt_inline, u32 tag, const u32** count_dev, PairSink sink = PairSink()) {
     const u32 tiles = (u32)ceil_div(m, kScanTile);
     if (tiles > ctx->scan_tiles) return ctx->fail_internal("scan tile state too small");
     ScanTileState ts{ctx->scan_words};
@@ -514,7 +500,7 @@ int launch_rerank(dark_bwt_ctx* ctx, const u64* keys, const u32* ids, u32 m, u32
     u32 *counter = nullptr, *count_copy = nullptr;  // two consecutive words: the tile counter, then the survivor count (device copy)
     if (int rc = next_counter(ctx, &counter)) return rc;
     if (int rc = next_counter(ctx, &count_copy)) return rc;
-    ctx->count_dev = count_copy;
+    if (count_dev) *count_dev = count_copy;
     CK(cudaMemsetAsync(ctx->scan_words, 0, sizeof(u64) * kScanWordsPerTile * tiles, ctx->stream));
     const u32 prefetch_ahead = 2u * (u32)ctx->num_sms;  // one wave of CTAs ahead (-2 %)
     auto kern = k_rerank<kScanThreads, kScanItems, ROUND0, PAIRS>;
@@ -522,7 +508,7 @@ int launch_rerank(dark_bwt_ctx* ctx, const u64* keys, const u32* ids, u32 m, u32
     kern<<<tiles, kScanThreads, smem, ctx->stream>>>(
         keys, ids, ROUND0 ? nullptr : ctx->ranks, m, n, K, kb, ctx->isa, sa, out_ids, ROUND0 ? ctx->ranks : ctx->ranks_alt, ts, counter,
         &ctx->mail_dev->count, sink.ids, sink.vals,
-        ctx->bucket_hist, sink.shift, text, bwt_inline, &ctx->mail_dev->origin, prefetch_ahead, (ROUND0 && !PAIRS) ? 0u : ctx->tag);
+        ctx->bucket_hist, sink.shift, text, bwt_inline, &ctx->mail_dev->origin, prefetch_ahead, (ROUND0 && !PAIRS) ? 0u : tag);
     LAUNCHED();
     if (!ROUND0) std::swap(ctx->ranks, ctx->ranks_alt);
     return 0;
@@ -557,22 +543,6 @@ int region_scatter(dark_bwt_ctx* ctx, const u32* ids, const u32* vals, u32 upper
 int fetch_count(dark_bwt_ctx* ctx, u32* out) {
     CK(sync_counted(ctx));
     *out = ctx->mail->count;
-    return 0;
-}
-
-// Queues the pairs check (suffix_kernels.cuh, k_pairs_detect) behind the re-rank that has just been launched: it reads the
-// survivor count from the device copy the re-rank leaves beside its tile counter, and its answer (ctx->mail->not_pairs) arrives with that count in the
-// round trip the round makes anyway.  `upper` bounds the count.
-int queue_pairs_check(dark_bwt_ctx* ctx, u32 upper, bool* queued) {
-    *queued = false;
-    if (ctx->count_dev == nullptr) return 0;
-    u32* seen = nullptr;
-    if (int rc = next_counter(ctx, &seen)) return rc;
-    ctx->mail->not_pairs = 0;
-    const u32 grid = (u32)std::min<u64>(std::max<u64>(ceil_div(upper, 256), 1), (u64)ctx->num_sms * 4);
-    k_pairs_detect<<<grid, 256, 0, ctx->stream>>>(ctx->ranks, 0u, ctx->count_dev, seen, &ctx->mail_dev->not_pairs);
-    LAUNCHED();
-    *queued = true;
     return 0;
 }
 
@@ -623,149 +593,229 @@ void finish_stats(dark_bwt_ctx* ctx, dark_bwt_stats* st) {
     st->host_syncs = ctx->syncs;
 }
 
-// The whole forward transform on device buffers (2 <= n <= capacity).  d_sa_user nullable.
-int forward_device(dark_bwt_ctx* ctx, const u8* d_text, u32 n, u8* d_bwt, u64* origin_out, u32* d_sa_user, dark_bwt_stats* st) {
-    if (int rc = begin_call(ctx)) return rc;
-    reset_stats(st, n);
-    u32* sa = d_sa_user ? d_sa_user : ctx->sa;
+// ---- the forward transform of one block: a driver (forward_device) and one function per phase
+// State of one forward_device call that crosses its phases.
+struct Fwd {
+    const u8* text;
+    u32 n;
+    u8* bwt;
+    u32* sa;
+    dark_bwt_stats st = {};  // the call's stats, copied to the caller's record at the end
+    int s_bits = 8, K = 8;  // alphabet: bits per symbol code, symbols per 64-bit key
+    int cur = 0;            // the (keys, ids) pair holding the active list
+    u32 m = 0;              // active suffixes
+    u64 h = 0;              // leading symbols known equal inside each group
+    int round = 0;
+    int kb = 0, passes_r = 0;      // bits of a rank + 1, radix passes of a doubling round
+    // The initial sort covered the key bits above `drop`: K0 whole leading symbols are known equal inside a
+    // tie group, Kc symbols were touched (a suffix shorter than Kc had padding compared).
+    int K0 = 0, Kc = 0, drop = 0;
+    bool emit_inline = false;  // the re-ranks emit each suffix's BWT byte as it settles (no gather pass at the end)
+    u32 tag = 0;               // bit carried by isa[] entries of active suffixes (0: not used)
+    bool bucketed = false;     // rank scatters of more than n/16 ranks go through bucket regions of 2^bshift suffixes
+    int bshift = 0;
+    PairSink regions = {};     // the regions the fused round-0 re-rank filled with every suffix's rank (ids null: not fused)
+};
 
-    // ---- alphabet: sigma, dense codes, symbols per key
-    int sp = span_begin(ctx, PH_INIT);
+// Alphabet scan: sigma, dense codes (ctx->lut), bits per symbol and symbols per key.
+int scan_alphabet(dark_bwt_ctx* ctx, Fwd& f) {
     CK(cudaMemsetAsync(ctx->present, 0, sizeof(u32) * 256, ctx->stream));
     CK(cudaMemsetAsync(ctx->hist, 0, sizeof(u32) * kMaxPasses * kRadix, ctx->stream));
     const int no_pack = (ctx->flags & DARK_BWT_F_NO_ALPHABET_PACKING) ? 1 : 0;
-    {
-        const u32 blocks = (u32)std::min<u64>(ceil_div(ceil_div(n, 16), 256), 148 * 8);
-        k_symbol_presence<256><<<std::max(blocks, 1u), 256, 0, ctx->stream>>>(d_text, n, ctx->present);
-        LAUNCHED();
-        k_build_lut<<<1, 256, 0, ctx->stream>>>(ctx->present, ctx->lut, &ctx->mail_dev->sigma, no_pack);
-        LAUNCHED();
-    }
+    const u32 blocks = (u32)std::min<u64>(ceil_div(ceil_div(f.n, 16), 256), 148 * 8);
+    k_symbol_presence<256><<<std::max(blocks, 1u), 256, 0, ctx->stream>>>(f.text, f.n, ctx->present);
+    LAUNCHED();
+    k_build_lut<<<1, 256, 0, ctx->stream>>>(ctx->present, ctx->lut, &ctx->mail_dev->sigma, no_pack);
+    LAUNCHED();
     CK(sync_counted(ctx));
     const u32 sigma = ctx->mail->sigma;
     if (sigma < 1 || sigma > 256) return ctx->fail_internal("alphabet scan returned an impossible sigma");
-    const int s_bits = no_pack ? 8 : std::max(1, bit_length(sigma - 1));
-    const int K = 64 / s_bits;
-    const int passes0 = kMaxPasses;  // the symbol field is MSB-aligned in the 64-bit key
-    if (st) {
-        st->sigma = sigma;
-        st->bits_per_symbol = s_bits;
-        st->symbols_per_key = K;
-    }
+    f.s_bits = no_pack ? 8 : std::max(1, bit_length(sigma - 1));
+    f.K = 64 / f.s_bits;
+    f.st.sigma = sigma;
+    f.st.bits_per_symbol = f.s_bits;
+    f.st.symbols_per_key = f.K;
+    return 0;
+}
 
-    // ---- round 0: keys of K symbols, ids descending
-    // Fused initial keys (s in {1,2,4,8}): the digit histograms come from the text's q-grams (suffix_kernels.cuh) and
-    // the first radix pass that runs builds the keys from the text (radix_sort.cuh, GEN).
-    const Knobs& kn = ctx->knobs;
-    const bool packed_s = s_bits == 1 || s_bits == 2 || s_bits == 4 || s_bits == 8;
-    const int lg_s = s_bits == 1 ? 0 : s_bits == 2 ? 1 : s_bits == 4 ? 2 : 3;
-    // packed widths: the keys (write) or the digit histograms counted key by key (!write); other widths: both
-    auto init_keys = [&](bool write) -> int {
-        const u32 blocks = (u32)std::min<u64>(ceil_div(n, kInitThreads * kInitItems), (u64)ctx->num_sms * 8);
+// Widths whose keys the packed kernels build: s in {1, 2, 4, 8}
+bool packed_width(int s_bits) { return s_bits == 1 || s_bits == 2 || s_bits == 4 || s_bits == 8; }
+int lg_width(int s_bits) { return s_bits == 1 ? 0 : s_bits == 2 ? 1 : s_bits == 4 ? 2 : 3; }
+
+// Round-0 keys of K symbols, ids descending, with their digit histograms (packed widths: the keys (write) or the
+// digit histograms counted key by key (!write); other widths: both).  The symbol field is MSB-aligned in the 64-bit key.
+int init_keys(dark_bwt_ctx* ctx, const Fwd& f, bool write) {
+    const u32 blocks = (u32)std::min<u64>(ceil_div(f.n, kInitThreads * kInitItems), (u64)ctx->num_sms * 8);
 #define INIT_PACKED(S)                                                                                                              \
     do {                                                                                                                            \
         if (write)                                                                                                                  \
             k_init_keys_packed<kInitThreads, kInitItems, S, true><<<blocks, kInitThreads, 0, ctx->stream>>>(                        \
-                d_text, n, ctx->lut, ctx->keys[0], ctx->ids[0], ctx->hist);                                                         \
+                f.text, f.n, ctx->lut, ctx->keys[0], ctx->ids[0], ctx->hist);                                                       \
         else                                                                                                                        \
             k_init_keys_packed<kInitThreads, kInitItems, S, false><<<blocks, kInitThreads, 0, ctx->stream>>>(                       \
-                d_text, n, ctx->lut, nullptr, nullptr, ctx->hist);                                                                  \
+                f.text, f.n, ctx->lut, nullptr, nullptr, ctx->hist);                                                                \
     } while (0)
-        switch (s_bits) {
-            case 1: INIT_PACKED(1); break;
-            case 2: INIT_PACKED(2); break;
-            case 4: INIT_PACKED(4); break;
-            case 8: INIT_PACKED(8); break;
-            default:
-                k_init_keys<kInitThreads, kInitItems><<<blocks, kInitThreads, 0, ctx->stream>>>(
-                    d_text, n, ctx->lut, s_bits, K, ctx->keys[0], ctx->ids[0], ctx->hist, passes0);
-        }
-#undef INIT_PACKED
-        LAUNCHED();
-        return 0;
-    };
-    if (packed_s) {
-        u32* gram = ctx->bucket_hist;  // 256 counters, free until the first rank scatter
-        CK(cudaMemsetAsync(gram, 0, sizeof(u32) * kRadix, ctx->stream));
-        const u32 blocks = (u32)std::min<u64>(ceil_div(n, 256 * 16), (u64)ctx->num_sms * 8);
-        switch (s_bits) {
-            case 1: k_gram_hist<256, 1><<<blocks, 256, 0, ctx->stream>>>(d_text, n, ctx->lut, gram); break;
-            case 2: k_gram_hist<256, 2><<<blocks, 256, 0, ctx->stream>>>(d_text, n, ctx->lut, gram); break;
-            case 4: k_gram_hist<256, 4><<<blocks, 256, 0, ctx->stream>>>(d_text, n, ctx->lut, gram); break;
-            default: k_gram_hist<256, 8><<<blocks, 256, 0, ctx->stream>>>(d_text, n, ctx->lut, gram); break;
-        }
-        LAUNCHED();
-        k_gram_expand<<<1, kRadix, 0, ctx->stream>>>(d_text, n, ctx->lut, lg_s, gram, ctx->hist);
-        LAUNCHED();
-        if (kn.check_hist) {  // test hook: compare with the histogram counted key by key
-            std::vector<u32> a(kMaxPasses * kRadix), b(kMaxPasses * kRadix);
-            CK(cudaMemcpyAsync(a.data(), ctx->hist, a.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
-            CK(cudaMemsetAsync(ctx->hist, 0, sizeof(u32) * kMaxPasses * kRadix, ctx->stream));
-            if (int rc = init_keys(false)) return rc;
-            CK(cudaMemcpyAsync(b.data(), ctx->hist, b.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
-            CK(sync_counted(ctx));
-            if (a != b) return ctx->fail_internal("q-gram histogram differs from the per-key histogram");
-            CK(cudaMemcpyAsync(ctx->hist, a.data(), a.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
-            CK(sync_counted(ctx));
-        }
-    } else {
-        if (int rc = init_keys(true)) return rc;
+    switch (f.s_bits) {
+        case 1: INIT_PACKED(1); break;
+        case 2: INIT_PACKED(2); break;
+        case 4: INIT_PACKED(4); break;
+        case 8: INIT_PACKED(8); break;
+        default:
+            k_init_keys<kInitThreads, kInitItems><<<blocks, kInitThreads, 0, ctx->stream>>>(
+                f.text, f.n, ctx->lut, f.s_bits, f.K, ctx->keys[0], ctx->ids[0], ctx->hist, kMaxPasses);
     }
-    span_end(ctx, sp);
+#undef INIT_PACKED
+    LAUNCHED();
+    return 0;
+}
 
-    int cur = 0;
-    int first_pass = 0;
-    sp = span_begin(ctx, PH_SORT);
+// Round 0, the digit histograms (and, for widths without a fused key build, the keys).  Packed widths: the histograms
+// come from the text's q-grams (suffix_kernels.cuh) and the first radix pass that runs builds the keys from the text
+// (radix_sort.cuh, GEN).
+int round0_keys(dark_bwt_ctx* ctx, const Fwd& f) {
+    if (!packed_width(f.s_bits)) return init_keys(ctx, f, true);
+    u32* gram = ctx->bucket_hist;  // 256 counters, free until the first rank scatter
+    CK(cudaMemsetAsync(gram, 0, sizeof(u32) * kRadix, ctx->stream));
+    const u32 blocks = (u32)std::min<u64>(ceil_div(f.n, 256 * 16), (u64)ctx->num_sms * 8);
+    switch (f.s_bits) {
+        case 1: k_gram_hist<256, 1><<<blocks, 256, 0, ctx->stream>>>(f.text, f.n, ctx->lut, gram); break;
+        case 2: k_gram_hist<256, 2><<<blocks, 256, 0, ctx->stream>>>(f.text, f.n, ctx->lut, gram); break;
+        case 4: k_gram_hist<256, 4><<<blocks, 256, 0, ctx->stream>>>(f.text, f.n, ctx->lut, gram); break;
+        default: k_gram_hist<256, 8><<<blocks, 256, 0, ctx->stream>>>(f.text, f.n, ctx->lut, gram); break;
+    }
+    LAUNCHED();
+    k_gram_expand<<<1, kRadix, 0, ctx->stream>>>(f.text, f.n, ctx->lut, lg_width(f.s_bits), gram, ctx->hist);
+    LAUNCHED();
+    if (ctx->knobs.check_hist) {  // test hook: compare with the histogram counted key by key
+        std::vector<u32> a(kMaxPasses * kRadix), b(kMaxPasses * kRadix);
+        CK(cudaMemcpyAsync(a.data(), ctx->hist, a.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaMemsetAsync(ctx->hist, 0, sizeof(u32) * kMaxPasses * kRadix, ctx->stream));
+        if (int rc = init_keys(ctx, f, false)) return rc;
+        CK(cudaMemcpyAsync(b.data(), ctx->hist, b.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(sync_counted(ctx));
+        if (a != b) return ctx->fail_internal("q-gram histogram differs from the per-key histogram");
+        CK(cudaMemcpyAsync(ctx->hist, a.data(), a.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
+        CK(sync_counted(ctx));
+    }
+    return 0;
+}
+
+// Pass pruning of the initial sort: an LSD sort of the top t digits alone orders the keys by their leading 8t bits;
+// whatever stays tied is finished by the doubling rounds.  With S_p the probability that two keys share digit p (from
+// the histogram), about m * prod(S_p) of the keys keep a partner after the top t digits, IF the digits are independent.
+// That holds for high-entropy blocks (packed DNA, random bytes) and fails badly for text, where a shallower initial
+// sort also slows every later round (h starts smaller).  So the low digits are dropped only when every digit is close
+// to uniform (S_p <= 1.5/256) and the estimate leaves < 1/64 of the block tied; measured: C2 8 -> 5 passes + one
+// 65,792-element round; C1/C5 unchanged.  Returns the lowest digit to sort.
+int round0_first_digit(const Mailbox* mail, u32 m) {
+    for (int p = 0; p < kMaxPasses; ++p)
+        if (mail->collide[p] > 1.5f / 256.0f) return 0;  // not a high-entropy block
+    double tied = (double)m;  // m * P(two keys agree on the top t digits) ~ fraction of keys left with a partner
+    int t = 0;
+    for (int p = kMaxPasses - 1; p >= 0; --p) {
+        tied *= (double)mail->collide[p];
+        ++t;
+        if (tied * 64.0 <= 1.0) break;
+    }
+    return std::max(0, kMaxPasses - t);
+}
+
+// Round 0, the sort: every digit, or the top ones of a pruned block (round0_first_digit; not without alphabet packing).
+int round0_sort(dark_bwt_ctx* ctx, Fwd& f) {
+    int sp = span_begin(ctx, PH_SORT);
+    if (int rc = scan_digits(ctx, f.n, kMaxPasses, true)) return rc;
+    const int first = (ctx->flags & DARK_BWT_F_NO_ALPHABET_PACKING) ? 0 : round0_first_digit(ctx->mail, f.n);
     // Inline emission: when the initial sort is pruned by >= 1 digit the BWT byte of each suffix travels in
     // the (unsorted) low key byte and is emitted as the suffix settles; no gather pass at the end.
-    const bool want_inline = kn.inline_emit;
-    bool emit_inline = false;
-    KeyGen gen;
-    gen.text = d_text;
-    gen.lut = ctx->lut;
-    gen.n = n;
-    gen.lg_s = lg_s;
-    gen.mode = 0;
-    gen.origin = 0;
-    bool gen_used = false;
-    if (int rc = run_sort(ctx, ctx->keys, ctx->ids, cur, n, 0, passes0, &cur, st, 0, /*prune=*/!no_pack, &first_pass,
-                          want_inline ? d_text : nullptr, &emit_inline, packed_s ? &gen : nullptr, &gen_used))
-        return rc;
-    if (packed_s && !gen_used) {  // every digit was trivial (one-symbol text): no pass ran, the re-rank still wants the keys
-        if (int rc = init_keys(true)) return rc;
-        cur = 0;
-    }
-    span_end(ctx, sp);
     // An unpruned block emits in a final gather pass.  Emitting it inline instead, the re-rank gathering T[id-1] for every
     // suffix as it settles, measured equal (C4: re-rank +38 ms, emission -37 ms: one random DRAM sector per suffix wherever
     // the read is issued, profiles/r2_rejected.md).
-    u8* bwt_inline = emit_inline ? d_bwt : nullptr;
-    // The sort covered the key bits above `drop`: K0 whole leading symbols are known equal inside a
-    // tie group, Kc symbols were touched (a suffix shorter than Kc had padding compared).
-    const int drop = first_pass * kRadixBits;
-    const int sorted_bits = 64 - drop;
-    const int K0 = std::min(K, sorted_bits / s_bits);
-    const int Kc = std::min(K, (sorted_bits + s_bits - 1) / s_bits);
-    if (K0 < 1) return ctx->fail_internal("initial sort covered less than one symbol");
-    if (st) st->initial_symbols = K0;
+    const bool patch = first >= 1 && ctx->knobs.inline_emit;
+    const bool packed = packed_width(f.s_bits);
+    const KeyGen gen{f.text, ctx->lut, f.n, lg_width(f.s_bits), 0, 0};
+    if (int rc = sort_passes(ctx, ctx->keys, ctx->ids, &f.cur, f.n, 0, first, kMaxPasses, &f.st, 0, false, patch ? f.text : nullptr,
+                             packed ? &gen : nullptr))
+        return rc;
+    const bool sorted = f.st.passes[0] > 0;  // some digit was not trivial
+    f.emit_inline = patch && sorted;
+    if (packed && !sorted) {  // every digit was trivial (one-symbol text): no pass ran, the re-rank still wants the keys
+        if (int rc = init_keys(ctx, f, true)) return rc;
+        f.cur = 0;
+    }
+    span_end(ctx, sp);
+    f.drop = first * kRadixBits;
+    const int sorted_bits = 64 - f.drop;
+    f.K0 = std::min(f.K, sorted_bits / f.s_bits);
+    f.Kc = std::min(f.K, (sorted_bits + f.s_bits - 1) / f.s_bits);
+    if (f.K0 < 1) return ctx->fail_internal("initial sort covered less than one symbol");
+    f.st.initial_symbols = f.K0;
+    f.kb = bit_length(f.n);  // rank2 = isa+1 in [0, n]
+    const int key_bits = f.kb + bit_length(((u64)f.n - 1) >> 1);  // high part = rank >> 1 (suffix_kernels.cuh, k_rerank)
+    f.passes_r = (key_bits + kRadixBits - 1) / kRadixBits;
+    return 0;
+}
 
-    const int kb = bit_length(n);  // rank2 = isa+1 in [0, n]
-    const int key_bits = kb + bit_length(((u64)n - 1) >> 1);  // high part = rank >> 1 (suffix_kernels.cuh, k_rerank)
-    const int passes_r = (key_bits + kRadixBits - 1) / kRadixBits;
+// Pairs mode: once every remaining group is a pair the rounds switch to the pairs kernel for good (groups only ever
+// split).  The check reads the rank list once; queued behind a re-rank (k_pairs_detect reads the survivor count from the
+// device copy the re-rank leaves), its answer (mail->not_pairs) arrives with that count in the round trip the round makes
+// anyway.  Otherwise it costs a round trip of its own, so it is skipped while most of the block is still active
+// (period-17: ten rounds of giant groups).  The kernel gathers from isa[], so it waits until every rank is there (few
+// survivors after round 0: the selective rounds).  DARK_BWT_PAIRS=0 switches it off.
+struct PairsMode {
+    bool enabled = true;
+    bool on = false;
+    bool checked = false;  // the check of the current list was queued behind its re-rank: the answer is in the mailbox
 
-    sp = span_begin(ctx, PH_RERANK);
-    u32 m = 0;
+    // After the re-rank of round f.round has been launched, with `upper` >= its survivor count.
+    int queue(dark_bwt_ctx* ctx, const Fwd& f, bool isa_complete, const u32* count_dev, u32 upper) {
+        if (!enabled || (f.round > 0 && !(isa_complete && upper <= f.n / 2))) return 0;
+        u32* seen = nullptr;
+        if (int rc = next_counter(ctx, &seen)) return rc;
+        ctx->mail->not_pairs = 0;
+        const u32 grid = (u32)std::min<u64>(std::max<u64>(ceil_div(upper, 256), 1), (u64)ctx->num_sms * 4);
+        k_pairs_detect<<<grid, 256, 0, ctx->stream>>>(ctx->ranks, 0u, count_dev, seen, &ctx->mail_dev->not_pairs);
+        LAUNCHED();
+        checked = true;
+        return 0;
+    }
+
+    // At the top of a round, with its f.m active suffixes: switches pairs mode on if every group is a pair.
+    int decide(dark_bwt_ctx* ctx, const Fwd& f, bool isa_complete) {
+        if (enabled && !on && isa_complete && (f.m & 1u) == 0 && (f.round == 1 || f.m <= f.n / 2)) {
+            if (checked) {  // answered in the round trip that fetched m
+                on = ctx->mail->not_pairs == 0;
+            } else {
+                ctx->mail->flag = 0;
+                u32* seen = nullptr;
+                if (int rc = next_counter(ctx, &seen)) return rc;
+                k_pairs_detect<<<(u32)std::min<u64>(ceil_div(f.m, 256), (u64)ctx->num_sms * 8), 256, 0, ctx->stream>>>(
+                    ctx->ranks, f.m, nullptr, seen, &ctx->mail_dev->flag);
+                LAUNCHED();
+                CK(sync_counted(ctx));
+                on = ctx->mail->flag == 0;
+            }
+        }
+        checked = false;
+        return 0;
+    }
+};
+
+// Round 0, the re-rank: settles the suffixes whose group is a singleton, compacts the others into ids[cur ^ 1] and
+// fetches their count.
+int round0_rerank(dark_bwt_ctx* ctx, Fwd& f, PairsMode& pairs) {
+    const Knobs& kn = ctx->knobs;
+    u8* bwt_inline = f.emit_inline ? f.bwt : nullptr;
+    int sp = span_begin(ctx, PH_RERANK);
     bool sparse_done = false;
-    bool pairs_checked = false;  // the pairs check of the current list was queued behind its re-rank: the answer is in the mailbox
     // Pruned initial sort with inline emission (high-entropy block: almost everything settles): the chain-free
     // sparse re-rank (suffix_kernels.cuh).  DARK_BWT_SPARSE_RERANK=0 keeps the scan-based kernel.
-    if (emit_inline && first_pass >= 1 && kn.sparse_rerank) {
+    if (f.emit_inline && kn.sparse_rerank) {
         u32 *total = nullptr, *ovf = nullptr;
         if (int rc = next_counter(ctx, &total)) return rc;
         if (int rc = next_counter(ctx, &ovf)) return rc;
-        const u32 tiles = (u32)ceil_div(n, kScanTile);
+        const u32 tiles = (u32)ceil_div(f.n, kScanTile);
         k_rerank0_sparse<kScanThreads, kScanItems><<<tiles, kScanThreads, 0, ctx->stream>>>(
-            ctx->keys[cur], ctx->ids[cur], n, Kc, drop, sa, bwt_inline, &ctx->mail_dev->origin, (u8*)ctx->bitmap, total);
+            ctx->keys[f.cur], ctx->ids[f.cur], f.n, f.Kc, f.drop, f.sa, bwt_inline, &ctx->mail_dev->origin, (u8*)ctx->bitmap, total);
         LAUNCHED();
         k_copy_u32<<<1, 1, 0, ctx->stream>>>(total, &ctx->mail_dev->count);
         LAUNCHED();
@@ -773,8 +823,8 @@ int forward_device(dark_bwt_ctx* ctx, const u8* d_text, u32 n, u8* d_bwt, u64* o
         if (int rc = fetch_count(ctx, &survivors)) return rc;
         if (survivors == 0) {
             sparse_done = true;
-        } else if (survivors <= n / 16) {
-            const u64 nbytes = ceil_div(n, 8);
+        } else if (survivors <= f.n / 16) {
+            const u64 nbytes = ceil_div(f.n, 8);
             const u32 nblocks = (u32)ceil_div(nbytes, kSparseChunk);
             u32* counts = (u32*)ctx->scan_words;  // n/32768 counters; the scan state is not in use
             u32* pos = ctx->ranks_alt;
@@ -784,234 +834,233 @@ int forward_device(dark_bwt_ctx* ctx, const u8* d_text, u32 n, u8* d_bwt, u64* o
             LAUNCHED();
             k_sparse_positions<<<nblocks, 256, 0, ctx->stream>>>((const u8*)ctx->bitmap, nbytes, counts, pos);
             LAUNCHED();
-            k_sparse_finalize<<<(u32)ceil_div(survivors, 256), 256, 0, ctx->stream>>>(pos, survivors, ctx->keys[cur], ctx->ids[cur], n, Kc, drop,
-                                                                                 ctx->ids[cur ^ 1], ctx->ranks, ovf);
+            k_sparse_finalize<<<(u32)ceil_div(survivors, 256), 256, 0, ctx->stream>>>(pos, survivors, ctx->keys[f.cur], ctx->ids[f.cur], f.n,
+                                                                                 f.Kc, f.drop, ctx->ids[f.cur ^ 1], ctx->ranks, ovf);
             LAUNCHED();
             k_copy_u32<<<1, 1, 0, ctx->stream>>>(ovf, &ctx->mail_dev->flag);
             LAUNCHED();
             CK(sync_counted(ctx));
             if (ctx->mail->flag == 0) {
                 sparse_done = true;
-                m = survivors;
+                f.m = survivors;
             }
         }
     }
     // isa[] entries of active suffixes carry bit 31 (blocks up to 2^31 bytes): the text-order key builder finds
     // them by it.  DARK_BWT_TEXT_BUILD=0 switches tag and builder off; =<k> uses the builder while m > n/k.
-    const int text_div = kn.text_div;
-    const u32 tag = (text_div > 0 && (u64)n <= (1ull << 31)) ? 0x80000000u : 0u;
-    ctx->tag = tag;
+    f.tag = (kn.text_div > 0 && (u64)f.n <= (1ull << 31)) ? 0x80000000u : 0u;
     // Scatters of more than n/16 ranks into an isa[] that outgrows L2 go through the bucketed path.
-    const bool bucketed = kn.bucketed >= 0 ? kn.bucketed != 0 : ((u64)n * 4 > (96ull << 20));
-    const int bshift = std::max(0, bit_length((u64)n - 1) - 8);
-    // A large block whose initial sort was not pruned is text-like: most suffixes survive round 0 and every rank is needed.
-    // Its round-0 re-rank then feeds the bucket regions of the rank scatter itself (every suffix reports its rank, settled
-    // ones their slot) instead of two partition passes over the SA and the survivor list afterwards.  DARK_BWT_FUSE_ROUND0=0
-    // keeps the separate passes.
-    const bool fused0 = !sparse_done && bucketed && first_pass == 0 && kn.fuse_round0;
-    PairSink sink0;
+    f.bucketed = kn.bucketed >= 0 ? kn.bucketed != 0 : ((u64)f.n * 4 > (96ull << 20));
+    f.bshift = std::max(0, bit_length((u64)f.n - 1) - 8);
     if (!sparse_done) {
-        if (fused0) {
-            sink0.ids = (u32*)ctx->keys[cur ^ 1];
-            sink0.vals = sink0.ids + align_up((size_t)n, 64);
-            sink0.shift = bshift;
+        // A large block whose initial sort was not pruned is text-like: most suffixes survive round 0 and every rank is
+        // needed.  Its round-0 re-rank then feeds the bucket regions of the rank scatter itself (every suffix reports its
+        // rank, settled ones their slot) instead of two partition passes over the SA and the survivor list afterwards.
+        // DARK_BWT_FUSE_ROUND0=0 keeps the separate passes.
+        const u32* count_dev = nullptr;
+        if (f.bucketed && f.drop == 0 && kn.fuse_round0) {
+            u32* ids = (u32*)ctx->keys[f.cur ^ 1];
+            f.regions = PairSink{ids, ids + align_up((size_t)f.n, 64), f.bshift};
             CK(cudaMemsetAsync(ctx->bucket_hist, 0, sizeof(u32) * 256, ctx->stream));
-            if (int rc = launch_rerank<true, true>(ctx, ctx->keys[cur], ctx->ids[cur], n, n, Kc, drop, sa, ctx->ids[cur ^ 1], d_text, bwt_inline, sink0)) return rc;
+            if (int rc = launch_rerank<true, true>(ctx, ctx->keys[f.cur], ctx->ids[f.cur], f.n, f.n, f.Kc, f.drop, f.sa, ctx->ids[f.cur ^ 1],
+                                                   f.text, bwt_inline, f.tag, &count_dev, f.regions))
+                return rc;
         } else {
-            if (int rc = launch_rerank<true, false>(ctx, ctx->keys[cur], ctx->ids[cur], n, n, Kc, drop, sa, ctx->ids[cur ^ 1], d_text, bwt_inline)) return rc;
+            if (int rc = launch_rerank<true, false>(ctx, ctx->keys[f.cur], ctx->ids[f.cur], f.n, f.n, f.Kc, f.drop, f.sa, ctx->ids[f.cur ^ 1],
+                                                    f.text, bwt_inline, f.tag, &count_dev))
+                return rc;
         }
-        if (kn.pairs)
-            if (int rc = queue_pairs_check(ctx, n, &pairs_checked)) return rc;
-        if (int rc = fetch_count(ctx, &m)) return rc;
+        if (int rc = pairs.queue(ctx, f, true, count_dev, f.n)) return rc;
+        if (int rc = fetch_count(ctx, &f.m)) return rc;
     }
     span_end(ctx, sp);
-    cur ^= 1;  // the compacted active ids now live in ids[cur]
+    f.cur ^= 1;  // the compacted active ids now live in ids[cur]
+    return 0;
+}
 
-    // Round 0 wrote no ranks.  If a round follows they are needed: all of them when many suffixes
-    // survive; otherwise only the survivors' now, and per round the few that are actually read.
-    bool isa_complete = true;
+// Which ranks isa[] holds.  Round 0 writes none.  If a round follows they are needed: all of them when many suffixes
+// survive; otherwise only the survivors' now, and per round the few that are actually read.
+struct RankFill {
+    bool complete = true;  // every rank a round may read is in isa[]
     int selective_rounds = 0;
-    const bool use_pairs = kn.pairs;
-    bool pairs_mode = false;
-    const bool use_search = kn.rank_search;
-    if (m > 0 && fused0) {  // the regions hold every suffix's rank already
-        sp = span_begin(ctx, PH_RERANK);
-        if (int rc = region_scatter(ctx, sink0.ids, sink0.vals, n, bshift)) return rc;
-        span_end(ctx, sp);
-    } else if (m > 0) {
-        sp = span_begin(ctx, PH_RERANK);
-        if (m > n / 16) {
-            if (bucketed) {  // every suffix gets its rank: settled ones their slot, survivors their group rank
-                CK(cudaMemsetAsync(ctx->bucket_hist, 0, sizeof(u32) * 256, ctx->stream));
-                u32* oi = (u32*)ctx->keys[0];
-                u32* ov = (u32*)ctx->keys[1];
-                if (int rc = bucket_partition(ctx, sa, nullptr, n, bshift, oi, ov)) return rc;
-                if (int rc = bucket_partition(ctx, ctx->ids[cur], ctx->ranks, m, bshift, oi, ov, tag)) return rc;
-                if (int rc = region_scatter(ctx, oi, ov, n, bshift)) return rc;
-            } else {
-                k_round0_isa<256><<<(u32)ceil_div(n, 256), 256, 0, ctx->stream>>>(sa, n, ctx->ids[cur], ctx->ranks, m, ctx->isa, tag);
-                LAUNCHED();
-            }
-        } else {
-            k_scatter_ranks<256><<<(u32)ceil_div(m, 256), 256, 0, ctx->stream>>>(ctx->ids[cur], ctx->ranks, m, ctx->isa, tag);
-            LAUNCHED();
-            isa_complete = false;
-        }
-        span_end(ctx, sp);
-    }
 
-    // ---- doubling rounds
-    u64 h = (u64)K0;
-    int round = 1;
-    while (m > 0) {
-        if (round >= DARK_BWT_MAX_ROUNDS || h >= 2 * (u64)n + 2) return ctx->fail_internal("prefix doubling did not converge");
-        if (st) {
-            st->active[round] = m;
-            st->rounds = round;
-        }
-        // Once every remaining group is a pair the rounds switch to the pairs kernel for good (groups
-        // only ever split).  The check reads the rank list once and costs a host round trip, so it is skipped
-        // while most of the block is still active (period-17: ten rounds of giant groups).  The kernel gathers
-        // from isa[], so it waits until every rank is there (few survivors after round 0: the selective rounds).
-        if (use_pairs && !pairs_mode && isa_complete && (m & 1u) == 0 && (round == 1 || m <= n / 2)) {
-            if (pairs_checked) {  // answered in the round trip that fetched m
-                if (ctx->mail->not_pairs == 0) pairs_mode = true;
-            } else {
-                ctx->mail->flag = 0;
-                u32* seen = nullptr;
-                if (int rc = next_counter(ctx, &seen)) return rc;
-                k_pairs_detect<<<(u32)std::min<u64>(ceil_div(m, 256), (u64)ctx->num_sms * 8), 256, 0, ctx->stream>>>(ctx->ranks, m, nullptr, seen,
-                                                                                                                    &ctx->mail_dev->flag);
-                LAUNCHED();
-                CK(sync_counted(ctx));
-                if (ctx->mail->flag == 0) {
-                    pairs_mode = true;
+    // After round 0 (f.round == 0, survivors left), or before the key build of round f.round; *keys_built: this fill
+    // built the round's keys too.
+    int fill(dark_bwt_ctx* ctx, const Fwd& f, bool* keys_built) {
+        if (f.round == 0) {
+            int sp = span_begin(ctx, PH_RERANK);
+            if (f.regions.ids) {  // the regions hold every suffix's rank already
+                if (int rc = region_scatter(ctx, f.regions.ids, f.regions.vals, f.n, f.bshift)) return rc;
+            } else if (f.m > f.n / 16) {
+                if (f.bucketed) {  // every suffix gets its rank: settled ones their slot, survivors their group rank
+                    CK(cudaMemsetAsync(ctx->bucket_hist, 0, sizeof(u32) * 256, ctx->stream));
+                    u32* oi = (u32*)ctx->keys[0];
+                    u32* ov = (u32*)ctx->keys[1];
+                    if (int rc = bucket_partition(ctx, f.sa, nullptr, f.n, f.bshift, oi, ov)) return rc;
+                    if (int rc = bucket_partition(ctx, ctx->ids[f.cur], ctx->ranks, f.m, f.bshift, oi, ov, f.tag)) return rc;
+                    if (int rc = region_scatter(ctx, oi, ov, f.n, f.bshift)) return rc;
+                } else {
+                    k_round0_isa<256><<<(u32)ceil_div(f.n, 256), 256, 0, ctx->stream>>>(f.sa, f.n, ctx->ids[f.cur], ctx->ranks, f.m, ctx->isa, f.tag);
+                    LAUNCHED();
                 }
+            } else {
+                k_scatter_ranks<256><<<(u32)ceil_div(f.m, 256), 256, 0, ctx->stream>>>(ctx->ids[f.cur], ctx->ranks, f.m, ctx->isa, f.tag);
+                LAUNCHED();
+                complete = false;
             }
-        }
-        pairs_checked = false;
-        if (pairs_mode) {
-            // every group is a pair: one kernel settles or keeps each pair (suffix_kernels.cuh, "pairs mode")
-            sp = span_begin(ctx, PH_RERANK);
-            constexpr int kPairThreads = 256, kPairsPerThread = 8;  // 4096 elements per tile, like the re-rank
-            const u32 tiles = (u32)ceil_div(m / 2, kPairThreads * kPairsPerThread);
-            if (tiles > ctx->scan_tiles) return ctx->fail_internal("scan tile state too small");
-            u32* counter = nullptr;
-            if (int rc = next_counter(ctx, &counter)) return rc;
-            CK(cudaMemsetAsync(ctx->scan_words, 0, sizeof(u64) * kScanWordsPerTile * tiles, ctx->stream));
-            ScanTileState ts{ctx->scan_words};
-            k_pairs_round<kPairThreads, kPairsPerThread><<<tiles, kPairThreads, 0, ctx->stream>>>(
-                ctx->ids[cur], ctx->ranks, m, n, h, ctx->isa, reinterpret_cast<uint2*>(ctx->keys[0]), sa, ctx->ids[cur ^ 1], ctx->ranks_alt, ts, counter,
-                &ctx->mail_dev->count, d_text, bwt_inline, &ctx->mail_dev->origin, tag);
-            LAUNCHED();
-            std::swap(ctx->ranks, ctx->ranks_alt);
             span_end(ctx, sp);
-            cur ^= 1;
-            if (st) st->pair_rounds += 1;
-            const u32 m_before = m;
-            if (int rc = fetch_count(ctx, &m)) return rc;
-            if (const u32 settled = (m_before - m) / 2) {
-                k_pairs_apply<<<(u32)ceil_div(settled, 256), 256, 0, ctx->stream>>>(reinterpret_cast<const uint2*>(ctx->keys[0]), settled, ctx->isa);
-                LAUNCHED();
-            }
-            h *= 2;
-            ++round;
-            continue;
+            return 0;
         }
-        sp = span_begin(ctx, PH_KEYBUILD);
-        CK(cudaMemsetAsync(ctx->hist, 0, sizeof(u32) * kMaxPasses * kRadix, ctx->stream));
-        bool keys_built = false;
-        if (!isa_complete) {
-            // ranks of suffixes settled in round 0 exist only where they are about to be read
-            if (round == 1 && use_search) {
-                // round 1: read the ranks off the sorted round-0 keys (still intact in keys[cur^1] / ids[cur^1])
-                k_build_keys_search<256><<<(u32)ceil_div(m, 256), 256, 0, ctx->stream>>>(
-                    ctx->ids[cur], ctx->ranks, m, n, h, kb, ctx->keys[cur ^ 1], ctx->ids[cur ^ 1], d_text, ctx->lut, s_bits, K, Kc,
-                    drop, ctx->keys[cur], ctx->hist, passes_r);
-                LAUNCHED();
-                keys_built = true;
-            } else if (selective_rounds < 2) {
-                const size_t words = (size_t)ceil_div(n, 32);
-                CK(cudaMemsetAsync(ctx->bitmap, 0, words * sizeof(u32), ctx->stream));
-                k_mark_needed<256><<<(u32)ceil_div(m, 256), 256, 0, ctx->stream>>>(ctx->ids[cur], m, n, h, ctx->bitmap);
-                LAUNCHED();
-                k_fill_needed<256><<<(u32)ceil_div(n, 256), 256, 0, ctx->stream>>>(sa, n, ctx->bitmap, ctx->isa);
-                LAUNCHED();
-                ++selective_rounds;
-            } else {  // still not done after two rounds: fill every settled rank once
-                k_round0_isa<256><<<(u32)ceil_div(n, 256), 256, 0, ctx->stream>>>(sa, n, ctx->ids[cur], ctx->ranks, 0u, ctx->isa, tag);
-                LAUNCHED();
-                isa_complete = true;
-            }
-        }
-        bool text_built = false;
-        if (!keys_built && tag != 0 && isa_complete && (u64)m * (u64)text_div > (u64)n) {
-            // many suffixes still active: sweep isa[] in text order instead of gathering from it (k_build_keys_text)
-            constexpr int kTextThreads = 512, kTextItems = 8;
-            const u32 tiles = (u32)ceil_div(n, kTextThreads * kTextItems);
-            if (tiles > ctx->scan_tiles) return ctx->fail_internal("scan tile state too small");
-            u32* counter = nullptr;
-            if (int rc = next_counter(ctx, &counter)) return rc;
-            CK(cudaMemsetAsync(ctx->scan_words, 0, sizeof(u64) * kScanWordsPerTile * tiles, ctx->stream));
-            auto kern = k_build_keys_text<kTextThreads, kTextItems>;
-            const size_t smem = kBuildTextSmem<kTextThreads, kTextItems>;
-            CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            const u32 grid = std::min<u32>(tiles, (u32)ctx->num_sms * 3);
-            kern<<<grid, kTextThreads, smem, ctx->stream>>>(ctx->isa, n, h, kb, tag, ctx->keys[cur], ctx->ids[cur], ctx->scan_words, counter,
-                                                            &ctx->mail_dev->flag, ctx->hist, passes_r);
+        if (complete) return 0;
+        // ranks of suffixes settled in round 0 exist only where they are about to be read
+        if (f.round == 1 && ctx->knobs.rank_search) {
+            // round 1: read the ranks off the sorted round-0 keys (still intact in keys[cur^1] / ids[cur^1])
+            k_build_keys_search<256><<<(u32)ceil_div(f.m, 256), 256, 0, ctx->stream>>>(
+                ctx->ids[f.cur], ctx->ranks, f.m, f.n, f.h, f.kb, ctx->keys[f.cur ^ 1], ctx->ids[f.cur ^ 1], f.text, ctx->lut, f.s_bits, f.K,
+                f.Kc, f.drop, ctx->keys[f.cur], ctx->hist, f.passes_r);
             LAUNCHED();
-            keys_built = true;
-            text_built = true;
-        }
-        if (!keys_built) {
-            const u32 blocks = (u32)ceil_div(m, kBuildThreads * kBuildItems);  // one tile per CTA: the gathers want every warp slot filled
-            k_build_keys<kBuildThreads, kBuildItems><<<blocks, kBuildThreads, 0, ctx->stream>>>(
-                ctx->ids[cur], ctx->ranks, m, n, h, kb, ctx->isa, tag, ctx->keys[cur], ctx->hist, passes_r);
+            *keys_built = true;
+        } else if (selective_rounds < 2) {
+            const size_t words = (size_t)ceil_div(f.n, 32);
+            CK(cudaMemsetAsync(ctx->bitmap, 0, words * sizeof(u32), ctx->stream));
+            k_mark_needed<256><<<(u32)ceil_div(f.m, 256), 256, 0, ctx->stream>>>(ctx->ids[f.cur], f.m, f.n, f.h, ctx->bitmap);
             LAUNCHED();
+            k_fill_needed<256><<<(u32)ceil_div(f.n, 256), 256, 0, ctx->stream>>>(f.sa, f.n, ctx->bitmap, ctx->isa);
+            LAUNCHED();
+            ++selective_rounds;
+        } else {  // still not done after two rounds: fill every settled rank once
+            k_round0_isa<256><<<(u32)ceil_div(f.n, 256), 256, 0, ctx->stream>>>(f.sa, f.n, ctx->ids[f.cur], ctx->ranks, 0u, ctx->isa, f.tag);
+            LAUNCHED();
+            complete = true;
         }
-        span_end(ctx, sp);
-
-        sp = span_begin(ctx, PH_SORT);
-        if (int rc = run_sort(ctx, ctx->keys, ctx->ids, cur, m, 0, passes_r, &cur, st, round, false, nullptr, nullptr, nullptr, nullptr, nullptr,
-                              /*all_passes=*/text_built))
-            return rc;
-        span_end(ctx, sp);
-
-        sp = span_begin(ctx, PH_RERANK);
-        if (bucketed && m > n / 16) {
-            // the re-rank appends each tile's rank updates to per-bucket regions (suffix_kernels.cuh, PAIRS); the
-            // regions are then scattered bucket by bucket, each bucket's slice of isa[] staying in L2
-            PairSink sink;
-            sink.ids = (u32*)ctx->keys[cur ^ 1];
-            sink.vals = sink.ids + align_up((size_t)n, 64);
-            sink.shift = bshift;
-            CK(cudaMemsetAsync(ctx->bucket_hist, 0, sizeof(u32) * 256, ctx->stream));
-            if (int rc = launch_rerank<false, true>(ctx, ctx->keys[cur], ctx->ids[cur], m, n, K, kb, sa, ctx->ids[cur ^ 1], d_text, bwt_inline, sink)) return rc;
-            if (int rc = region_scatter(ctx, sink.ids, sink.vals, m, bshift)) return rc;
-        } else {
-            if (int rc = launch_rerank<false, false>(ctx, ctx->keys[cur], ctx->ids[cur], m, n, K, kb, sa, ctx->ids[cur ^ 1], d_text, bwt_inline)) return rc;
-        }
-        span_end(ctx, sp);
-        cur ^= 1;
-        const u32 m_sorted = m;
-        if (use_pairs && isa_complete && m_sorted <= n / 2) {  // the list that comes out may be all pairs: ask now, read with the count
-            if (int rc = queue_pairs_check(ctx, m_sorted, &pairs_checked)) return rc;
-        }
-        if (int rc = fetch_count(ctx, &m)) return rc;
-        if (text_built && ctx->mail->flag != m_sorted) return ctx->fail_internal("tagged isa[] entries disagree with the active list");
-        h *= 2;
-        ++round;
+        return 0;
     }
+};
+
+// A doubling round in pairs mode: one kernel settles or keeps each pair (suffix_kernels.cuh, "pairs mode").
+int pairs_round(dark_bwt_ctx* ctx, Fwd& f) {
+    int sp = span_begin(ctx, PH_RERANK);
+    constexpr int kPairThreads = 256, kPairsPerThread = 8;  // 4096 elements per tile, like the re-rank
+    const u32 tiles = (u32)ceil_div(f.m / 2, kPairThreads * kPairsPerThread);
+    if (tiles > ctx->scan_tiles) return ctx->fail_internal("scan tile state too small");
+    u32* counter = nullptr;
+    if (int rc = next_counter(ctx, &counter)) return rc;
+    CK(cudaMemsetAsync(ctx->scan_words, 0, sizeof(u64) * kScanWordsPerTile * tiles, ctx->stream));
+    ScanTileState ts{ctx->scan_words};
+    k_pairs_round<kPairThreads, kPairsPerThread><<<tiles, kPairThreads, 0, ctx->stream>>>(
+        ctx->ids[f.cur], ctx->ranks, f.m, f.n, f.h, ctx->isa, reinterpret_cast<uint2*>(ctx->keys[0]), f.sa, ctx->ids[f.cur ^ 1], ctx->ranks_alt,
+        ts, counter, &ctx->mail_dev->count, f.text, f.emit_inline ? f.bwt : nullptr, &ctx->mail_dev->origin, f.tag);
+    LAUNCHED();
+    std::swap(ctx->ranks, ctx->ranks_alt);
+    span_end(ctx, sp);
+    f.cur ^= 1;
+    f.st.pair_rounds += 1;
+    const u32 m_before = f.m;
+    if (int rc = fetch_count(ctx, &f.m)) return rc;
+    if (const u32 settled = (m_before - f.m) / 2) {
+        k_pairs_apply<<<(u32)ceil_div(settled, 256), 256, 0, ctx->stream>>>(reinterpret_cast<const uint2*>(ctx->keys[0]), settled, ctx->isa);
+        LAUNCHED();
+    }
+    return 0;
+}
+
+// One doubling round: keys (rank[i], rank[i+h]) -> radix sort -> re-rank/compact, or a pairs round.
+int doubling_round(dark_bwt_ctx* ctx, Fwd& f, RankFill& ranks, PairsMode& pairs) {
+    if (f.round >= DARK_BWT_MAX_ROUNDS || f.h >= 2 * (u64)f.n + 2) return ctx->fail_internal("prefix doubling did not converge");
+    f.st.active[f.round] = f.m;
+    f.st.rounds = f.round;
+    if (int rc = pairs.decide(ctx, f, ranks.complete)) return rc;
+    if (pairs.on) return pairs_round(ctx, f);
+    int sp = span_begin(ctx, PH_KEYBUILD);
+    CK(cudaMemsetAsync(ctx->hist, 0, sizeof(u32) * kMaxPasses * kRadix, ctx->stream));
+    bool keys_built = false;
+    if (int rc = ranks.fill(ctx, f, &keys_built)) return rc;
+    const bool text_built = !keys_built && f.tag != 0 && ranks.complete && (u64)f.m * (u64)ctx->knobs.text_div > (u64)f.n;
+    if (text_built) {
+        // many suffixes still active: sweep isa[] in text order instead of gathering from it (k_build_keys_text)
+        constexpr int kTextThreads = 512, kTextItems = 8;
+        const u32 tiles = (u32)ceil_div(f.n, kTextThreads * kTextItems);
+        if (tiles > ctx->scan_tiles) return ctx->fail_internal("scan tile state too small");
+        u32* counter = nullptr;
+        if (int rc = next_counter(ctx, &counter)) return rc;
+        CK(cudaMemsetAsync(ctx->scan_words, 0, sizeof(u64) * kScanWordsPerTile * tiles, ctx->stream));
+        auto kern = k_build_keys_text<kTextThreads, kTextItems>;
+        const size_t smem = kBuildTextSmem<kTextThreads, kTextItems>;
+        CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        const u32 grid = std::min<u32>(tiles, (u32)ctx->num_sms * 3);
+        kern<<<grid, kTextThreads, smem, ctx->stream>>>(ctx->isa, f.n, f.h, f.kb, f.tag, ctx->keys[f.cur], ctx->ids[f.cur], ctx->scan_words,
+                                                        counter, &ctx->mail_dev->flag, ctx->hist, f.passes_r);
+        LAUNCHED();
+    } else if (!keys_built) {
+        const u32 blocks = (u32)ceil_div(f.m, kBuildThreads * kBuildItems);  // one tile per CTA: the gathers want every warp slot filled
+        k_build_keys<kBuildThreads, kBuildItems><<<blocks, kBuildThreads, 0, ctx->stream>>>(
+            ctx->ids[f.cur], ctx->ranks, f.m, f.n, f.h, f.kb, ctx->isa, f.tag, ctx->keys[f.cur], ctx->hist, f.passes_r);
+        LAUNCHED();
+    }
+    span_end(ctx, sp);
+
+    sp = span_begin(ctx, PH_SORT);
+    if (int rc = run_sort(ctx, ctx->keys, ctx->ids, f.cur, f.m, 0, f.passes_r, &f.cur, &f.st, f.round, nullptr, /*all_passes=*/text_built))
+        return rc;
+    span_end(ctx, sp);
+
+    sp = span_begin(ctx, PH_RERANK);
+    u8* bwt_inline = f.emit_inline ? f.bwt : nullptr;
+    const u32* count_dev = nullptr;
+    if (f.bucketed && f.m > f.n / 16) {
+        // the re-rank appends each tile's rank updates to per-bucket regions (suffix_kernels.cuh, PAIRS); the
+        // regions are then scattered bucket by bucket, each bucket's slice of isa[] staying in L2
+        u32* ids = (u32*)ctx->keys[f.cur ^ 1];
+        const PairSink sink{ids, ids + align_up((size_t)f.n, 64), f.bshift};
+        CK(cudaMemsetAsync(ctx->bucket_hist, 0, sizeof(u32) * 256, ctx->stream));
+        if (int rc = launch_rerank<false, true>(ctx, ctx->keys[f.cur], ctx->ids[f.cur], f.m, f.n, f.K, f.kb, f.sa, ctx->ids[f.cur ^ 1], f.text,
+                                                bwt_inline, f.tag, &count_dev, sink))
+            return rc;
+        if (int rc = region_scatter(ctx, sink.ids, sink.vals, f.m, f.bshift)) return rc;
+    } else {
+        if (int rc = launch_rerank<false, false>(ctx, ctx->keys[f.cur], ctx->ids[f.cur], f.m, f.n, f.K, f.kb, f.sa, ctx->ids[f.cur ^ 1], f.text,
+                                                 bwt_inline, f.tag, &count_dev))
+            return rc;
+    }
+    span_end(ctx, sp);
+    f.cur ^= 1;
+    const u32 m_sorted = f.m;
+    if (int rc = pairs.queue(ctx, f, ranks.complete, count_dev, m_sorted)) return rc;  // the list that comes out may be all pairs
+    if (int rc = fetch_count(ctx, &f.m)) return rc;
+    if (text_built && ctx->mail->flag != m_sorted) return ctx->fail_internal("tagged isa[] entries disagree with the active list");
+    return 0;
+}
+
+// The whole forward transform on device buffers (2 <= n <= capacity).  d_sa_user and st_out nullable.
+int forward_device(dark_bwt_ctx* ctx, const u8* d_text, u32 n, u8* d_bwt, u64* origin_out, u32* d_sa_user, dark_bwt_stats* st_out) {
+    if (int rc = begin_call(ctx)) return rc;
+    Fwd f{d_text, n, d_bwt, d_sa_user ? d_sa_user : ctx->sa};
+    f.st.h2d_ms = st_out ? st_out->h2d_ms : 0.f;
+    reset_stats(&f.st, n);
+
+    int sp = span_begin(ctx, PH_INIT);
+    if (int rc = scan_alphabet(ctx, f)) return rc;
+    if (int rc = round0_keys(ctx, f)) return rc;
+    span_end(ctx, sp);
+    PairsMode pairs{ctx->knobs.pairs};
+    RankFill ranks;
+    if (int rc = round0_sort(ctx, f)) return rc;
+    if (int rc = round0_rerank(ctx, f, pairs)) return rc;
+    if (f.m > 0)
+        if (int rc = ranks.fill(ctx, f, nullptr)) return rc;
+    for (f.h = (u64)f.K0, f.round = 1; f.m > 0; f.h *= 2, ++f.round)
+        if (int rc = doubling_round(ctx, f, ranks, pairs)) return rc;
 
     // ---- BWT bytes + origin
     sp = span_begin(ctx, PH_EMIT);
-    if (!emit_inline)
-        if (int rc = emit(ctx, d_text, n, sa, d_bwt)) return rc;
+    if (!f.emit_inline)
+        if (int rc = emit(ctx, d_text, n, f.sa, d_bwt)) return rc;
     span_end(ctx, sp);
     CK(cudaEventRecord(ctx->call_stop, ctx->stream));
     CK(sync_counted(ctx));
     *origin_out = ctx->mail->origin;
-    finish_stats(ctx, st);
+    finish_stats(ctx, &f.st);
+    if (st_out) *st_out = f.st;
     return DARK_BWT_OK;
 }
 
@@ -1054,7 +1103,7 @@ int forward_many_device(dark_bwt_ctx* ctx, const u8* d_text, u32 n, u32 B, u8* d
     span_end(ctx, sp);
     sp = span_begin(ctx, PH_RERANK);
     // no "short suffix" special case (K = 1 disables it): the padding code 0 orders proper prefixes first
-    if (int rc = launch_rerank<true, false>(ctx, ctx->keys[cur], ctx->ids[cur], n, n, 1, 0, ctx->sa, ctx->ids[cur ^ 1], d_text, nullptr)) return rc;
+    if (int rc = launch_rerank<true, false>(ctx, ctx->keys[cur], ctx->ids[cur], n, n, 1, 0, ctx->sa, ctx->ids[cur ^ 1], d_text, nullptr, 0u, nullptr)) return rc;
     span_end(ctx, sp);
     cur ^= 1;
     u32 m = 0;
@@ -1086,7 +1135,7 @@ int forward_many_device(dark_bwt_ctx* ctx, const u8* d_text, u32 n, u32 B, u8* d
         if (int rc = run_sort(ctx, ctx->keys, ctx->ids, cur, m, 0, passes_r, &cur, st, round)) return rc;
         span_end(ctx, sp);
         sp = span_begin(ctx, PH_RERANK);
-        if (int rc = launch_rerank<false, false>(ctx, ctx->keys[cur], ctx->ids[cur], m, n, K, kb, ctx->sa, ctx->ids[cur ^ 1], d_text, nullptr)) return rc;
+        if (int rc = launch_rerank<false, false>(ctx, ctx->keys[cur], ctx->ids[cur], m, n, K, kb, ctx->sa, ctx->ids[cur ^ 1], d_text, nullptr, 0u, nullptr)) return rc;
         span_end(ctx, sp);
         cur ^= 1;
         if (int rc = fetch_count(ctx, &m)) return rc;
@@ -1225,12 +1274,10 @@ int inverse_device(dark_bwt_ctx* ctx, const u8* d_bwt, u32 n, u32 origin, const 
         gen.lg_s = 3;
         gen.mode = 1;
         gen.origin = origin;
-        bool gen_used = false;
-        if (int rc = run_sort(ctx, ctx->keys, ctx->ids, 0, n, 0, 1, &cur, nullptr, 0, false, nullptr, nullptr, nullptr, &gen, &gen_used)) return rc;
-        if (!gen_used) {  // one-symbol BWT: the pass is the identity and did not run; psi is the row list itself
+        if (int rc = run_sort(ctx, ctx->keys, ctx->ids, 0, n, 0, 1, &cur, nullptr, 0, &gen)) return rc;
+        if (cur == 0) {  // one-symbol BWT: the pass is the identity and did not run; psi is the row list itself
             k_ibwt_elements<<<(u32)ceil_div(n, 256), 256, 0, ctx->stream>>>(d_bwt, n, origin, ctx->keys[0], ctx->ids[0]);
             LAUNCHED();
-            cur = 0;
         }
         // k_ibwt_walk finds first symbols in the symbol bases (exclusive digit counts of pass 0, left in ctx->hist by run_sort)
     } else {

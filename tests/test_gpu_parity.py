@@ -724,18 +724,21 @@ def test_inverse_forced_paths(env_extra):
     assert out.returncode == 0 and "ok" in out.stdout, out.stderr[-2000:]
 
 
-def test_sparse_rerank_fallbacks(saca, oracle, torch):
-    """Pruned round 0 (uniform DNA digits) whose survivors defeat the sparse re-rank: a motif planted 150 times (groups
-    longer than the walk limit -> scan kernel), and a block whose second half repeats the first (more than n/16
-    survivors -> scan kernel).  Both must still give the oracle's bytes."""
+def _sparse_fallback_inputs():
     rng = np.random.default_rng(21)
     a = (rng.integers(0, 4, 1_500_000).astype(np.uint8) + 65)
     motif = (rng.integers(0, 4, 300).astype(np.uint8) + 65)
     for k in range(150):
         a[5000 + 9000 * k: 5000 + 9000 * k + 300] = motif
     half = (rng.integers(0, 4, 600_000).astype(np.uint8) + 65)
-    b = np.concatenate([half, half])
-    for t in (a, b):
+    return {"planted_motif": a, "repeated_half": np.concatenate([half, half])}
+
+
+def test_sparse_rerank_fallbacks(saca, oracle, torch):
+    """Pruned round 0 (uniform DNA digits) whose survivors defeat the sparse re-rank: a motif planted 150 times (groups
+    longer than the walk limit -> scan kernel), and a block whose second half repeats the first (more than n/16
+    survivors -> scan kernel).  Both must still give the oracle's bytes."""
+    for t in _sparse_fallback_inputs().values():
         bwt_o, origin_o, sa_o = oracle.bwt_forward(t, want_sa=True)
         with saca.Constructor(t.size) as con:
             bwt, origin, sa = con.bwt_and_sa(t)
