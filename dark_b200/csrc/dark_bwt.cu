@@ -11,10 +11,10 @@
 //   emit                            BWT gather + origin (unless the re-ranks emitted the bytes inline)
 //
 // forward_device drives these phases.  What crosses them lives in one Fwd record; RankFill owns which ranks isa[]
-// holds, PairsMode owns pairs mode.
+// holds, PairsMode owns pairs mode, SortStatus owns which rows of the radix passes' status buffer may hold stale words.
 //
 // All device memory is carved from one arena allocated at create (Constructor::new allocates its
-// arena up front too, saca.rs:351-360); the forward calls allocate nothing.
+// arena up front too, saca.rs:351-360) by carve_arena; the forward calls allocate nothing.
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -26,6 +26,7 @@
 #include <future>
 #include <new>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/dark_bwt.h"
@@ -150,6 +151,40 @@ struct DcSlot {
     u8* item_rank = nullptr;
 };
 
+// The tile status words of the radix passes (decoupled look-back), carved from the arena: every row a pass reads must
+// be zero when it starts.  Sorts of at most 2^31 pairs on the TMA pass use the buffer as two halves in turn: the workers
+// of a pass zero the rows of the OTHER half (onesweep_tma.cuh), so only what they did not cover is cleared by a memset.
+// The round-1 kernel, a TMA pass with 64-bit words and distance coding use the buffer from its start instead.
+class SortStatus {
+   public:
+    void init(void* base, size_t bytes) {
+        base_ = base;
+        bytes_ = bytes;
+        all_stale();
+    }
+    // The round-1 kernel or a TMA pass with 64-bit words: the first `bytes` of the buffer, zeroed.
+    int take_whole(dark_bwt_ctx* ctx, size_t bytes, void** use);
+    // A TMA pass with 32-bit words over `tiles` tiles that reads `rows` rows: *use is its half, zero in those rows; *clean
+    // the other half, whose rows [0, tiles) the pass' workers zero for the next such pass.
+    int take_half(dark_bwt_ctx* ctx, u32 tiles, u32 rows, void** use, void** clean);
+    // The whole buffer as scratch (the last-occurrence tables of distance coding on tiny blocks).
+    void* borrow() {
+        all_stale();
+        return base_;
+    }
+
+   private:
+    u32 half_rows() const { return (u32)(bytes_ / 2 / (kRadix * sizeof(u32))); }
+    void all_stale() {
+        for (int h = 0; h < 2; ++h) lo_[h] = 0u, hi_[h] = half_rows();
+    }
+
+    void* base_ = nullptr;
+    size_t bytes_ = 0;
+    int cur_ = 0;                              // the half the next TMA pass with 32-bit words uses
+    u32 lo_[2] = {0u, 0u}, hi_[2] = {0u, 0u};  // rows [lo_[h], hi_[h]) of half h may hold stale words
+};
+
 struct dark_bwt_ctx {
     int device = 0;
     Knobs knobs;
@@ -179,13 +214,7 @@ struct dark_bwt_ctx {
     u32* present = nullptr;
     u8* lut = nullptr;
     unsigned long long* bad = nullptr;  // dark_bwt_verify_sa_device: violation counter (device atomics)
-    void* sort_status = nullptr;
-    size_t sort_status_bytes = 0;
-    // Sorts of at most 2^31 pairs use 32-bit status words and the buffer as two halves in turn: the workers of a pass zero
-    // the rows of the OTHER half (onesweep_tma.cuh), so only what they did not cover is cleared by a memset.  Rows [lo, hi)
-    // of half h may hold stale words.
-    int status_cur = 0;
-    u32 status_dirty_lo[2] = {0u, 0u}, status_dirty_hi[2] = {0u, 0u};
+    SortStatus status;
     u32* counters = nullptr;
     u64* scan_words = nullptr;
     u32* bucket_hist = nullptr;  // 256 counters / cursors of the bucketed rank scatter
@@ -233,6 +262,30 @@ struct dark_bwt_ctx {
         ctx->launches += 1;   \
         CK(cudaGetLastError()); \
     } while (0)
+
+int SortStatus::take_whole(dark_bwt_ctx* ctx, size_t bytes, void** use) {
+    if (bytes > bytes_) return ctx->fail_internal("sort status buffer too small");
+    CK(cudaMemsetAsync(base_, 0, bytes, ctx->stream));
+    all_stale();
+    *use = base_;
+    return 0;
+}
+
+int SortStatus::take_half(dark_bwt_ctx* ctx, u32 tiles, u32 rows, void** use, void** clean) {
+    if (rows > half_rows()) return ctx->fail_internal("sort status buffer too small");
+    const int h = cur_, o = h ^ 1;
+    u32* base_h = (u32*)base_ + (size_t)h * half_rows() * kRadix;
+    if (hi_[h] > lo_[h])  // what the previous pass' workers did not zero (usually nothing)
+        CK(cudaMemsetAsync(base_h + (size_t)lo_[h] * kRadix, 0, (size_t)(hi_[h] - lo_[h]) * kRadix * sizeof(u32), ctx->stream));
+    lo_[h] = 0u;  // this pass writes rows [0, tiles) of its half ...
+    hi_[h] = tiles;
+    if (hi_[o] <= tiles) lo_[o] = hi_[o] = 0u;  // ... and zeroes rows [0, tiles) of the other
+    else lo_[o] = std::max(lo_[o], tiles);
+    cur_ = o;
+    *use = base_h;
+    *clean = (u32*)base_ + (size_t)o * half_rows() * kRadix;
+    return 0;
+}
 
 namespace {
 
@@ -287,120 +340,84 @@ void span_end(dark_bwt_ctx* ctx, int span) {
     ctx->spans[span].e1 = e1;
 }
 
-template <typename K>
-int set_smem(dark_bwt_ctx* ctx, K kernel, size_t bytes) {
-    CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-    return 0;
-}
-
 int next_counter(dark_bwt_ctx* ctx, u32** out) {
     if (ctx->next_counter >= kMaxCounters) return ctx->fail_internal("tile counters exhausted");
     *out = ctx->counters + ctx->next_counter++;
     return 0;
 }
 
-template <int THREADS, int ITEMS, int MINBLOCKS, int ILP, typename StatusT, bool ALIGNED, bool GEN = false>
-int launch_pass_kernel(dark_bwt_ctx* ctx, const u64* kin, const u32* vin, u64* kout, u32* vout, u32 m, int shift,
-                       const u32* digit_base, u32* counter, u32 tiles, const u8* prev_text, u32 n_text, KeyGen gen = KeyGen()) {
-    typedef OnesweepSmem<THREADS, ITEMS> Smem;
-    auto kern = k_onesweep_pass<THREADS, ITEMS, MINBLOCKS, ILP, StatusT, ALIGNED, GEN>;
-    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)));  // per device
-    // persistent grid: as many CTAs as stay resident (SMs x MINBLOCKS), each claiming tiles until none are left
-    const u32 grid = std::min<u32>(tiles, (u32)ctx->num_sms * MINBLOCKS);
+// Tilings of the radix passes: threads, items per thread, CTAs per SM, ranking items in flight per warp.  The pipelined
+// pass (onesweep_tma.cuh), and the round-1 kernel k_onesweep_pass (radix_sort.cuh), best of the tiling sweeps in
+// profiles/r1_sort_variants_*.log.
+constexpr int kPassThreads = 256, kPassItems = 16, kPassCtas = 2, kPassIlp = 2;
+constexpr int kRound1Threads = 256, kRound1Items = 16, kRound1Ctas = 3, kRound1Ilp = 2;
+
+// f(BoolC<b>()): a runtime choice as a template argument of the kernel f launches.  A function template, not a lambda:
+// the pass kernels are then instantiated after the kernels launched directly, and that order of the module's extern
+// shared arrays decides the offset of k_build_keys_text's dynamic shared memory.
+template <typename F>
+int with_bool(bool b, const F& f) {
+    return b ? f(BoolC<true>()) : f(BoolC<false>());
+}
+
+// The TMA-staged, software-pipelined pass: byte-aligned digits, 16-byte aligned inputs, plain or key-generating (GEN mode 0).
+int launch_pass_tma(dark_bwt_ctx* ctx, const u64* kin, const u32* vin, u64* kout, u32* vout, u32 m, int shift, const u32* digit_base,
+                    u32* counter, bool wide, const u8* prev_text, const KeyGen* gen) {
+    typedef PipeSmem<kPassThreads, kPassItems> Smem;
+    const u32 tiles = (u32)ceil_div(m, Smem::kTile);
+    const u32 rows = tiles + 3 * kScannerBatch;  // the scanners read ahead
+    void *status = nullptr, *status_clean = nullptr;
+    if (int rc = wide ? ctx->status.take_whole(ctx, (size_t)rows * kRadix * sizeof(u64), &status)
+                      : ctx->status.take_half(ctx, tiles, rows, &status, &status_clean))
+        return rc;
+    const u32 grid = std::min<u32>(tiles + kScanners, (u32)ctx->num_sms * kPassCtas);  // kScanners CTAs scan, the rest sort
+    const KeyGen g = gen ? *gen : KeyGen();
+    auto run = [&](auto wide_c, auto gen_c, auto hi_c) {
+        typedef std::conditional_t<decltype(wide_c)::value, u64, u32> StatusT;
+        auto kern = k_onesweep_tma<kPassThreads, kPassItems, kPassCtas, kPassIlp, StatusT, decltype(gen_c)::value, decltype(hi_c)::value>;
+        CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)));
+        kern<<<grid, kPassThreads, sizeof(Smem), ctx->stream>>>(kin, vin, kout, vout, m, shift, digit_base, (StatusT*)status,
+                                                                 (StatusT*)status_clean, counter, g, prev_text);
+        LAUNCHED();
+        return 0;
+    };
+    return with_bool(gen != nullptr, [&](auto gen_c) {
+        return with_bool(wide, [&](auto wide_c) {
+            return with_bool(shift >= 32, [&](auto hi_c) { return run(wide_c, gen_c, hi_c); });
+        });
+    });
+}
+
+// The round-1 kernel: any digit, any 8-byte aligned input, plain or key-generating (GEN modes 0 and 1).
+int launch_pass_round1(dark_bwt_ctx* ctx, const u64* kin, const u32* vin, u64* kout, u32* vout, u32 m, int shift,
+                       const u32* digit_base, u32* counter, bool wide, const u8* prev_text, u32 n_text, const KeyGen* gen) {
+    typedef OnesweepSmem<kRound1Threads, kRound1Items> Smem;
+    const u32 tiles = (u32)ceil_div(m, Smem::kTile);
+    void* status = nullptr;
+    if (int rc = ctx->status.take_whole(ctx, (size_t)tiles * kRadix * (wide ? sizeof(u64) : sizeof(u32)), &status)) return rc;
+    const bool aligned = (shift & 7) == 0;  // always true for the suffix sorter; the public sort may differ
+    if (gen && !aligned) return ctx->fail_internal("key-generating pass needs a byte-aligned digit");
+    // persistent grid: as many CTAs as stay resident (SMs x CTAs per SM), each claiming tiles until none are left
+    const u32 grid = std::min<u32>(tiles, (u32)ctx->num_sms * kRound1Ctas);
     // L2 prefetch distance in tiles: two thirds of a wave of claims (the persistent grid; 148..444 measured alike, beyond
     // one wave the gain fades)
     const u32 prefetch_ahead = std::max(1u, grid * 2 / 3);
-    kern<<<grid, THREADS, sizeof(Smem), ctx->stream>>>(kin, vin, kout, vout, m, shift, digit_base, (StatusT*)ctx->sort_status, counter,
-                                                        prev_text, n_text, gen, prefetch_ahead);
-    LAUNCHED();
-    return 0;
-}
-
-template <int THREADS, int ITEMS, int MINBLOCKS, int ILP>
-int launch_pass_variant(dark_bwt_ctx* ctx, const u64* kin, const u32* vin, u64* kout, u32* vout, u32 m, int shift,
-                        const u32* digit_base, u32* counter, bool wide, const u8* prev_text, u32 n_text, const KeyGen* gen = nullptr) {
-    typedef OnesweepSmem<THREADS, ITEMS> Smem;
-    const u32 tiles = (u32)ceil_div(m, Smem::kTile);
-    const size_t bytes = (size_t)tiles * kRadix * (wide ? sizeof(u64) : sizeof(u32));
-    if (bytes > ctx->sort_status_bytes) return ctx->fail_internal("sort status buffer too small");
-    CK(cudaMemsetAsync(ctx->sort_status, 0, bytes, ctx->stream));
-    {  // this kernel uses the buffer from its start: both halves of the TMA pass' bookkeeping are stale now
-        const u32 half_rows = (u32)(ctx->sort_status_bytes / 2 / (kRadix * sizeof(u32)));
-        for (int h = 0; h < 2; ++h) ctx->status_dirty_lo[h] = 0u, ctx->status_dirty_hi[h] = half_rows;
-    }
-    const bool aligned = (shift & 7) == 0;  // always true for the suffix sorter; the public sort may differ
-#define LP(ST, AL) launch_pass_kernel<THREADS, ITEMS, MINBLOCKS, ILP, ST, AL>(ctx, kin, vin, kout, vout, m, shift, digit_base, counter, tiles, prev_text, n_text)
-    if (gen != nullptr) {  // keys built from the text inside the pass (default tiling, byte-aligned digits only)
-        if (!aligned) return ctx->fail_internal("key-generating pass needs a byte-aligned digit");
-        if (wide)
-            return launch_pass_kernel<THREADS, ITEMS, MINBLOCKS, ILP, u64, true, true>(ctx, kin, vin, kout, vout, m, shift, digit_base, counter,
-                                                                                       tiles, prev_text, n_text, *gen);
-        return launch_pass_kernel<THREADS, ITEMS, MINBLOCKS, ILP, u32, true, true>(ctx, kin, vin, kout, vout, m, shift, digit_base, counter,
-                                                                                   tiles, prev_text, n_text, *gen);
-    }
-    if (!aligned) return wide ? LP(u64, false) : LP(u32, false);
-    return wide ? LP(u64, true) : LP(u32, true);
-#undef LP
-}
-
-// The TMA-staged, software-pipelined pass (onesweep_tma.cuh): byte-aligned digits, 16-byte aligned inputs, plain or
-// key-generating (GEN mode 0).  Returns 1 if this pass is not eligible (the caller then runs k_onesweep_pass).
-template <int THREADS, int ITEMS, int MINBLOCKS, int ILP>
-int launch_pass_tma(dark_bwt_ctx* ctx, const u64* kin, const u32* vin, u64* kout, u32* vout, u32 m, int shift, const u32* digit_base,
-                    u32* counter, bool wide, const u8* prev_text, const KeyGen* gen) {
-    typedef PipeSmem<THREADS, ITEMS> Smem;
-    const u32 tiles = (u32)ceil_div(m, Smem::kTile);
-    const u32 rows_needed = tiles + 3 * kScannerBatch;  // the scanners read ahead
-    const u32 half_rows = (u32)(ctx->sort_status_bytes / 2 / (kRadix * sizeof(u32)));
-    void* st_use = ctx->sort_status;
-    void* st_clean = nullptr;
-    if (wide) {
-        const size_t bytes = (size_t)rows_needed * kRadix * sizeof(u64);
-        if (bytes > ctx->sort_status_bytes) return ctx->fail_internal("sort status buffer too small");
-        CK(cudaMemsetAsync(ctx->sort_status, 0, bytes, ctx->stream));
-        for (int h = 0; h < 2; ++h) ctx->status_dirty_lo[h] = 0u, ctx->status_dirty_hi[h] = half_rows;
-    } else {
-        if (rows_needed > half_rows) return ctx->fail_internal("sort status buffer too small");
-        const int h = ctx->status_cur, o = h ^ 1;
-        u32* base_h = (u32*)ctx->sort_status + (size_t)h * half_rows * kRadix;
-        u32* base_o = (u32*)ctx->sort_status + (size_t)o * half_rows * kRadix;
-        if (ctx->status_dirty_hi[h] > ctx->status_dirty_lo[h]) {  // what the previous pass' workers did not zero (usually nothing)
-            CK(cudaMemsetAsync(base_h + (size_t)ctx->status_dirty_lo[h] * kRadix, 0,
-                               (size_t)(ctx->status_dirty_hi[h] - ctx->status_dirty_lo[h]) * kRadix * sizeof(u32), ctx->stream));
-        }
-        ctx->status_dirty_lo[h] = 0u;  // this pass writes rows [0, tiles) of its half ...
-        ctx->status_dirty_hi[h] = tiles;
-        if (ctx->status_dirty_hi[o] <= tiles) ctx->status_dirty_lo[o] = ctx->status_dirty_hi[o] = 0u;  // ... and zeroes rows [0, tiles) of the other
-        else ctx->status_dirty_lo[o] = std::max(ctx->status_dirty_lo[o], tiles);
-        ctx->status_cur = o;
-        st_use = base_h;
-        st_clean = base_o;
-    }
-    const u32 grid = std::min<u32>(tiles + kScanners, (u32)ctx->num_sms * MINBLOCKS);  // kScanners CTAs scan, the rest sort
     const KeyGen g = gen ? *gen : KeyGen();
-    const bool hi = shift >= 32;
-#define LT(ST, GEN)                                                                                                          \
-    do {                                                                                                                     \
-        auto kern = hi ? k_onesweep_tma<THREADS, ITEMS, MINBLOCKS, ILP, ST, GEN, true>                                       \
-                       : k_onesweep_tma<THREADS, ITEMS, MINBLOCKS, ILP, ST, GEN, false>;                                     \
-        CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)));                      \
-        kern<<<grid, THREADS, sizeof(Smem), ctx->stream>>>(kin, vin, kout, vout, m, shift, digit_base, (ST*)st_use, (ST*)st_clean, \
-                                                           counter, g, prev_text);                                           \
-    } while (0)
-    if (gen) {
-        if (wide) LT(u64, true);
-        else LT(u32, true);
-    } else {
-        if (wide) LT(u64, false);
-        else LT(u32, false);
-    }
-#undef LT
-    LAUNCHED();
-    return 0;
+    auto run = [&](auto wide_c, auto aligned_c, auto gen_c) {
+        typedef std::conditional_t<decltype(wide_c)::value, u64, u32> StatusT;
+        auto kern = k_onesweep_pass<kRound1Threads, kRound1Items, kRound1Ctas, kRound1Ilp, StatusT, decltype(aligned_c)::value,
+                                    decltype(gen_c)::value>;
+        CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)));  // per device
+        kern<<<grid, kRound1Threads, sizeof(Smem), ctx->stream>>>(kin, vin, kout, vout, m, shift, digit_base, (StatusT*)status, counter,
+                                                                   prev_text, n_text, g, prefetch_ahead);
+        LAUNCHED();
+        return 0;
+    };
+    if (gen) return with_bool(wide, [&](auto wide_c) { return run(wide_c, BoolC<true>(), BoolC<true>()); });  // keys built from the text inside the pass
+    return with_bool(aligned, [&](auto aligned_c) {
+        return with_bool(wide, [&](auto wide_c) { return run(wide_c, aligned_c, BoolC<false>()); });
+    });
 }
-
-// Tiling of the pipelined pass: threads, items per thread, CTAs per SM, ranking items in flight per warp
-constexpr int kPassThreads = 256, kPassItems = 16, kPassCtas = 2, kPassIlp = 2;
 
 // One onesweep pass over m pairs: buffers[cur] -> buffers[cur^1].
 int launch_pass(dark_bwt_ctx* ctx, const u64* kin, const u32* vin, u64* kout, u32* vout, u32 m, int shift,
@@ -420,10 +437,8 @@ int launch_pass(dark_bwt_ctx* ctx, const u64* kin, const u32* vin, u64* kout, u3
     const bool eligible = (shift & 7) == 0 && (gen == nullptr || gen->mode == 0) &&
                           (gen != nullptr || (prev_text == nullptr && ((uintptr_t)kin & 15) == 0 && ((uintptr_t)vin & 15) == 0));
     if (ctx->knobs.pass_impl != 0 && eligible)
-        return launch_pass_tma<kPassThreads, kPassItems, kPassCtas, kPassIlp>(ctx, kin, vin, kout, vout, m, shift, digit_base, counter, wide_tma,
-                                                                              prev_text, gen);
-    // the round-1 kernel: 256 threads x 16 items, 3 CTAs/SM, best of the tiling sweeps in profiles/r1_sort_variants_*.log
-    return launch_pass_variant<256, 16, 3, 2>(ctx, kin, vin, kout, vout, m, shift, digit_base, counter, wide, prev_text, n_text, gen);
+        return launch_pass_tma(ctx, kin, vin, kout, vout, m, shift, digit_base, counter, wide_tma, prev_text, gen);
+    return launch_pass_round1(ctx, kin, vin, kout, vout, m, shift, digit_base, counter, wide, prev_text, n_text, gen);
 }
 
 // The digit statistics of the histograms in ctx->hist: mail->trivial[p] (every key has the same digit p) and
@@ -1382,11 +1397,7 @@ int dc_device(dark_bwt_ctx* ctx, const u8* d_bwt, u32 n, const BlockList* blocks
     const u32 nblocks = (u32)ceil_div(n, kDcBlock);
     // last-occurrence tables: (nblocks + ngroups) x 256 words = n/4 + n/1024 bytes (+ 2 KB): inside the 4n-byte rank buffer for
     // all but tiny blocks, which borrow the sort's status buffer (>= 256 KB)
-    u32* tab = ctx->ranks;
-    if (n <= 65536u) {
-        tab = (u32*)ctx->sort_status;
-        for (int h = 0; h < 2; ++h) ctx->status_dirty_lo[h] = 0u, ctx->status_dirty_hi[h] = (u32)(ctx->sort_status_bytes / 2 / (kRadix * sizeof(u32)));
-    }
+    u32* tab = n <= 65536u ? (u32*)ctx->status.borrow() : ctx->ranks;
     u32* run_counts = ctx->ranks_alt;
     u32* first = ctx->bucket_hist;
     u32* final_last = ctx->bucket_hist + 256;
@@ -1687,64 +1698,61 @@ int run_pipelined(dark_bwt_ctx* ctx, const u8* const* ins, const uint64_t* ns, u
     return DARK_BWT_OK;
 }
 
-// Where dark_bwt_create_ex carves each buffer of the arena: byte offsets, and `bytes` in all.  Pure host arithmetic, shared
-// with dark_bwt_arena_bytes.  Returns false for a capacity or flags create rejects.
-struct ArenaLayout {
-    size_t keys[2], ids[2], ranks, ranks2, isa, sa;
-    size_t text, bwt, text2, bwt2;  // host-entry staging pairs (none with DARK_BWT_F_DEVICE_ONLY); text2 == text with one pair
-    size_t hist, present, lut, bad, status, counters, bhist, bitmap, swords, mstarts, morigins, mlut, dcinfo;
-    size_t slot[2][5];  // DARK_BWT_F_DC_BATCH: dist, item_pos, item_dist, item_sym, item_rank
-    size_t sort_status_bytes, scan_tiles, bytes;
-    int staging_pairs;
-};
-
-bool arena_layout(uint64_t max_n, uint32_t flags, ArenaLayout* L) {
-    *L = ArenaLayout{};
-    if (flags & ~(DARK_BWT_F_NO_ALPHABET_PACKING | DARK_BWT_F_DEVICE_ONLY | DARK_BWT_F_DC_BATCH)) return false;
+// The arguments dark_bwt_create_ex checks before it looks for a device, in its order: DARK_BWT_OK or the code it returns.
+int check_create_args(uint64_t max_n, uint32_t flags) {
+    if (flags & ~(DARK_BWT_F_NO_ALPHABET_PACKING | DARK_BWT_F_DEVICE_ONLY | DARK_BWT_F_DC_BATCH)) return DARK_BWT_E_INVALID_ARG;
     // the DC batch is a host-buffer entry: it needs the staging a device-only context does not have
-    if ((flags & DARK_BWT_F_DC_BATCH) && (flags & DARK_BWT_F_DEVICE_ONLY)) return false;
-    if (max_n < 2 || max_n > 0xFFFFFFFEull) return false;
-    const size_t N = (size_t)max_n;
-    const size_t sort_tiles = ceil_div(N, kSortTile);
-    L->sort_status_bytes = (sort_tiles + 128) * kRadix * sizeof(u64);  // + rows the scanner CTA reads ahead
-    L->scan_tiles = ceil_div(N, std::min(kScanTile, 4096));  // the pairs kernel and the text-order builder scan 4,096-suffix tiles
-    const bool staging = !(flags & DARK_BWT_F_DEVICE_ONLY);
-    const bool dc_batch = flags & DARK_BWT_F_DC_BATCH;
+    if ((flags & DARK_BWT_F_DC_BATCH) && (flags & DARK_BWT_F_DEVICE_ONLY)) return DARK_BWT_E_INVALID_ARG;
+    if (max_n < 2 || max_n > 0xFFFFFFFEull) return DARK_BWT_E_INVALID_N;
+    return DARK_BWT_OK;
+}
+
+// The arena of a context of ctx->capacity and ctx->flags (checked): every device buffer, carved in one order.  Returns the
+// arena's bytes.  With ctx->arena null it only sizes (dark_bwt_arena_bytes, and create before its cudaMalloc); with the
+// allocation it also points the context's buffers into it.
+size_t carve_arena(dark_bwt_ctx* ctx) {
+    const size_t N = (size_t)ctx->capacity;
+    const bool staging = !(ctx->flags & DARK_BWT_F_DEVICE_ONLY);
+    const bool dc_batch = ctx->flags & DARK_BWT_F_DC_BATCH;
     // Above 2^31 the second pair (2 N bytes) is what keeps a context of 2^32 - 2 inside a B200: the batch entries then run
     // their blocks one after another through one pair.  The DC batch keeps two pairs: its output slots pair with them.
-    L->staging_pairs = !staging ? 0 : (max_n > (1ull << 31) && !dc_batch) ? 1 : 2;
+    ctx->pipeline_depth = !staging ? 0 : (ctx->capacity > (1ull << 31) && !dc_batch) ? 1 : 2;
+    ctx->scan_tiles = ceil_div(N, std::min(kScanTile, 4096));  // the pairs kernel and the text-order builder scan 4,096-suffix tiles
 
+    char* const base = (char*)ctx->arena;
     size_t off = 0;
-    auto carve = [&](size_t bytes) {
-        size_t o = off;
+    auto carve = [&](auto& ptr, size_t bytes) {
+        if (base) ptr = (std::remove_reference_t<decltype(ptr)>)(base + off);
         off = align_up(off + bytes, 256);
-        return o;
     };
-    L->keys[0] = carve(N * 8 + 1024), L->keys[1] = carve(N * 8 + 1024);  // slack: pair lists are split at a 64-aligned offset
-    L->ids[0] = carve(N * 4 + 16), L->ids[1] = carve(N * 4 + 16);
-    L->ranks = carve(N * 4 + 16), L->ranks2 = carve(N * 4 + 16), L->isa = carve(N * 4 + 16), L->sa = carve(N * 4 + 16);
-    L->text = staging ? carve(N + 16) : 0, L->bwt = staging ? carve(N + 16) : 0;
-    L->text2 = L->staging_pairs == 2 ? carve(N + 16) : L->text, L->bwt2 = L->staging_pairs == 2 ? carve(N + 16) : L->bwt;
-    L->hist = carve(sizeof(u32) * kMaxPasses * kRadix);
-    L->present = carve(sizeof(u32) * 256);
-    L->lut = carve(256);
-    L->bad = carve(sizeof(unsigned long long));
-    L->status = carve(L->sort_status_bytes);
-    L->counters = carve(sizeof(u32) * kMaxCounters);
-    L->bhist = carve(sizeof(u32) * 1280);  // 256 bucket counters/cursors + 257 chunk prefixes; DC: first/last occurrences + dense alphabet
-    L->bitmap = carve(sizeof(u32) * (ceil_div(N, 32) + 1) + 1024);  // + one tile of flag bytes past the end
-    L->swords = carve(sizeof(u64) * kScanWordsPerTile * L->scan_tiles);
-    L->mstarts = carve(sizeof(u32) * (kMaxManyBlocks + 1));
-    L->morigins = carve(sizeof(unsigned long long) * kMaxManyBlocks);
-    L->mlut = carve(sizeof(u16) * 256);
-    L->dcinfo = carve(sizeof(DcInfoDev) + 16);
+    for (u64*& k : ctx->keys) carve(k, N * 8 + 1024);  // slack: pair lists are split at a 64-aligned offset
+    for (u32*& i : ctx->ids) carve(i, N * 4 + 16);
+    carve(ctx->ranks, N * 4 + 16), carve(ctx->ranks_alt, N * 4 + 16), carve(ctx->isa, N * 4 + 16), carve(ctx->sa, N * 4 + 16);
+    if (staging) carve(ctx->d_text, N + 16), carve(ctx->d_bwt, N + 16);  // host-entry staging
+    if (ctx->pipeline_depth == 2) carve(ctx->d_text2, N + 16), carve(ctx->d_bwt2, N + 16);
+    else ctx->d_text2 = ctx->d_text, ctx->d_bwt2 = ctx->d_bwt;  // one pair (or none)
+    carve(ctx->hist, sizeof(u32) * kMaxPasses * kRadix);
+    carve(ctx->present, sizeof(u32) * 256);
+    carve(ctx->lut, 256);
+    carve(ctx->bad, sizeof(unsigned long long));
+    const size_t status_bytes = (ceil_div(N, kSortTile) + 128) * kRadix * sizeof(u64);  // + rows the scanner CTA reads ahead
+    void* status = nullptr;
+    carve(status, status_bytes);
+    ctx->status.init(status, status_bytes);
+    carve(ctx->counters, sizeof(u32) * kMaxCounters);
+    carve(ctx->bucket_hist, sizeof(u32) * 1280);  // 256 bucket counters/cursors + 257 chunk prefixes; DC: first/last occurrences + dense alphabet
+    carve(ctx->bitmap, sizeof(u32) * (ceil_div(N, 32) + 1) + 1024);  // + one tile of flag bytes past the end
+    carve(ctx->scan_words, sizeof(u64) * kScanWordsPerTile * ctx->scan_tiles);
+    carve(ctx->many_starts, sizeof(u32) * (kMaxManyBlocks + 1));
+    carve(ctx->many_origins, sizeof(unsigned long long) * kMaxManyBlocks);
+    carve(ctx->many_lut, sizeof(u16) * 256);
+    carve(ctx->dc_info, sizeof(DcInfoDev) + 16);
     if (dc_batch)
-        for (auto& s : L->slot) {
-            for (int a = 0; a < 3; ++a) s[a] = carve(N * 4 + 16);
-            for (int a = 3; a < 5; ++a) s[a] = carve(N + 16);
+        for (DcSlot& s : ctx->dc_slot) {
+            carve(s.dist, N * 4 + 16), carve(s.item_pos, N * 4 + 16), carve(s.item_dist, N * 4 + 16);
+            carve(s.item_sym, N + 16), carve(s.item_rank, N + 16);
         }
-    L->bytes = off;
-    return true;
+    return off;
 }
 
 }  // namespace
@@ -1771,8 +1779,11 @@ uint64_t dark_bwt_capacity(const dark_bwt_ctx* ctx) { return ctx ? ctx->capacity
 void* dark_bwt_stream(const dark_bwt_ctx* ctx) { return ctx ? (void*)ctx->stream : nullptr; }
 
 uint64_t dark_bwt_arena_bytes(uint64_t max_n, uint32_t flags) {
-    ArenaLayout L;
-    return arena_layout(max_n, flags, &L) ? (uint64_t)L.bytes : 0;
+    if (check_create_args(max_n, flags) != DARK_BWT_OK) return 0;
+    dark_bwt_ctx sizing;
+    sizing.capacity = max_n;
+    sizing.flags = flags;
+    return carve_arena(&sizing);
 }
 
 int dark_bwt_create(uint64_t max_n, int device, dark_bwt_ctx** out) {
@@ -1782,9 +1793,7 @@ int dark_bwt_create(uint64_t max_n, int device, dark_bwt_ctx** out) {
 int dark_bwt_create_ex(uint64_t max_n, int device, uint32_t flags, dark_bwt_ctx** out) {
     if (!out) return DARK_BWT_E_INVALID_ARG;
     *out = nullptr;
-    if (flags & ~(DARK_BWT_F_NO_ALPHABET_PACKING | DARK_BWT_F_DEVICE_ONLY | DARK_BWT_F_DC_BATCH)) return DARK_BWT_E_INVALID_ARG;
-    if ((flags & DARK_BWT_F_DC_BATCH) && (flags & DARK_BWT_F_DEVICE_ONLY)) return DARK_BWT_E_INVALID_ARG;
-    if (max_n < 2 || max_n > 0xFFFFFFFEull) return DARK_BWT_E_INVALID_N;
+    if (int rc = check_create_args(max_n, flags)) return rc;
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return DARK_BWT_E_CUDA;  // no CPU fallback
     if (device < 0 || device >= ndev) return DARK_BWT_E_INVALID_ARG;
@@ -1801,14 +1810,7 @@ int dark_bwt_create_ex(uint64_t max_n, int device, uint32_t flags, dark_bwt_ctx*
     ctx->flags = flags;
     ctx->knobs.read_env();
 
-    ArenaLayout L;
-    arena_layout(max_n, flags, &L);
-    ctx->sort_status_bytes = L.sort_status_bytes;
-    ctx->scan_tiles = L.scan_tiles;
-    const bool staging = !(flags & DARK_BWT_F_DEVICE_ONLY);
-    const bool dc_batch = flags & DARK_BWT_F_DC_BATCH;
-    ctx->arena_bytes = L.bytes;
-
+    ctx->arena_bytes = carve_arena(ctx);
     auto bail = [&](int code) {
         dark_bwt_destroy(ctx);
         return code;
@@ -1818,41 +1820,10 @@ int dark_bwt_create_ex(uint64_t max_n, int device, uint32_t flags, dark_bwt_ctx*
         ctx->arena = nullptr;
         return bail(DARK_BWT_E_NOMEM);
     }
-    char* base = (char*)ctx->arena;
-    ctx->keys[0] = (u64*)(base + L.keys[0]);
-    ctx->keys[1] = (u64*)(base + L.keys[1]);
-    ctx->ids[0] = (u32*)(base + L.ids[0]);
-    ctx->ids[1] = (u32*)(base + L.ids[1]);
-    ctx->ranks = (u32*)(base + L.ranks);
-    ctx->ranks_alt = (u32*)(base + L.ranks2);
-    ctx->isa = (u32*)(base + L.isa);
-    ctx->sa = (u32*)(base + L.sa);
-    ctx->d_text = staging ? (u8*)(base + L.text) : nullptr;
-    ctx->d_bwt = staging ? (u8*)(base + L.bwt) : nullptr;
-    ctx->d_text2 = staging ? (u8*)(base + L.text2) : nullptr;  // one pair: the same buffers as d_text and d_bwt
-    ctx->d_bwt2 = staging ? (u8*)(base + L.bwt2) : nullptr;
-    ctx->pipeline_depth = L.staging_pairs;
-    ctx->hist = (u32*)(base + L.hist);
-    ctx->present = (u32*)(base + L.present);
-    ctx->lut = (u8*)(base + L.lut);
-    ctx->bad = (unsigned long long*)(base + L.bad);
-    ctx->sort_status = base + L.status;
-    for (int h = 0; h < 2; ++h) ctx->status_dirty_lo[h] = 0u, ctx->status_dirty_hi[h] = (u32)(ctx->sort_status_bytes / 2 / (kRadix * sizeof(u32)));
-    ctx->counters = (u32*)(base + L.counters);
-    ctx->scan_words = (u64*)(base + L.swords);
-    ctx->bitmap = (u32*)(base + L.bitmap);
-    ctx->bucket_hist = (u32*)(base + L.bhist);
-    ctx->many_starts = (u32*)(base + L.mstarts);
-    ctx->many_origins = (unsigned long long*)(base + L.morigins);
-    ctx->many_lut = (u16*)(base + L.mlut);
-    ctx->dc_info = (DcInfoDev*)(base + L.dcinfo);
-    if (dc_batch)
-        for (int b = 0; b < 2; ++b)
-            ctx->dc_slot[b] = DcSlot{(u32*)(base + L.slot[b][0]), (u32*)(base + L.slot[b][1]), (u32*)(base + L.slot[b][2]),
-                                     (u8*)(base + L.slot[b][3]), (u8*)(base + L.slot[b][4])};
+    carve_arena(ctx);
 
     if (cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking) != cudaSuccess) return bail(DARK_BWT_E_CUDA);
-    if (staging) {
+    if (!(flags & DARK_BWT_F_DEVICE_ONLY)) {
         if (cudaStreamCreateWithFlags(&ctx->copy_in, cudaStreamNonBlocking) != cudaSuccess ||
             cudaStreamCreateWithFlags(&ctx->copy_out, cudaStreamNonBlocking) != cudaSuccess)
             return bail(DARK_BWT_E_CUDA);

@@ -253,28 +253,39 @@ def test_pageable_host_buffers_through_the_staging_lanes(oracle, idx):
 
 # ---- building blocks (SURVEY §4 T1) -------------------------------------------------------------
 @pytest.mark.parametrize("m,begin,end", [(1, 0, 64), (100, 0, 64), (4096, 0, 64), (4097, 0, 64), (1000003, 0, 64),
-                                         (300000, 0, 40), (300000, 16, 48), (50000, 0, 8)])
-def test_radix_sort_pairs_is_a_stable_sort(saca, torch, m, begin, end):
+                                         (300000, 0, 40), (300000, 16, 48), (50000, 0, 8), (300000, 3, 40)])
+def test_radix_sort_pairs_is_a_stable_sort(saca, oracle, torch, m, begin, end):
+    from dark_b200 import synth
     rng = np.random.default_rng(m + begin)
     keys = rng.integers(0, 1 << 63, m, dtype=np.uint64) * 2 + rng.integers(0, 2, m, dtype=np.uint64)
     if m > 1000:
         keys[: m // 2] &= np.uint64(0x00FF00FF00FF00FF)      # skewed digits, many ties
     vals = np.arange(m, dtype=np.uint32)
-    con = saca.Constructor(max(m, 2))
-    dk = torch.from_numpy(keys.view(np.int64)).cuda()
-    dv = torch.from_numpy(vals.view(np.int32)).cuda()
-    dk2, dv2 = torch.empty_like(dk), torch.empty_like(dv)
-    in_alt, _ = con.sort_pairs_device(dk.data_ptr(), dv.data_ptr(), dk2.data_ptr(), dv2.data_ptr(), m, begin, end)
-    torch.cuda.synchronize()
-    rk = (dk2 if in_alt else dk).cpu().numpy().view(np.uint64)
-    rv = (dv2 if in_alt else dv).cpu().numpy().view(np.uint32)
     nbits = end - begin
     passes = (nbits + 7) // 8
     mask = np.uint64((1 << min(64 - begin, passes * 8)) - 1)
     sub = (keys >> np.uint64(begin)) & mask                   # whole 8-bit digits take part
     order = np.argsort(sub, kind="stable")
-    assert np.array_equal(rv, vals[order])
-    assert np.array_equal(rk, keys[order])
+    con = saca.Constructor(max(m, 2))
+    # off = 1: keys and values one element past 16-byte alignment, so the passes that read them take the round-1 kernel
+    # (k_onesweep_pass) and those that read the aligned alt buffers take the TMA pass
+    for off in (0, 1):
+        dk = torch.empty(m + off, dtype=torch.int64, device="cuda")[off:]
+        dv = torch.empty(m + off, dtype=torch.int32, device="cuda")[off:]
+        dk.copy_(torch.from_numpy(keys.view(np.int64)))
+        dv.copy_(torch.from_numpy(vals.view(np.int32)))
+        dk2, dv2 = torch.empty_like(dk), torch.empty_like(dv)
+        in_alt, _ = con.sort_pairs_device(dk.data_ptr(), dv.data_ptr(), dk2.data_ptr(), dv2.data_ptr(), m, begin, end)
+        torch.cuda.synchronize()
+        rk = (dk2 if in_alt else dk).cpu().numpy().view(np.uint64)
+        rv = (dv2 if in_alt else dv).cpu().numpy().view(np.uint32)
+        assert np.array_equal(rv, vals[order]), off
+        assert np.array_equal(rk, keys[order]), off
+    # a forward on the same context: its passes take over the sort status buffer from the sort's
+    t = synth.generate("text", m, max(m, 2))
+    b, o = con.bwt(t)
+    rb, ro = oracle.bwt_forward(t)
+    assert o == ro and np.array_equal(b, rb)
     con.close()
 
 
