@@ -142,13 +142,15 @@ struct HostStage {
     cudaEvent_t slot_done[kMaxLanes][2] = {{nullptr}};  // the DMA out of / into a lane's slot has completed
 };
 
-// One distance-coding output slot of dark_bwt_forward_dc_batch (DARK_BWT_F_DC_BATCH): room for N entries in each array.
-struct DcSlot {
-    u32* dist = nullptr;
-    u32* item_pos = nullptr;
+// Where distance coding writes.  Every device pointer is nullable: the context's own arena is used for what the caller does
+// not want, and dc_device sets the pointer to where the data is.
+struct DcBuffers {
+    u32* dist = nullptr;         // n
+    u32* item_pos = nullptr;     // num_items
     u32* item_dist = nullptr;
     u8* item_sym = nullptr;
     u8* item_rank = nullptr;
+    u32* item_starts = nullptr;  // many blocks: count + 1
 };
 
 // The tile status words of the radix passes (decoupled look-back), carved from the arena: every row a pass reads must
@@ -207,7 +209,7 @@ struct dark_bwt_ctx {
     u8* d_text2 = nullptr;  // second pair for the pipelined batch entries (== d_text, d_bwt on a one-pair context)
     u8* d_bwt2 = nullptr;
     int pipeline_depth = 0;  // staging pairs: 2, or 1 above 2^31 (the batch entries then run their blocks serially)
-    DcSlot dc_slot[2];  // DARK_BWT_F_DC_BATCH: block k of a pipelined DC batch is coded into slot k & 1
+    DcBuffers dc_slot[2];  // DARK_BWT_F_DC_BATCH: block k of a pipelined DC batch is coded into slot k & 1 (N entries each)
     cudaStream_t copy_in = nullptr, copy_out = nullptr;
     cudaEvent_t ev_in[2] = {nullptr, nullptr}, ev_comp[2] = {nullptr, nullptr}, ev_out[2] = {nullptr, nullptr};
     u32* hist = nullptr;
@@ -1370,18 +1372,6 @@ int inverse_device(dark_bwt_ctx* ctx, const u8* d_bwt, u32 n, u32 origin, const 
 }
 
 // ---- distance coding ----------------------------------------------------------------------------
-// Where distance coding writes.  Every device pointer is nullable: the context's own arena is used for what the caller does
-// not want, and dc_device sets the pointer to where the data is.
-struct DcBuffers {
-    u32* dist = nullptr;         // n
-    u32* item_pos = nullptr;     // num_items
-    u32* item_dist = nullptr;
-    u8* item_sym = nullptr;
-    u8* item_rank = nullptr;
-    u32* item_starts = nullptr;  // many blocks: count + 1
-    std::vector<u32> item_starts_host;  // many blocks: item_starts, read back
-};
-
 // The per-block records of the many-block pass are staged in the sort's second key buffer (8 N + 1 KiB bytes), which distance
 // coding leaves free: count * sizeof(DcRecDev) <= 8 * capacity + 1024.
 bool dc_many_records_fit(const dark_bwt_ctx* ctx, u64 count) {
@@ -1390,9 +1380,10 @@ bool dc_many_records_fit(const dark_bwt_ctx* ctx, u64 count) {
 
 // Distance coding + MTF on device buffers (dc_kernels.cuh) of one BWT block d_bwt[0..n) (`blocks` null; 1 <= n <= capacity),
 // or in one pass of the checked list `blocks`, back to back in d_bwt and loaded into ctx->many_starts (the records fit).
-// One block: infos[0] gets the result header.  Many: infos[0..count) get the per-block records, io->item_starts_host the
-// item offsets.
-int dc_device(dark_bwt_ctx* ctx, const u8* d_bwt, u32 n, const BlockList* blocks, DcBuffers* io, dark_bwt_dc_info* infos) {
+// One block: infos[0] gets the result header.  Many: infos[0..count) get the per-block records, *item_starts_host the
+// item offsets, read back.
+int dc_device(dark_bwt_ctx* ctx, const u8* d_bwt, u32 n, const BlockList* blocks, DcBuffers* io, dark_bwt_dc_info* infos,
+              std::vector<u32>* item_starts_host) {
     CK(cudaSetDevice(ctx->device));
     const u32 nblocks = (u32)ceil_div(n, kDcBlock);
     // last-occurrence tables: (nblocks + ngroups) x 256 words = n/4 + n/1024 bytes (+ 2 KB): inside the 4n-byte rank buffer for
@@ -1459,7 +1450,7 @@ int dc_device(dark_bwt_ctx* ctx, const u8* d_bwt, u32 n, const BlockList* blocks
     }
     const u32 count = many.count;
     std::vector<DcRecDev> recs(count);
-    std::vector<u32>& hs = io->item_starts_host;
+    std::vector<u32>& hs = *item_starts_host;
     hs.resize((size_t)count + 1);
     CK(cudaMemcpyAsync(recs.data(), many.recs, sizeof(DcRecDev) * count, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaMemcpyAsync(hs.data(), io->item_starts, sizeof(u32) * ((size_t)count + 1), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1488,6 +1479,18 @@ bool is_pageable(const void* p) {
     return a.type == cudaMemoryTypeUnregistered;
 }
 
+void stage_release(HostStage& st) {
+    for (int i = 0; i < HostStage::kMaxLanes; ++i) {
+        if (st.streams[i]) cudaStreamDestroy(st.streams[i]);
+        for (int k = 0; k < 2; ++k)
+            if (st.slot_done[i][k]) cudaEventDestroy(st.slot_done[i][k]);
+    }
+    if (st.pinned) cudaFreeHost(st.pinned);
+    st = HostStage();
+}
+
+// Sets up the lanes of `st` once: 0 when they are ready, 1 when there are none (switched off, or no pinned memory), or a
+// CUDA error code.  A failure part-way releases what was made, so that the next call starts from a clean state.
 int stage_prepare(dark_bwt_ctx* ctx, HostStage& st) {
     if (st.lanes > 0) return 0;
     const int lanes = ctx->knobs.host_threads;
@@ -1498,24 +1501,19 @@ int stage_prepare(dark_bwt_ctx* ctx, HostStage& st) {
         st.pinned = nullptr;
         return 1;  // no pinned memory to be had: fall back to the driver's own staging
     }
+    auto release = [&](int rc) {
+        stage_release(st);
+        return rc;
+    };
     for (int i = 0; i < lanes; ++i) {
-        if (cudaStreamCreateWithFlags(&st.streams[i], cudaStreamNonBlocking) != cudaSuccess) return ctx->fail_cuda(cudaGetLastError(), "staging stream", __LINE__);
+        if (cudaStreamCreateWithFlags(&st.streams[i], cudaStreamNonBlocking) != cudaSuccess)
+            return release(ctx->fail_cuda(cudaGetLastError(), "staging stream", __LINE__));
         for (int k = 0; k < 2; ++k)
             if (cudaEventCreateWithFlags(&st.slot_done[i][k], cudaEventDisableTiming) != cudaSuccess)
-                return ctx->fail_cuda(cudaGetLastError(), "staging event", __LINE__);
+                return release(ctx->fail_cuda(cudaGetLastError(), "staging event", __LINE__));
     }
     st.lanes = lanes;
     return 0;
-}
-
-void stage_release(HostStage& st) {
-    for (int i = 0; i < HostStage::kMaxLanes; ++i) {
-        if (st.streams[i]) cudaStreamDestroy(st.streams[i]);
-        for (int k = 0; k < 2; ++k)
-            if (st.slot_done[i][k]) cudaEventDestroy(st.slot_done[i][k]);
-    }
-    if (st.pinned) cudaFreeHost(st.pinned);
-    st = HostStage();
 }
 
 // Copies `bytes` between a pageable host buffer and device memory through the lanes of `st`; returns when done.
@@ -1575,67 +1573,83 @@ int staged_copy(dark_bwt_ctx* ctx, HostStage& st, void* dev, void* host, size_t 
 
 constexpr size_t kStageMinBytes = 1u << 20;  // smaller copies go straight to cudaMemcpyAsync
 
-// host -> device on `stream` semantics: returns after the copy has completed
-int copy_in_blocking(dark_bwt_ctx* ctx, u8* dev, const u8* host, size_t bytes, cudaStream_t stream) {
-    if (bytes >= kStageMinBytes && is_pageable(host)) {
-        const int rc = stage_prepare(ctx, ctx->stage_in);
-        if (rc > 1) return rc;
-        if (rc == 0) return staged_copy(ctx, ctx->stage_in, dev, (void*)host, bytes, true);
-    }
-    CK(cudaMemcpyAsync(dev, host, bytes, cudaMemcpyHostToDevice, stream));
-    CK(cudaStreamSynchronize(stream));
-    return 0;
-}
-int copy_out_blocking(dark_bwt_ctx* ctx, void* host, const void* dev, size_t bytes, cudaStream_t stream) {
-    if (bytes >= kStageMinBytes && is_pageable(host)) {
-        const int rc = stage_prepare(ctx, ctx->stage_out);
-        if (rc > 1) return rc;
-        if (rc == 0) return staged_copy(ctx, ctx->stage_out, (void*)dev, host, bytes, false);
-    }
-    CK(cudaMemcpyAsync(host, dev, bytes, cudaMemcpyDeviceToHost, stream));
-    CK(cudaStreamSynchronize(stream));
-    return 0;
+// The staging rule of every host copy in direction `kind`: a pageable host buffer of kStageMinBytes or more goes through the
+// context's lanes for that direction (*stage), anything else straight to cudaMemcpyAsync (*stage null), and so does every
+// buffer when the lanes are switched off or no pinned memory is to be had.  Returns 0 or a CUDA error code.
+int stage_for(dark_bwt_ctx* ctx, const void* host, size_t bytes, cudaMemcpyKind kind, HostStage** stage) {
+    *stage = nullptr;
+    if (bytes < kStageMinBytes || !is_pageable(host)) return 0;
+    HostStage& st = kind == cudaMemcpyHostToDevice ? ctx->stage_in : ctx->stage_out;
+    const int rc = stage_prepare(ctx, st);
+    if (rc == 0) *stage = &st;
+    return rc == 1 ? 0 : rc;
 }
 
-// The device -> host copies of one block's results, issued in order.  Absent outputs (null host pointers) and empty copies
-// are left out.  `serial`: a source is single-buffered (the next block overwrites it), so the copies must be complete
-// before the next block is transformed.
-struct OutCopies {
+// Copies between caller host buffers and device buffers in one direction, issued in order.  Absent buffers (null host
+// pointers) and empty copies are left out.  `serial` (the pipelined copy-out): a source is single-buffered (the next block
+// overwrites it), so the copies must be complete before the next block is transformed.
+struct CopyList {
     struct Copy {
         void* host;
-        const void* dev;
+        void* dev;
         size_t bytes;
     };
     Copy list[6];  // the most any entry copies: BWT, distances and the four item arrays
     int count = 0;
     bool serial = false;
-    void add(void* host, const void* dev, size_t bytes) {
-        if (host && bytes) list[count++] = Copy{host, dev, bytes};
+    void add(const void* host, const void* dev, size_t bytes) {
+        if (host && bytes) list[count++] = Copy{(void*)host, (void*)dev, bytes};
     }
 };
+
+// Runs `copies` in direction `kind` and returns when every one has completed: the staged ones through the lanes, the others
+// with cudaMemcpyAsync on `stream` and one synchronise.  The caller has made sure that the device side is ready.
+int copy_blocking(dark_bwt_ctx* ctx, const CopyList& copies, cudaMemcpyKind kind, cudaStream_t stream) {
+    const bool to_device = kind == cudaMemcpyHostToDevice;
+    bool direct = false;
+    for (int i = 0; i < copies.count; ++i) {
+        const CopyList::Copy& c = copies.list[i];
+        HostStage* st;
+        if (int rc = stage_for(ctx, c.host, c.bytes, kind, &st)) return rc;
+        if (st) {
+            if (int rc = staged_copy(ctx, *st, c.dev, c.host, c.bytes, to_device)) return rc;
+        } else {
+            CK(cudaMemcpyAsync(to_device ? c.dev : c.host, to_device ? c.host : c.dev, c.bytes, kind, stream));
+            direct = true;
+        }
+    }
+    if (direct) CK(cudaStreamSynchronize(stream));
+    return 0;
+}
+
+// A block's distance-coding outputs, where dc_device left them in `io`, to the caller's host arrays (each nullable): the
+// distances (n entries) and the four item arrays (`items` entries).
+void add_dc_outputs(CopyList* out, const DcBuffers& io, u64 n, u64 items, uint32_t* dist, uint32_t* item_pos,
+                    uint32_t* item_dist, uint8_t* item_sym, uint8_t* item_rank) {
+    out->add(dist, io.dist, n * sizeof(u32));
+    out->add(item_pos, io.item_pos, items * sizeof(u32));
+    out->add(item_dist, io.item_dist, items * sizeof(u32));
+    out->add(item_sym, io.item_sym, items);
+    out->add(item_rank, io.item_rank, items);
+}
 
 // The pipelined loop of the batch entries: `count` host blocks ins[k] (ns[k] bytes).  While block k is transformed
 // (transform(k, b, d_in[b], &copies), synchronous on the context's stream; b = k & 1 selects the block's device buffers),
 // block k+1 is copied into the other input buffer and the copies of block k-1 run out of the other buffers.  Pinned host
-// buffers ride on the two copy streams; a list with a pageable buffer of 1 MiB or more is sent one copy after another by a
-// helper thread, the pageable copies through the staging lanes.  A context with one staging pair (pipeline_depth 1: above
-// 2^31) has only b = 0: the copy-in of block k+1 starts once transform k has returned and the copies of block k have drained.
+// buffers ride on the two copy streams; a list with a staged copy (stage_for) is sent by a helper thread through
+// copy_blocking.  A context with one staging pair (pipeline_depth 1: above 2^31) has only b = 0: the copy-in of block k+1
+// starts once transform k has returned and the copies of block k have drained.
 template <typename Transform>
 int run_pipelined(dark_bwt_ctx* ctx, const u8* const* ins, const uint64_t* ns, uint64_t count, u8* const d_in[2], Transform transform) {
     bool comp_recorded[2] = {false, false}, out_recorded[2] = {false, false};
     std::future<int> fin[2], fout;
-    auto staged_in = [&](uint64_t k) { return ns[k] >= kStageMinBytes && is_pageable(ins[k]) && stage_prepare(ctx, ctx->stage_in) == 0; };
-    auto staged_out = [&](const OutCopies& oc) {
-        for (int i = 0; i < oc.count; ++i)
-            if (oc.list[i].bytes >= kStageMinBytes && is_pageable(oc.list[i].host) && stage_prepare(ctx, ctx->stage_out) == 0) return true;
-        return false;
-    };
     auto start_in = [&](uint64_t k, int buf) -> int {  // the transform that read d_in[buf] has returned (it is synchronous)
-        if (staged_in(k)) {
-            u8* dst = d_in[buf];
-            const u8* src = ins[k];
-            const size_t bytes = ns[k];
-            fin[buf] = std::async(std::launch::async, [ctx, dst, src, bytes] { return staged_copy(ctx, ctx->stage_in, dst, (void*)src, bytes, true); });
+        HostStage* st;
+        if (int rc = stage_for(ctx, ins[k], ns[k], cudaMemcpyHostToDevice, &st)) return rc;
+        if (st) {
+            fin[buf] = std::async(std::launch::async, [ctx, st, dst = d_in[buf], src = ins[k], bytes = ns[k]] {
+                return staged_copy(ctx, *st, dst, (void*)src, bytes, true);
+            });
             return 0;
         }
         if (comp_recorded[buf]) CK(cudaStreamWaitEvent(ctx->copy_in, ctx->ev_comp[buf], 0));
@@ -1663,7 +1677,7 @@ int run_pipelined(dark_bwt_ctx* ctx, const u8* const* ins, const uint64_t* ns, u
             if (int rc = start_in(k + 1, nb)) { drain(); return rc; }
         // (a staged copy-out of block k-1 may still be reading the OTHER buffers; these were drained before it began)
         if (out_recorded[b]) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_out[b], 0));  // output buffers b drained
-        OutCopies oc;
+        CopyList oc;
         int rc = transform(k, b, (const u8*)d_in[b], &oc);
         if (rc) { drain(); return rc; }
         if (depth == 1) oc.serial = true;
@@ -1671,12 +1685,13 @@ int run_pipelined(dark_bwt_ctx* ctx, const u8* const* ins, const uint64_t* ns, u
         comp_recorded[b] = true;
         if (fout.valid())
             if (int rc2 = fout.get()) { drain(); return rc2; }  // one staged copy-out at a time (they share the lanes)
-        if (staged_out(oc)) {
+        HostStage* staged = nullptr;  // one staged copy sends the whole list to the helper thread
+        for (int i = 0; i < oc.count && !staged; ++i)
+            if (int rc2 = stage_for(ctx, oc.list[i].host, oc.list[i].bytes, cudaMemcpyDeviceToHost, &staged)) { drain(); return rc2; }
+        if (staged) {
             fout = std::async(std::launch::async, [ctx, oc] {
                 if (cudaSetDevice(ctx->device) != cudaSuccess) return ctx->fail_cuda(cudaGetLastError(), "helper thread device", __LINE__);
-                for (int i = 0; i < oc.count; ++i)
-                    if (int r = copy_out_blocking(ctx, oc.list[i].host, oc.list[i].dev, oc.list[i].bytes, ctx->copy_out)) return r;
-                return 0;
+                return copy_blocking(ctx, oc, cudaMemcpyDeviceToHost, ctx->copy_out);
             });
             if (oc.serial)
                 if (int rc2 = fout.get()) { drain(); return rc2; }
@@ -1748,7 +1763,7 @@ size_t carve_arena(dark_bwt_ctx* ctx) {
     carve(ctx->many_lut, sizeof(u16) * 256);
     carve(ctx->dc_info, sizeof(DcInfoDev) + 16);
     if (dc_batch)
-        for (DcSlot& s : ctx->dc_slot) {
+        for (DcBuffers& s : ctx->dc_slot) {
             carve(s.dist, N * 4 + 16), carve(s.item_pos, N * 4 + 16), carve(s.item_dist, N * 4 + 16);
             carve(s.item_sym, N + 16), carve(s.item_rank, N + 16);
         }
@@ -1882,18 +1897,18 @@ int dark_bwt_forward_device(dark_bwt_ctx* ctx, const uint8_t* d_text, uint64_t n
 static int forward_host(dark_bwt_ctx* ctx, const uint8_t* text, uint64_t n, uint8_t* bwt_out, uint64_t* origin_out, uint32_t* sa_out,
                         dark_bwt_stats* stats) {
     CK(cudaSetDevice(ctx->device));
-    // pinned (or registered) buffers are copied directly, pageable ones through the context's pinned staging lanes
     typedef std::chrono::steady_clock Clock;
     auto ms_since = [](Clock::time_point t0) { return std::chrono::duration<float, std::milli>(Clock::now() - t0).count(); };
+    CopyList in, out;
+    in.add(text, ctx->d_text, n);
+    out.add(bwt_out, ctx->d_bwt, n);
+    out.add(sa_out, ctx->sa, n * sizeof(u32));
     Clock::time_point t0 = Clock::now();
-    if (int rc = copy_in_blocking(ctx, ctx->d_text, text, n, ctx->stream)) return rc;
+    if (int rc = copy_blocking(ctx, in, cudaMemcpyHostToDevice, ctx->stream)) return rc;
     if (stats) stats->h2d_ms = ms_since(t0);
     if (int rc = forward_device(ctx, ctx->d_text, (u32)n, ctx->d_bwt, origin_out, nullptr, stats)) return rc;
     t0 = Clock::now();
-    if (bwt_out)
-        if (int rc = copy_out_blocking(ctx, bwt_out, ctx->d_bwt, n, ctx->stream)) return rc;
-    if (sa_out)
-        if (int rc = copy_out_blocking(ctx, sa_out, ctx->sa, n * sizeof(u32), ctx->stream)) return rc;
+    if (int rc = copy_blocking(ctx, out, cudaMemcpyDeviceToHost, ctx->stream)) return rc;
     if (stats) stats->d2h_ms = ms_since(t0);
     return DARK_BWT_OK;
 }
@@ -1920,7 +1935,7 @@ int dark_bwt_forward_batch(dark_bwt_ctx* ctx, const uint8_t* const* texts, const
     CK(cudaSetDevice(ctx->device));
     u8* const d_text[2] = {ctx->d_text, ctx->d_text2};
     u8* const d_bwt[2] = {ctx->d_bwt, ctx->d_bwt2};
-    return run_pipelined(ctx, texts, ns, count, d_text, [&](uint64_t k, int b, const u8* din, OutCopies* out) {
+    return run_pipelined(ctx, texts, ns, count, d_text, [&](uint64_t k, int b, const u8* din, CopyList* out) {
         dark_bwt_stats* st = stats ? stats + k : nullptr;
         if (st) st->h2d_ms = 0.f;
         if (int rc = forward_device(ctx, din, (u32)ns[k], d_bwt[b], origins_out + k, nullptr, st)) return rc;
@@ -1947,7 +1962,7 @@ int dark_bwt_inverse_batch(dark_bwt_ctx* ctx, const uint8_t* const* bwts, const 
     CK(cudaSetDevice(ctx->device));
     u8* const d_bwt[2] = {ctx->d_bwt, ctx->d_bwt2};
     u8* const d_text[2] = {ctx->d_text, ctx->d_text2};
-    return run_pipelined(ctx, bwts, ns, count, d_bwt, [&](uint64_t k, int b, const u8* din, OutCopies* out) {
+    return run_pipelined(ctx, bwts, ns, count, d_bwt, [&](uint64_t k, int b, const u8* din, CopyList* out) {
         if (int rc = inverse_device(ctx, din, (u32)ns[k], (u32)origins[k], nullptr, d_text[b], ms_out ? ms_out + k : nullptr)) return rc;
         out->add(text_outs[k], d_text[b], ns[k]);
         return 0;
@@ -2019,9 +2034,12 @@ int dark_bwt_inverse(dark_bwt_ctx* ctx, const uint8_t* bwt, uint64_t n, uint64_t
     if (origin >= n) return DARK_BWT_E_INVALID_ARG;
     ctx->err[0] = 0;
     CK(cudaSetDevice(ctx->device));
-    if (int rc = copy_in_blocking(ctx, ctx->d_bwt, bwt, n, ctx->stream)) return rc;
+    CopyList in, out;
+    in.add(bwt, ctx->d_bwt, n);
+    out.add(text_out, ctx->d_text, n);
+    if (int rc = copy_blocking(ctx, in, cudaMemcpyHostToDevice, ctx->stream)) return rc;
     if (int rc = inverse_device(ctx, ctx->d_bwt, (u32)n, (u32)origin, nullptr, ctx->d_text, nullptr)) return rc;
-    return copy_out_blocking(ctx, text_out, ctx->d_text, n, ctx->stream);
+    return copy_blocking(ctx, out, cudaMemcpyDeviceToHost, ctx->stream);
 }
 
 int dark_bwt_inverse_many(dark_bwt_ctx* ctx, const uint8_t* const* bwts, const uint64_t* ns, const uint64_t* origins,
@@ -2052,35 +2070,13 @@ int dark_bwt_inverse_many_device(dark_bwt_ctx* ctx, const uint8_t* d_bwt, const 
     return inverse_device(ctx, d_bwt, bl.total(), 0, &bl, d_text_out, ms_out);
 }
 
-// Host copies of what dc_device left in `io`, one copy per array (`items` runs in all); null host pointers are skipped.
-static int dc_copy_out(dark_bwt_ctx* ctx, u64 n, u64 items, const DcBuffers& io, uint32_t* dist_out, uint32_t* item_starts,
-                       uint32_t* item_pos, uint32_t* item_dist, uint8_t* item_sym, uint8_t* item_rank) {
-    if (dist_out)
-        if (int rc = copy_out_blocking(ctx, dist_out, io.dist, n * sizeof(u32), ctx->stream)) return rc;
-    if (item_starts) memcpy(item_starts, io.item_starts_host.data(), io.item_starts_host.size() * sizeof(u32));
-    if (item_pos && items)
-        if (int rc = copy_out_blocking(ctx, item_pos, io.item_pos, items * sizeof(u32), ctx->stream)) return rc;
-    if (item_dist && items)
-        if (int rc = copy_out_blocking(ctx, item_dist, io.item_dist, items * sizeof(u32), ctx->stream)) return rc;
-    if (item_sym && items)
-        if (int rc = copy_out_blocking(ctx, item_sym, io.item_sym, items, ctx->stream)) return rc;
-    if (item_rank && items)
-        if (int rc = copy_out_blocking(ctx, item_rank, io.item_rank, items, ctx->stream)) return rc;
-    return DARK_BWT_OK;
-}
-
 int dark_bwt_dc_encode_device(dark_bwt_ctx* ctx, const uint8_t* d_bwt, uint64_t n, uint32_t* d_dist_out, uint32_t* d_item_pos,
                               uint32_t* d_item_dist, uint8_t* d_item_sym, uint8_t* d_item_rank, dark_bwt_dc_info* info) {
     if (!ctx || !d_bwt || !info) return DARK_BWT_E_INVALID_ARG;
     if (int rc = check_n(ctx, n, 1)) return rc;
     ctx->err[0] = 0;
-    DcBuffers io;
-    io.dist = d_dist_out;
-    io.item_pos = d_item_pos;
-    io.item_dist = d_item_dist;
-    io.item_sym = d_item_sym;
-    io.item_rank = d_item_rank;
-    return dc_device(ctx, d_bwt, (u32)n, nullptr, &io, info);
+    DcBuffers io{d_dist_out, d_item_pos, d_item_dist, d_item_sym, d_item_rank};
+    return dc_device(ctx, d_bwt, (u32)n, nullptr, &io, info, nullptr);
 }
 
 int dark_bwt_dc_encode(dark_bwt_ctx* ctx, const uint8_t* bwt, uint64_t n, uint32_t* dist_out, uint32_t* item_pos, uint32_t* item_dist,
@@ -2090,10 +2086,13 @@ int dark_bwt_dc_encode(dark_bwt_ctx* ctx, const uint8_t* bwt, uint64_t n, uint32
     if (int rc = check_n(ctx, n, 1)) return rc;
     ctx->err[0] = 0;
     CK(cudaSetDevice(ctx->device));
-    if (int rc = copy_in_blocking(ctx, ctx->d_bwt, bwt, n, ctx->stream)) return rc;
+    CopyList in, out;
+    in.add(bwt, ctx->d_bwt, n);
+    if (int rc = copy_blocking(ctx, in, cudaMemcpyHostToDevice, ctx->stream)) return rc;
     DcBuffers io;
-    if (int rc = dc_device(ctx, ctx->d_bwt, (u32)n, nullptr, &io, info)) return rc;
-    return dc_copy_out(ctx, n, info->num_items, io, dist_out, nullptr, item_pos, item_dist, item_sym, item_rank);
+    if (int rc = dc_device(ctx, ctx->d_bwt, (u32)n, nullptr, &io, info, nullptr)) return rc;
+    add_dc_outputs(&out, io, n, info->num_items, dist_out, item_pos, item_dist, item_sym, item_rank);
+    return copy_blocking(ctx, out, cudaMemcpyDeviceToHost, ctx->stream);
 }
 
 int dark_bwt_forward_dc(dark_bwt_ctx* ctx, const uint8_t* text, uint64_t n, uint8_t* bwt_out, uint64_t* origin_out, uint32_t* dist_out,
@@ -2106,8 +2105,10 @@ int dark_bwt_forward_dc(dark_bwt_ctx* ctx, const uint8_t* text, uint64_t n, uint
     if (int rc = forward_host(ctx, text, n, bwt_out, origin_out, nullptr, stats)) return rc;
     // the BWT is still in HBM: distance coding reads it there
     DcBuffers io;
-    if (int rc = dc_device(ctx, ctx->d_bwt, (u32)n, nullptr, &io, info)) return rc;
-    return dc_copy_out(ctx, n, info->num_items, io, dist_out, nullptr, item_pos, item_dist, item_sym, item_rank);
+    if (int rc = dc_device(ctx, ctx->d_bwt, (u32)n, nullptr, &io, info, nullptr)) return rc;
+    CopyList out;
+    add_dc_outputs(&out, io, n, info->num_items, dist_out, item_pos, item_dist, item_sym, item_rank);
+    return copy_blocking(ctx, out, cudaMemcpyDeviceToHost, ctx->stream);
 }
 
 int dark_bwt_forward_dc_batch(dark_bwt_ctx* ctx, const uint8_t* const* texts, const uint64_t* ns, uint64_t count, uint8_t* const* bwt_outs,
@@ -2128,26 +2129,16 @@ int dark_bwt_forward_dc_batch(dark_bwt_ctx* ctx, const uint8_t* const* texts, co
     // Block k: the forward into d_bwt[b], then distance coding of it into slot b (b = k & 1).  Its scratch (run starts,
     // tables, run counts, the status buffer a small block borrows) is consumed before block k+1's forward starts on the
     // same stream; what the copies read stays untouched until the wait on ev_out[b] before block k+2.
-    return run_pipelined(ctx, texts, ns, count, d_text, [&](uint64_t k, int b, const u8* din, OutCopies* out) {
+    return run_pipelined(ctx, texts, ns, count, d_text, [&](uint64_t k, int b, const u8* din, CopyList* out) {
         const u64 n = ns[k];
         dark_bwt_stats* st = stats ? stats + k : nullptr;
         if (st) st->h2d_ms = 0.f;
         if (int rc = forward_device(ctx, din, (u32)n, d_bwt[b], origins_out + k, nullptr, st)) return rc;
-        const DcSlot& slot = ctx->dc_slot[b];
-        DcBuffers io;
-        io.dist = slot.dist;
-        io.item_pos = slot.item_pos;
-        io.item_dist = slot.item_dist;
-        io.item_sym = slot.item_sym;
-        io.item_rank = slot.item_rank;
-        if (int rc = dc_device(ctx, d_bwt[b], (u32)n, nullptr, &io, infos + k)) return rc;
-        const u64 items = infos[k].num_items;
+        DcBuffers io = ctx->dc_slot[b];
+        if (int rc = dc_device(ctx, d_bwt[b], (u32)n, nullptr, &io, infos + k, nullptr)) return rc;
         out->add(bwt_outs ? bwt_outs[k] : nullptr, d_bwt[b], n);
-        out->add(dist_outs ? dist_outs[k] : nullptr, slot.dist, n * sizeof(u32));
-        out->add(item_pos ? item_pos[k] : nullptr, slot.item_pos, items * sizeof(u32));
-        out->add(item_dist ? item_dist[k] : nullptr, slot.item_dist, items * sizeof(u32));
-        out->add(item_sym ? item_sym[k] : nullptr, slot.item_sym, items);
-        out->add(item_rank ? item_rank[k] : nullptr, slot.item_rank, items);
+        add_dc_outputs(out, io, n, infos[k].num_items, dist_outs ? dist_outs[k] : nullptr, item_pos ? item_pos[k] : nullptr,
+                       item_dist ? item_dist[k] : nullptr, item_sym ? item_sym[k] : nullptr, item_rank ? item_rank[k] : nullptr);
         return 0;
     });
 }
@@ -2162,14 +2153,9 @@ int dark_bwt_dc_encode_many_device(dark_bwt_ctx* ctx, const uint8_t* d_bwt, cons
     if (int rc = check_blocks(ctx, count, nullptr, d_starts, nullptr, 1, 0, nullptr, nullptr, &bl)) return rc;
     if (!dc_many_records_fit(ctx, count)) return DARK_BWT_E_INVALID_N;
     if (int rc = load_blocks(ctx, bl)) return rc;
-    DcBuffers io;
-    io.dist = d_dist_out;
-    io.item_starts = d_item_starts;
-    io.item_pos = d_item_pos;
-    io.item_dist = d_item_dist;
-    io.item_sym = d_item_sym;
-    io.item_rank = d_item_rank;
-    if (int rc = dc_device(ctx, d_bwt, bl.total(), &bl, &io, infos)) return rc;
+    DcBuffers io{d_dist_out, d_item_pos, d_item_dist, d_item_sym, d_item_rank, d_item_starts};
+    std::vector<u32> starts;
+    if (int rc = dc_device(ctx, d_bwt, bl.total(), &bl, &io, infos, &starts)) return rc;
     if (ms_out) *ms_out = infos[0].device_ms;
     return DARK_BWT_OK;
 }
@@ -2190,9 +2176,13 @@ int dark_bwt_dc_encode_many(dark_bwt_ctx* ctx, const uint8_t* const* bwts, const
     CK(cudaSetDevice(ctx->device));
     if (int rc = load_blocks(ctx, bl, bwts, ctx->d_bwt)) return rc;
     DcBuffers io;
-    if (int rc = dc_device(ctx, ctx->d_bwt, bl.total(), &bl, &io, infos)) return rc;
+    std::vector<u32> starts;
+    if (int rc = dc_device(ctx, ctx->d_bwt, bl.total(), &bl, &io, infos, &starts)) return rc;
     if (ms_out) *ms_out = infos[0].device_ms;
-    return dc_copy_out(ctx, bl.total(), io.item_starts_host.back(), io, dist_out, item_starts, item_pos, item_dist, item_sym, item_rank);
+    if (item_starts) memcpy(item_starts, starts.data(), starts.size() * sizeof(u32));
+    CopyList out;
+    add_dc_outputs(&out, io, bl.total(), starts.back(), dist_out, item_pos, item_dist, item_sym, item_rank);
+    return copy_blocking(ctx, out, cudaMemcpyDeviceToHost, ctx->stream);
 }
 
 int dark_bwt_forward_dc_many(dark_bwt_ctx* ctx, const uint8_t* const* texts, const uint64_t* ns, uint64_t count, uint8_t* const* bwt_outs,
@@ -2211,8 +2201,12 @@ int dark_bwt_forward_dc_many(dark_bwt_ctx* ctx, const uint8_t* const* texts, con
     if (int rc = forward_many_host(ctx, texts, bwt_outs, origins_out, bl, stats)) return rc;
     // the BWTs are still in HBM at the same offsets, and ctx->many_starts still holds them
     DcBuffers io;
-    if (int rc = dc_device(ctx, ctx->d_bwt, bl.total(), &bl, &io, infos)) return rc;
-    return dc_copy_out(ctx, bl.total(), io.item_starts_host.back(), io, dist_out, item_starts, item_pos, item_dist, item_sym, item_rank);
+    std::vector<u32> starts;
+    if (int rc = dc_device(ctx, ctx->d_bwt, bl.total(), &bl, &io, infos, &starts)) return rc;
+    if (item_starts) memcpy(item_starts, starts.data(), starts.size() * sizeof(u32));
+    CopyList out;
+    add_dc_outputs(&out, io, bl.total(), starts.back(), dist_out, item_pos, item_dist, item_sym, item_rank);
+    return copy_blocking(ctx, out, cudaMemcpyDeviceToHost, ctx->stream);
 }
 
 int dark_bwt_reuse(dark_bwt_ctx* ctx, uint32_t** words_out, uint64_t* count_out) {
