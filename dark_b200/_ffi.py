@@ -20,7 +20,13 @@ SYMBOLS = [
     "dark_bwt_stream", "dark_bwt_sort_pairs_device", "dark_bwt_verify_sa_device", "dark_bwt_emit_device", "dark_bwt_lcp_profile_device",
     "dark_bwt_synth", "dark_bwt_dc_encode_device", "dark_bwt_dc_encode", "dark_bwt_forward_dc", "dark_bwt_dc_encode_many",
     "dark_bwt_dc_encode_many_device", "dark_bwt_forward_dc_many", "dark_bwt_forward_dc_batch",
+    "dark_bwt_dc_encode_packed_device", "dark_bwt_forward_dc_packed", "dark_bwt_forward_dc_packed_batch",
 ]
+
+
+def dc_packed_max(n):
+    """DARK_BWT_DC_PACKED_MAX(n): the most bytes the packed item stream of an n-byte block takes."""
+    return 8 * int(n)
 
 
 class Stats(ctypes.Structure):
@@ -122,6 +128,10 @@ def lib():
     L.dark_bwt_dc_encode_many_device.argtypes = [vp, vp, vp, u64, vp, vp, vp, vp, vp, vp, vp, ctypes.POINTER(ctypes.c_float)]
     L.dark_bwt_forward_dc_many.argtypes = [vp, vp, vp, u64, vp, vp, vp, vp, vp, vp, vp, vp, vp, ctypes.POINTER(Stats)]
     L.dark_bwt_forward_dc_batch.argtypes = [vp, vp, vp, u64, vp, vp, vp, vp, vp, vp, vp, vp, vp]
+    L.dark_bwt_dc_encode_packed_device.argtypes = [vp, vp, u64, vp, u64, ctypes.POINTER(u64), ctypes.POINTER(DcInfo)]
+    L.dark_bwt_forward_dc_packed.argtypes = [vp, vp, u64, vp, ctypes.POINTER(u64), vp, u64, ctypes.POINTER(u64),
+                                             ctypes.POINTER(DcInfo), ctypes.POINTER(Stats)]
+    L.dark_bwt_forward_dc_packed_batch.argtypes = [vp, vp, vp, u64, vp, vp, vp, vp, vp, vp, vp]
     _lib = L
     return L
 

@@ -65,6 +65,7 @@ struct Mailbox {  // pinned host memory the device results are copied into
     u32 not_pairs;  // the same answer from the check queued behind a re-rank (read with the survivor count)
     u32 bad_block;  // inverse: the lowest block whose list does not cover its rows (with `count` = how many do not)
     u32 bad_dist;   // inverse: the rows that block's list covers
+    unsigned long long packed_bytes;  // distance coding: the size of the packed item stream
 };
 
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
@@ -1469,6 +1470,35 @@ int dc_device(dark_bwt_ctx* ctx, const u8* d_bwt, u32 n, const BlockList* blocks
     return DARK_BWT_OK;
 }
 
+// The packed item stream (include/dark_bwt.h; kernels in dc_kernels.cuh) of the `items` items dc_device left in `io`, into
+// d_out, which holds `capacity` bytes.  *bytes_out = the stream's size, which the scan leaves in the mailbox; a size above
+// the capacity is DARK_BWT_E_INVALID_ARG before anything is written.  The tile sums and offsets go to ranks_alt and ranks
+// (at most 12 bytes per 2,048 items), which dc_device has finished with.  Returns after the stream is complete; adds the
+// pack's device time to *ms.
+int dc_pack(dark_bwt_ctx* ctx, const DcBuffers& io, u64 items, u8* d_out, u64 capacity, uint64_t* bytes_out, float* ms) {
+    const u32 ntiles = (u32)ceil_div(items, kPackTile);
+    u32* tile_bytes = ctx->ranks_alt;
+    u64* tile_off = (u64*)ctx->ranks;
+    CK(cudaEventRecord(ctx->call_start, ctx->stream));
+    k_dc_pack_sizes<<<ntiles, kPackThreads, 0, ctx->stream>>>(io.item_pos, io.item_dist, items, tile_bytes);
+    LAUNCHED();
+    k_dc_pack_scan<<<1, 1024, 0, ctx->stream>>>(tile_bytes, ntiles, tile_off, &ctx->mail_dev->packed_bytes);
+    LAUNCHED();
+    CK(cudaStreamSynchronize(ctx->stream));
+    *bytes_out = ctx->mail->packed_bytes;
+    if (*bytes_out > capacity) {
+        snprintf(ctx->err, sizeof(ctx->err), "the packed item stream needs %llu bytes, the buffer holds %llu",
+                 (unsigned long long)*bytes_out, (unsigned long long)capacity);
+        return DARK_BWT_E_INVALID_ARG;
+    }
+    k_dc_pack_write<<<ntiles, kPackThreads, 0, ctx->stream>>>(io.item_pos, io.item_dist, io.item_sym, io.item_rank, items, tile_off, d_out);
+    LAUNCHED();
+    CK(cudaEventRecord(ctx->call_stop, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    *ms += call_ms(ctx);
+    return DARK_BWT_OK;
+}
+
 // ---- pageable host buffers ---------------------------------------------------------------------
 bool is_pageable(const void* p) {
     cudaPointerAttributes a;
@@ -1657,11 +1687,13 @@ int run_pipelined(dark_bwt_ctx* ctx, const u8* const* ins, const uint64_t* ns, u
         CK(cudaEventRecord(ctx->ev_in[buf], ctx->copy_in));
         return 0;
     };
-    auto drain = [&]() {  // never leave a helper thread behind
+    auto drain = [&]() {  // never leave a helper thread or a copy behind: on an error, the blocks before it are complete
         int rc = 0;
         for (int i = 0; i < 2; ++i)
             if (fin[i].valid()) rc |= fin[i].get();
         if (fout.valid()) rc |= fout.get();
+        cudaStreamSynchronize(ctx->copy_out);
+        cudaStreamSynchronize(ctx->copy_in);
         return rc;
     };
     const uint64_t depth = (uint64_t)ctx->pipeline_depth;
@@ -2139,6 +2171,76 @@ int dark_bwt_forward_dc_batch(dark_bwt_ctx* ctx, const uint8_t* const* texts, co
         out->add(bwt_outs ? bwt_outs[k] : nullptr, d_bwt[b], n);
         add_dc_outputs(out, io, n, infos[k].num_items, dist_outs ? dist_outs[k] : nullptr, item_pos ? item_pos[k] : nullptr,
                        item_dist ? item_dist[k] : nullptr, item_sym ? item_sym[k] : nullptr, item_rank ? item_rank[k] : nullptr);
+        return 0;
+    });
+}
+
+int dark_bwt_dc_encode_packed_device(dark_bwt_ctx* ctx, const uint8_t* d_bwt, uint64_t n, uint8_t* d_stream_out, uint64_t stream_capacity,
+                                     uint64_t* stream_bytes_out, dark_bwt_dc_info* info) {
+    if (!ctx || !d_bwt || !d_stream_out || !stream_bytes_out || !info) return DARK_BWT_E_INVALID_ARG;
+    if (int rc = check_n(ctx, n, 1)) return rc;
+    ctx->err[0] = 0;
+    DcBuffers io;
+    if (int rc = dc_device(ctx, d_bwt, (u32)n, nullptr, &io, info, nullptr)) return rc;
+    return dc_pack(ctx, io, info->num_items, d_stream_out, stream_capacity, stream_bytes_out, &info->device_ms);
+}
+
+int dark_bwt_forward_dc_packed(dark_bwt_ctx* ctx, const uint8_t* text, uint64_t n, uint8_t* bwt_out, uint64_t* origin_out, uint8_t* stream_out,
+                               uint64_t stream_capacity, uint64_t* stream_bytes_out, dark_bwt_dc_info* info, dark_bwt_stats* stats) {
+    if (!ctx || !text || !origin_out || !stream_out || !stream_bytes_out || !info) return DARK_BWT_E_INVALID_ARG;
+    if (int rc = check_staging(ctx)) return rc;
+    if (int rc = check_n(ctx, n, 2)) return rc;
+    ctx->err[0] = 0;
+    if (int rc = forward_host(ctx, text, n, bwt_out, origin_out, nullptr, stats)) return rc;
+    DcBuffers io;
+    if (int rc = dc_device(ctx, ctx->d_bwt, (u32)n, nullptr, &io, info, nullptr)) return rc;
+    // the sort's second key buffer (8 N + 1 KiB), which single-block distance coding leaves free, holds any stream (<= 8 n)
+    u8* const d_stream = (u8*)ctx->keys[1];
+    if (int rc = dc_pack(ctx, io, info->num_items, d_stream, stream_capacity, stream_bytes_out, &info->device_ms)) return rc;
+    CopyList out;
+    out.add(stream_out, d_stream, *stream_bytes_out);
+    return copy_blocking(ctx, out, cudaMemcpyDeviceToHost, ctx->stream);
+}
+
+int dark_bwt_forward_dc_packed_batch(dark_bwt_ctx* ctx, const uint8_t* const* texts, const uint64_t* ns, uint64_t count,
+                                     uint8_t* const* bwt_outs, uint64_t* origins_out, uint8_t* const* stream_outs,
+                                     const uint64_t* stream_capacities, uint64_t* stream_bytes_out, dark_bwt_dc_info* infos,
+                                     dark_bwt_stats* stats) {
+    if (!ctx || !texts || !ns || !origins_out || !stream_outs || !stream_capacities || !stream_bytes_out || !infos)
+        return DARK_BWT_E_INVALID_ARG;
+    if (int rc = check_staging(ctx)) return rc;
+    if (!(ctx->flags & DARK_BWT_F_DC_BATCH)) return DARK_BWT_E_INVALID_ARG;  // no DC output slots
+    ctx->err[0] = 0;
+    for (uint64_t k = 0; k < count; ++k) {
+        if (!texts[k] || !stream_outs[k]) return DARK_BWT_E_INVALID_ARG;
+        if (int rc = check_n(ctx, ns[k], 2)) return rc;
+    }
+    if (count == 0) return DARK_BWT_OK;
+    CK(cudaSetDevice(ctx->device));
+    u8* const d_text[2] = {ctx->d_text, ctx->d_text2};
+    u8* const d_bwt[2] = {ctx->d_bwt, ctx->d_bwt2};
+    // Block k: the forward into d_bwt[b], distance coding into the context's scratch as in the single call, and the pack into
+    // slot b (b = k & 1): its dist and item_pos arrays, carved back to back, are 8 N + 32 bytes or more, room for any stream.
+    // The scratch is consumed before block k+1's forward starts on the same stream; what the copies read stays untouched
+    // until the wait on ev_out[b] before block k+2.
+    return run_pipelined(ctx, texts, ns, count, d_text, [&](uint64_t k, int b, const u8* din, CopyList* out) {
+        const u64 n = ns[k];
+        dark_bwt_stats* st = stats ? stats + k : nullptr;
+        if (st) st->h2d_ms = 0.f;
+        if (int rc = forward_device(ctx, din, (u32)n, d_bwt[b], origins_out + k, nullptr, st)) return rc;
+        DcBuffers io;
+        if (int rc = dc_device(ctx, d_bwt[b], (u32)n, nullptr, &io, infos + k, nullptr)) return rc;
+        u8* const d_stream = (u8*)ctx->dc_slot[b].dist;
+        if (int rc = dc_pack(ctx, io, infos[k].num_items, d_stream, stream_capacities[k], stream_bytes_out + k, &infos[k].device_ms)) {
+            if (rc == DARK_BWT_E_INVALID_ARG) {
+                char what[sizeof(ctx->err)];
+                memcpy(what, ctx->err, sizeof(what));
+                snprintf(ctx->err, sizeof(ctx->err), "block %llu: %.280s", (unsigned long long)k, what);
+            }
+            return rc;
+        }
+        out->add(stream_outs[k], d_stream, stream_bytes_out[k]);
+        out->add(bwt_outs ? bwt_outs[k] : nullptr, d_bwt[b], n);
         return 0;
     });
 }

@@ -431,4 +431,158 @@ k_dc_stream(const u32* __restrict__ run_start, const unsigned long long* __restr
     }
 }
 
+// ---- the packed item stream (include/dark_bwt.h): per item sym, rank, varint(run length - 1), varint(dist) ----------
+// The items k_dc_stream wrote, m of them, become one byte string in three launches over tiles of kPackTile items:
+//   k_dc_pack_sizes   each tile's byte count                                     (reads pos, dist: 8 B per item)
+//   k_dc_pack_scan    one CTA: the tile counts -> u64 tile offsets and the total (a stream can pass 2^32 bytes)
+//   k_dc_pack_write   each tile again: sizes, block scan, the tile's bytes built in shared memory, then stored as one
+//                     contiguous span with 16-byte stores (bytes one by one only in the span's first and last 16-byte word)
+constexpr int kPackThreads = 256;
+constexpr int kPackItems = 8;  // consecutive items per thread
+constexpr int kPackTile = kPackThreads * kPackItems;
+constexpr int kPackMaxItemBytes = 12;  // sym + rank + two varints of at most 5 bytes
+
+__device__ __forceinline__ u32 varint_bytes(u32 v) {
+    return 1u + (v >= (1u << 7)) + (v >= (1u << 14)) + (v >= (1u << 21)) + (v >= (1u << 28));
+}
+
+// run length - 1 of item k is pos[k] - pos[k-1] - 1 with pos[-1] = -1: in u32 arithmetic, prev = 0xFFFFFFFF for k = 0
+__global__ void __launch_bounds__(kPackThreads)
+k_dc_pack_sizes(const u32* __restrict__ pos, const u32* __restrict__ dist, u64 m, u32* __restrict__ tile_bytes) {
+    __shared__ u32 s_warp[kPackThreads / 32];
+    const u64 k0 = (u64)blockIdx.x * kPackTile + threadIdx.x;
+    u32 bytes = 0;
+#pragma unroll
+    for (int j = 0; j < kPackItems; ++j) {
+        const u64 k = k0 + (u64)j * kPackThreads;
+        if (k < m) {
+            const u32 prev = k ? pos[k - 1] : 0xFFFFFFFFu;
+            bytes += 2u + varint_bytes(pos[k] - prev - 1u) + varint_bytes(dist[k]);
+        }
+    }
+    bytes = __reduce_add_sync(0xffffffffu, bytes);
+    if ((threadIdx.x & 31) == 0) s_warp[threadIdx.x >> 5] = bytes;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        u32 t = 0;
+#pragma unroll
+        for (int w = 0; w < kPackThreads / 32; ++w) t += s_warp[w];
+        tile_bytes[blockIdx.x] = t;
+    }
+}
+
+// One CTA of 1024 threads, 4 tiles per thread and step: tile_off[t] = bytes of the tiles before t; *total = all of them
+// (the context's mapped mailbox: the host reads it after one synchronise).
+__global__ void __launch_bounds__(1024, 1)
+k_dc_pack_scan(const u32* __restrict__ tile_bytes, u32 ntiles, u64* __restrict__ tile_off, unsigned long long* __restrict__ total) {
+    __shared__ u64 s_warp[32];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    u64 carry = 0;
+    for (u32 base = 0; base < ntiles; base += 4096) {
+        const u32 i0 = base + 4u * (u32)tid;
+        u32 v[4];
+        u64 sum = 0;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            v[j] = i0 + j < ntiles ? tile_bytes[i0 + j] : 0u;
+            sum += v[j];
+        }
+        u64 x = sum;  // inclusive scan over the warp
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const u64 y = __shfl_up_sync(0xffffffffu, x, o);
+            if (lane >= o) x += y;
+        }
+        if (lane == 31) s_warp[warp] = x;
+        __syncthreads();
+        if (warp == 0) {
+            u64 w = s_warp[lane];
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const u64 y = __shfl_up_sync(0xffffffffu, w, o);
+                if (lane >= o) w += y;
+            }
+            s_warp[lane] = w;
+        }
+        __syncthreads();
+        u64 off = carry + (warp ? s_warp[warp - 1] : 0ull) + x - sum;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            if (i0 + j < ntiles) tile_off[i0 + j] = off;
+            off += v[j];
+        }
+        carry += s_warp[31];
+        __syncthreads();  // s_warp is rewritten by the next step
+    }
+    if (tid == 0) *total = carry;
+}
+
+// Thread t of a tile codes its items tile0 + 8t .. 8t+7 into s_buf at shift + (bytes of the tile's items before them),
+// shift = the address of the tile's first byte mod 16, so that s_buf's 16-byte words line up with out's.
+__global__ void __launch_bounds__(kPackThreads)
+k_dc_pack_write(const u32* __restrict__ pos, const u32* __restrict__ dist, const u8* __restrict__ sym, const u8* __restrict__ rank,
+                u64 m, const u64* __restrict__ tile_off, u8* __restrict__ out) {
+    __shared__ __align__(16) u8 s_buf[kPackTile * kPackMaxItemBytes + 16];
+    __shared__ u32 s_warp[kPackThreads / 32];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const u64 k0 = (u64)blockIdx.x * kPackTile + (u64)tid * kPackItems;
+    u32 p[kPackItems], d[kPackItems];
+    u32 prev = k0 > 0 && k0 < m ? pos[k0 - 1] : 0xFFFFFFFFu;
+    u32 bytes = 0;
+    {
+        u32 q = prev;
+#pragma unroll
+        for (int j = 0; j < kPackItems; ++j) {
+            const u64 k = k0 + j;
+            p[j] = k < m ? pos[k] : 0u;
+            d[j] = k < m ? dist[k] : 0u;
+            if (k < m) bytes += 2u + varint_bytes(p[j] - q - 1u) + varint_bytes(d[j]);
+            q = p[j];
+        }
+    }
+    u32 x = bytes;  // exclusive block scan of the threads' byte counts
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const u32 y = __shfl_up_sync(0xffffffffu, x, o);
+        if (lane >= o) x += y;
+    }
+    if (lane == 31) s_warp[warp] = x;
+    __syncthreads();
+    u32 before = 0, tile_bytes = 0;
+#pragma unroll
+    for (int w = 0; w < kPackThreads / 32; ++w) {
+        const u32 t = s_warp[w];
+        if (w < warp) before += t;
+        tile_bytes += t;
+    }
+    const u64 base = tile_off[blockIdx.x];
+    const u32 shift = (u32)(((uintptr_t)out + base) & 15u);
+    u32 o = shift + before + x - bytes;
+    DARK_ASSERT(o + bytes <= sizeof(s_buf));
+#pragma unroll
+    for (int j = 0; j < kPackItems; ++j) {
+        if (k0 + j >= m) break;
+        s_buf[o++] = sym[k0 + j];
+        s_buf[o++] = rank[k0 + j];
+        u32 v = p[j] - prev - 1u;
+        prev = p[j];
+        for (; v >= 0x80u; v >>= 7) s_buf[o++] = (u8)(v | 0x80u);
+        s_buf[o++] = (u8)v;
+        v = d[j];
+        for (; v >= 0x80u; v >>= 7) s_buf[o++] = (u8)(v | 0x80u);
+        s_buf[o++] = (u8)v;
+    }
+    __syncthreads();
+    u8* const dst = (u8*)((uintptr_t)out + base - shift);  // 16-byte aligned; only [shift, end) of it is written
+    const u32 end = shift + tile_bytes;
+    for (u32 w = (u32)tid; w * 16u < end; w += kPackThreads) {
+        const u32 lo = w * 16u, hi = lo + 16u;
+        if (lo >= shift && hi <= end) {
+            *(uint4*)(dst + lo) = *(const uint4*)(s_buf + lo);
+        } else {
+            for (u32 b = max(lo, shift); b < min(hi, end); ++b) dst[b] = s_buf[b];
+        }
+    }
+}
+
 }  // namespace dark

@@ -283,6 +283,55 @@ class Constructor:
                                                      ctypes.byref(info)), self._ctx, "dc::encode")
         return info
 
+    # -- the packed item stream (include/dark_bwt.h): sym, rank, varint(run length - 1), varint(dist) per item ----------
+    def bwt_dc_packed(self, input, want_bwt=False):
+        """block/dc.rs:45-52 with the items packed on the GPU (dark_bwt_forward_dc_packed): (bwt or None, origin,
+        stream np.uint8 of its exact length, DcInfo)."""
+        t = _as_u8(input)
+        n = t.size
+        out = np.empty(n, dtype=np.uint8) if want_bwt else None
+        stream = np.empty(_ffi.dc_packed_max(n), dtype=np.uint8)
+        info, origin, nbytes = _ffi.DcInfo(), ctypes.c_uint64(0), ctypes.c_uint64(0)
+        _ffi.check(self._L.dark_bwt_forward_dc_packed(self._ctx, t.ctypes.data, n, out.ctypes.data if want_bwt else None,
+                                                      ctypes.byref(origin), stream.ctypes.data, stream.size, ctypes.byref(nbytes),
+                                                      ctypes.byref(info), ctypes.byref(self.stats)), self._ctx, "bwt + dc::encode (packed)")
+        return out, int(origin.value), stream[:nbytes.value], info
+
+    def bwt_dc_packed_batch_into(self, text_ptrs, ns, stream_ptrs, capacities, bwt_ptrs=None, want_stats=False):
+        """Pipelined dark_bwt_forward_dc_packed over several blocks (dark_bwt_forward_dc_packed_batch; raw host addresses,
+        ideally pinned; needs a Constructor made with flags including _ffi.F_DC_BATCH).  Returns (origins, stream sizes,
+        DcInfo records) and the per-block stats if asked."""
+        cnt = len(ns)
+        assert len(text_ptrs) == cnt and len(stream_ptrs) == cnt and len(capacities) == cnt
+        m = max(cnt, 1)
+        arr = lambda ptrs: (ctypes.c_void_p * m)(*ptrs) if ptrs is not None else None  # noqa: E731
+        O, B = (ctypes.c_uint64 * m)(), (ctypes.c_uint64 * m)()
+        infos = (_ffi.DcInfo * m)()
+        S = (_ffi.Stats * m)() if want_stats else None
+        _ffi.check(self._L.dark_bwt_forward_dc_packed_batch(self._ctx, arr(text_ptrs), (ctypes.c_uint64 * m)(*[int(x) for x in ns]), cnt,
+                                                            arr(bwt_ptrs), O, arr(stream_ptrs), (ctypes.c_uint64 * m)(*[int(c) for c in capacities]),
+                                                            B, infos, S), self._ctx, "bwt + dc::encode (packed batch)")
+        res = ([int(O[i]) for i in range(cnt)], [int(B[i]) for i in range(cnt)], [infos[i] for i in range(cnt)])
+        return res + ([S[i].as_dict() for i in range(cnt)],) if want_stats else res
+
+    def bwt_dc_packed_blocks(self, texts, want_bwt=False):
+        """bwt_dc_packed for a run of host blocks through the pipelined batch entry: [(bwt or None, origin, stream, DcInfo), ...]."""
+        ts = [_as_u8(t) for t in texts]
+        ns = [t.size for t in ts]
+        bwts = [np.empty(n, dtype=np.uint8) for n in ns] if want_bwt else None
+        streams = [np.empty(_ffi.dc_packed_max(n), dtype=np.uint8) for n in ns]
+        origins, sizes, infos = self.bwt_dc_packed_batch_into([t.ctypes.data for t in ts], ns, [s.ctypes.data for s in streams],
+                                                              [s.size for s in streams], [b.ctypes.data for b in bwts] if want_bwt else None)
+        return [(bwts[k] if want_bwt else None, origins[k], streams[k][:sizes[k]], infos[k]) for k in range(len(ts))]
+
+    def dc_encode_packed_device(self, d_bwt, n, d_stream, capacity):
+        """Device pointers: distance coding of d_bwt[0..n) with its items packed into d_stream (capacity bytes).  Returns
+        (stream bytes, DcInfo)."""
+        info, nbytes = _ffi.DcInfo(), ctypes.c_uint64(0)
+        _ffi.check(self._L.dark_bwt_dc_encode_packed_device(self._ctx, d_bwt, int(n), d_stream, int(capacity), ctypes.byref(nbytes),
+                                                            ctypes.byref(info)), self._ctx, "dc::encode (packed)")
+        return int(nbytes.value), info
+
     # -- distance coding of many small blocks in one device pass -----------------------------------------------------
     def _dc_many_results(self, infos, ns, dist, item_starts, pos, idist, sym, rank):
         """Per-block dicts shaped like _dc_result, cut out of the concatenated outputs."""

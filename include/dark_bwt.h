@@ -237,6 +237,44 @@ int dark_bwt_forward_dc_batch(dark_bwt_ctx *ctx, const uint8_t *const *texts, co
                               uint32_t *const *item_pos, uint32_t *const *item_dist, uint8_t *const *item_sym,
                               uint8_t *const *item_rank, dark_bwt_dc_info *infos, dark_bwt_stats *stats);
 
+/* ---- the packed item stream: the items of one block as one byte string ---------------------------------------------
+ * The four item arrays cost 10 bytes per run on the way out; most of those bytes are zero.  The packed entries below code
+ * a block's info->num_items items, k = 0, 1, ..., as one byte string, per item in this order:
+ *     item_sym[k]                                    1 byte
+ *     item_rank[k]                                   1 byte
+ *     varint(item_pos[k] - item_pos[k-1] - 1)        run length - 1, with item_pos[-1] = -1
+ *     varint(item_dist[k])
+ * varint = unsigned LEB128: 7 bits per byte, the low group first, bit 7 set on every byte but the last (a u32 takes at
+ * most 5 bytes).  A consumer keeps a running run end, pos = -1 before the first item and pos += 1 + the first varint at
+ * each item; that is item_pos[k], and Context.distance_limit = n - pos.  init[], the MTF list, num_unique and num_items stay in dark_bwt_dc_info.  About 4 bytes per run on DNA and
+ * text blocks instead of 10.
+ * Size: the run lengths add up to n, and varint(len - 1) <= len bytes, so a block of n bytes packs into at most
+ * 2 + 5 bytes per item plus n, at most DARK_BWT_DC_PACKED_MAX(n) bytes: a buffer of that size never fails the capacity
+ * check.  Capacity: the stream's size is always written to *stream_bytes_out (stream_bytes_out[k]); a size above the
+ * buffer's capacity is DARK_BWT_E_INVALID_ARG, nothing is written to the stream buffer, dark_bwt_last_error() names the
+ * bytes needed (and, in the batch, the block), and the context stays usable.  info->device_ms includes the pack kernels. */
+#define DARK_BWT_DC_PACKED_MAX(n) (8ull * (uint64_t)(n))
+/* Device buffers: distance coding of d_bwt[0..n), its items packed into d_stream_out (stream_capacity bytes).  The item
+ * arrays stay in the context's arena.  1 <= n <= capacity.  Returns after the work has completed on the stream. */
+int dark_bwt_dc_encode_packed_device(dark_bwt_ctx *ctx, const uint8_t *d_bwt, uint64_t n, uint8_t *d_stream_out,
+                                     uint64_t stream_capacity, uint64_t *stream_bytes_out, dark_bwt_dc_info *info);
+/* dark_bwt_forward_dc with the packed stream as the only DC output: only the stream (and the BWT, if bwt_out is non-null)
+ * crosses PCIe.  Host buffers, pageable or pinned; 2 <= n <= capacity; stats nullable. */
+int dark_bwt_forward_dc_packed(dark_bwt_ctx *ctx, const uint8_t *text, uint64_t n, uint8_t *bwt_out /* nullable */,
+                               uint64_t *origin_out, uint8_t *stream_out, uint64_t stream_capacity,
+                               uint64_t *stream_bytes_out, dark_bwt_dc_info *info, dark_bwt_stats *stats /* nullable */);
+/* `count` host blocks through dark_bwt_forward_dc_packed, pipelined like dark_bwt_forward_dc_batch (a context created with
+ * DARK_BWT_F_DC_BATCH; block k's stream is packed into its DC output slot).  Block k gets exactly what
+ * dark_bwt_forward_dc_packed(texts[k], ...) gives.  Required: texts, ns, origins_out, stream_outs (every entry),
+ * stream_capacities, stream_bytes_out, infos (`count` records each).  Nullable: bwt_outs and its entries, stats.
+ * DARK_BWT_E_INVALID_ARG, before any device work, for a context without DARK_BWT_F_DC_BATCH or a null required pointer;
+ * DARK_BWT_E_INVALID_N for any ns[k] outside [2, capacity].  count == 0 is DARK_BWT_OK.  A block whose stream does not fit
+ * its buffer ends the call: every block before it is complete, stream_bytes_out[k] holds the size it needs. */
+int dark_bwt_forward_dc_packed_batch(dark_bwt_ctx *ctx, const uint8_t *const *texts, const uint64_t *ns, uint64_t count,
+                                     uint8_t *const *bwt_outs /* nullable, entries too */, uint64_t *origins_out,
+                                     uint8_t *const *stream_outs, const uint64_t *stream_capacities,
+                                     uint64_t *stream_bytes_out, dark_bwt_dc_info *infos, dark_bwt_stats *stats /* nullable */);
+
 /* MANY SMALL blocks distance-coded in ONE pass.  Block k gives exactly what dark_bwt_dc_encode gives on that block alone:
  * every value is block-relative (filler and last-run distances use n_k, init[c] is the first occurrence inside the block
  * or n_k, item_pos is the run end inside the block, runs never merge across a boundary).  Outputs:

@@ -7,6 +7,8 @@ pub const DARK_BWT_OK: c_int = 0;
 pub const DARK_BWT_MAX_ROUNDS: usize = 40;
 /// dark_bwt_create_ex flag: the two DC output slots dark_bwt_forward_dc_batch needs (73 N bytes of HBM in all).
 pub const DARK_BWT_F_DC_BATCH: u32 = 4;
+/// DARK_BWT_DC_PACKED_MAX(n): a stream buffer of this many bytes never fails the capacity check.
+pub const fn dark_bwt_dc_packed_max(n: u64) -> u64 { 8 * n }
 
 #[repr(C)]
 pub struct dark_bwt_ctx { _private: [u8; 0] }
@@ -76,6 +78,16 @@ extern "C" {
                                      bwt_outs: *const *mut u8, origins_out: *mut u64, dist_outs: *const *mut u32,
                                      item_pos: *const *mut u32, item_dist: *const *mut u32, item_sym: *const *mut u8,
                                      item_rank: *const *mut u8, infos: *mut dark_bwt_dc_info, stats: *mut dark_bwt_stats) -> c_int;
+    // the packed item stream: per item sym, rank, LEB128(run length - 1), LEB128(dist); at most DARK_BWT_DC_PACKED_MAX(n) bytes
+    pub fn dark_bwt_dc_encode_packed_device(ctx: *mut dark_bwt_ctx, d_bwt: *const u8, n: u64, d_stream_out: *mut u8,
+                                            stream_capacity: u64, stream_bytes_out: *mut u64, info: *mut dark_bwt_dc_info) -> c_int;
+    pub fn dark_bwt_forward_dc_packed(ctx: *mut dark_bwt_ctx, text: *const u8, n: u64, bwt_out: *mut u8, origin_out: *mut u64,
+                                      stream_out: *mut u8, stream_capacity: u64, stream_bytes_out: *mut u64,
+                                      info: *mut dark_bwt_dc_info, stats: *mut dark_bwt_stats) -> c_int;
+    pub fn dark_bwt_forward_dc_packed_batch(ctx: *mut dark_bwt_ctx, texts: *const *const u8, ns: *const u64, count: u64,
+                                            bwt_outs: *const *mut u8, origins_out: *mut u64, stream_outs: *const *mut u8,
+                                            stream_capacities: *const u64, stream_bytes_out: *mut u64,
+                                            infos: *mut dark_bwt_dc_info, stats: *mut dark_bwt_stats) -> c_int;
     pub fn dark_bwt_create(max_n: u64, device: c_int, out: *mut *mut dark_bwt_ctx) -> c_int;
     pub fn dark_bwt_create_ex(max_n: u64, device: c_int, flags: u32, out: *mut *mut dark_bwt_ctx) -> c_int;
     pub fn dark_bwt_arena_bytes(max_n: u64, flags: u32) -> u64;
