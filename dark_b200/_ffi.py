@@ -21,6 +21,7 @@ SYMBOLS = [
     "dark_bwt_synth", "dark_bwt_dc_encode_device", "dark_bwt_dc_encode", "dark_bwt_forward_dc", "dark_bwt_dc_encode_many",
     "dark_bwt_dc_encode_many_device", "dark_bwt_forward_dc_many", "dark_bwt_forward_dc_batch",
     "dark_bwt_dc_encode_packed_device", "dark_bwt_forward_dc_packed", "dark_bwt_forward_dc_packed_batch",
+    "dark_bwt_dc_encode_packed_many_device", "dark_bwt_forward_dc_packed_many",
 ]
 
 
@@ -132,6 +133,9 @@ def lib():
     L.dark_bwt_forward_dc_packed.argtypes = [vp, vp, u64, vp, ctypes.POINTER(u64), vp, u64, ctypes.POINTER(u64),
                                              ctypes.POINTER(DcInfo), ctypes.POINTER(Stats)]
     L.dark_bwt_forward_dc_packed_batch.argtypes = [vp, vp, vp, u64, vp, vp, vp, vp, vp, vp, vp]
+    L.dark_bwt_dc_encode_packed_many_device.argtypes = [vp, vp, vp, u64, vp, u64, vp, ctypes.POINTER(u64), vp,
+                                                        ctypes.POINTER(ctypes.c_float)]
+    L.dark_bwt_forward_dc_packed_many.argtypes = [vp, vp, vp, u64, vp, vp, vp, u64, vp, ctypes.POINTER(u64), vp, ctypes.POINTER(Stats)]
     _lib = L
     return L
 

@@ -14,7 +14,10 @@
 // holds, PairsMode owns pairs mode, SortStatus owns which rows of the radix passes' status buffer may hold stale words.
 //
 // All device memory is carved from one arena allocated at create (Constructor::new allocates its
-// arena up front too, saca.rs:351-360) by carve_arena; the forward calls allocate nothing.
+// arena up front too, saca.rs:351-360) by carve_arena; the forward calls allocate nothing.  The packed item stream
+// (dc_pack) reuses what distance coding has finished with: the host entries' stream lives in keys[1]; the tile counts in
+// ranks_alt, or for many blocks (whose item offsets are in ranks_alt) in ranks behind the per-block stream offsets of
+// dark_bwt_forward_dc_packed_many and the tile offsets; the first-item bitmap of many blocks in `bitmap`.
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -1475,12 +1478,28 @@ int dc_device(dark_bwt_ctx* ctx, const u8* d_bwt, u32 n, const BlockList* blocks
 // the capacity is DARK_BWT_E_INVALID_ARG before anything is written.  The tile sums and offsets go to ranks_alt and ranks
 // (at most 12 bytes per 2,048 items), which dc_device has finished with.  Returns after the stream is complete; adds the
 // pack's device time to *ms.
-int dc_pack(dark_bwt_ctx* ctx, const DcBuffers& io, u64 items, u8* d_out, u64 capacity, uint64_t* bytes_out, float* ms) {
+// Many blocks (d_stream_starts non-null): the items of the `count` blocks of a many-block pass, at io.item_starts.  Each
+// block's stream is what the block alone packs to, the streams back to back; d_stream_starts[0..count] (device) gets their
+// offsets, [count] = the total, only when the stream fits.  The first-item bitmap goes to ctx->bitmap, which the pass has
+// finished with.  ranks_alt holds the item starts, so the tile sums go to ranks instead: ranks holds count + 1 words of 8
+// bytes first (where dark_bwt_forward_dc_packed_many keeps the offsets), then the tile offsets, then the tile sums.
+int dc_pack(dark_bwt_ctx* ctx, const DcBuffers& io, u64 items, u8* d_out, u64 capacity, uint64_t* bytes_out, float* ms,
+            u32 count = 0, u64* d_stream_starts = nullptr) {
     const u32 ntiles = (u32)ceil_div(items, kPackTile);
-    u32* tile_bytes = ctx->ranks_alt;
-    u64* tile_off = (u64*)ctx->ranks;
+    const bool many = d_stream_starts != nullptr;
+    u64* tile_off = (u64*)ctx->ranks + (many ? count + 1 : 0);
+    u32* tile_bytes = many ? (u32*)(tile_off + ntiles) : ctx->ranks_alt;
+    PackMany pm{};  // zero in the single-block instantiations
     CK(cudaEventRecord(ctx->call_start, ctx->stream));
-    k_dc_pack_sizes<<<ntiles, kPackThreads, 0, ctx->stream>>>(io.item_pos, io.item_dist, items, tile_bytes);
+    if (many) {
+        pm = PackMany{ctx->bitmap, io.item_starts, count, d_stream_starts};
+        CK(cudaMemsetAsync(ctx->bitmap, 0, sizeof(u32) * ceil_div(items, 32), ctx->stream));
+        k_dc_mark_items<<<(u32)ceil_div(count, 256), 256, 0, ctx->stream>>>(io.item_starts, count, ctx->bitmap);
+        LAUNCHED();
+        k_dc_pack_sizes<true><<<ntiles, kPackThreads, 0, ctx->stream>>>(io.item_pos, io.item_dist, items, tile_bytes, pm);
+    } else {
+        k_dc_pack_sizes<false><<<ntiles, kPackThreads, 0, ctx->stream>>>(io.item_pos, io.item_dist, items, tile_bytes, pm);
+    }
     LAUNCHED();
     k_dc_pack_scan<<<1, 1024, 0, ctx->stream>>>(tile_bytes, ntiles, tile_off, &ctx->mail_dev->packed_bytes);
     LAUNCHED();
@@ -1491,11 +1510,31 @@ int dc_pack(dark_bwt_ctx* ctx, const DcBuffers& io, u64 items, u8* d_out, u64 ca
                  (unsigned long long)*bytes_out, (unsigned long long)capacity);
         return DARK_BWT_E_INVALID_ARG;
     }
-    k_dc_pack_write<<<ntiles, kPackThreads, 0, ctx->stream>>>(io.item_pos, io.item_dist, io.item_sym, io.item_rank, items, tile_off, d_out);
+    if (many) {
+        static_assert(sizeof(ctx->mail->packed_bytes) == sizeof(u64), "the total is copied as it is");
+        CK(cudaMemcpyAsync(d_stream_starts + count, &ctx->mail->packed_bytes, sizeof(u64), cudaMemcpyHostToDevice, ctx->stream));
+        k_dc_pack_write<true><<<ntiles, kPackThreads, 0, ctx->stream>>>(io.item_pos, io.item_dist, io.item_sym, io.item_rank, items,
+                                                                        tile_off, d_out, pm);
+    } else {
+        k_dc_pack_write<false><<<ntiles, kPackThreads, 0, ctx->stream>>>(io.item_pos, io.item_dist, io.item_sym, io.item_rank, items,
+                                                                         tile_off, d_out, pm);
+    }
     LAUNCHED();
     CK(cudaEventRecord(ctx->call_stop, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     *ms += call_ms(ctx);
+    return DARK_BWT_OK;
+}
+
+// dc_pack of the `count` blocks dc_device coded in one pass (item offsets `starts`, read back): every infos[k].device_ms, and
+// *ms_out (nullable), becomes the time of the pass and the pack.
+int dc_pack_many(dark_bwt_ctx* ctx, const DcBuffers& io, const std::vector<u32>& starts, u8* d_out, u64 capacity,
+                 u64* d_stream_starts, uint64_t* bytes_out, dark_bwt_dc_info* infos, float* ms_out) {
+    const u32 count = (u32)starts.size() - 1;
+    float ms = infos[0].device_ms;
+    if (int rc = dc_pack(ctx, io, starts.back(), d_out, capacity, bytes_out, &ms, count, d_stream_starts)) return rc;
+    for (u32 k = 0; k < count; ++k) infos[k].device_ms = ms;
+    if (ms_out) *ms_out = ms;
     return DARK_BWT_OK;
 }
 
@@ -1624,11 +1663,10 @@ struct CopyList {
         void* dev;
         size_t bytes;
     };
-    Copy list[6];  // the most any entry copies: BWT, distances and the four item arrays
-    int count = 0;
+    std::vector<Copy> list;  // dark_bwt_forward_dc_packed_many: a BWT per block besides the stream and its offsets
     bool serial = false;
     void add(const void* host, const void* dev, size_t bytes) {
-        if (host && bytes) list[count++] = Copy{(void*)host, (void*)dev, bytes};
+        if (host && bytes) list.push_back(Copy{(void*)host, (void*)dev, bytes});
     }
 };
 
@@ -1637,8 +1675,7 @@ struct CopyList {
 int copy_blocking(dark_bwt_ctx* ctx, const CopyList& copies, cudaMemcpyKind kind, cudaStream_t stream) {
     const bool to_device = kind == cudaMemcpyHostToDevice;
     bool direct = false;
-    for (int i = 0; i < copies.count; ++i) {
-        const CopyList::Copy& c = copies.list[i];
+    for (const CopyList::Copy& c : copies.list) {
         HostStage* st;
         if (int rc = stage_for(ctx, c.host, c.bytes, kind, &st)) return rc;
         if (st) {
@@ -1718,7 +1755,7 @@ int run_pipelined(dark_bwt_ctx* ctx, const u8* const* ins, const uint64_t* ns, u
         if (fout.valid())
             if (int rc2 = fout.get()) { drain(); return rc2; }  // one staged copy-out at a time (they share the lanes)
         HostStage* staged = nullptr;  // one staged copy sends the whole list to the helper thread
-        for (int i = 0; i < oc.count && !staged; ++i)
+        for (size_t i = 0; i < oc.list.size() && !staged; ++i)
             if (int rc2 = stage_for(ctx, oc.list[i].host, oc.list[i].bytes, cudaMemcpyDeviceToHost, &staged)) { drain(); return rc2; }
         if (staged) {
             fout = std::async(std::launch::async, [ctx, oc] {
@@ -1730,8 +1767,8 @@ int run_pipelined(dark_bwt_ctx* ctx, const u8* const* ins, const uint64_t* ns, u
             out_recorded[b] = false;
         } else {
             CK(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_comp[b], 0));
-            for (int i = 0; i < oc.count; ++i)
-                CK(cudaMemcpyAsync(oc.list[i].host, oc.list[i].dev, oc.list[i].bytes, cudaMemcpyDeviceToHost, ctx->copy_out));
+            for (const CopyList::Copy& c : oc.list)
+                CK(cudaMemcpyAsync(c.host, c.dev, c.bytes, cudaMemcpyDeviceToHost, ctx->copy_out));
             if (oc.serial) CK(cudaStreamSynchronize(ctx->copy_out));
             CK(cudaEventRecord(ctx->ev_out[b], ctx->copy_out));
             out_recorded[b] = true;
@@ -2309,6 +2346,60 @@ int dark_bwt_forward_dc_many(dark_bwt_ctx* ctx, const uint8_t* const* texts, con
     CopyList out;
     add_dc_outputs(&out, io, bl.total(), starts.back(), dist_out, item_pos, item_dist, item_sym, item_rank);
     return copy_blocking(ctx, out, cudaMemcpyDeviceToHost, ctx->stream);
+}
+
+int dark_bwt_dc_encode_packed_many_device(dark_bwt_ctx* ctx, const uint8_t* d_bwt, const uint32_t* d_starts, uint64_t count,
+                                          uint8_t* d_stream_out, uint64_t stream_capacity, uint64_t* d_stream_starts,
+                                          uint64_t* stream_bytes_out, dark_bwt_dc_info* infos, float* ms_out) {
+    if (!ctx || !d_bwt || !d_starts || !d_stream_out || !d_stream_starts || !stream_bytes_out || !infos) return DARK_BWT_E_INVALID_ARG;
+    ctx->err[0] = 0;
+    if (count == 0) {
+        *stream_bytes_out = 0;
+        return DARK_BWT_OK;
+    }
+    BlockList bl;
+    if (int rc = check_blocks(ctx, count, nullptr, d_starts, nullptr, 1, 0, nullptr, nullptr, &bl)) return rc;
+    if (!dc_many_records_fit(ctx, count)) return DARK_BWT_E_INVALID_N;
+    if (int rc = load_blocks(ctx, bl)) return rc;
+    DcBuffers io;
+    std::vector<u32> starts;
+    if (int rc = dc_device(ctx, d_bwt, bl.total(), &bl, &io, infos, &starts)) return rc;
+    return dc_pack_many(ctx, io, starts, d_stream_out, stream_capacity, d_stream_starts, stream_bytes_out, infos, ms_out);
+}
+
+int dark_bwt_forward_dc_packed_many(dark_bwt_ctx* ctx, const uint8_t* const* texts, const uint64_t* ns, uint64_t count,
+                                    uint8_t* const* bwt_outs, uint64_t* origins_out, uint8_t* stream_out, uint64_t stream_capacity,
+                                    uint64_t* stream_starts, uint64_t* stream_bytes_out, dark_bwt_dc_info* infos, dark_bwt_stats* stats) {
+    if (!ctx || !texts || !ns || !origins_out || !stream_out || !stream_starts || !stream_bytes_out || !infos) return DARK_BWT_E_INVALID_ARG;
+    if (int rc = check_staging(ctx)) return rc;
+    ctx->err[0] = 0;
+    if (count == 0) {
+        *stream_bytes_out = 0;
+        stream_starts[0] = 0;
+        return DARK_BWT_OK;
+    }
+    BlockList bl;
+    if (int rc = check_blocks(ctx, count, ns, nullptr, nullptr, 2, 0, texts, nullptr, &bl)) return rc;
+    if (!dc_many_records_fit(ctx, count)) return DARK_BWT_E_INVALID_N;
+    // the BWTs stay in HBM for distance coding and are copied out with the stream
+    if (int rc = forward_many_host(ctx, texts, nullptr, origins_out, bl, stats)) return rc;
+    DcBuffers io;
+    std::vector<u32> starts;
+    if (int rc = dc_device(ctx, ctx->d_bwt, bl.total(), &bl, &io, infos, &starts)) return rc;
+    // dc_device has read the per-block records back out of the sort's second key buffer (8 N + 1 KiB): it holds any stream
+    // (<= 8 sum(ns)).  The offsets go to the head of ranks, in front of the pack's tile scratch (dc_pack).
+    u8* const d_stream = (u8*)ctx->keys[1];
+    u64* const d_offsets = (u64*)ctx->ranks;
+    if (int rc = dc_pack_many(ctx, io, starts, d_stream, stream_capacity, d_offsets, stream_bytes_out, infos, nullptr)) return rc;
+    CopyList out;
+    out.add(stream_out, d_stream, *stream_bytes_out);
+    out.add(stream_starts, d_offsets, sizeof(u64) * (count + 1));
+    if (bwt_outs)
+        for (u32 k = 0; k < bl.count(); ++k) out.add(bwt_outs[k], ctx->d_bwt + bl.starts[k], bl.starts[k + 1] - bl.starts[k]);
+    const auto t0 = std::chrono::steady_clock::now();
+    if (int rc = copy_blocking(ctx, out, cudaMemcpyDeviceToHost, ctx->stream)) return rc;
+    if (stats) stats->d2h_ms += std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    return DARK_BWT_OK;
 }
 
 int dark_bwt_reuse(dark_bwt_ctx* ctx, uint32_t** words_out, uint64_t* count_out) {

@@ -437,6 +437,10 @@ k_dc_stream(const u32* __restrict__ run_start, const unsigned long long* __restr
 //   k_dc_pack_scan    one CTA: the tile counts -> u64 tile offsets and the total (a stream can pass 2^32 bytes)
 //   k_dc_pack_write   each tile again: sizes, block scan, the tile's bytes built in shared memory, then stored as one
 //                     contiguous span with 16-byte stores (bytes one by one only in the span's first and last 16-byte word)
+// MANY = true: the items of a many-block pass, back to back in block order (item_pos block-relative).  Each block's stream
+// is what the block alone packs to: at an item that opens a block (a bit of k_dc_mark_items' bitmap) the previous run end
+// is -1 again, so the streams of the blocks are simply concatenated, and the thread that codes a block's first item writes
+// where it lands to stream_starts[block].  k_dc_pack_scan serves both forms.
 constexpr int kPackThreads = 256;
 constexpr int kPackItems = 8;  // consecutive items per thread
 constexpr int kPackTile = kPackThreads * kPackItems;
@@ -446,9 +450,27 @@ __device__ __forceinline__ u32 varint_bytes(u32 v) {
     return 1u + (v >= (1u << 7)) + (v >= (1u << 14)) + (v >= (1u << 21)) + (v >= (1u << 28));
 }
 
+// What the many-block instantiations of the pack read and write besides the single-block arguments (zero in the others).
+struct PackMany {
+    const u32* first_bits;   // bit k set: item k is the first item of a block
+    const u32* item_starts;  // [0..count]: index of each block's first item (k_dc_ranks), [count] = all items
+    u32 count;
+    u64* stream_starts;      // [0..count): offset of each block's first byte in the stream
+};
+
+// The first-item bitmap of the pack (bits zeroed before): blocks hold at least one run, so item_starts[b] are distinct.
+__global__ void __launch_bounds__(256) k_dc_mark_items(const u32* __restrict__ item_starts, u32 count, u32* __restrict__ bits) {
+    const u32 b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b < count) atomicOr(&bits[item_starts[b] >> 5], 1u << (item_starts[b] & 31));
+}
+
+__device__ __forceinline__ bool first_item(const PackMany& many, u64 k) { return (many.first_bits[k >> 5] >> (k & 31)) & 1u; }
+
 // run length - 1 of item k is pos[k] - pos[k-1] - 1 with pos[-1] = -1: in u32 arithmetic, prev = 0xFFFFFFFF for k = 0
+// (MANY: and for the first item of every block)
+template <bool MANY>
 __global__ void __launch_bounds__(kPackThreads)
-k_dc_pack_sizes(const u32* __restrict__ pos, const u32* __restrict__ dist, u64 m, u32* __restrict__ tile_bytes) {
+k_dc_pack_sizes(const u32* __restrict__ pos, const u32* __restrict__ dist, u64 m, u32* __restrict__ tile_bytes, PackMany many) {
     __shared__ u32 s_warp[kPackThreads / 32];
     const u64 k0 = (u64)blockIdx.x * kPackTile + threadIdx.x;
     u32 bytes = 0;
@@ -456,7 +478,9 @@ k_dc_pack_sizes(const u32* __restrict__ pos, const u32* __restrict__ dist, u64 m
     for (int j = 0; j < kPackItems; ++j) {
         const u64 k = k0 + (u64)j * kPackThreads;
         if (k < m) {
-            const u32 prev = k ? pos[k - 1] : 0xFFFFFFFFu;
+            u32 prev = k ? pos[k - 1] : 0xFFFFFFFFu;
+            if constexpr (MANY)
+                if (first_item(many, k)) prev = 0xFFFFFFFFu;
             bytes += 2u + varint_bytes(pos[k] - prev - 1u) + varint_bytes(dist[k]);
         }
     }
@@ -519,15 +543,20 @@ k_dc_pack_scan(const u32* __restrict__ tile_bytes, u32 ntiles, u64* __restrict__
 
 // Thread t of a tile codes its items tile0 + 8t .. 8t+7 into s_buf at shift + (bytes of the tile's items before them),
 // shift = the address of the tile's first byte mod 16, so that s_buf's 16-byte words line up with out's.
+// MANY: a thread's 8 items (k0 is a multiple of 8) have their first-item bits in one bitmap word.
+template <bool MANY>
 __global__ void __launch_bounds__(kPackThreads)
 k_dc_pack_write(const u32* __restrict__ pos, const u32* __restrict__ dist, const u8* __restrict__ sym, const u8* __restrict__ rank,
-                u64 m, const u64* __restrict__ tile_off, u8* __restrict__ out) {
+                u64 m, const u64* __restrict__ tile_off, u8* __restrict__ out, PackMany many) {
     __shared__ __align__(16) u8 s_buf[kPackTile * kPackMaxItemBytes + 16];
     __shared__ u32 s_warp[kPackThreads / 32];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const u64 k0 = (u64)blockIdx.x * kPackTile + (u64)tid * kPackItems;
     u32 p[kPackItems], d[kPackItems];
     u32 prev = k0 > 0 && k0 < m ? pos[k0 - 1] : 0xFFFFFFFFu;
+    u32 firsts = 0;  // MANY: bit j set: item k0 + j is the first item of a block
+    if constexpr (MANY)
+        if (k0 < m) firsts = (many.first_bits[k0 >> 5] >> (k0 & 31)) & 0xFFu;
     u32 bytes = 0;
     {
         u32 q = prev;
@@ -536,6 +565,8 @@ k_dc_pack_write(const u32* __restrict__ pos, const u32* __restrict__ dist, const
             const u64 k = k0 + j;
             p[j] = k < m ? pos[k] : 0u;
             d[j] = k < m ? dist[k] : 0u;
+            if constexpr (MANY)
+                if ((firsts >> j) & 1u) q = 0xFFFFFFFFu;
             if (k < m) bytes += 2u + varint_bytes(p[j] - q - 1u) + varint_bytes(d[j]);
             q = p[j];
         }
@@ -562,6 +593,12 @@ k_dc_pack_write(const u32* __restrict__ pos, const u32* __restrict__ dist, const
 #pragma unroll
     for (int j = 0; j < kPackItems; ++j) {
         if (k0 + j >= m) break;
+        if constexpr (MANY) {
+            if ((firsts >> j) & 1u) {
+                prev = 0xFFFFFFFFu;
+                many.stream_starts[dc_block_of(many.item_starts, many.count, (u32)(k0 + j))] = base + (o - shift);
+            }
+        }
         s_buf[o++] = sym[k0 + j];
         s_buf[o++] = rank[k0 + j];
         u32 v = p[j] - prev - 1u;

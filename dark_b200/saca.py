@@ -393,6 +393,36 @@ class Constructor:
                    self._ctx, "dc::encode (many)")
         return [infos[k] for k in range(int(count))], float(ms.value)
 
+    # -- many small blocks with the packed item stream: the blocks' streams back to back, u64 offsets ------------------
+    def bwt_dc_packed_many(self, texts, want_bwt=False):
+        """bwt_dc_packed for many small blocks in one sort and one DC pass (dark_bwt_forward_dc_packed_many):
+        [(bwt or None, origin, stream, DcInfo), ...] like bwt_dc_packed_blocks; the streams are slices of one buffer."""
+        ts = [_as_u8(t) for t in texts]
+        cnt, ns = len(ts), [t.size for t in ts]
+        m = max(cnt, 1)
+        outs = [np.empty(n, dtype=np.uint8) for n in ns] if want_bwt else None
+        stream = np.empty(_ffi.dc_packed_max(sum(ns)), dtype=np.uint8)
+        starts = np.empty(cnt + 1, dtype=np.uint64)
+        infos, origins, nbytes = (_ffi.DcInfo * m)(), (ctypes.c_uint64 * m)(), ctypes.c_uint64(0)
+        bwt_ptrs = (ctypes.c_void_p * m)(*[o.ctypes.data for o in outs]) if want_bwt else None
+        _ffi.check(self._L.dark_bwt_forward_dc_packed_many(self._ctx, (ctypes.c_void_p * m)(*[t.ctypes.data for t in ts]),
+                                                           (ctypes.c_uint64 * m)(*ns), cnt, bwt_ptrs, origins, stream.ctypes.data,
+                                                           stream.size, starts.ctypes.data, ctypes.byref(nbytes), infos,
+                                                           ctypes.byref(self.stats)), self._ctx, "bwt + dc::encode (packed many)")
+        assert int(starts[cnt]) == nbytes.value
+        return [(outs[k] if want_bwt else None, int(origins[k]), stream[int(starts[k]):int(starts[k + 1])], infos[k])
+                for k in range(cnt)]
+
+    def dc_encode_packed_many_device(self, d_bwt, d_starts, count, d_stream, capacity, d_stream_starts):
+        """Device pointers, the layout dc_encode_many_device reads: the blocks' packed item streams back to back into d_stream
+        (capacity bytes), their offsets into d_stream_starts (count + 1 u64).  Returns (total bytes, list of DcInfo, device ms)."""
+        infos = (_ffi.DcInfo * max(int(count), 1))()
+        nbytes, ms = ctypes.c_uint64(0), ctypes.c_float(0)
+        _ffi.check(self._L.dark_bwt_dc_encode_packed_many_device(self._ctx, d_bwt, d_starts, int(count), d_stream, int(capacity),
+                                                                 d_stream_starts, ctypes.byref(nbytes), infos, ctypes.byref(ms)),
+                   self._ctx, "dc::encode (packed many)")
+        return int(nbytes.value), [infos[k] for k in range(int(count))], float(ms.value)
+
     # -- device-resident form (benches, pipelines that keep the block in HBM) ------------------
     def bwt_device(self, d_text, n, d_bwt, d_sa=None):
         """Raw device pointers (ints).  Returns origin; self.stats holds the device timings."""

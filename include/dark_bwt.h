@@ -303,6 +303,31 @@ int dark_bwt_forward_dc_many(dark_bwt_ctx *ctx, const uint8_t *const *texts, con
                              uint32_t *item_pos, uint32_t *item_dist, uint8_t *item_sym, uint8_t *item_rank,
                              dark_bwt_dc_info *infos, dark_bwt_stats *stats);
 
+/* MANY SMALL blocks with the packed item stream: the pass above, each block's items packed as the packed entries pack them.
+ * Block k's bytes are exactly what dark_bwt_dc_encode_packed_device / dark_bwt_forward_dc_packed give for that block alone;
+ * the blocks' streams lie back to back in block order, and count + 1 u64 offsets locate them: block k is
+ * stream[stream_starts[k] .. stream_starts[k+1]), stream_starts[0] = 0, stream_starts[count] = *stream_bytes_out = the
+ * total, at most DARK_BWT_DC_PACKED_MAX(sum(ns)).  Limits and errors are those of the entries above (count <=
+ * DARK_BWT_MAX_MANY_BLOCKS, sum(ns) <= capacity, the record bound count * 1288 <= 8 * capacity + 1024).  The capacity rule
+ * is the packed entries': the total is always written to *stream_bytes_out; a total above stream_capacity is
+ * DARK_BWT_E_INVALID_ARG, neither the stream nor the offsets are written, dark_bwt_last_error() names the bytes needed, and
+ * the context stays usable.  infos[k].device_ms (and *ms_out) = the time of the pass and the pack.  count == 0 is
+ * DARK_BWT_OK with *stream_bytes_out = 0 (and, in the host form, stream_starts[0] = 0). */
+/* Device buffers, the layout of dark_bwt_dc_encode_many_device: the blocks (each >= 1 byte) back to back in d_bwt at the u32
+ * offsets d_starts[0..count]; the stream goes to d_stream_out (stream_capacity bytes), the offsets to d_stream_starts
+ * (count + 1 u64, on the device).  infos (count records), stream_bytes_out and ms_out (nullable) are host pointers.  The
+ * item arrays stay in the context's arena.  Returns after the work has completed on the stream. */
+int dark_bwt_dc_encode_packed_many_device(dark_bwt_ctx *ctx, const uint8_t *d_bwt, const uint32_t *d_starts, uint64_t count,
+                                          uint8_t *d_stream_out, uint64_t stream_capacity, uint64_t *d_stream_starts,
+                                          uint64_t *stream_bytes_out, dark_bwt_dc_info *infos, float *ms_out);
+/* Host buffers: dark_bwt_forward_many of texts[0..count) (each >= 2 bytes), then the pass above while the BWTs are in HBM;
+ * only the stream, its offsets (stream_starts: a host array of count + 1) and the BWTs, if asked for, cross PCIe.  Pageable
+ * or pinned; bwt_outs (and its entries) and stats nullable.  DARK_BWT_E_INVALID_ARG with a device-only context. */
+int dark_bwt_forward_dc_packed_many(dark_bwt_ctx *ctx, const uint8_t *const *texts, const uint64_t *ns, uint64_t count,
+                                    uint8_t *const *bwt_outs /* nullable, entries too */, uint64_t *origins_out,
+                                    uint8_t *stream_out, uint64_t stream_capacity, uint64_t *stream_starts,
+                                    uint64_t *stream_bytes_out, dark_bwt_dc_info *infos, dark_bwt_stats *stats /* nullable */);
+
 /* Constructor::reuse — lends >= capacity host u32 words of scratch (DC distances in
  * block/dc.rs:51).  Allocated on first use; owned by the context. */
 int dark_bwt_reuse(dark_bwt_ctx *ctx, uint32_t **words_out, uint64_t *count_out);

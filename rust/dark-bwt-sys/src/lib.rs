@@ -88,6 +88,14 @@ extern "C" {
                                             bwt_outs: *const *mut u8, origins_out: *mut u64, stream_outs: *const *mut u8,
                                             stream_capacities: *const u64, stream_bytes_out: *mut u64,
                                             infos: *mut dark_bwt_dc_info, stats: *mut dark_bwt_stats) -> c_int;
+    // many small blocks: one stream, block k at [stream_starts[k], stream_starts[k + 1]); at most DARK_BWT_DC_PACKED_MAX(sum(ns))
+    pub fn dark_bwt_dc_encode_packed_many_device(ctx: *mut dark_bwt_ctx, d_bwt: *const u8, d_starts: *const u32, count: u64,
+                                                 d_stream_out: *mut u8, stream_capacity: u64, d_stream_starts: *mut u64,
+                                                 stream_bytes_out: *mut u64, infos: *mut dark_bwt_dc_info, ms_out: *mut f32) -> c_int;
+    pub fn dark_bwt_forward_dc_packed_many(ctx: *mut dark_bwt_ctx, texts: *const *const u8, ns: *const u64, count: u64,
+                                           bwt_outs: *const *mut u8, origins_out: *mut u64, stream_out: *mut u8,
+                                           stream_capacity: u64, stream_starts: *mut u64, stream_bytes_out: *mut u64,
+                                           infos: *mut dark_bwt_dc_info, stats: *mut dark_bwt_stats) -> c_int;
     pub fn dark_bwt_create(max_n: u64, device: c_int, out: *mut *mut dark_bwt_ctx) -> c_int;
     pub fn dark_bwt_create_ex(max_n: u64, device: c_int, flags: u32, out: *mut *mut dark_bwt_ctx) -> c_int;
     pub fn dark_bwt_arena_bytes(max_n: u64, flags: u32) -> u64;
