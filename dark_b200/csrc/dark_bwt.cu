@@ -1243,9 +1243,8 @@ int check_blocks(dark_bwt_ctx* ctx, u64 count, const uint64_t* ns, const u32* d_
     return DARK_BWT_OK;
 }
 
-// Puts a checked list where the kernels read it: the offsets into ctx->many_starts, the inverse's origins into ctx->many_origins,
-// and the host blocks `ins` (if given) into `dst` at their offsets.
-int load_blocks(dark_bwt_ctx* ctx, const BlockList& bl, const uint8_t* const* ins = nullptr, u8* dst = nullptr) {
+// Puts a checked list where the kernels read it: the offsets into ctx->many_starts, the inverse's origins into ctx->many_origins.
+int load_blocks(dark_bwt_ctx* ctx, const BlockList& bl) {
     const size_t count = bl.count();
     if (bl.d_starts) CK(cudaMemcpyAsync(ctx->many_starts, bl.d_starts, sizeof(u32) * (count + 1), cudaMemcpyDeviceToDevice, ctx->stream));
     else CK(cudaMemcpyAsync(ctx->many_starts, bl.starts.data(), sizeof(u32) * (count + 1), cudaMemcpyHostToDevice, ctx->stream));
@@ -1253,9 +1252,6 @@ int load_blocks(dark_bwt_ctx* ctx, const BlockList& bl, const uint8_t* const* in
     if (bl.d_origins) CK(cudaMemcpyAsync(ctx->many_origins, bl.d_origins, sizeof(uint64_t) * count, cudaMemcpyDeviceToDevice, ctx->stream));
     else if (!bl.origins.empty())
         CK(cudaMemcpyAsync(ctx->many_origins, bl.origins.data(), sizeof(uint64_t) * count, cudaMemcpyHostToDevice, ctx->stream));
-    if (ins)
-        for (size_t k = 0; k < count; ++k)
-            CK(cudaMemcpyAsync(dst + bl.starts[k], ins[k], bl.starts[k + 1] - bl.starts[k], cudaMemcpyHostToDevice, ctx->stream));
     return 0;
 }
 
@@ -1385,7 +1381,8 @@ bool dc_many_records_fit(const dark_bwt_ctx* ctx, u64 count) {
 // Distance coding + MTF on device buffers (dc_kernels.cuh) of one BWT block d_bwt[0..n) (`blocks` null; 1 <= n <= capacity),
 // or in one pass of the checked list `blocks`, back to back in d_bwt and loaded into ctx->many_starts (the records fit).
 // One block: infos[0] gets the result header.  Many: infos[0..count) get the per-block records, *item_starts_host the
-// item offsets, read back.
+// item offsets, read back.  Neither it nor dc_pack writes ctx->d_bwt or ctx->many_origins: the forward + DC host entries
+// copy the BWTs and origins out with the DC outputs.
 int dc_device(dark_bwt_ctx* ctx, const u8* d_bwt, u32 n, const BlockList* blocks, DcBuffers* io, dark_bwt_dc_info* infos,
               std::vector<u32>* item_starts_host) {
     CK(cudaSetDevice(ctx->device));
@@ -1663,10 +1660,17 @@ struct CopyList {
         void* dev;
         size_t bytes;
     };
-    std::vector<Copy> list;  // dark_bwt_forward_dc_packed_many: a BWT per block besides the stream and its offsets
+    std::vector<Copy> list;  // the many-block entries: one copy per block
     bool serial = false;
-    void add(const void* host, const void* dev, size_t bytes) {
+    CopyList& add(const void* host, const void* dev, size_t bytes) {
         if (host && bytes) list.push_back(Copy{(void*)host, (void*)dev, bytes});
+        return *this;
+    }
+    // The blocks of `bl` between the caller's host blocks hosts[k] and `dev` at their offsets (`hosts` and its entries nullable).
+    CopyList& add_blocks(const BlockList& bl, const uint8_t* const* hosts, const u8* dev) {
+        if (hosts)
+            for (u32 k = 0; k < bl.count(); ++k) add(hosts[k], dev + bl.starts[k], bl.starts[k + 1] - bl.starts[k]);
+        return *this;
     }
 };
 
@@ -1687,6 +1691,25 @@ int copy_blocking(dark_bwt_ctx* ctx, const CopyList& copies, cudaMemcpyKind kind
     }
     if (direct) CK(cudaStreamSynchronize(stream));
     return 0;
+}
+
+// The frame of every blocking host entry: the caller's buffers `in` to the device, then device(&out), which runs the device
+// drivers (they return with their work complete) and adds the call's outputs to `out`, then `out` to the caller's buffers.
+// st (nullable) gets the host-clock time of each direction's copies in h2d_ms and d2h_ms.
+template <typename Device>
+int run_blocking(dark_bwt_ctx* ctx, const CopyList& in, dark_bwt_stats* st, Device device) {
+    typedef std::chrono::steady_clock Clock;
+    auto ms_since = [](Clock::time_point t0) { return std::chrono::duration<float, std::milli>(Clock::now() - t0).count(); };
+    CK(cudaSetDevice(ctx->device));
+    Clock::time_point t0 = Clock::now();
+    if (int rc = copy_blocking(ctx, in, cudaMemcpyHostToDevice, ctx->stream)) return rc;
+    if (st) st->h2d_ms = ms_since(t0);
+    CopyList out;
+    if (int rc = device(&out)) return rc;
+    t0 = Clock::now();
+    if (int rc = copy_blocking(ctx, out, cudaMemcpyDeviceToHost, ctx->stream)) return rc;
+    if (st) st->d2h_ms = ms_since(t0);
+    return DARK_BWT_OK;
 }
 
 // A block's distance-coding outputs, where dc_device left them in `io`, to the caller's host arrays (each nullable): the
@@ -1961,34 +1984,18 @@ int dark_bwt_forward_device(dark_bwt_ctx* ctx, const uint8_t* d_text, uint64_t n
     return forward_device(ctx, d_text, (u32)n, d_bwt_out, origin_out, d_sa_out, stats);
 }
 
-// dark_bwt_forward and dark_bwt_forward_dc after their argument checks: the host text in, the transform, the BWT (bwt_out
-// nullable) and the SA (sa_out nullable) out, h2d_ms and d2h_ms on the host clock.  The BWT stays in ctx->d_bwt.
-static int forward_host(dark_bwt_ctx* ctx, const uint8_t* text, uint64_t n, uint8_t* bwt_out, uint64_t* origin_out, uint32_t* sa_out,
-                        dark_bwt_stats* stats) {
-    CK(cudaSetDevice(ctx->device));
-    typedef std::chrono::steady_clock Clock;
-    auto ms_since = [](Clock::time_point t0) { return std::chrono::duration<float, std::milli>(Clock::now() - t0).count(); };
-    CopyList in, out;
-    in.add(text, ctx->d_text, n);
-    out.add(bwt_out, ctx->d_bwt, n);
-    out.add(sa_out, ctx->sa, n * sizeof(u32));
-    Clock::time_point t0 = Clock::now();
-    if (int rc = copy_blocking(ctx, in, cudaMemcpyHostToDevice, ctx->stream)) return rc;
-    if (stats) stats->h2d_ms = ms_since(t0);
-    if (int rc = forward_device(ctx, ctx->d_text, (u32)n, ctx->d_bwt, origin_out, nullptr, stats)) return rc;
-    t0 = Clock::now();
-    if (int rc = copy_blocking(ctx, out, cudaMemcpyDeviceToHost, ctx->stream)) return rc;
-    if (stats) stats->d2h_ms = ms_since(t0);
-    return DARK_BWT_OK;
-}
-
 int dark_bwt_forward(dark_bwt_ctx* ctx, const uint8_t* text, uint64_t n, uint8_t* bwt_out, uint64_t* origin_out,
                      uint32_t* sa_out, dark_bwt_stats* stats) {
     if (!ctx || !text || !bwt_out || !origin_out) return DARK_BWT_E_INVALID_ARG;
     if (int rc = check_staging(ctx)) return rc;
     if (int rc = check_n(ctx, n, 2)) return rc;
     ctx->err[0] = 0;
-    return forward_host(ctx, text, n, bwt_out, origin_out, sa_out, stats);
+    return run_blocking(ctx, CopyList().add(text, ctx->d_text, n), stats, [&](CopyList* out) {
+        if (int rc = forward_device(ctx, ctx->d_text, (u32)n, ctx->d_bwt, origin_out, nullptr, stats)) return rc;
+        out->add(bwt_out, ctx->d_bwt, n);
+        out->add(sa_out, ctx->sa, n * sizeof(u32));
+        return 0;
+    });
 }
 
 int dark_bwt_forward_batch(dark_bwt_ctx* ctx, const uint8_t* const* texts, const uint64_t* ns, uint8_t* const* bwt_outs,
@@ -2038,29 +2045,6 @@ int dark_bwt_inverse_batch(dark_bwt_ctx* ctx, const uint8_t* const* bwts, const 
     });
 }
 
-// dark_bwt_forward_many and dark_bwt_forward_dc_many after their argument checks; bwt_outs (and its entries) may be null: the
-// BWTs stay in ctx->d_bwt, and ctx->many_starts keeps their offsets.
-static int forward_many_host(dark_bwt_ctx* ctx, const uint8_t* const* texts, uint8_t* const* bwt_outs, uint64_t* origins_out,
-                             const BlockList& bl, dark_bwt_stats* stats) {
-    const u32 count = bl.count();
-    CK(cudaSetDevice(ctx->device));
-    CK(cudaEventRecord(ctx->call_start, ctx->stream));
-    if (int rc = load_blocks(ctx, bl, texts, ctx->d_text)) return rc;
-    CK(cudaEventRecord(ctx->call_stop, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    if (stats) stats->h2d_ms = call_ms(ctx);
-    if (int rc = forward_many_device(ctx, ctx->d_text, bl.total(), count, ctx->d_bwt, nullptr, stats)) return rc;
-    CK(cudaEventRecord(ctx->call_start, ctx->stream));
-    for (u32 k = 0; k < count; ++k)
-        if (bwt_outs && bwt_outs[k])
-            CK(cudaMemcpyAsync(bwt_outs[k], ctx->d_bwt + bl.starts[k], bl.starts[k + 1] - bl.starts[k], cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(origins_out, ctx->many_origins, sizeof(uint64_t) * count, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaEventRecord(ctx->call_stop, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    if (stats) stats->d2h_ms = call_ms(ctx);
-    return DARK_BWT_OK;
-}
-
 int dark_bwt_forward_many(dark_bwt_ctx* ctx, const uint8_t* const* texts, const uint64_t* ns, uint8_t* const* bwt_outs,
                           uint64_t* origins_out, uint64_t count, dark_bwt_stats* stats) {
     if (!ctx || !texts || !ns || !bwt_outs || !origins_out) return DARK_BWT_E_INVALID_ARG;
@@ -2069,7 +2053,13 @@ int dark_bwt_forward_many(dark_bwt_ctx* ctx, const uint8_t* const* texts, const 
     if (count == 0) return DARK_BWT_OK;
     BlockList bl;
     if (int rc = check_blocks(ctx, count, ns, nullptr, nullptr, 2, 0, texts, bwt_outs, &bl)) return rc;
-    return forward_many_host(ctx, texts, bwt_outs, origins_out, bl, stats);
+    return run_blocking(ctx, CopyList().add_blocks(bl, texts, ctx->d_text), stats, [&](CopyList* out) {
+        if (int rc = load_blocks(ctx, bl)) return rc;
+        if (int rc = forward_many_device(ctx, ctx->d_text, bl.total(), bl.count(), ctx->d_bwt, nullptr, stats)) return rc;
+        out->add_blocks(bl, bwt_outs, ctx->d_bwt);
+        out->add(origins_out, ctx->many_origins, sizeof(uint64_t) * count);
+        return 0;
+    });
 }
 
 int dark_bwt_forward_many_device(dark_bwt_ctx* ctx, const uint8_t* d_text, const uint32_t* d_starts, uint64_t count,
@@ -2102,13 +2092,11 @@ int dark_bwt_inverse(dark_bwt_ctx* ctx, const uint8_t* bwt, uint64_t n, uint64_t
     if (int rc = check_n(ctx, n, 1)) return rc;
     if (origin >= n) return DARK_BWT_E_INVALID_ARG;
     ctx->err[0] = 0;
-    CK(cudaSetDevice(ctx->device));
-    CopyList in, out;
-    in.add(bwt, ctx->d_bwt, n);
-    out.add(text_out, ctx->d_text, n);
-    if (int rc = copy_blocking(ctx, in, cudaMemcpyHostToDevice, ctx->stream)) return rc;
-    if (int rc = inverse_device(ctx, ctx->d_bwt, (u32)n, (u32)origin, nullptr, ctx->d_text, nullptr)) return rc;
-    return copy_blocking(ctx, out, cudaMemcpyDeviceToHost, ctx->stream);
+    return run_blocking(ctx, CopyList().add(bwt, ctx->d_bwt, n), nullptr, [&](CopyList* out) {
+        if (int rc = inverse_device(ctx, ctx->d_bwt, (u32)n, (u32)origin, nullptr, ctx->d_text, nullptr)) return rc;
+        out->add(text_out, ctx->d_text, n);
+        return 0;
+    });
 }
 
 int dark_bwt_inverse_many(dark_bwt_ctx* ctx, const uint8_t* const* bwts, const uint64_t* ns, const uint64_t* origins,
@@ -2119,13 +2107,12 @@ int dark_bwt_inverse_many(dark_bwt_ctx* ctx, const uint8_t* const* bwts, const u
     if (count == 0) return DARK_BWT_OK;
     BlockList bl;
     if (int rc = check_blocks(ctx, count, ns, nullptr, origins, 1, 1, bwts, text_outs, &bl)) return rc;
-    CK(cudaSetDevice(ctx->device));
-    if (int rc = load_blocks(ctx, bl, bwts, ctx->d_bwt)) return rc;
-    if (int rc = inverse_device(ctx, ctx->d_bwt, bl.total(), 0, &bl, ctx->d_text, ms_out)) return rc;
-    for (uint64_t k = 0; k < count; ++k)
-        CK(cudaMemcpyAsync(text_outs[k], ctx->d_text + bl.starts[k], ns[k], cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    return DARK_BWT_OK;
+    return run_blocking(ctx, CopyList().add_blocks(bl, bwts, ctx->d_bwt), nullptr, [&](CopyList* out) {
+        if (int rc = load_blocks(ctx, bl)) return rc;
+        if (int rc = inverse_device(ctx, ctx->d_bwt, bl.total(), 0, &bl, ctx->d_text, ms_out)) return rc;
+        out->add_blocks(bl, text_outs, ctx->d_text);
+        return 0;
+    });
 }
 
 int dark_bwt_inverse_many_device(dark_bwt_ctx* ctx, const uint8_t* d_bwt, const uint32_t* d_starts, const uint64_t* d_origins,
@@ -2154,14 +2141,12 @@ int dark_bwt_dc_encode(dark_bwt_ctx* ctx, const uint8_t* bwt, uint64_t n, uint32
     if (int rc = check_staging(ctx)) return rc;
     if (int rc = check_n(ctx, n, 1)) return rc;
     ctx->err[0] = 0;
-    CK(cudaSetDevice(ctx->device));
-    CopyList in, out;
-    in.add(bwt, ctx->d_bwt, n);
-    if (int rc = copy_blocking(ctx, in, cudaMemcpyHostToDevice, ctx->stream)) return rc;
-    DcBuffers io;
-    if (int rc = dc_device(ctx, ctx->d_bwt, (u32)n, nullptr, &io, info, nullptr)) return rc;
-    add_dc_outputs(&out, io, n, info->num_items, dist_out, item_pos, item_dist, item_sym, item_rank);
-    return copy_blocking(ctx, out, cudaMemcpyDeviceToHost, ctx->stream);
+    return run_blocking(ctx, CopyList().add(bwt, ctx->d_bwt, n), nullptr, [&](CopyList* out) {
+        DcBuffers io;
+        if (int rc = dc_device(ctx, ctx->d_bwt, (u32)n, nullptr, &io, info, nullptr)) return rc;
+        add_dc_outputs(out, io, n, info->num_items, dist_out, item_pos, item_dist, item_sym, item_rank);
+        return 0;
+    });
 }
 
 int dark_bwt_forward_dc(dark_bwt_ctx* ctx, const uint8_t* text, uint64_t n, uint8_t* bwt_out, uint64_t* origin_out, uint32_t* dist_out,
@@ -2171,13 +2156,14 @@ int dark_bwt_forward_dc(dark_bwt_ctx* ctx, const uint8_t* text, uint64_t n, uint
     if (int rc = check_staging(ctx)) return rc;
     if (int rc = check_n(ctx, n, 2)) return rc;
     ctx->err[0] = 0;
-    if (int rc = forward_host(ctx, text, n, bwt_out, origin_out, nullptr, stats)) return rc;
-    // the BWT is still in HBM: distance coding reads it there
-    DcBuffers io;
-    if (int rc = dc_device(ctx, ctx->d_bwt, (u32)n, nullptr, &io, info, nullptr)) return rc;
-    CopyList out;
-    add_dc_outputs(&out, io, n, info->num_items, dist_out, item_pos, item_dist, item_sym, item_rank);
-    return copy_blocking(ctx, out, cudaMemcpyDeviceToHost, ctx->stream);
+    return run_blocking(ctx, CopyList().add(text, ctx->d_text, n), stats, [&](CopyList* out) {
+        if (int rc = forward_device(ctx, ctx->d_text, (u32)n, ctx->d_bwt, origin_out, nullptr, stats)) return rc;
+        DcBuffers io;
+        if (int rc = dc_device(ctx, ctx->d_bwt, (u32)n, nullptr, &io, info, nullptr)) return rc;
+        out->add(bwt_out, ctx->d_bwt, n);
+        add_dc_outputs(out, io, n, info->num_items, dist_out, item_pos, item_dist, item_sym, item_rank);
+        return 0;
+    });
 }
 
 int dark_bwt_forward_dc_batch(dark_bwt_ctx* ctx, const uint8_t* const* texts, const uint64_t* ns, uint64_t count, uint8_t* const* bwt_outs,
@@ -2228,15 +2214,17 @@ int dark_bwt_forward_dc_packed(dark_bwt_ctx* ctx, const uint8_t* text, uint64_t 
     if (int rc = check_staging(ctx)) return rc;
     if (int rc = check_n(ctx, n, 2)) return rc;
     ctx->err[0] = 0;
-    if (int rc = forward_host(ctx, text, n, bwt_out, origin_out, nullptr, stats)) return rc;
-    DcBuffers io;
-    if (int rc = dc_device(ctx, ctx->d_bwt, (u32)n, nullptr, &io, info, nullptr)) return rc;
-    // the sort's second key buffer (8 N + 1 KiB), which single-block distance coding leaves free, holds any stream (<= 8 n)
-    u8* const d_stream = (u8*)ctx->keys[1];
-    if (int rc = dc_pack(ctx, io, info->num_items, d_stream, stream_capacity, stream_bytes_out, &info->device_ms)) return rc;
-    CopyList out;
-    out.add(stream_out, d_stream, *stream_bytes_out);
-    return copy_blocking(ctx, out, cudaMemcpyDeviceToHost, ctx->stream);
+    return run_blocking(ctx, CopyList().add(text, ctx->d_text, n), stats, [&](CopyList* out) {
+        if (int rc = forward_device(ctx, ctx->d_text, (u32)n, ctx->d_bwt, origin_out, nullptr, stats)) return rc;
+        DcBuffers io;
+        if (int rc = dc_device(ctx, ctx->d_bwt, (u32)n, nullptr, &io, info, nullptr)) return rc;
+        // the sort's second key buffer (8 N + 1 KiB), which single-block distance coding leaves free, holds any stream (<= 8 n)
+        u8* const d_stream = (u8*)ctx->keys[1];
+        if (int rc = dc_pack(ctx, io, info->num_items, d_stream, stream_capacity, stream_bytes_out, &info->device_ms)) return rc;
+        out->add(bwt_out, ctx->d_bwt, n);
+        out->add(stream_out, d_stream, *stream_bytes_out);
+        return 0;
+    });
 }
 
 int dark_bwt_forward_dc_packed_batch(dark_bwt_ctx* ctx, const uint8_t* const* texts, const uint64_t* ns, uint64_t count,
@@ -2312,16 +2300,16 @@ int dark_bwt_dc_encode_many(dark_bwt_ctx* ctx, const uint8_t* const* bwts, const
     BlockList bl;
     if (int rc = check_blocks(ctx, count, ns, nullptr, nullptr, 1, 0, bwts, nullptr, &bl)) return rc;
     if (!dc_many_records_fit(ctx, count)) return DARK_BWT_E_INVALID_N;
-    CK(cudaSetDevice(ctx->device));
-    if (int rc = load_blocks(ctx, bl, bwts, ctx->d_bwt)) return rc;
-    DcBuffers io;
-    std::vector<u32> starts;
-    if (int rc = dc_device(ctx, ctx->d_bwt, bl.total(), &bl, &io, infos, &starts)) return rc;
-    if (ms_out) *ms_out = infos[0].device_ms;
-    if (item_starts) memcpy(item_starts, starts.data(), starts.size() * sizeof(u32));
-    CopyList out;
-    add_dc_outputs(&out, io, bl.total(), starts.back(), dist_out, item_pos, item_dist, item_sym, item_rank);
-    return copy_blocking(ctx, out, cudaMemcpyDeviceToHost, ctx->stream);
+    return run_blocking(ctx, CopyList().add_blocks(bl, bwts, ctx->d_bwt), nullptr, [&](CopyList* out) {
+        if (int rc = load_blocks(ctx, bl)) return rc;
+        DcBuffers io;
+        std::vector<u32> starts;
+        if (int rc = dc_device(ctx, ctx->d_bwt, bl.total(), &bl, &io, infos, &starts)) return rc;
+        if (ms_out) *ms_out = infos[0].device_ms;
+        if (item_starts) memcpy(item_starts, starts.data(), starts.size() * sizeof(u32));
+        add_dc_outputs(out, io, bl.total(), starts.back(), dist_out, item_pos, item_dist, item_sym, item_rank);
+        return 0;
+    });
 }
 
 int dark_bwt_forward_dc_many(dark_bwt_ctx* ctx, const uint8_t* const* texts, const uint64_t* ns, uint64_t count, uint8_t* const* bwt_outs,
@@ -2337,15 +2325,18 @@ int dark_bwt_forward_dc_many(dark_bwt_ctx* ctx, const uint8_t* const* texts, con
     BlockList bl;
     if (int rc = check_blocks(ctx, count, ns, nullptr, nullptr, 2, 0, texts, nullptr, &bl)) return rc;
     if (!dc_many_records_fit(ctx, count)) return DARK_BWT_E_INVALID_N;
-    if (int rc = forward_many_host(ctx, texts, bwt_outs, origins_out, bl, stats)) return rc;
-    // the BWTs are still in HBM at the same offsets, and ctx->many_starts still holds them
-    DcBuffers io;
-    std::vector<u32> starts;
-    if (int rc = dc_device(ctx, ctx->d_bwt, bl.total(), &bl, &io, infos, &starts)) return rc;
-    if (item_starts) memcpy(item_starts, starts.data(), starts.size() * sizeof(u32));
-    CopyList out;
-    add_dc_outputs(&out, io, bl.total(), starts.back(), dist_out, item_pos, item_dist, item_sym, item_rank);
-    return copy_blocking(ctx, out, cudaMemcpyDeviceToHost, ctx->stream);
+    return run_blocking(ctx, CopyList().add_blocks(bl, texts, ctx->d_text), stats, [&](CopyList* out) {
+        if (int rc = load_blocks(ctx, bl)) return rc;
+        if (int rc = forward_many_device(ctx, ctx->d_text, bl.total(), bl.count(), ctx->d_bwt, nullptr, stats)) return rc;
+        DcBuffers io;
+        std::vector<u32> starts;
+        if (int rc = dc_device(ctx, ctx->d_bwt, bl.total(), &bl, &io, infos, &starts)) return rc;
+        if (item_starts) memcpy(item_starts, starts.data(), starts.size() * sizeof(u32));
+        out->add_blocks(bl, bwt_outs, ctx->d_bwt);
+        out->add(origins_out, ctx->many_origins, sizeof(uint64_t) * count);
+        add_dc_outputs(out, io, bl.total(), starts.back(), dist_out, item_pos, item_dist, item_sym, item_rank);
+        return 0;
+    });
 }
 
 int dark_bwt_dc_encode_packed_many_device(dark_bwt_ctx* ctx, const uint8_t* d_bwt, const uint32_t* d_starts, uint64_t count,
@@ -2381,25 +2372,23 @@ int dark_bwt_forward_dc_packed_many(dark_bwt_ctx* ctx, const uint8_t* const* tex
     BlockList bl;
     if (int rc = check_blocks(ctx, count, ns, nullptr, nullptr, 2, 0, texts, nullptr, &bl)) return rc;
     if (!dc_many_records_fit(ctx, count)) return DARK_BWT_E_INVALID_N;
-    // the BWTs stay in HBM for distance coding and are copied out with the stream
-    if (int rc = forward_many_host(ctx, texts, nullptr, origins_out, bl, stats)) return rc;
-    DcBuffers io;
-    std::vector<u32> starts;
-    if (int rc = dc_device(ctx, ctx->d_bwt, bl.total(), &bl, &io, infos, &starts)) return rc;
-    // dc_device has read the per-block records back out of the sort's second key buffer (8 N + 1 KiB): it holds any stream
-    // (<= 8 sum(ns)).  The offsets go to the head of ranks, in front of the pack's tile scratch (dc_pack).
-    u8* const d_stream = (u8*)ctx->keys[1];
-    u64* const d_offsets = (u64*)ctx->ranks;
-    if (int rc = dc_pack_many(ctx, io, starts, d_stream, stream_capacity, d_offsets, stream_bytes_out, infos, nullptr)) return rc;
-    CopyList out;
-    out.add(stream_out, d_stream, *stream_bytes_out);
-    out.add(stream_starts, d_offsets, sizeof(u64) * (count + 1));
-    if (bwt_outs)
-        for (u32 k = 0; k < bl.count(); ++k) out.add(bwt_outs[k], ctx->d_bwt + bl.starts[k], bl.starts[k + 1] - bl.starts[k]);
-    const auto t0 = std::chrono::steady_clock::now();
-    if (int rc = copy_blocking(ctx, out, cudaMemcpyDeviceToHost, ctx->stream)) return rc;
-    if (stats) stats->d2h_ms += std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    return DARK_BWT_OK;
+    return run_blocking(ctx, CopyList().add_blocks(bl, texts, ctx->d_text), stats, [&](CopyList* out) {
+        if (int rc = load_blocks(ctx, bl)) return rc;
+        if (int rc = forward_many_device(ctx, ctx->d_text, bl.total(), bl.count(), ctx->d_bwt, nullptr, stats)) return rc;
+        DcBuffers io;
+        std::vector<u32> starts;
+        if (int rc = dc_device(ctx, ctx->d_bwt, bl.total(), &bl, &io, infos, &starts)) return rc;
+        // dc_device has read the per-block records back out of the sort's second key buffer (8 N + 1 KiB): it holds any stream
+        // (<= 8 sum(ns)).  The offsets go to the head of ranks, in front of the pack's tile scratch (dc_pack).
+        u8* const d_stream = (u8*)ctx->keys[1];
+        u64* const d_offsets = (u64*)ctx->ranks;
+        if (int rc = dc_pack_many(ctx, io, starts, d_stream, stream_capacity, d_offsets, stream_bytes_out, infos, nullptr)) return rc;
+        out->add_blocks(bl, bwt_outs, ctx->d_bwt);
+        out->add(origins_out, ctx->many_origins, sizeof(uint64_t) * count);
+        out->add(stream_out, d_stream, *stream_bytes_out);
+        out->add(stream_starts, d_offsets, sizeof(u64) * (count + 1));
+        return 0;
+    });
 }
 
 int dark_bwt_reuse(dark_bwt_ctx* ctx, uint32_t** words_out, uint64_t* count_out) {

@@ -91,8 +91,9 @@ typedef struct dark_bwt_stats {
     float keybuild_ms;        /* (rank[i], rank[i+h]) key construction                    */
     float rerank_ms;          /* re-rank + compaction scans                               */
     float emit_ms;            /* BWT gather + origin                                      */
-    float h2d_ms;             /* host entry point only                                    */
-    float d2h_ms;             /* host entry point only                                    */
+    float h2d_ms;             /* blocking host entries: host-clock time of all copies of the caller's buffers to the
+                                 device; 0 in the pipelined batch entries and the device entries */
+    float d2h_ms;             /* the same for the copies back to the caller's buffers     */
     /* the key-generating first pass (reads 1 B of text and writes 12 B per suffix instead of 12 + 12), part of the figures above */
     uint32_t gen_passes;      /* key-generating pass launches (0 or 1)                    */
     float gen_pass_ms;        /* their share of pass_ms                                   */
@@ -141,7 +142,8 @@ int dark_bwt_forward_batch(dark_bwt_ctx *ctx, const uint8_t *const *texts, const
  * for a fraction of its 0.5 ms of launches; `count` such blocks (each >= 2 bytes, sum <= capacity, count <=
  * DARK_BWT_MAX_MANY_BLOCKS) are concatenated and their suffixes sorted together, every suffix ending at the end
  * of its own block.  Results are identical to `count` dark_bwt_forward calls: bwt_outs[k][0..ns[k]) and
- * origins_out[k].  One H2D copy per block into one device text, one device pass, one D2H copy per block.
+ * origins_out[k].  One H2D copy per block into one device text, one device pass, one D2H copy per block (pageable blocks
+ * of 1 MiB or more go through the staging lanes, as in dark_bwt_forward).
  * (src/main.rs:87-113: the reference's CLI feeds its blocks one after another through one Encoder.) */
 #define DARK_BWT_MAX_MANY_BLOCKS 65536u
 int dark_bwt_forward_many(dark_bwt_ctx *ctx, const uint8_t *const *texts, const uint64_t *ns, uint8_t *const *bwt_outs,
@@ -178,8 +180,9 @@ int dark_bwt_inverse_batch(dark_bwt_ctx *ctx, const uint8_t *const *bwts, const 
  * origins[k] < ns[k], count <= DARK_BWT_MAX_MANY_BLOCKS) give text_outs[k][0..ns[k]), what dark_bwt_inverse(bwts[k],
  * ns[k], origins[k]) gives.  The blocks share one row space of sum(ns) + count rows (one '$' row per block), which must
  * fit: sum(ns) + count <= capacity, else DARK_BWT_E_INVALID_N.  One H2D copy per block, one device pass, one D2H copy per
- * block.  ms_out (nullable) = device time of the pass.  DARK_BWT_E_INVALID_ARG if some (bwt, origin) is not the forward
- * transform of any text; dark_bwt_last_error() then names the first such block. */
+ * block (pageable blocks of 1 MiB or more go through the staging lanes).  ms_out (nullable) = device time of the pass.
+ * DARK_BWT_E_INVALID_ARG if some (bwt, origin) is not the forward transform of any text; dark_bwt_last_error() then names
+ * the first such block. */
 int dark_bwt_inverse_many(dark_bwt_ctx *ctx, const uint8_t *const *bwts, const uint64_t *ns, const uint64_t *origins,
                           uint8_t *const *text_outs, uint64_t count, float *ms_out);
 /* Same on device buffers, the layout dark_bwt_forward_many_device writes: d_bwt holds the blocks back to back,
@@ -285,7 +288,8 @@ int dark_bwt_forward_dc_packed_batch(dark_bwt_ctx *ctx, const uint8_t *const *te
  * Every output but `infos` is nullable.  Limits: count <= DARK_BWT_MAX_MANY_BLOCKS (else DARK_BWT_E_INVALID_ARG), each
  * block >= 1 byte, sum(ns) <= capacity and <= 2^32-2, and the per-block records (1,288 bytes each) are staged in an
  * 8 * capacity + 1 KiB buffer: count * 1288 <= 8 * capacity + 1024 (blocks of about 161 bytes or more on average at full
- * capacity), else DARK_BWT_E_INVALID_N.  One H2D copy per block, one device pass, one D2H copy per output array.
+ * capacity), else DARK_BWT_E_INVALID_N.  One H2D copy per block, one device pass, one D2H copy per output array (pageable
+ * blocks and arrays of 1 MiB or more go through the staging lanes).
  * DARK_BWT_E_INVALID_ARG with a device-only context. */
 int dark_bwt_dc_encode_many(dark_bwt_ctx *ctx, const uint8_t *const *bwts, const uint64_t *ns, uint64_t count, uint32_t *dist_out,
                             uint32_t *item_starts, uint32_t *item_pos, uint32_t *item_dist, uint8_t *item_sym, uint8_t *item_rank,
