@@ -22,6 +22,7 @@ SYMBOLS = [
     "dark_bwt_dc_encode_many_device", "dark_bwt_forward_dc_many", "dark_bwt_forward_dc_batch",
     "dark_bwt_dc_encode_packed_device", "dark_bwt_forward_dc_packed", "dark_bwt_forward_dc_packed_batch",
     "dark_bwt_dc_encode_packed_many_device", "dark_bwt_forward_dc_packed_many",
+    "dark_bwt_dc_decode_packed_device", "dark_bwt_inverse_dc_packed",
 ]
 
 
@@ -136,6 +137,8 @@ def lib():
     L.dark_bwt_dc_encode_packed_many_device.argtypes = [vp, vp, vp, u64, vp, u64, vp, ctypes.POINTER(u64), vp,
                                                         ctypes.POINTER(ctypes.c_float)]
     L.dark_bwt_forward_dc_packed_many.argtypes = [vp, vp, vp, u64, vp, vp, vp, u64, vp, ctypes.POINTER(u64), vp, ctypes.POINTER(Stats)]
+    L.dark_bwt_dc_decode_packed_device.argtypes = [vp, vp, u64, u64, vp, ctypes.POINTER(DcInfo)]
+    L.dark_bwt_inverse_dc_packed.argtypes = [vp, vp, u64, u64, u64, vp, vp, ctypes.POINTER(DcInfo)]
     _lib = L
     return L
 

@@ -17,7 +17,8 @@
 // arena up front too, saca.rs:351-360) by carve_arena; the forward calls allocate nothing.  The packed item stream
 // (dc_pack) reuses what distance coding has finished with: the host entries' stream lives in keys[1]; the tile counts in
 // ranks_alt, or for many blocks (whose item offsets are in ranks_alt) in ranks behind the per-block stream offsets of
-// dark_bwt_forward_dc_packed_many and the tile offsets; the first-item bitmap of many blocks in `bitmap`.
+// dark_bwt_forward_dc_packed_many and the tile offsets; the first-item bitmap of many blocks in `bitmap`.  Decoding a packed
+// stream (dc_decode) parses into keys[0] and re-packs there for its check; the host entry's stream lives in keys[1].
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -69,6 +70,8 @@ struct Mailbox {  // pinned host memory the device results are copied into
     u32 bad_block;  // inverse: the lowest block whose list does not cover its rows (with `count` = how many do not)
     u32 bad_dist;   // inverse: the rows that block's list covers
     unsigned long long packed_bytes;  // distance coding: the size of the packed item stream
+    UnpackTotals unpack;              // decoding a packed stream: the parse's totals (k_dc_unpack_chain)
+    unsigned long long unpack_diff;   // ... the first byte at which the stream differs from the decoded block's, ~0 if none
 };
 
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
@@ -1191,6 +1194,13 @@ int check_n(const dark_bwt_ctx* ctx, u64 n, u64 min_n) {
 // The host-buffer entries stage through device buffers that a DARK_BWT_F_DEVICE_ONLY context does not have.
 int check_staging(const dark_bwt_ctx* ctx) { return (ctx->flags & DARK_BWT_F_DEVICE_ONLY) ? DARK_BWT_E_INVALID_ARG : DARK_BWT_OK; }
 
+// A packed item stream of stream_bytes for a block of n bytes (the decode entries, after their pointer checks).
+int check_decode_args(const dark_bwt_ctx* ctx, uint64_t stream_bytes, uint64_t n) {
+    if (int rc = check_n(ctx, n, 1)) return rc;
+    if (stream_bytes == 0 || stream_bytes > DARK_BWT_DC_PACKED_MAX(n)) return DARK_BWT_E_INVALID_ARG;  // no valid stream is that long
+    return DARK_BWT_OK;
+}
+
 // The blocks of a many-block entry, back to back: block k is [starts[k], starts[k+1]).
 struct BlockList {
     std::vector<u32> starts;              // count + 1 offsets
@@ -1532,6 +1542,79 @@ int dc_pack_many(dark_bwt_ctx* ctx, const DcBuffers& io, const std::vector<u32>&
     if (int rc = dc_pack(ctx, io, starts.back(), d_out, capacity, bytes_out, &ms, count, d_stream_starts)) return rc;
     for (u32 k = 0; k < count; ++k) infos[k].device_ms = ms;
     if (ms_out) *ms_out = ms;
+    return DARK_BWT_OK;
+}
+
+// The inverse of dark_bwt_dc_encode_packed_device (kernels in dc_kernels.cuh, DESIGN.md §3.9): d_bwt[0..n) gets the block
+// whose packed stream is d_stream[0..bytes), 1 <= bytes <= 8 n, or the call is DARK_BWT_E_INVALID_ARG with ctx->err saying
+// why.  Parse (tiles, chain), one host round trip for the chain's totals, which must be those of a stream of n bytes, and
+// only then the items and the expansion into d_bwt; the check is dc_device + dc_pack of d_bwt and a byte compare with the
+// stream.  *info = what the encoder gives for the block, device_ms = the whole call.
+// Scratch: run starts (4 n), symbols (n) and the tile summaries and bases (96 bytes per 8 KiB of stream: <= 0.1 n + 96) in
+// keys[0] (8 N + 1 KiB), which the check then takes for DC's distances and the re-pack (<= 8 n): the pack reads neither.  A
+// host entry's stream in keys[1] and the caller's buffers are only read.
+int dc_decode(dark_bwt_ctx* ctx, const u8* d_stream, u64 bytes, u32 n, u8* d_bwt, dark_bwt_dc_info* info) {
+    if (int rc = begin_call(ctx)) return rc;
+    cudaEvent_t ev_start = ctx->events[0], ev_stop = ctx->events[1];
+    CK(cudaEventRecord(ev_start, ctx->stream));
+    u8* const scratch = (u8*)ctx->keys[0];
+    u32* const run_start = (u32*)scratch;
+    u8* const run_sym = scratch + (size_t)n * 4;
+    const u32 ntiles = (u32)ceil_div(bytes, kUnpackTile);
+    UnpackSum* const tiles = (UnpackSum*)(scratch + align_up((size_t)n * 5, 16));
+    UnpackBase* const bases = (UnpackBase*)(tiles + ntiles);
+    k_dc_unpack_tiles<<<ntiles, kUnpackThreads, 0, ctx->stream>>>(d_stream, bytes, tiles);
+    LAUNCHED();
+    k_dc_unpack_chain<<<1, kChainThreads, 0, ctx->stream>>>(tiles, ntiles, bases, &ctx->mail_dev->unpack);
+    LAUNCHED();
+    CK(cudaStreamSynchronize(ctx->stream));
+    const UnpackTotals t = ctx->mail->unpack;
+    if (t.err != ~0ull) {
+        snprintf(ctx->err, sizeof(ctx->err), "packed item stream: malformed item at byte %llu (a varint of more than 5 bytes or "
+                 "above 2^32 - 1, or an item cut off by the end)", t.err);
+        return DARK_BWT_E_INVALID_ARG;
+    }
+    if (t.state != 0) {
+        snprintf(ctx->err, sizeof(ctx->err), "packed item stream: the %llu bytes end inside an item", (unsigned long long)bytes);
+        return DARK_BWT_E_INVALID_ARG;
+    }
+    if (t.sum != n) {
+        snprintf(ctx->err, sizeof(ctx->err), "packed item stream: the run lengths of its %llu items add up to %s%llu, not n = %u",
+                 t.items, t.sum >= kUnpackSumCap ? "at least " : "", t.sum, n);
+        return DARK_BWT_E_INVALID_ARG;
+    }
+    // every item is well formed and the run lengths (each >= 1) add up to n: at most n items, run starts increasing below n
+    k_dc_unpack_items<<<ntiles, kUnpackThreads, 0, ctx->stream>>>(d_stream, bytes, bases, n, run_start, run_sym);
+    LAUNCHED();
+    k_dc_unpack_expand<<<(u32)ceil_div((u64)n + ((uintptr_t)d_bwt & 15u), kExpandWords * 16), kExpandWords, 0, ctx->stream>>>(
+        run_start, run_sym, (u32)t.items, n, d_bwt);
+    LAUNCHED();
+    // the check: the decoded block's own stream must be the input, byte for byte (distances and ranks have no cheaper test)
+    DcBuffers io;
+    if (int rc = dc_device(ctx, d_bwt, n, nullptr, &io, info, nullptr)) return rc;
+    u8* const repack = (u8*)ctx->keys[0];
+    u64 repacked = 0;
+    float pack_ms = 0.f;
+    if (int rc = dc_pack(ctx, io, info->num_items, repack, (u64)n * 8, &repacked, &pack_ms)) return rc;
+    if (repacked != bytes) {
+        snprintf(ctx->err, sizeof(ctx->err), "packed item stream: the decoded block packs to %llu bytes, the stream has %llu",
+                 (unsigned long long)repacked, (unsigned long long)bytes);
+        return DARK_BWT_E_INVALID_ARG;
+    }
+    u32* done = nullptr;
+    if (int rc = next_counter(ctx, &done)) return rc;
+    CK(cudaMemsetAsync(ctx->bad, 0xFF, sizeof(unsigned long long), ctx->stream));
+    const u32 cgrid = (u32)std::min<u64>(ceil_div(bytes, 256), (u64)ctx->num_sms * 8);
+    k_dc_unpack_compare<<<cgrid, 256, 0, ctx->stream>>>(d_stream, repack, bytes, ctx->bad, done, &ctx->mail_dev->unpack_diff);
+    LAUNCHED();
+    CK(cudaEventRecord(ev_stop, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (ctx->mail->unpack_diff != ~0ull) {
+        snprintf(ctx->err, sizeof(ctx->err), "packed item stream: differs from the decoded block's own stream at byte %llu",
+                 ctx->mail->unpack_diff);
+        return DARK_BWT_E_INVALID_ARG;
+    }
+    cudaEventElapsedTime(&info->device_ms, ev_start, ev_stop);
     return DARK_BWT_OK;
 }
 
@@ -2266,6 +2349,34 @@ int dark_bwt_forward_dc_packed_batch(dark_bwt_ctx* ctx, const uint8_t* const* te
         }
         out->add(stream_outs[k], d_stream, stream_bytes_out[k]);
         out->add(bwt_outs ? bwt_outs[k] : nullptr, d_bwt[b], n);
+        return 0;
+    });
+}
+
+int dark_bwt_dc_decode_packed_device(dark_bwt_ctx* ctx, const uint8_t* d_stream, uint64_t stream_bytes, uint64_t n, uint8_t* d_bwt_out,
+                                     dark_bwt_dc_info* info) {
+    if (!ctx || !d_stream || !d_bwt_out) return DARK_BWT_E_INVALID_ARG;
+    if (int rc = check_decode_args(ctx, stream_bytes, n)) return rc;
+    ctx->err[0] = 0;
+    dark_bwt_dc_info local;
+    return dc_decode(ctx, d_stream, stream_bytes, (u32)n, d_bwt_out, info ? info : &local);
+}
+
+int dark_bwt_inverse_dc_packed(dark_bwt_ctx* ctx, const uint8_t* stream, uint64_t stream_bytes, uint64_t n, uint64_t origin,
+                               uint8_t* text_out, uint8_t* bwt_out, dark_bwt_dc_info* info) {
+    if (!ctx || !stream || !text_out) return DARK_BWT_E_INVALID_ARG;
+    if (int rc = check_staging(ctx)) return rc;
+    if (int rc = check_decode_args(ctx, stream_bytes, n)) return rc;
+    if (origin >= n) return DARK_BWT_E_INVALID_ARG;
+    ctx->err[0] = 0;
+    dark_bwt_dc_info local;
+    // the stream goes to the sort's second key buffer (8 N + 1 KiB >= 8 n), the block to d_bwt, which the inverse reads
+    u8* const d_stream = (u8*)ctx->keys[1];
+    return run_blocking(ctx, CopyList().add(stream, d_stream, stream_bytes), nullptr, [&](CopyList* out) {
+        if (int rc = dc_decode(ctx, d_stream, stream_bytes, (u32)n, ctx->d_bwt, info ? info : &local)) return rc;
+        if (int rc = inverse_device(ctx, ctx->d_bwt, (u32)n, (u32)origin, nullptr, ctx->d_text, nullptr)) return rc;
+        out->add(text_out, ctx->d_text, n);
+        out->add(bwt_out, ctx->d_bwt, n);
         return 0;
     });
 }

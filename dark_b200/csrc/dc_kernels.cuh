@@ -622,4 +622,364 @@ k_dc_pack_write(const u32* __restrict__ pos, const u32* __restrict__ dist, const
     }
 }
 
+// ---- decoding the packed item stream (the inverse of the pack; DESIGN.md §3.9) ---------------------------------------
+// Item boundaries are sequential: sym and rank bytes are arbitrary, only the varints end on a byte with bit 7 clear.  A
+// stretch of the stream is summarised for each of the four states it may be entered in (0 = at an item's sym byte, 1 = at
+// its rank byte, 2 = inside the run-length varint, 3 = inside the distance varint) and the summaries compose, so the
+// boundaries are found in parallel:
+//   k_dc_unpack_tiles   per tile of kUnpackTile bytes: its summary (a block scan of the threads' 32-byte chunks)
+//   k_dc_unpack_chain   one CTA: the tiles chained from state 0 at byte 0 -> each tile's entry state, item base and run
+//                       start base; the totals and the first malformed item into the mailbox (the host checks them)
+//   k_dc_unpack_items   each tile again from its entry state: every item's run start and symbol
+//   k_dc_unpack_expand  per 4 KiB of output: the tile's runs by binary search, its bytes with 16-byte stores
+//   k_dc_unpack_compare the first byte at which the stream differs from the decoded block's re-pack
+// An item is decoded whole by the thread whose chunk holds its sym byte, which reads at most kPackMaxItemBytes bytes and
+// never at or past the end of the stream; a varint of more than 5 bytes, one above 2^32 - 1, or an item cut off by the end
+// is malformed.  The walks jump from item to item, so a chunk costs at most its 32 bytes whatever the bytes are.
+constexpr int kUnpackThreads = 256;
+constexpr int kUnpackChunk = 32;  // bytes per thread
+constexpr int kUnpackTile = kUnpackThreads * kUnpackChunk;
+constexpr u32 kUnpackNone = 0xFFFFFFFFu;
+constexpr u64 kUnpackSumCap = 1ull << 40;  // the chain saturates run-length sums here (a valid stream sums to n < 2^32)
+
+// A stretch of the stream, for each entry state s.  Composing stretch a, then b: b is entered in a's exit state.
+struct UnpackSum {
+    u64 sum[4];    // run lengths of the items whose sym byte lies in the stretch
+    u32 items[4];  // those items
+    u32 err[4];    // tile-relative offset of the first malformed one, kUnpackNone if none
+    u32 exit;      // 2 bits per s: the state after the stretch
+    u32 pad_;
+};
+
+struct UnpackBase {  // a tile as the chain enters it
+    u64 item;  // index of the first item whose sym byte lies in the tile
+    u64 pos;   // its run start
+    u32 state;
+    u32 pad_;
+};
+
+template <typename T>
+__device__ __forceinline__ T unpack_pick(const T (&a)[4], u32 s) {  // a[s] without dynamic indexing (no local memory)
+    return s == 0 ? a[0] : s == 1 ? a[1] : s == 2 ? a[2] : a[3];
+}
+
+__device__ __forceinline__ UnpackSum unpack_identity() {
+    UnpackSum r;
+#pragma unroll
+    for (int s = 0; s < 4; ++s) r.sum[s] = 0, r.items[s] = 0, r.err[s] = kUnpackNone;
+    r.exit = 0xE4u;  // s -> s
+    r.pad_ = 0;
+    return r;
+}
+
+__device__ __forceinline__ UnpackSum unpack_then(const UnpackSum& a, const UnpackSum& b) {
+    UnpackSum r;
+    r.exit = 0;
+    r.pad_ = 0;
+#pragma unroll
+    for (int s = 0; s < 4; ++s) {
+        const u32 t = (a.exit >> (2 * s)) & 3u;
+        r.exit |= ((b.exit >> (2 * t)) & 3u) << (2 * s);
+        r.items[s] = a.items[s] + unpack_pick(b.items, t);
+        r.sum[s] = a.sum[s] + unpack_pick(b.sum, t);
+        r.err[s] = a.err[s] != kUnpackNone ? a.err[s] : unpack_pick(b.err, t);
+    }
+    return r;
+}
+
+__device__ __forceinline__ UnpackSum unpack_shfl_up(const UnpackSum& v, int o) {
+    UnpackSum r;
+#pragma unroll
+    for (int s = 0; s < 4; ++s) {
+        r.sum[s] = __shfl_up_sync(0xffffffffu, v.sum[s], o);
+        r.items[s] = __shfl_up_sync(0xffffffffu, v.items[s], o);
+        r.err[s] = __shfl_up_sync(0xffffffffu, v.err[s], o);
+    }
+    r.exit = __shfl_up_sync(0xffffffffu, v.exit, o);
+    r.pad_ = 0;
+    return r;
+}
+
+// Exclusive block scan of the threads' summaries in thread order (blockDim.x = 32 * warps); *total = all of them.
+template <int WARPS>
+__device__ __forceinline__ UnpackSum unpack_block_scan(const UnpackSum& v, UnpackSum* s_warp /* [WARPS] */, UnpackSum* total) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    UnpackSum x = v;  // inclusive scan over the warp
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const UnpackSum y = unpack_shfl_up(x, o);
+        if (lane >= o) x = unpack_then(y, x);
+    }
+    UnpackSum ex = unpack_shfl_up(x, 1);
+    if (lane == 0) ex = unpack_identity();
+    if (lane == 31) s_warp[warp] = x;
+    __syncthreads();
+    if (warp == 0) {  // the warps' totals, scanned in place
+        UnpackSum w = lane < WARPS ? s_warp[lane] : unpack_identity();
+#pragma unroll
+        for (int o = 1; o < WARPS; o <<= 1) {
+            const UnpackSum y = unpack_shfl_up(w, o);
+            if (lane >= o) w = unpack_then(y, w);
+        }
+        if (lane < WARPS) s_warp[lane] = w;
+    }
+    __syncthreads();
+    *total = s_warp[WARPS - 1];
+    const UnpackSum r = warp ? unpack_then(s_warp[warp - 1], ex) : ex;
+    __syncthreads();  // s_warp may be rewritten by the caller's next scan
+    return r;
+}
+
+// One unsigned LEB128 of at most 5 bytes at buf[q], not reaching lim: the offset after it, or 0 if malformed (*val = its value).
+__device__ __forceinline__ u32 unpack_varint(const u8* buf, u32 q, u32 lim, u32* val) {
+    u64 v = 0;
+    u32 b = 0x80u;
+    int k = 0;
+    for (; k < 5 && (b & 0x80u) && q < lim; ++k, ++q) {
+        b = buf[q];
+        v |= (u64)(b & 0x7Fu) << (7 * k);
+    }
+    *val = (u32)v;
+    return (b & 0x80u) || v > 0xFFFFFFFFull ? 0u : q;
+}
+
+// Walks buf[c0, c1) entered in `state`; lim = the stream's bytes in buf (>= c1).  Items whose sym byte lies in the chunk
+// are decoded whole (they may reach past c1, never to lim); emit(sym, run length) is called for each in order.
+// *err_at = the chunk's first malformed item (kUnpackNone: none); the walk stops there.  Returns the exit state.
+template <typename Emit>
+__device__ __forceinline__ u32 unpack_walk(const u8* buf, u32 c0, u32 c1, u32 lim, u32 state, u32* err_at, Emit emit) {
+    *err_at = kUnpackNone;
+    u32 p = c0;
+    while (p < c1) {
+        if (state == 0) {
+            u32 len1 = 0, d = 0;
+            const u32 len_end = p + 1 < lim ? unpack_varint(buf, p + 2, lim, &len1) : 0u;
+            const u32 q = len_end ? unpack_varint(buf, len_end, lim, &d) : 0u;
+            if (!q) {
+                *err_at = p;
+                return 0;
+            }
+            emit((u32)buf[p], (u64)len1 + 1u);
+            if (q <= c1) {
+                p = q;
+                continue;
+            }
+            return c1 == p + 1 ? 1u : c1 < len_end ? 2u : 3u;  // the item goes on past the chunk
+        }
+        const u32 b = buf[p++];
+        if (state == 1) state = 2;
+        else if (!(b & 0x80u)) state = state == 2 ? 3u : 0u;
+    }
+    return state;
+}
+
+// The tile's bytes [tile0, tile0 + kUnpackTile + 16) into shared memory (zero past the stream); returns the stream's bytes
+// in it (the walks' lim) and sets *len = those of the tile proper.
+__device__ __forceinline__ u32 unpack_load_tile(const u8* __restrict__ stream, u64 bytes, u64 tile0, u8* s_buf, u32* len) {
+    const u64 left = bytes - tile0;
+    const u32 lim = (u32)min(left, (u64)kUnpackTile + 16);
+    for (u32 i = threadIdx.x; i < (u32)kUnpackTile + 16; i += blockDim.x) s_buf[i] = i < lim ? stream[tile0 + i] : (u8)0;
+    *len = min(lim, (u32)kUnpackTile);
+    __syncthreads();
+    return lim;
+}
+
+// The summary of this thread's chunk for each entry state.
+__device__ __forceinline__ UnpackSum unpack_chunk(const u8* s_buf, u32 len, u32 lim) {
+    const u32 c0 = min((u32)threadIdx.x * kUnpackChunk, len), c1 = min(c0 + kUnpackChunk, len);
+    UnpackSum v;
+    v.exit = 0;
+    v.pad_ = 0;
+#pragma unroll
+    for (int s = 0; s < 4; ++s) {
+        u32 items = 0;
+        u64 sum = 0;
+        const u32 x = unpack_walk(s_buf, c0, c1, lim, (u32)s, &v.err[s], [&](u32, u64 run) {
+            ++items;
+            sum += run;
+        });
+        v.exit |= x << (2 * s);
+        v.items[s] = items;
+        v.sum[s] = sum;
+    }
+    return v;
+}
+
+__global__ void __launch_bounds__(kUnpackThreads, 1)
+k_dc_unpack_tiles(const u8* __restrict__ stream, u64 bytes, UnpackSum* __restrict__ tiles) {
+    __shared__ __align__(16) u8 s_buf[kUnpackTile + 16];
+    __shared__ UnpackSum s_warp[kUnpackThreads / 32];
+    u32 len;
+    const u32 lim = unpack_load_tile(stream, bytes, (u64)blockIdx.x * kUnpackTile, s_buf, &len);
+    UnpackSum total;
+    unpack_block_scan<kUnpackThreads / 32>(unpack_chunk(s_buf, len, lim), s_warp, &total);
+    if (threadIdx.x == 0) tiles[blockIdx.x] = total;
+}
+
+// Mailbox fields the chain writes (the context's mapped mailbox; the host reads them after one synchronise).
+struct UnpackTotals {
+    unsigned long long items;  // items of the whole stream
+    unsigned long long sum;    // their run lengths (saturated at kUnpackSumCap)
+    unsigned long long err;    // byte offset of the first malformed item, ~0 if none
+    u32 state;                 // the state after the last byte (0: the stream ends at an item boundary)
+    u32 pad_;
+};
+
+// One CTA of kChainThreads threads, kChainTiles tiles per thread and step: the tiles in order from state 0, item 0, run start 0.
+constexpr int kChainThreads = 512, kChainTiles = 8;
+__global__ void __launch_bounds__(kChainThreads, 1)
+k_dc_unpack_chain(const UnpackSum* __restrict__ tiles, u32 ntiles, UnpackBase* __restrict__ bases, UnpackTotals* __restrict__ out) {
+    __shared__ UnpackSum s_warp[kChainThreads / 32];
+    __shared__ unsigned long long s_err;
+    if (threadIdx.x == 0) s_err = ~0ull;
+    u32 state = 0;
+    u64 item = 0, pos = 0;
+    for (u32 base = 0; base < ntiles; base += kChainThreads * kChainTiles) {
+        const u32 i0 = base + (u32)kChainTiles * threadIdx.x;
+        UnpackSum mine = unpack_identity();
+#pragma unroll 1
+        for (int j = 0; j < kChainTiles; ++j)
+            if (i0 + j < ntiles) mine = unpack_then(mine, tiles[i0 + j]);
+        UnpackSum total;
+        const UnpackSum before = unpack_block_scan<kChainThreads / 32>(mine, s_warp, &total);
+        u32 st = (before.exit >> (2 * state)) & 3u;
+        u64 it = item + unpack_pick(before.items, state), ps = pos + unpack_pick(before.sum, state);
+#pragma unroll 1
+        for (int j = 0; j < kChainTiles; ++j) {
+            if (i0 + j >= ntiles) break;
+            const UnpackSum& t = tiles[i0 + j];
+            bases[i0 + j] = UnpackBase{it, ps, st, 0u};
+            const u32 e = unpack_pick(t.err, st);
+            if (e != kUnpackNone) atomicMin(&s_err, (unsigned long long)(i0 + j) * kUnpackTile + e);
+            it += unpack_pick(t.items, st);
+            ps += unpack_pick(t.sum, st);
+            st = (t.exit >> (2 * st)) & 3u;
+        }
+        item += unpack_pick(total.items, state);
+        pos = min(pos + unpack_pick(total.sum, state), kUnpackSumCap);
+        state = (total.exit >> (2 * state)) & 3u;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        out->items = item;
+        out->sum = pos;
+        out->err = s_err;
+        out->state = state;
+    }
+}
+
+// Each tile from its entry state: run_start[k] and run_sym[k] of every item k whose sym byte lies in it.  The host has
+// checked the chain's totals (no malformed item, the run lengths add up to n), so k < n and every start is below n; the
+// bound is kept anyway.
+__global__ void __launch_bounds__(kUnpackThreads, 1)
+k_dc_unpack_items(const u8* __restrict__ stream, u64 bytes, const UnpackBase* __restrict__ bases, u32 n, u32* __restrict__ run_start,
+                  u8* __restrict__ run_sym) {
+    __shared__ __align__(16) u8 s_buf[kUnpackTile + 16];
+    __shared__ UnpackSum s_warp[kUnpackThreads / 32];
+    u32 len;
+    const u32 lim = unpack_load_tile(stream, bytes, (u64)blockIdx.x * kUnpackTile, s_buf, &len);
+    const UnpackBase tb = bases[blockIdx.x];
+    UnpackSum total;
+    const UnpackSum before = unpack_block_scan<kUnpackThreads / 32>(unpack_chunk(s_buf, len, lim), s_warp, &total);
+    const u32 state = (before.exit >> (2 * tb.state)) & 3u;
+    u64 k = tb.item + unpack_pick(before.items, tb.state);
+    u64 pos = tb.pos + unpack_pick(before.sum, tb.state);
+    const u32 c0 = min((u32)threadIdx.x * kUnpackChunk, len), c1 = min(c0 + kUnpackChunk, len);
+    u32 err;
+    unpack_walk(s_buf, c0, c1, lim, state, &err, [&](u32 sym, u64 run) {
+        DARK_ASSERT(k < n && pos < n);
+        if (k < n) {
+            run_start[k] = (u32)pos;
+            run_sym[k] = (u8)sym;
+        }
+        ++k;
+        pos += run;
+    });
+}
+
+// Output tile b covers the 16-byte words [256 b, 256 b + 256) of out's aligned address space; thread t writes word 256 b + t
+// (16-byte store where all its bytes are in [0, n)).  run_start[0..m) strictly increases from 0 (the host's checks): the
+// tile's runs are the lo..hi found by binary search, at most 4,096 of them, staged in shared memory.
+constexpr int kExpandWords = 256;
+__global__ void __launch_bounds__(kExpandWords)
+k_dc_unpack_expand(const u32* __restrict__ run_start, const u8* __restrict__ run_sym, u32 m, u32 n, u8* __restrict__ out) {
+    __shared__ u32 s_start[kExpandWords * 16];
+    __shared__ u8 s_sym[kExpandWords * 16];
+    __shared__ u32 s_run[2];
+    const u32 shift = (u32)((uintptr_t)out & 15u);
+    const u64 v0 = (u64)blockIdx.x * kExpandWords * 16;  // the tile's first position in the aligned space (output byte v0 - shift)
+    if (threadIdx.x < 2) {  // the runs holding the tile's first (thread 0) and last (thread 1) byte: the largest r with run_start[r] <= p
+        const u32 p = threadIdx.x ? (u32)min(v0 + kExpandWords * 16 - shift, (u64)n) - 1u : (u32)(v0 > shift ? v0 - shift : 0);
+        u32 lo = 0, hi = m - 1;
+        while (lo < hi) {
+            const u32 mid = lo + (hi - lo + 1) / 2;
+            if (run_start[mid] <= p) lo = mid;
+            else hi = mid - 1;
+        }
+        s_run[threadIdx.x] = lo;
+    }
+    __syncthreads();
+    const u32 lo = s_run[0], cnt = min(s_run[1] - lo + 1u, (u32)kExpandWords * 16);
+    DARK_ASSERT(s_run[1] >= lo && s_run[1] - lo < (u32)kExpandWords * 16);
+    for (u32 j = threadIdx.x; j < cnt; j += kExpandWords) {
+        s_start[j] = run_start[lo + j];
+        s_sym[j] = run_sym[lo + j];
+    }
+    __syncthreads();
+    const u64 w0 = v0 + (u64)threadIdx.x * 16;  // this thread's word; its bytes are output positions w0 - shift + 0..15
+    if (w0 + 16 <= shift || w0 >= (u64)n + shift) return;
+    const u32 a = (u32)(w0 > shift ? w0 - shift : 0), b = (u32)min(w0 + 16 - shift, (u64)n);  // [a, b) valid
+    u32 j = 0, hi = cnt - 1;  // the run holding a
+    while (j < hi) {
+        const u32 mid = j + (hi - j + 1) / 2;
+        if (s_start[mid] <= a) j = mid;
+        else hi = mid - 1;
+    }
+    u32 word[4] = {0u, 0u, 0u, 0u};
+#pragma unroll
+    for (int k = 0; k < 16; ++k) {
+        const u64 p = w0 + k - shift;  // wraps below 0 for the bytes before out: those are never stored
+        if (p >= a && p < b) {
+            while (j + 1 < cnt && s_start[j + 1] <= (u32)p) ++j;
+            word[k >> 2] |= (u32)s_sym[j] << (8 * (k & 3));
+        }
+    }
+    if (b - a == 16) {
+        *(uint4*)(out + (w0 - shift)) = make_uint4(word[0], word[1], word[2], word[3]);
+    } else {
+#pragma unroll
+        for (int k = 0; k < 16; ++k) {
+            const u64 p = w0 + k - shift;
+            if (p >= a && p < b) out[p] = (u8)(word[k >> 2] >> (8 * (k & 3)));
+        }
+    }
+}
+
+// *first = min(*first, the first offset < bytes where a and b differ); first preset to ~0, *done to 0.  The last CTA to
+// finish copies the answer into the mailbox (*out).
+__global__ void __launch_bounds__(256)
+k_dc_unpack_compare(const u8* __restrict__ a, const u8* __restrict__ b, u64 bytes, unsigned long long* first, u32* done,
+                    unsigned long long* out) {
+    __shared__ unsigned long long s_first;
+    __shared__ bool s_last;
+    if (threadIdx.x == 0) s_first = ~0ull;
+    __syncthreads();
+    unsigned long long mine = ~0ull;
+    const u64 stride = (u64)gridDim.x * blockDim.x;
+    for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < bytes; i += stride)
+        if (a[i] != b[i]) {
+            mine = i;
+            break;  // later offsets of this thread are larger
+        }
+    if (mine != ~0ull) atomicMin(&s_first, mine);
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        if (s_first != ~0ull) atomicMin(first, s_first);
+        __threadfence();
+        s_last = atomicAdd(done, 1u) == gridDim.x - 1;
+    }
+    __syncthreads();
+    if (s_last && threadIdx.x == 0) *out = atomicMin(first, ~0ull);
+}
+
 }  // namespace dark

@@ -332,6 +332,29 @@ class Constructor:
                                                             ctypes.byref(info)), self._ctx, "dc::encode (packed)")
         return int(nbytes.value), info
 
+    # -- decoding the packed item stream: its block back, checked by re-encoding, then the text -------------------------------
+    def inverse_dc_packed(self, stream, n, origin, want_bwt=False):
+        """The unpack side of bwt_dc_packed (dark_bwt_inverse_dc_packed): (text np.uint8[n], bwt or None, DcInfo) from the
+        packed item stream of the block's BWT and its origin.  A stream that is not exactly the packed stream of some block of
+        n bytes raises DarkBwtError(E_INVALID_ARG)."""
+        s = _as_u8(stream)
+        n = int(n)
+        text = np.empty(n, dtype=np.uint8)
+        bwt = np.empty(n, dtype=np.uint8) if want_bwt else None
+        info = _ffi.DcInfo()
+        _ffi.check(self._L.dark_bwt_inverse_dc_packed(self._ctx, s.ctypes.data if s.size else None, s.size, n, int(origin),
+                                                      text.ctypes.data if n else None, bwt.ctypes.data if want_bwt and n else None,
+                                                      ctypes.byref(info)), self._ctx, "dc::decode (packed) + bwt::decode")
+        return text, bwt, info
+
+    def dc_decode_packed_device(self, d_stream, stream_bytes, n, d_bwt):
+        """Device pointers: d_bwt[0..n) gets the block whose packed item stream is d_stream[0..stream_bytes)
+        (dark_bwt_dc_decode_packed_device).  Returns the DcInfo the encoder gives for that block."""
+        info = _ffi.DcInfo()
+        _ffi.check(self._L.dark_bwt_dc_decode_packed_device(self._ctx, d_stream, int(stream_bytes), int(n), d_bwt, ctypes.byref(info)),
+                   self._ctx, "dc::decode (packed)")
+        return info
+
     # -- distance coding of many small blocks in one device pass -----------------------------------------------------
     def _dc_many_results(self, infos, ns, dist, item_starts, pos, idist, sym, rank):
         """Per-block dicts shaped like _dc_result, cut out of the concatenated outputs."""

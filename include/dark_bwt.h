@@ -332,6 +332,30 @@ int dark_bwt_forward_dc_packed_many(dark_bwt_ctx *ctx, const uint8_t *const *tex
                                     uint8_t *stream_out, uint64_t stream_capacity, uint64_t *stream_starts,
                                     uint64_t *stream_bytes_out, dark_bwt_dc_info *infos, dark_bwt_stats *stats /* nullable */);
 
+/* ---- decoding the packed item stream: the unpack side of the packed entries ------------------------------------------
+ * A stream is valid for n when it is byte for byte what dark_bwt_dc_encode_packed_device writes for some block of n bytes;
+ * the symbols and run lengths fix that block, and the decoders return it.  Any other byte string is
+ * DARK_BWT_E_INVALID_ARG (wrong distances or ranks, non-canonical varints such as 0x80 0x00, two adjacent items with the
+ * same symbol, trailing bytes included), and the context stays usable.  The decoders are safe for any input bytes: they
+ * read nothing past stream_bytes, write nothing past n output bytes, and end in bounded time. */
+/* The inverse of dark_bwt_dc_encode_packed_device: d_bwt_out[0..n) gets the block whose packed item stream is
+ * d_stream[0..stream_bytes) (device buffers, any alignment).  1 <= n <= capacity.  DARK_BWT_E_INVALID_ARG unless the
+ * stream is exactly the packed stream of some block of n bytes (dark_bwt_last_error() says why: where the parse failed,
+ * the run lengths' sum against n, or the first byte at which the stream differs from the decoded block's); d_bwt_out is
+ * then unspecified.  info (nullable) gets what dark_bwt_dc_encode_packed_device gives for the decoded block, device_ms =
+ * this call's device time.  Returns after the work has completed on the stream. */
+int dark_bwt_dc_decode_packed_device(dark_bwt_ctx *ctx, const uint8_t *d_stream, uint64_t stream_bytes, uint64_t n,
+                                     uint8_t *d_bwt_out, dark_bwt_dc_info *info);
+/* The unpack side of dark_bwt_forward_dc_packed in one call: the stream (host, pageable or pinned) is decoded into the BWT,
+ * which stays in HBM and is inverted with `origin` into text_out[0..n).  bwt_out and info nullable.  1 <= n <= capacity,
+ * origin < n.  DARK_BWT_E_INVALID_ARG as above, or when (BWT, origin) is not the transform of any text (the inverse's own
+ * check); neither text_out nor bwt_out is written then.  DARK_BWT_E_INVALID_ARG with a device-only context.
+ * Both entries, before any device work: a null required pointer is DARK_BWT_E_INVALID_ARG, n outside [1, capacity]
+ * DARK_BWT_E_INVALID_N, stream_bytes == 0 or above DARK_BWT_DC_PACKED_MAX(n) (no valid stream is that long) and
+ * origin >= n DARK_BWT_E_INVALID_ARG. */
+int dark_bwt_inverse_dc_packed(dark_bwt_ctx *ctx, const uint8_t *stream, uint64_t stream_bytes, uint64_t n, uint64_t origin,
+                               uint8_t *text_out, uint8_t *bwt_out, dark_bwt_dc_info *info);
+
 /* Constructor::reuse — lends >= capacity host u32 words of scratch (DC distances in
  * block/dc.rs:51).  Allocated on first use; owned by the context. */
 int dark_bwt_reuse(dark_bwt_ctx *ctx, uint32_t **words_out, uint64_t *count_out);

@@ -96,6 +96,11 @@ extern "C" {
                                            bwt_outs: *const *mut u8, origins_out: *mut u64, stream_out: *mut u8,
                                            stream_capacity: u64, stream_starts: *mut u64, stream_bytes_out: *mut u64,
                                            infos: *mut dark_bwt_dc_info, stats: *mut dark_bwt_stats) -> c_int;
+    // the unpack side: the block back from its packed stream (checked by re-encoding), then the text
+    pub fn dark_bwt_dc_decode_packed_device(ctx: *mut dark_bwt_ctx, d_stream: *const u8, stream_bytes: u64, n: u64,
+                                            d_bwt_out: *mut u8, info: *mut dark_bwt_dc_info) -> c_int;
+    pub fn dark_bwt_inverse_dc_packed(ctx: *mut dark_bwt_ctx, stream: *const u8, stream_bytes: u64, n: u64, origin: u64,
+                                      text_out: *mut u8, bwt_out: *mut u8, info: *mut dark_bwt_dc_info) -> c_int;
     pub fn dark_bwt_create(max_n: u64, device: c_int, out: *mut *mut dark_bwt_ctx) -> c_int;
     pub fn dark_bwt_create_ex(max_n: u64, device: c_int, flags: u32, out: *mut *mut dark_bwt_ctx) -> c_int;
     pub fn dark_bwt_arena_bytes(max_n: u64, flags: u32) -> u64;
